@@ -224,6 +224,10 @@ SIGNATURES = {
     'b2r_c51_project': (c_int, [c_int32, c_int32, c_void_p, c_void_p, c_void_p,
                                 c_void_p, c_void_p]),
     'b2r_c51_loss': (c_int, [P(C51Args), c_void_p]),
+    'b2r_c51_loss_sharded': (c_int, [P(C51Args), c_void_p, c_int32, c_void_p]),
+    'b2r_sample_transition_batch_sharded_device': (c_int, [
+        c_void_p, c_void_p, c_int32, c_uint64, c_uint64, P(Batch), c_void_p, c_void_p,
+        c_int32, c_void_p, c_void_p]),
     'b2r_dqn_loss': (c_int, [P(DqnArgs), c_void_p]),
     'b2r_train_step_device': (c_int, [c_void_p, c_int32, c_uint64, c_uint64,
                                       P(Batch), P(C51Args), c_void_p]),

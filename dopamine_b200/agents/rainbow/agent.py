@@ -339,3 +339,125 @@ class RainbowAgent(RainbowLearner, dqn_agent.ActingLoop):
     "the maximum ever seen", is resolved on the device when the row is applied)."""
     if not self.eval_mode:
       self.store_transition(last_observation, action, reward, is_terminal, priority)
+
+
+class ShardedRainbowLearner(RainbowLearner):
+  """`RainbowLearner` on ONE global prioritized batch sharded over the ranks of
+  torch.distributed (SURVEY.md section 8(d), config 5 fed by config 4's sampler).
+
+  Every rank owns one replay shard of `replay_capacity` transitions and a peer-memory
+  exchange.  `batch_size` is the GLOBAL batch: its strata are apportioned over the
+  shards by their priority totals (`ShardedPrioritizedReplay`), so the update is the
+  reference's update (rainbow_agent.py:253-305) on that global batch, up to the order of
+  floating-point sums.  One update:
+    1. `sample()`: sharded sampler + frame copies into `max_rows` rows (default
+       `share_bound`; the rank's share is counted on the device);
+    2. `loss_backward()`: both networks on all `max_rows` rows, the sharded C51 loss
+       (IS weights normalised over every rank's minimum, mean over the global batch,
+       zero gradients for padded rows) and backward into one flat buffer;
+    3. `reduce()`: ONE all-reduce (sum) of that buffer — every parameter's gradient
+       and, appended, the partial loss, so the reported loss is the global mean;
+    4. `apply()`: TF-form Adam and the counted priority write-back.
+  The shapes are static, so `cuda_graph=True` captures the whole update, all-reduce
+  included.  Errors latched on the device (a share beyond `max_rows`, a peer that did not
+  answer) are raised by `check()`, which `sync_target()` calls.  Pass `exchange`
+  (`PeerExchange.emulated`) to run the phases of several ranks on one device without
+  torch.distributed (tests); `reduce()` then is the caller's.
+  """
+
+  def __init__(self, num_actions, batch_size=32, max_rows=None, exchange=None,
+               group=None, exchange_timeout_s=2.0, ddp=False, **kwargs):
+    torch = _torch()
+    import torch.distributed as dist  # pylint: disable=g-import-not-at-top
+    from dopamine_b200.replay_memory import sharded_replay  # pylint: disable=g-import-not-at-top
+    if ddp:
+      raise ValueError('the sharded learner reduces its gradients itself (ddp=False)')
+    self._dist = dist if exchange is None else None
+    if exchange is None:
+      if not (dist.is_available() and dist.is_initialized()):
+        raise RuntimeError('ShardedRainbowLearner needs torch.distributed initialised')
+      exchange = sharded_replay.PeerExchange(group=group, timeout_s=exchange_timeout_s)
+    self._group = group
+    RainbowLearner.__init__(self, num_actions, batch_size=batch_size, **kwargs)
+    self.exchange = exchange
+    self.rank, self.world = exchange.rank, exchange.world
+    self.sharded = sharded_replay.ShardedPrioritizedReplay(
+        self.memory, rank=self.rank, world_size=self.world,
+        seed=kwargs.get('seed', 0), exchange=exchange)
+    self.max_rows = (sharded_replay.share_bound(batch_size, self.world)
+                     if max_rows is None else min(int(max_rows), int(batch_size)))
+    params = list(self.online.parameters())
+    if self._dist is not None:
+      with torch.no_grad():
+        for p in params:
+          self._dist.broadcast(p, 0, group=group)
+      RainbowLearner.sync_target(self)
+    # every gradient views one flat buffer; the partial loss rides at its end
+    total = sum(p.numel() for p in params)
+    self._flat = torch.zeros(total + 1, dtype=torch.float32, device='cuda')
+    offset = 0
+    for p in params:
+      p.grad = self._flat[offset:offset + p.numel()].view_as(p)
+      offset += p.numel()
+    self.loss = self._flat[total:]
+    self._sample = None
+
+  # -- phases ------------------------------------------------------------------------
+  def sample(self):
+    """(slots, count, batch tuple, min_probability) of this rank's share."""
+    self._sample = self.sharded.sample_transition_batch_sharded(self.batch_size,
+                                                                self.max_rows)
+    return self._sample
+
+  def loss_backward(self):
+    """Networks, sharded loss and backward: the flat buffer holds this rank's partial
+    gradients and partial mean.  Returns the per-row priorities."""
+    torch = _torch()
+    _, count, batch, min_probability = self._sample
+    (state, action, reward, next_state, _, _, terminal, _, probs) = batch[:9]
+    with torch.no_grad():
+      target_logits = self.target(next_state)
+    online_logits = self.online(state)
+    scheme_probs = probs if self.replay_scheme == 'prioritized' else None
+    mean, priorities, _, _ = rainbow_agent.ShardedC51Loss.apply(
+        online_logits, target_logits, action, reward, terminal, scheme_probs,
+        self.support, self.cumulative_gamma,
+        (self.exchange, self.batch_size, count, min_probability))
+    self._flat.zero_()
+    mean.backward()  # (accumulates into the views of the flat buffer)
+    self.loss.copy_(mean.detach().view(1))
+    return priorities
+
+  def reduce(self):
+    """The one all-reduce of the update: gradients and loss summed over the ranks."""
+    self._dist.all_reduce(self._flat, group=self._group)
+
+  def apply(self, priorities):
+    """Adam on the reduced gradients, then this rank's priority write-back."""
+    self.optimizer.step()
+    if self.replay_scheme == 'prioritized':  # rainbow_agent.py:289-295
+      slots, count, batch, _ = self._sample
+      del slots
+      self.sharded.set_priority(batch[7], priorities, count)
+
+  def _update(self):
+    self.sample()
+    priorities = self.loss_backward()
+    self.reduce()
+    self.apply(priorities)
+    if not self._cuda_graph or self._graph is None:
+      self.updates += 1
+    return self.loss
+
+  def check(self):
+    """Raises what the device latched since the last check (synchronises); also
+    verifies that backward left every gradient in the flat buffer."""
+    lo, hi = self._flat.data_ptr(), self._flat.data_ptr() + 4 * self._flat.numel()
+    for p in self.online.parameters():
+      if p.grad is None or not lo <= p.grad.data_ptr() < hi:
+        raise RuntimeError('a gradient left the all-reduced buffer')
+    self.sharded.check()
+
+  def sync_target(self):
+    self.check()
+    RainbowLearner.sync_target(self)

@@ -105,7 +105,8 @@ def project_distribution(supports, weights, target_support,
 
 def c51_loss(online_logits, target_logits, actions, rewards, terminals,
              sampling_probabilities, support, cumulative_gamma,
-             want_target=False, want_grad=False, want_mean=True, out=None):
+             want_target=False, want_grad=False, want_mean=True, out=None,
+             sharded=None):
   """Fused Rainbow update math for one batch, all on the device.
 
   Args:
@@ -121,6 +122,13 @@ def c51_loss(online_logits, target_logits, actions, rewards, terminals,
     'grad_logits' (B, A, N) = d mean_weighted_loss / d online_logits.
     `out` (a dict returned by an earlier call with the same shapes) is reused
     instead of allocating.
+    sharded: (exchange, global_batch, count, min_probability) — the rows are one
+    rank's share of a global batch of `global_batch` strata, as
+    `ShardedPrioritizedReplay.sample_transition_batch_sharded` returns it
+    (b2r_c51_loss_sharded): the first `count` (device) rows are valid, the weights are
+    normalised over every rank's minimum sampling probability, and the mean and its
+    gradient are this rank's part of the global batch's (divisor global_batch; padded
+    rows get zero gradients).
   """
   torch = _torch()
   b, a, n = online_logits.shape
@@ -166,8 +174,17 @@ def c51_loss(online_logits, target_logits, actions, rewards, terminals,
   args.mean_weighted_loss = (out['mean_weighted_loss'].data_ptr()
                              if want_mean else None)
   args.grad_logits = out['grad_logits'].data_ptr() if want_grad else None
-  _native.check(_native.lib().b2r_c51_loss(ctypes.byref(args),
-                                           _native.current_stream()))
+  if sharded is None:
+    _native.check(_native.lib().b2r_c51_loss(ctypes.byref(args),
+                                             _native.current_stream()))
+    return out
+  exchange, global_batch, count, min_probability = sharded
+  args.batch_count = count.data_ptr()
+  if sampling_probabilities is not None:
+    args.min_probability = min_probability.data_ptr()
+  _native.check(_native.lib().b2r_c51_loss_sharded(
+      ctypes.byref(args), exchange._h, int(global_batch),  # pylint: disable=protected-access
+      _native.current_stream()))
   return out
 
 
@@ -207,10 +224,10 @@ class C51Loss(object):
 
         @staticmethod
         def forward(ctx, online_logits, target_logits, actions, rewards,
-                    terminals, probs, support, gamma_n):
+                    terminals, probs, support, gamma_n, sharded):
           out = c51_loss(online_logits.detach(), target_logits.detach(), actions,
                          rewards, terminals, probs, support, gamma_n,
-                         want_grad=True)
+                         want_grad=True, sharded=sharded)
           ctx.save_for_backward(out['grad_logits'])
           ctx.mark_non_differentiable(out['priorities'], out['loss'],
                                       out['weights'])
@@ -221,7 +238,7 @@ class C51Loss(object):
         def backward(ctx, grad_mean, *unused):
           (grad_logits,) = ctx.saved_tensors
           return (grad_logits * grad_mean, None, None, None, None, None, None,
-                  None)
+                  None, None)
 
       cls._fn = _Fn
     return cls._fn
@@ -231,7 +248,22 @@ class C51Loss(object):
             sampling_probabilities, support, gamma_n):
     return cls._function().apply(online_logits, target_logits, actions, rewards,
                                  terminals, sampling_probabilities, support,
-                                 gamma_n)
+                                 gamma_n, None)
+
+
+class ShardedC51Loss(C51Loss):
+  """`C51Loss` over one rank's share of a sharded global batch (b2r_c51_loss_sharded):
+  `mean, priorities, loss, weights = ShardedC51Loss.apply(..., sharded)` with `sharded`
+  as in `c51_loss`.  `mean` is this rank's partial mean (its rows' weighted losses over
+  the global batch size) and backward gives its gradient; summed over the ranks both
+  are the global batch's."""
+
+  @classmethod
+  def apply(cls, online_logits, target_logits, actions, rewards, terminals,
+            sampling_probabilities, support, gamma_n, sharded):
+    return cls._function().apply(online_logits, target_logits, actions, rewards,
+                                 terminals, sampling_probabilities, support,
+                                 gamma_n, tuple(sharded))
 
 
 # ---------------------------------------------------------------------------

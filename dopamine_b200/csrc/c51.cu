@@ -90,8 +90,24 @@ c51_project_kernel(int batch, int n, const float *__restrict__ supports,
     out[(size_t)b * n + i] = project_atom(s, w, n, z[i], z0, zlast, dz);
 }
 
+// b2r_c51_loss_sharded: this rank's rows of a global batch of global_batch strata.  The
+// IS normaliser is the minimum over the G ranks' local minima (the rank's own one is
+// args->min_probability, the peers' are polled from the local mailbox for the step the
+// sampler has just closed), the mean and its gradient use global_batch as the divisor and
+// rows >= count get zero gradients: summed over the ranks, the means and the gradients
+// are those of the whole global batch.
+struct ShardedLoss {
+  int global_batch = 0;        // 0: not sharded
+  int world = 1, rank = 0;
+  const uint64_t *mins = nullptr;  // this rank's mailbox, local-minimum region
+  const uint64_t *seq = nullptr;   // device step counter (advanced by the sampler)
+  int64_t timeout_ns = 0;
+  int64_t *latched = nullptr;      // nullable: B2R_ERR_EXCHANGE on a peer's timeout
+};
+
 struct LossArgs {
   b2r_c51_args u;
+  ShardedLoss sh;
   float *weighted;        // scratch (B,): w_b * loss_b, reduced by the last CTA
   unsigned int *ticket;   // scratch: CTAs finished (self-resetting)
   int warps;              // warps per CTA = min(num_actions, 32)
@@ -115,6 +131,91 @@ struct LossArgs {
   // sampled indices are final (tree.cuh: TreeGo); go.go == nullptr: nobody does.
   TreeGo go;
 };
+
+__device__ __forceinline__ uint64_t timer_ns() {
+  uint64_t t;
+  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
+  return t;
+}
+
+// Minimum of `own` and the peers' local minima of the current step (see ShardedLoss).  A
+// peer's word carries the step number in-band: a stale or early word is waited on, never
+// read as a value.  A peer that does not publish within the timeout latches
+// B2R_ERR_EXCHANGE (later launches then skip the wait) and is left out.
+__device__ __noinline__ float sharded_min_probability(const ShardedLoss &x, float own) {
+  const uint64_t seq = *x.seq;
+  const uint32_t tag = (uint32_t)seq;
+  const uint64_t *box = x.mins + (size_t)(seq & 1) * x.world;
+  float m = own;
+  for (int g = 0; g < x.world; ++g) {
+    if (g == x.rank) continue;
+    bool broken = x.timeout_ns <= 0 || (x.latched != nullptr && x.latched[0] == B2R_ERR_EXCHANGE);
+    const uint64_t t0 = timer_ns();
+    while (!broken) {
+      const uint64_t w = ld_sys_u64(box + g);
+      if ((uint32_t)w == tag) {
+        m = fminf(m, __uint_as_float((uint32_t)(w >> 32)));
+        break;
+      }
+      if (timer_ns() - t0 > (uint64_t)x.timeout_ns) {
+        if (x.latched != nullptr) {
+          x.latched[0] = B2R_ERR_EXCHANGE;
+          x.latched[1] = g;
+        }
+        broken = true;
+      }
+    }
+  }
+  return m;
+}
+
+// Last CTA of a launch to get here (every thread calls; s_last in shared memory).
+__device__ __forceinline__ bool last_cta(unsigned int *ticket, bool *s_last) {
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const unsigned int done = atomicAdd(ticket, 1u);
+    *s_last = (done == gridDim.x - 1);
+    if (*s_last) *ticket = 0u;  // ready for the next launch
+  }
+  __syncthreads();
+  if (*s_last) __threadfence();
+  return *s_last;
+}
+
+// By the last CTA: sum of weighted[0, n) in a fixed order (thread t takes k = t mod
+// blockDim, butterfly per warp, warps in order) / divisor into *out.
+__device__ __forceinline__ void mean_of_weighted(const float *weighted, int n, float divisor,
+                                                 float *s_red, float *out) {
+  float acc = 0.f;
+  for (int k = threadIdx.x; k < n; k += blockDim.x) acc = __fadd_rn(acc, __ldcg(weighted + k));
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) acc = __fadd_rn(acc, __shfl_xor_sync(0xffffffffu, acc, o));
+  if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float total = 0.f;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) total = __fadd_rn(total, s_red[w]);
+    *out = __fdiv_rn(total, divisor);
+  }
+}
+
+// A sharded launch's rows past the count: zero gradient rows, and the CTA still takes its
+// ticket so that the last CTA forms this rank's part of the mean.
+__device__ void sharded_padding(const LossArgs &a, int b0, int nrows, int rows, float *s_red,
+                                bool *s_last) {
+  const int AN = a.u.num_actions * a.u.num_atoms;
+  if (a.u.grad_logits != nullptr)
+    for (int r = 0; r < nrows; ++r) {
+      const int b = b0 + r;
+      if (b < rows || b >= a.u.batch) continue;
+      float *g = a.u.grad_logits + (size_t)b * AN;
+      for (int k = threadIdx.x; k < AN; k += blockDim.x) g[k] = 0.f;
+    }
+  if (a.u.mean_weighted_loss == nullptr) return;
+  if (!last_cta(a.ticket, s_last)) return;
+  mean_of_weighted(a.weighted, rows, (float)a.sh.global_batch, s_red, a.u.mean_weighted_loss);
+}
 
 // One CTA per batch row, one warp per action (rainbow_agent.py:200-293):
 //   A. every warp: softmax of its action's target logits, q = sum z*p
@@ -160,7 +261,11 @@ c51_loss_kernel(LossArgs a) {
   if (blockIdx.x == 0 && threadIdx.x == 0) tree_go_signal(a.go);
   B2R_MARK(1);
   const int rows = a.u.batch_count ? min(*a.u.batch_count, a.u.batch) : a.u.batch;
-  if (b >= rows) return;  // (mean_weighted_loss is not supported with batch_count)
+  const bool sharded = a.sh.global_batch > 0;
+  if (b >= rows) {  // (mean_weighted_loss with batch_count: sharded only)
+    if (sharded) sharded_padding(a, b, 1, rows, s_red, &s_last);
+    return;
+  }
 
   // ---- every global load the row needs is issued here, before the first use:
   // the kernel is latency-bound at batch 32 and this keeps it to one round trip.
@@ -377,6 +482,7 @@ c51_loss_kernel(LossArgs a) {
     float w = 1.f;
     if (a.u.sampling_probabilities) {
       float mn = pmin;  // handed over by the sampler, or reduced per warp above
+      if (sharded) mn = sharded_min_probability(a.sh, mn);
       if (!a.u.min_probability) {
         mn = s_red[0];
 #pragma unroll 1
@@ -396,7 +502,7 @@ c51_loss_kernel(LossArgs a) {
   // ---- D. gradient of mean(w * ce) w.r.t. the online logits
   if (a.u.grad_logits) {
     const float tsum = s_scalar[0], w = s_scalar[1], m = s_scalar[2], denom = s_scalar[3];
-    const float scale = __fmul_rn(w, __fdiv_rn(1.0f, (float)rows));
+    const float scale = __fmul_rn(w, __fdiv_rn(1.0f, (float)(sharded ? a.sh.global_batch : rows)));
     float *g = a.u.grad_logits + (size_t)b * A * N;
     for (int k = threadIdx.x; k < A * N; k += blockDim.x) {
       const int act = k / N, i = k - act * N;
@@ -429,17 +535,9 @@ c51_loss_kernel(LossArgs a) {
     B2R_MARK_END(9);
   }
   if (a.u.mean_weighted_loss == nullptr) return;
-  float acc = 0.f;
-  for (int k = threadIdx.x; k < a.u.batch; k += blockDim.x)
-    acc = __fadd_rn(acc, __ldcg(a.weighted + k));
-  acc = warp_sum(acc);
-  if (lane == 0) s_red[warp] = acc;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float total = 0.f;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) total = __fadd_rn(total, s_red[w]);
-    *a.u.mean_weighted_loss = __fdiv_rn(total, (float)a.u.batch);
-  }
+  mean_of_weighted(a.weighted, sharded ? rows : a.u.batch,
+                   (float)(sharded ? a.sh.global_batch : a.u.batch), s_red,
+                   a.u.mean_weighted_loss);
 }
 
 // ---- throughput instance (batches above 256 rows, num_atoms <= 64) ----------
@@ -493,7 +591,11 @@ c51_loss_rows_kernel(LossArgs a) {
   if (blockIdx.x == 0 && threadIdx.x == 0) tree_go_signal(a.go);
   B2R_MARK(11);
   const int rows = a.u.batch_count ? min(*a.u.batch_count, a.u.batch) : a.u.batch;
-  if ((int)blockIdx.x * kRowWarps >= rows) return;  // (no mean loss with batch_count)
+  const bool sharded = a.sh.global_batch > 0;
+  if ((int)blockIdx.x * kRowWarps >= rows) {  // (mean loss with batch_count: sharded only)
+    if (sharded) sharded_padding(a, blockIdx.x * kRowWarps, kRowWarps, rows, s_red, &s_last);
+    return;
+  }
   const int b = blockIdx.x * kRowWarps + warp;
   const bool row_ok = b < rows;
 
@@ -503,6 +605,7 @@ c51_loss_rows_kernel(LossArgs a) {
   if (a.u.sampling_probabilities) {
     if (a.u.min_probability) {
       pmin = *a.u.min_probability;
+      if (sharded) pmin = sharded_min_probability(a.sh, pmin);
     } else {
       for (int k = threadIdx.x; k < rows; k += blockDim.x)
         pmin = fminf(pmin, a.u.sampling_probabilities[k]);
@@ -698,7 +801,8 @@ c51_loss_rows_kernel(LossArgs a) {
 
     // ---- D. gradient of mean(w * ce) w.r.t. the online logits
     if (a.u.grad_logits) {
-      const float scale = __fmul_rn(w, __fdiv_rn(1.0f, (float)rows));
+      const float scale =
+          __fmul_rn(w, __fdiv_rn(1.0f, (float)(sharded ? a.sh.global_batch : rows)));
       float *g = a.u.grad_logits + (size_t)b * A * N;
       float v[2] = {0.f, 0.f};
 #pragma unroll
@@ -717,32 +821,18 @@ c51_loss_rows_kernel(LossArgs a) {
         }
       }
     }
+  } else if (sharded && a.u.grad_logits != nullptr && b < a.u.batch) {
+    float *g = a.u.grad_logits + (size_t)b * A * N;  // a padded row of this CTA
+    for (int k = lane; k < A * N; k += 32) g[k] = 0.f;
   }
 
   B2R_MARK_END(12);
   // ---- mean weighted loss: the last CTA to finish reduces in a fixed order.
   if (a.u.mean_weighted_loss == nullptr) return;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int done = atomicAdd(a.ticket, 1u);
-    s_last = (done == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  float acc = 0.f;
-  for (int k = threadIdx.x; k < a.u.batch; k += blockDim.x)
-    acc = __fadd_rn(acc, __ldcg(a.weighted + k));
-  acc = group_sum<32>(acc);
-  if (lane == 0) s_red[warp] = acc;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    float total = 0.f;
-    for (int k = 0; k < kRowWarps; ++k) total = __fadd_rn(total, s_red[k]);
-    *a.u.mean_weighted_loss = __fdiv_rn(total, (float)a.u.batch);
-    *a.ticket = 0u;  // ready for the next launch
-  }
+  if (!last_cta(a.ticket, &s_last)) return;
+  mean_of_weighted(a.weighted, sharded ? rows : a.u.batch,
+                   (float)(sharded ? a.sh.global_batch : a.u.batch), s_red,
+                   a.u.mean_weighted_loss);
 }
 
 // ---- the loss in two halves (the fused step) --------------------------------------
@@ -1411,6 +1501,8 @@ bool c51_can_fuse_writeback(const b2r_c51_args *args, const b2r_tree *tree) {
 
 int c51_loss_launch(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
                     const int32_t *indices);
+int launch_loss(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
+                const int32_t *indices, const ShardedLoss &sh);
 
 }  // namespace b2r
 
@@ -1418,6 +1510,29 @@ extern "C" {
 
 int b2r_c51_loss(const b2r_c51_args *args, b2r_stream stream) {
   return b2r::c51_loss_launch(args, as_stream(stream), nullptr, nullptr);
+}
+
+int b2r_c51_loss_sharded(const b2r_c51_args *args, b2r_exchange *exchange,
+                         int32_t global_batch, b2r_stream stream) {
+  if (!args) return fail(B2R_ERR_INVALID_ARGUMENT, "args is NULL");
+  if (!args->batch_count)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "a shard's loss needs batch_count");
+  if (global_batch < 1) return fail(B2R_ERR_INVALID_ARGUMENT, "global_batch must be >= 1");
+  if (args->sampling_probabilities && !args->min_probability)
+    return fail(B2R_ERR_INVALID_ARGUMENT,
+                "sampling_probabilities need the sampler's min_probability");
+  if (!exchange) return fail(B2R_ERR_INVALID_ARGUMENT, "exchange is NULL");
+  if (!exchange->connected)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "the exchange is not connected");
+  b2r::ShardedLoss sh;
+  sh.global_batch = global_batch;
+  sh.world = exchange->world;
+  sh.rank = exchange->rank;
+  sh.mins = exchange->mailbox + b2r::kMinWordsOffset;
+  sh.seq = exchange->seq;
+  sh.timeout_ns = exchange->timeout_ns;
+  sh.latched = exchange->latched;
+  return b2r::launch_loss(args, as_stream(stream), nullptr, nullptr, sh);
 }
 
 }  // extern "C"
@@ -1578,9 +1693,14 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
 // tree != nullptr (c51_can_fuse_writeback): also set_priority(indices, priorities).
 int c51_loss_launch(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
                     const int32_t *indices) {
+  return launch_loss(args, s, tree, indices, ShardedLoss());
+}
+
+int launch_loss(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
+                const int32_t *indices, const ShardedLoss &sh) {
   if (!args || args->batch <= 0 || args->num_atoms < 2 || args->num_actions <= 0)
     return fail(B2R_ERR_INVALID_ARGUMENT, "bad C51 shape");
-  if (args->batch_count && args->mean_weighted_loss)
+  if (args->batch_count && args->mean_weighted_loss && sh.global_batch == 0)
     return fail(B2R_ERR_UNSUPPORTED,
                 "mean_weighted_loss cannot be combined with batch_count");
   if (!args->support || !args->target_logits || !args->online_logits ||
@@ -1589,6 +1709,7 @@ int c51_loss_launch(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
     return fail(B2R_ERR_INVALID_ARGUMENT, "a required C51 pointer is NULL");
   b2r::LossArgs a;
   a.u = *args;
+  a.sh = sh;
   a.fuse_tree = 0;
   a.err = nullptr;
   a.count_copy = nullptr;

@@ -11,7 +11,8 @@
 using b2r::fail;
 
 namespace {
-constexpr size_t kMailboxBytes = 2 * b2r::kMaxShards * 2 * sizeof(uint64_t);
+// totals [2][kMaxShards][2 words], then local minima [2][kMaxShards] (tree.cuh)
+constexpr size_t kMailboxBytes = b2r::kMailboxWords * sizeof(uint64_t);
 }
 
 namespace {

@@ -369,6 +369,9 @@ struct b2r_exchange {
   // sharded step publishes the shard total itself, and the staged adds of a step call are
   // flushed at the END of that call (they become visible to the next step's sampler).
   bool early_publish = false;
+  // Latch of the buffer last sampled through b2r_sample_transition_batch_sharded_device:
+  // where b2r_c51_loss_sharded reports a peer whose minimum never arrived.
+  int64_t *latched = nullptr;
 };
 
 namespace b2r {
@@ -397,7 +400,7 @@ int launch_sample_sharded(b2r_buffer *buf, int32_t global_batch, int32_t num_sha
                           int32_t *out_count, cudaStream_t stream,
                           const b2r_batch *scalars = nullptr,
                           float *min_prob_out = nullptr, int32_t max_rows = 0,
-                          const PreSync *pre = nullptr);
+                          const PreSync *pre = nullptr, bool publish_min = false);
 void fill_valid_ctx(const b2r_buffer *buf, ValidCtx *ctx);
 int ensure_ctx(b2r_buffer *buf, cudaStream_t stream);
 // tree.cu: largest batch the one-CTA tree kernel takes, and the fused flush launch

@@ -79,7 +79,16 @@ struct PerSampleArgs {
   // Rows the caller's outputs hold (a sharded step sizes them by a bound on its share of
   // the global batch): rows beyond it are dropped and B2R_ERR_UNSUPPORTED is latched.
   int out_cap;
+  // Exchange mode: the closing thread also stores min_prob_out's value into every peer's
+  // mailbox for this step (b2r_sample_transition_batch_sharded_device).
+  int publish_min;
 };
+
+// The local minimum of step `seq`, for the peers' sharded loss (b2r_c51_loss_sharded).
+__device__ __forceinline__ void publish_local_min(const PerSampleArgs &a, bool exchange,
+                                                  float m, uint64_t seq) {
+  if (a.publish_min && exchange) exchange_publish_min(a.xchg, a.num_shards, a.rank, m, seq);
+}
 
 __device__ __forceinline__ uint64_t global_timer_ns() {
   uint64_t t;
@@ -236,6 +245,7 @@ __global__ void __launch_bounds__(MAX_THREADS) per_sample_kernel(const __grid_co
       a.info[1] = 0; a.info[2] = 0; a.info[3] = 0;
       if (a.count_out) *a.count_out = 0;
       if (a.min_prob_out) *a.min_prob_out = INFINITY;
+      publish_local_min(a, exchange, INFINITY, xseq);
       if (a.counter) *a.counter = draws_before + 1;  // ranks stay in lockstep
       pre_sync_consume(a.pre);
       if (exchange) *a.xchg.seq = xseq;
@@ -376,6 +386,7 @@ __global__ void __launch_bounds__(MAX_THREADS) per_sample_kernel(const __grid_co
         a.info[3] = rows;
         if (a.count_out) *a.count_out = rows;
         if (want_min) *a.min_prob_out = m;
+        if (want_min) publish_local_min(a, exchange, m, xseq);
         if (all > rows && a.latched && a.latched[0] == 0) {  // the share outgrew the buffers
           a.latched[0] = B2R_ERR_UNSUPPORTED;
           a.latched[1] = all;
@@ -522,6 +533,7 @@ __global__ void __launch_bounds__(MAX_THREADS) per_sample_kernel(const __grid_co
       for (int t = 0; t < n_tiles; ++t)
         m = fminf(m, *(volatile float *)(a.tile_min + t));
       *a.min_prob_out = m;
+      publish_local_min(a, exchange, m, xseq);
     }
   }
   if (threadIdx.x == 0) pre_sync_consume(a.pre);
@@ -721,6 +733,7 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       a.info[1] = 0; a.info[2] = 0; a.info[3] = 0;
       if (a.count_out) *a.count_out = 0;
       if (a.min_prob_out) *a.min_prob_out = INFINITY;
+      publish_local_min(a, exchange, INFINITY, xseq);
       if (a.counter) *a.counter = draws_before + 1;
       if (exchange) *a.xchg.seq = xseq;
       if (a.latched && a.latched[0] == 0) a.latched[0] = B2R_ERR_EMPTY_TREE;
@@ -957,6 +970,7 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
         a.info[3] = n_mine;
         if (a.count_out) *a.count_out = n_mine;
         if (want_min) *a.min_prob_out = m;
+        if (want_min) publish_local_min(a, exchange, m, xseq);
         if (hand_over) st_release_u32(a.flags.final_word, row_tag);
         pre_sync_consume(a.pre, peek);
       }
@@ -1193,7 +1207,10 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
   }
   if (want_min) {
     const float m = block_min(fminf(min_seen, fix_min), warp_mins);
-    if (threadIdx.x == 0) *a.min_prob_out = m;
+    if (threadIdx.x == 0) {
+      *a.min_prob_out = m;
+      publish_local_min(a, exchange, m, xseq);
+    }
   }
   if (hand_over && threadIdx.x == 0) st_release_u32(a.flags.final_word, row_tag);
   if (threadIdx.x == 0) pre_sync_consume(a.pre);
@@ -1451,6 +1468,7 @@ int launch_sample(b2r_buffer *b, int32_t batch, bool philox, uint64_t seed,
   a.count_out = nullptr;
   a.shard_ranges = 0;
   a.out_cap = batch;
+  a.publish_min = 0;
   a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
   if (pre != nullptr) a.pre = *pre;
   a.xchg.local = nullptr;
@@ -1498,7 +1516,7 @@ int launch_sample_sharded(b2r_buffer *b, int32_t global_batch, int32_t num_shard
                           uint64_t offset, int32_t *out_slots, int32_t *out_indices,
                           int32_t *out_count, cudaStream_t s,
                           const b2r_batch *scalars, float *min_prob_out,
-                          int32_t max_rows, const PreSync *pre) {
+                          int32_t max_rows, const PreSync *pre, bool publish_min) {
   if (!b->tree) return fail(B2R_ERR_UNSUPPORTED, "not a prioritized buffer");
   if (global_batch <= 0 || num_shards <= 0 || num_shards > kMaxShards || rank < 0 ||
       rank >= num_shards)
@@ -1567,6 +1585,7 @@ int launch_sample_sharded(b2r_buffer *b, int32_t global_batch, int32_t num_shard
   a.count_out = out_count;
   a.shard_ranges = ranges ? 1 : 0;
   a.out_cap = cap;
+  a.publish_min = publish_min ? 1 : 0;
   a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
   if (pre != nullptr) a.pre = *pre;
   a.xchg.local = nullptr;

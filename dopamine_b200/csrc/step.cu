@@ -72,6 +72,11 @@ struct ShardSpec {
   // global batch.  Every launch behind the sampler is sized by it, not by the global
   // batch; 0 = global batch rows.
   int32_t max_rows;
+  // b2r_sample_transition_batch_sharded_device: the step ends after the sampler and the
+  // frame copies (no loss, no write-back); the sampler leaves its minimum sampling
+  // probability in min_probability and publishes it to the peers.
+  bool sample_only;
+  float *min_probability;
 };
 
 // The host-facing trainer without copy calls: the first half of the loss reads both
@@ -94,7 +99,8 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
                       const b2r_batch *out, const b2r_c51_args *c51, cudaStream_t s,
                       cudaEvent_t wait_before_loss, cudaEvent_t loss_done,
                       const ShardSpec *shard = nullptr, const DirectIO *direct = nullptr) {
-  if (!b || !out || !c51) return fail(B2R_ERR_INVALID_ARGUMENT, "NULL argument");
+  const bool sample_only = shard != nullptr && shard->sample_only;
+  if (!b || !out || (!c51 && !sample_only)) return fail(B2R_ERR_INVALID_ARGUMENT, "NULL argument");
   if (!b->tree) return fail(B2R_ERR_UNSUPPORTED, "not a prioritized buffer");
   if (batch <= 0 || batch > 60000)
     return fail(B2R_ERR_INVALID_ARGUMENT, "batch must be in [1, 60000]");
@@ -115,13 +121,14 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   const int32_t rows_cap =
       shard && shard->max_rows > 0 && shard->max_rows < batch ? shard->max_rows : batch;
   g_host_trace.lap(1);
-  b2r_c51_args loss = *c51;
+  b2r_c51_args loss = c51 ? *c51 : b2r_c51_args{};
   loss.batch = rows_cap;
   loss.actions = static_cast<const int32_t *>(out->action);
   loss.rewards = static_cast<const float *>(out->reward);
   loss.terminals = static_cast<const uint8_t *>(out->terminal);
   loss.sampling_probabilities = out->sampling_probabilities;
-  loss.min_probability = b->min_prob;
+  float *const min_out = sample_only ? shard->min_probability : b->min_prob;
+  loss.min_probability = min_out;
   loss.batch_count = count;
   if (count) loss.mean_weighted_loss = nullptr;
   // The half of the loss that needs the network outputs only (every action's softmax
@@ -129,7 +136,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   // sampler; the tail that needs the sampled rows follows the sampler (c51.cu).
   // (A shard does not know its row count before it has sampled: the first half covers
   // every row its logits hold.)
-  const bool split_loss = !debug_skip() && c51_can_split(&loss);
+  const bool split_loss = !sample_only && !debug_skip() && c51_can_split(&loss);
   if (direct != nullptr && direct->online_src != nullptr && !split_loss)
     return fail(B2R_ERR_INVALID_ARGUMENT, "direct logits need the loss in two halves");
   const bool unjoined = direct != nullptr && split_loss;  // (see DirectIO)
@@ -181,9 +188,10 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   // this call are applied behind the write-back, at the end of the call, and are seen by
   // the next step's sampler: the order of effects on the tree stays the reference's
   // add, sample, set_priority, add, ... with the adds one call later.
-  const b2r_exchange *early =
-      shard && shard->exchange->early_publish && shard->exchange->world > 1 ? shard->exchange
-                                                                           : nullptr;
+  const b2r_exchange *early = shard && !sample_only && shard->exchange->early_publish &&
+                                      shard->exchange->world > 1
+                                  ? shard->exchange
+                                  : nullptr;
   if (!early) B2R_TRY(flush_queue(b, s, batch > split_min()));
   const bool flush_behind = early != nullptr && b->q_entries > 0;
   g_host_trace.lap(2);
@@ -231,8 +239,8 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
     B2R_TRY(launch_sample_sharded(
         b, batch, shard->exchange->world, shard->exchange->rank, nullptr,
         shard->exchange, nullptr, b->cfg.max_sample_attempts, nullptr, seed, offset,
-        shard->out_slots, sample_idx, const_cast<int32_t *>(count), s, out, b->min_prob,
-        rows_cap, split_loss ? &pre_sync : nullptr));
+        shard->out_slots, sample_idx, const_cast<int32_t *>(count), s, out, min_out,
+        rows_cap, split_loss ? &pre_sync : nullptr, sample_only));
   else
     B2R_TRY(launch_sample(b, batch, true, seed, offset, nullptr, nullptr, 0,
                           sample_idx, b->info, s, out, b->min_prob,
@@ -260,7 +268,8 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
     if (off != nullptr && std::atoi(off) == 0) return 0;
     return e != nullptr ? std::atoi(e) : 1024;
   }();
-  const bool groupable = tree_can_presort(rows_cap, expected_rows) && !(debug_skip() & 6);
+  const bool groupable =
+      !sample_only && tree_can_presort(rows_cap, expected_rows) && !(debug_skip() & 6);
   const int64_t likely_rows = expected_rows >= 0 ? expected_rows : rows_cap;
   const bool early_tree = groupable && split_loss && likely_rows <= tree_early_max;
   const bool presort = groupable && !early_tree;
@@ -288,6 +297,10 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
     }
   }
   g_host_trace.lap(4);
+  if (sample_only) {
+    if (frames) B2R_CUDA(cudaStreamWaitEvent(s, b->ev_join, 0));
+    return B2R_OK;
+  }
   // (Measured: waiting for the logits before the sampler, or recording "loss done"
   // after the write-back, serialises the input copy of the next step behind this
   // step's tail and costs 13 us per update.)
@@ -461,8 +474,28 @@ int b2r_train_step_sharded_device(b2r_buffer *b, b2r_exchange *x,
                                   int32_t *out_count, int32_t max_rows,
                                   b2r_stream stream) {
   if (max_rows < 0) return fail(B2R_ERR_INVALID_ARGUMENT, "max_rows must be >= 0");
-  b2r::ShardSpec shard = {x, out_slots, out_count, max_rows};
+  b2r::ShardSpec shard = {x, out_slots, out_count, max_rows, false, nullptr};
   return b2r::train_step(b, global_batch, seed, offset, out, c51, as_stream(stream),
+                         nullptr, nullptr, &shard);
+}
+
+int b2r_sample_transition_batch_sharded_device(b2r_buffer *b, b2r_exchange *x,
+                                               int32_t global_batch, uint64_t seed,
+                                               uint64_t offset, const b2r_batch *out,
+                                               int32_t *out_slots, int32_t *out_count,
+                                               int32_t max_rows, float *min_probability,
+                                               b2r_stream stream) {
+  if (global_batch < 1) return fail(B2R_ERR_INVALID_ARGUMENT, "global_batch must be >= 1");
+  if (max_rows < 0) return fail(B2R_ERR_INVALID_ARGUMENT, "max_rows must be >= 0");
+  if (!b || !x || !out || !out_slots || !out_count || !min_probability)
+    return fail(B2R_ERR_INVALID_ARGUMENT,
+                "buffer, exchange, out, out_slots, out_count and min_probability are "
+                "required");
+  if (!x->connected) return fail(B2R_ERR_INVALID_ARGUMENT, "the exchange is not connected");
+  // the sharded loss of this step latches a peer that never published into this buffer
+  x->latched = b->status;
+  b2r::ShardSpec shard = {x, out_slots, out_count, max_rows, true, min_probability};
+  return b2r::train_step(b, global_batch, seed, offset, out, nullptr, as_stream(stream),
                          nullptr, nullptr, &shard);
 }
 
@@ -644,7 +677,8 @@ int b2r_trainer_step_host(b2r_trainer *t, const float *online_logits,
       io.loss_host = t->ring_dev + (size_t)slot * (t->cfg.logit_rows + 1);
       // the buffers of this set were last read by the tail of step n - 2
       io.first_half_after = n >= 2 ? t->ev_done[(size_t)((n - 2) % t->ring)] : nullptr;
-      b2r::ShardSpec shard = {t->exchange, t->slots, t->count_buf[set], t->cfg.logit_rows};
+      b2r::ShardSpec shard = {t->exchange, t->slots, t->count_buf[set], t->cfg.logit_rows,
+                              false, nullptr};
       // (the result slot of step n is read by the host after ev_done[slot], recorded
       // behind the tail; with ring = depth + 1 slots it was collected before this call)
       B2R_TRY(b2r::train_step(t->buf, t->cfg.batch, t->cfg.seed, 0, &t->batch, &c51, s,
@@ -699,7 +733,8 @@ int b2r_trainer_step_host(b2r_trainer *t, const float *online_logits,
     c51.online_logits = t->logits[set][0];
     c51.target_logits = t->logits[set][1];
     c51.loss = t->loss_buf[set];
-    b2r::ShardSpec shard = {t->exchange, t->slots, t->count_buf[set], t->cfg.logit_rows};
+    b2r::ShardSpec shard = {t->exchange, t->slots, t->count_buf[set], t->cfg.logit_rows,
+                            false, nullptr};
     B2R_TRY(b2r::train_step(t->buf, t->cfg.batch, t->cfg.seed, 0, &t->batch, &c51, s,
                             t->ev_in[set], after_loss, &shard, &hints));
   } else if (t->cfg.use_graph && n >= 2) {

@@ -322,6 +322,25 @@ __device__ __forceinline__ void exchange_publish(const ExchangeArgs &x, int worl
 }
 #endif  // __CUDACC__
 
+// Second region of a mailbox: the ranks' local minimum sampling probabilities of a step
+// (the IS-weight normaliser of a sharded batch, read by b2r_c51_loss_sharded).  Layout
+// [2 parities][world] words after the totals; a word is the f32 value in the high half
+// and the step number in the low half, written with ONE 8-byte store.
+constexpr int kMinWordsOffset = 2 * kMaxShards * 2;
+constexpr int kMailboxWords = kMinWordsOffset + 2 * kMaxShards;
+
+#ifdef __CUDACC__
+// Called by ONE thread: stores this rank's local minimum of step `seq` into every peer's
+// mailbox (the own value stays with the caller: its min_probability).
+__device__ __forceinline__ void exchange_publish_min(const ExchangeArgs &x, int world,
+                                                     int rank, float local_min,
+                                                     uint64_t seq) {
+  const uint64_t word = ((uint64_t)__float_as_uint(local_min) << 32) | (uint32_t)seq;
+  for (int g = 0; g < world; ++g)
+    if (g != rank) st_sys_u64(x.peer[g] + kMinWordsOffset + (seq & 1) * world + rank, word);
+}
+#endif  // __CUDACC__
+
 // "The sampled indices are final": what the kernel in front of the early write-back
 // (tree.cu, kEarly) tells it through memory, so that the write-back can be resident and
 // start on the indices the moment they are — a programmatic dependent launch would only

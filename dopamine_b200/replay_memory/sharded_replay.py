@@ -175,6 +175,39 @@ class ShardedPrioritizedReplay(object):
         ctypes.byref(batch), _native.current_stream()))
     return slots, count, tuple(arrays)
 
+  def sample_transition_batch_sharded(self, global_batch, max_rows=None):
+    """This rank's share of a global batch in one call over the peer exchange
+    (b2r_sample_transition_batch_sharded_device): sharded sampler, scalar columns and
+    frame copies.  Returns (slots, count, batch tuple, min_probability), CUDA tensors
+    sized by `max_rows` rows (default `share_bound`); rows [0, count) are this rank's
+    strata in ascending order, the rest are left from earlier calls.  min_probability
+    (1,) is the minimum sampling probability of this rank's rows; the sampler has also
+    published it to the peers for `rainbow_agent.c51_loss(..., sharded=...)`.  The
+    tensors are reused by every call with the same sizes (static for CUDA graphs)."""
+    if self.exchange is None:
+      raise ValueError('sample_transition_batch_sharded needs a PeerExchange')
+    torch = self._torch
+    global_batch = int(global_batch)
+    rows = (share_bound(global_batch, self.world) if max_rows is None
+            else min(int(max_rows), global_batch))
+    key = (global_batch, rows)
+    if getattr(self, '_share_out', None) is None or self._share_out[0] != key:
+      _, arrays, batch = self.memory._alloc_outputs(rows, True)  # pylint: disable=protected-access
+      self._share_out = (key, torch.zeros(rows, dtype=torch.int32, device='cuda'),
+                         tuple(arrays), batch,
+                         torch.zeros(1, dtype=torch.float32, device='cuda'))
+    _, slots, arrays, batch, min_probability = self._share_out
+    _native.check(self._lib.b2r_sample_transition_batch_sharded_device(
+        self._h, self.exchange._h, global_batch, self.seed, 0,  # pylint: disable=protected-access
+        ctypes.byref(batch), slots.data_ptr(), self._count.data_ptr(), rows,
+        min_probability.data_ptr(), _native.current_stream()))
+    return slots, self._count, arrays, min_probability
+
+  def check(self):
+    """Raises the error latched by an earlier asynchronous call (a share beyond
+    max_rows, a peer that did not answer in time, ...).  Synchronises."""
+    _native.check(self._lib.b2r_check(self._h, _native.current_stream()))
+
   def set_priority(self, indices, priorities, count):
     """Batched priority write-back for the first `count` (device) entries."""
     _native.check(self._lib.b2r_set_priority_device_counted(

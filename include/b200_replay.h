@@ -377,6 +377,24 @@ int b2r_sample_indices_sharded_p2p_device(b2r_buffer *buf, b2r_exchange *exchang
                                           int32_t *out_indices, int32_t *out_count,
                                           b2r_stream stream);
 
+/* The first half of b2r_train_step_sharded_device alone: the sharded sampler (totals
+ * over the exchange, this rank's strata compacted at the front of `out`, *out_count of
+ * them, out_slots[r] = stratum of row r; the scalar columns written by the sampler) and
+ * the frame copies, joined into `stream` before the call returns.  No loss, no
+ * write-back: a learner runs its networks on the max_rows rows of `out` next, then
+ * b2r_c51_loss_sharded and b2r_set_priority_device_counted.  *min_probability
+ * (DEVICE) receives the minimum sampling probability of this rank's rows, and the
+ * sampler publishes it to every peer of the exchange for this step.  max_rows as in
+ * b2r_train_step_sharded_device (0 = global_batch); a share above it latches
+ * B2R_ERR_UNSUPPORTED (b2r_check).  Early publish is not used by this call.
+ * DEVICE pointers; asynchronous; can be captured in a CUDA graph. */
+int b2r_sample_transition_batch_sharded_device(b2r_buffer *buf, b2r_exchange *exchange,
+                                               int32_t global_batch, uint64_t seed,
+                                               uint64_t offset, const b2r_batch *out,
+                                               int32_t *out_slots, int32_t *out_count,
+                                               int32_t max_rows, float *min_probability,
+                                               b2r_stream stream);
+
 /* Variants whose element count lives on the DEVICE (*count <= max_...): what a
  * shard serves of a global batch is only known there.  Rows past *count are
  * skipped.  Asynchronous. */
@@ -428,6 +446,21 @@ typedef struct {
 /* Bellman target + projection + softmax cross-entropy + new priorities + IS
  * weights in one launch (RA:200-293). */
 int b2r_c51_loss(const b2r_c51_args *args, b2r_stream stream);
+
+/* The loss of one shard of a global batch of `global_batch` strata, sampled by
+ * b2r_sample_transition_batch_sharded_device over the same exchange (the call that
+ * closed the exchange's current step).  The same arithmetic per row as b2r_c51_loss;
+ * args->batch is the rank's max_rows, args->batch_count (required) its row count and
+ * args->min_probability (required with sampling_probabilities) the sampler's local
+ * minimum.  The IS-weight normaliser is the minimum over every rank's published local
+ * minimum, so the weights are those of the whole global batch (RA:279-280);
+ * mean_weighted_loss = (sum over this rank's rows of w * loss) / global_batch and
+ * grad_logits its derivative, with rows >= count written as zeros.  Summed over the
+ * ranks, the means and the gradients are the global batch's (RA:293).  A peer whose
+ * minimum does not arrive within the exchange's timeout latches B2R_ERR_EXCHANGE in
+ * the sampled buffer (b2r_check).  DEVICE pointers; asynchronous. */
+int b2r_c51_loss_sharded(const b2r_c51_args *args, b2r_exchange *exchange,
+                         int32_t global_batch, b2r_stream stream);
 
 /* DQN (dqn_agent.py:283-322): Bellman target r + gamma^n max_a Q_target(s') (1 - t),
  * Huber loss (delta 1) against Q_online(s, a), optional mean and gradient.  f32,

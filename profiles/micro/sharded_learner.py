@@ -1,0 +1,147 @@
+"""ms per update and transitions/s of ShardedRainbowLearner at 1/2/4/8 GPUs: a global
+batch of 32 rows per GPU, a replay shard of 1M transitions per GPU, eager and
+replayed as a CUDA graph.  Also reports the rows the networks computed (max_rows per
+rank, the padding that keeps the shapes static) next to the useful rows (the global
+batch), and the card's name and power limit read in the same run.
+
+  python profiles/micro/sharded_learner.py [--gpus 1,2,4,8] [--steps 200] [--out F]
+
+Each configuration runs in fresh processes (one per GPU, NCCL); rank 0 times `--steps`
+updates between CUDA events after `--warmup` updates.  The frames of the shards are
+left as allocated (only the scalar columns and the priorities are written): the
+timing does not depend on pixel values.
+"""
+import argparse
+import json
+import os
+import socket
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+if ROOT not in sys.path:
+  sys.path.insert(0, ROOT)
+
+import numpy as np  # noqa: E402
+
+PER_GPU_BATCH = 32
+CAPACITY = 1000000
+ACTIONS = 18
+
+
+def _shard(cap, seed, batch):
+  from dopamine_b200.replay_memory import prioritized_replay_buffer as prb
+  rng = np.random.RandomState(seed)
+  mem = prb.OutOfGraphPrioritizedReplayBuffer(
+      (84, 84), 4, cap, batch, update_horizon=3, gamma=0.99, output='torch',
+      rng='device', seed=seed, reuse_outputs=True)
+  mem._store['action'] = rng.randint(0, ACTIONS, size=cap).astype(np.int32)
+  mem._store['reward'] = np.clip(rng.randn(cap), -1, 1).astype(np.float32)
+  mem._store['terminal'] = (rng.rand(cap) < 0.01).astype(np.uint8)
+  mem.add_count = cap + 1000
+  mem.invalid_range = np.array([(1000 - 3 + i) % cap for i in range(7)])
+  mem.set_priority(np.arange(cap, dtype=np.int32),
+                   np.sqrt(np.abs(rng.randn(cap)) + 1e-10).astype(np.float32))
+  return mem
+
+
+def _worker(rank, world, port, graph, steps, warmup, out_path):
+  import torch
+  import torch.distributed as dist
+  from dopamine_b200.agents.rainbow import agent
+  torch.cuda.set_device(rank)
+  os.environ['MASTER_ADDR'] = '127.0.0.1'
+  os.environ['MASTER_PORT'] = str(port)
+  dist.init_process_group('nccl', rank=rank, world_size=world,
+                          device_id=torch.device('cuda', rank))
+  try:
+    global_batch = PER_GPU_BATCH * world
+    learner = agent.ShardedRainbowLearner(
+        ACTIONS, batch_size=global_batch, memory=_shard(CAPACITY, 10 + rank, global_batch),
+        replay_capacity=CAPACITY, seed=1, cuda_graph=graph)
+    for _ in range(warmup):
+      learner.train_step()
+    torch.cuda.synchronize()
+    dist.barrier()
+    start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    start.record()
+    for _ in range(steps):
+      learner.train_step()
+    end.record()
+    torch.cuda.synchronize()
+    learner.check()
+    ms = start.elapsed_time(end) / steps
+    if rank == 0:
+      result = dict(gpus=world, mode='graph' if graph else 'eager', steps=steps,
+                    ms_per_update=round(ms, 4),
+                    transitions_per_s=round(global_batch / ms * 1e3, 1),
+                    useful_rows=global_batch, max_rows_per_rank=learner.max_rows,
+                    network_rows=learner.max_rows * world,
+                    loss=float(learner.loss.item()))
+      with open(out_path, 'w') as f:
+        json.dump(result, f)
+    dist.barrier()
+  finally:
+    dist.destroy_process_group()
+
+
+def _free_port():
+  with socket.socket() as s:
+    s.bind(('127.0.0.1', 0))
+    return s.getsockname()[1]
+
+
+def main():
+  import torch
+  import torch.multiprocessing as mp
+  p = argparse.ArgumentParser()
+  p.add_argument('--gpus', default='1,2,4,8')
+  p.add_argument('--steps', type=int, default=200)
+  p.add_argument('--warmup', type=int, default=20)
+  p.add_argument('--out', default=None)
+  a = p.parse_args()
+  if not torch.cuda.is_available():
+    sys.exit('needs CUDA devices')
+  card = subprocess.check_output(
+      ['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader']
+  ).decode().strip().splitlines()
+  lines = [json.dumps(dict(cards=card))]
+  print(lines[0], flush=True)
+  tmp = os.environ.get('TMPDIR', '/tmp')
+  for n in [int(x) for x in a.gpus.split(',')]:
+    if n > torch.cuda.device_count():
+      lines.append(json.dumps(dict(gpus=n, skipped='only {} devices'.format(
+          torch.cuda.device_count()))))
+      print(lines[-1], flush=True)
+      continue
+    for graph in (False, True):
+      out_path = os.path.join(tmp, 'sharded_learner_{}_{}.json'.format(n, int(graph)))
+      ctx = mp.get_context('spawn')
+      port = _free_port()
+      procs = [ctx.Process(target=_worker,
+                           args=(r, n, port, graph, a.steps, a.warmup, out_path))
+               for r in range(n)]
+      for q in procs:
+        q.start()
+      for q in procs:
+        q.join(timeout=1200)
+      for q in procs:
+        if q.is_alive():
+          q.terminate()
+          q.join(timeout=60)
+      codes = [q.exitcode for q in procs]
+      if any(c != 0 for c in codes):
+        lines.append(json.dumps(dict(gpus=n, mode='graph' if graph else 'eager',
+                                     failed=codes)))
+      else:
+        with open(out_path) as f:
+          lines.append(f.read())
+      print(lines[-1], flush=True)
+  if a.out:
+    os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
+    with open(a.out, 'w') as f:
+      f.write('\n'.join(lines) + '\n')
+
+
+if __name__ == '__main__':
+  main()
