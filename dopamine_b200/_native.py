@@ -264,6 +264,7 @@ SIGNATURES = {
     'b2r_trainer_drain': (c_int, [c_void_p, c_void_p, P(c_int64), c_void_p]),
     'b2r_trainer_views': (c_int, [c_void_p, P(Batch), P(C51Args)]),
     'b2r_iqn_loss': (c_int, [P(IqnArgs), c_void_p]),
+    'b2r_iqn_loss_sharded': (c_int, [P(IqnArgs), c_void_p, c_int32, c_void_p]),
     'b2r_actor_create': (c_int, [c_int64, c_int32, c_int32, c_int32, P(c_void_p)]),
     'b2r_actor_destroy': (c_int, [c_void_p]),
     'b2r_actor_reset': (c_int, [c_void_p, c_void_p, c_void_p]),

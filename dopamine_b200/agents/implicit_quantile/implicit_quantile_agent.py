@@ -30,7 +30,7 @@ def cumulative_gamma(gamma, update_horizon):
 def quantile_huber_loss(online_quantile_values, quantiles, target_quantile_values,
                         action_quantile_values, actions, rewards, terminals,
                         cumulative_gamma, kappa=1.0, want_grad=False,  # pylint: disable=redefined-outer-name
-                        want_mean=True, out=None):
+                        want_mean=True, out=None, sharded=None):
   """Per-row IQN loss for one replay batch, on the device.
 
   Args:
@@ -44,6 +44,12 @@ def quantile_huber_loss(online_quantile_values, quantiles, target_quantile_value
   Returns:
     dict with 'loss' (B,), 'next_action' (B,) int32, optionally 'mean_loss'
     (scalar) and 'grad' (N * B, A) = d mean(loss) / d online_quantile_values.
+    sharded: (global_batch, count) — the B rows are one rank's share of a global batch
+    of `global_batch` strata, as `ShardedPrioritizedReplay.sample_transition_batch_sharded`
+    returns it (b2r_iqn_loss_sharded): the first `count` rows ((1,) int32 CUDA tensor)
+    are valid, the mean and its gradient are this rank's part of the global batch's
+    (divisor global_batch), rows past the count get loss 0 and zero gradients and keep
+    their old next_action.
   """
   torch = _torch()
   if not kappa > 0:
@@ -69,6 +75,13 @@ def quantile_huber_loss(online_quantile_values, quantiles, target_quantile_value
   n, n_prime, k = sizes
   if quantiles.numel() != n * batch:
     raise ValueError('quantiles must hold one tau per online row')
+  if sharded is not None:
+    global_batch, count = sharded
+    if (not isinstance(count, torch.Tensor) or count.dtype != torch.int32 or
+        not count.is_cuda or tuple(count.shape) != (1,)):
+      raise ValueError('count must be a (1,) int32 CUDA tensor')
+    if int(global_batch) < 1:
+      raise ValueError('global_batch must be >= 1, got {}'.format(global_batch))
   dev = online_quantile_values.device
   if out is None:
     out = {'loss': torch.empty(batch, dtype=torch.float32, device=dev),
@@ -97,8 +110,12 @@ def quantile_huber_loss(online_quantile_values, quantiles, target_quantile_value
   args.next_action = out['next_action'].data_ptr() if 'next_action' in out else None
   args.mean_loss = out['mean_loss'].data_ptr() if 'mean_loss' in out else None
   args.grad_quantile_values = out['grad'].data_ptr() if 'grad' in out else None
-  _native.check(_native.lib().b2r_iqn_loss(ctypes.byref(args),
-                                           _native.current_stream()))
+  if sharded is None:
+    _native.check(_native.lib().b2r_iqn_loss(ctypes.byref(args),
+                                             _native.current_stream()))
+    return out
+  _native.check(_native.lib().b2r_iqn_loss_sharded(
+      ctypes.byref(args), count.data_ptr(), int(global_batch), _native.current_stream()))
   return out
 
 
@@ -110,8 +127,7 @@ class QuantileHuberLoss(object):
   _fn = None
 
   @classmethod
-  def apply(cls, online_quantile_values, quantiles, target_quantile_values,
-            action_quantile_values, actions, rewards, terminals, gamma_n, kappa=1.0):
+  def _function(cls):
     if cls._fn is None:
       torch = _torch()
 
@@ -119,10 +135,10 @@ class QuantileHuberLoss(object):
 
         @staticmethod
         def forward(ctx, online, taus, target, action_net, actions, rewards,  # pylint: disable=redefined-outer-name
-                    terminals, gamma_n, kappa):  # pylint: disable=redefined-outer-name
+                    terminals, gamma_n, kappa, sharded):  # pylint: disable=redefined-outer-name
           out = quantile_huber_loss(online.detach(), taus.detach(), target.detach(),
                                     action_net.detach(), actions, rewards, terminals,
-                                    gamma_n, kappa, want_grad=True)
+                                    gamma_n, kappa, want_grad=True, sharded=sharded)
           ctx.save_for_backward(out['grad'])
           ctx.mark_non_differentiable(out['loss'])
           return out['mean_loss'], out['loss']
@@ -130,9 +146,30 @@ class QuantileHuberLoss(object):
         @staticmethod
         def backward(ctx, grad_mean, *unused):
           (grad,) = ctx.saved_tensors
-          return (grad * grad_mean,) + (None,) * 8
+          return (grad * grad_mean,) + (None,) * 9
 
       cls._fn = _Fn
-    return cls._fn.apply(online_quantile_values, quantiles, target_quantile_values,
-                         action_quantile_values, actions, rewards, terminals, gamma_n,
-                         kappa)
+    return cls._fn
+
+  @classmethod
+  def apply(cls, online_quantile_values, quantiles, target_quantile_values,
+            action_quantile_values, actions, rewards, terminals, gamma_n, kappa=1.0):
+    return cls._function().apply(online_quantile_values, quantiles,
+                                 target_quantile_values, action_quantile_values, actions,
+                                 rewards, terminals, gamma_n, kappa, None)
+
+
+class ShardedQuantileHuberLoss(QuantileHuberLoss):
+  """`QuantileHuberLoss` over one rank's share of a sharded global batch
+  (b2r_iqn_loss_sharded): `mean, loss = ShardedQuantileHuberLoss.apply(..., kappa,
+  sharded)` with `sharded` = (global_batch, count) as in `quantile_huber_loss`.  `mean`
+  is this rank's partial mean (its rows' losses over the global batch size) and backward
+  gives its gradient; summed over the ranks both are the global batch's."""
+
+  @classmethod
+  def apply(cls, online_quantile_values, quantiles, target_quantile_values,
+            action_quantile_values, actions, rewards, terminals, gamma_n, kappa,
+            sharded):
+    return cls._function().apply(online_quantile_values, quantiles,
+                                 target_quantile_values, action_quantile_values, actions,
+                                 rewards, terminals, gamma_n, kappa, tuple(sharded))

@@ -11,6 +11,9 @@ target sync.  Uniform replay through the prioritized buffer class, as the refere
 """
 import math
 
+import numpy as np
+
+from dopamine_b200.agents import sharded_learner
 from dopamine_b200.agents.dqn import learner as dqn_learner
 from dopamine_b200.agents.implicit_quantile import implicit_quantile_agent as iqn
 from dopamine_b200.agents.rainbow import agent as conv
@@ -149,3 +152,101 @@ class IQNLearner(object):
       self.sync_target()
     self.training_steps += 1
     return loss
+
+
+class ShardedIQNLearner(sharded_learner.ShardedLearner, IQNLearner):
+  """`IQNLearner` on ONE global batch sharded over the ranks of torch.distributed.
+
+  Every rank owns one replay shard of `replay_capacity` transitions (unit priorities, as
+  the reference's IQN uses its prioritized buffer, implicit_quantile.gin:23-24) and a
+  peer-memory exchange.  `batch_size` is the GLOBAL batch: its strata are apportioned
+  over the shards by their totals, i.e. by their transition counts, so the update is the
+  reference's update (implicit_quantile_agent.py:166-321) on one uniform batch of a
+  virtual replay of every shard's transitions.  One update:
+    1. `sample()`: sharded sampler + frame copies into `max_rows` rows (default
+       `share_bound`), then fresh taus for the three networks;
+    2. `loss_backward()`: the online net on `state` with N taus, the target net on
+       `next_state` with N' taus and the action-picking net (target net; online net with
+       `double_dqn`) with K taus, all on `max_rows` rows, then the sharded
+       quantile-Huber loss (mean and gradient over the global batch, zero gradients for
+       padded rows) and backward into one flat buffer;
+    3. `reduce()`: ONE all-reduce (sum) of that buffer — every gradient and, appended,
+       the partial loss, so the reported loss is the global mean;
+    4. `apply()`: TF-form Adam.  Priorities stay 1: there is no write-back.
+  IQN has no importance weights, so the loss exchanges nothing between the ranks.  The
+  taus are drawn into three static buffers, `online_taus` (N * max_rows, 1),
+  `target_taus` (N' * max_rows, 1) and `action_taus` (K * max_rows, 1), refilled in
+  place by every `sample()` from a CUDA generator seeded with (seed, rank): an emulated
+  rank and a process of the same rank draw the same taus, and a replayed graph draws
+  fresh ones.  `cuda_graph=True` captures the whole update, all-reduce included.  Errors
+  latched on the device are raised by `check()`, which `sync_target()` calls.  Pass
+  `exchange` (`PeerExchange.emulated`) to run the phases of several ranks on one device
+  without torch.distributed (tests); `reduce()` then is the caller's.
+  """
+
+  def __init__(self, num_actions, batch_size=32, max_rows=None, exchange=None,
+               group=None, exchange_timeout_s=2.0, ddp=False, cuda_graph=False,
+               **kwargs):
+    torch = _torch()
+    exchange = self._connect(exchange, group, exchange_timeout_s, ddp)
+    IQNLearner.__init__(self, num_actions, batch_size=batch_size, **kwargs)
+    self._cuda_graph = bool(cuda_graph)
+    self._graph = None
+    self._static_loss = None
+    if self._cuda_graph:  # Adam's step count on the device, so that it can be captured
+      adam = self.optimizer.param_groups[0]
+      self.optimizer = conv.make_tf_adam(self.online.parameters(), lr=adam['lr'],
+                                         epsilon=adam['epsilon'], capturable=True)
+    seed = kwargs.get('seed', 0)
+    self._shard(exchange, max_rows, seed)
+    self._generator = torch.Generator(device='cuda')
+    self._generator.manual_seed(
+        int(np.random.SeedSequence([int(seed), self.rank]).generate_state(1)[0]))
+    taus = lambda samples: torch.zeros(samples * self.max_rows, 1, device='cuda')
+    self.online_taus = taus(self.num_tau_samples)
+    self.target_taus = taus(self.num_tau_prime_samples)
+    self.action_taus = taus(self.num_quantile_samples)
+
+  def _graph_generators(self):
+    return (self._generator,)
+
+  # -- phases (reduce: ShardedLearner's) ----------------------------------------------
+  def sample(self):
+    """This rank's share of the global batch, then fresh taus (:180-181)."""
+    sample = super(ShardedIQNLearner, self).sample()
+    for t in (self.online_taus, self.target_taus, self.action_taus):
+      t.uniform_(0., 1., generator=self._generator)
+    return sample
+
+  def loss_backward(self):
+    """Networks, sharded loss and backward: the flat buffer holds this rank's partial
+    gradients and partial mean.  Returns the per-row losses."""
+    torch = _torch()
+    _, count, batch, _ = self._sample
+    state, action, reward, next_state, _, _, terminal = batch[:7]
+    with torch.no_grad():
+      target_values, _ = self.target(next_state, self.num_tau_prime_samples,
+                                     self.target_taus)
+      picker = self.online if self.double_dqn else self.target
+      action_values, _ = picker(next_state, self.num_quantile_samples, self.action_taus)
+    online_values, _ = self.online(state, self.num_tau_samples, self.online_taus)
+    mean, rows = iqn.ShardedQuantileHuberLoss.apply(
+        online_values, self.online_taus, target_values, action_values, action, reward,
+        terminal, self.cumulative_gamma, self.kappa, (self.batch_size, count))
+    self._flat.zero_()
+    mean.backward()  # (accumulates into the views of the flat buffer)
+    self.loss.copy_(mean.detach().view(1))
+    return rows
+
+  def apply(self):
+    """Adam on the reduced gradients."""
+    self.optimizer.step()
+
+  def _update(self):
+    self.sample()
+    self.loss_backward()
+    self.reduce()
+    self.apply()
+    if not self._cuda_graph or self._graph is None:
+      self.updates += 1
+    return self.loss

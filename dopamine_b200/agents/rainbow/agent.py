@@ -22,6 +22,7 @@ import math
 
 import numpy as np
 
+from dopamine_b200.agents import sharded_learner
 from dopamine_b200.agents.dqn import dqn_agent
 from dopamine_b200.agents.rainbow import rainbow_agent
 from dopamine_b200.replay_memory import prioritized_replay_buffer
@@ -165,7 +166,7 @@ def make_tf_adam(params, lr, beta1=0.9, beta2=0.999, epsilon=1e-8, capturable=Fa
   return TFAdam()
 
 
-class RainbowLearner(object):
+class RainbowLearner(sharded_learner.GraphedUpdate):
   """Replay + train op of RainbowAgent (rainbow_agent.py:93-337)."""
 
   def __init__(self, num_actions, observation_shape=(84, 84), stack_size=4,
@@ -233,32 +234,7 @@ class RainbowLearner(object):
       probs = torch.softmax(self.online(state), dim=2)
       return (probs * self.support).sum(dim=2)
 
-  # -- the train op (rainbow_agent.py:253-305) ---------------------------------------
-  def train_step(self):
-    """One update; returns the scalar training loss (a CUDA tensor, no sync)."""
-    if not self._cuda_graph:
-      return self._update()
-    if self._graph is None:
-      self._capture()
-    self.memory._flush()  # pylint: disable=protected-access
-    self._graph.replay()
-    self.updates += 1
-    return self._static_loss
-
-  def _capture(self):
-    torch = _torch()
-    side = torch.cuda.Stream()
-    side.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(side):
-      for _ in range(3):  # lazy allocations, cuDNN algorithm selection, Adam state
-        self._update()
-    torch.cuda.current_stream().wait_stream(side)
-    torch.cuda.synchronize()
-    self.memory._flush()  # pylint: disable=protected-access
-    self._graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(self._graph):
-      self._static_loss = self._update()
-
+  # -- the train op (rainbow_agent.py:253-305); train_step() is GraphedUpdate's ------
   def _update(self):
     torch = _torch()
     batch = self.memory.sample_transition_batch(self.batch_size)
@@ -341,7 +317,7 @@ class RainbowAgent(RainbowLearner, dqn_agent.ActingLoop):
       self.store_transition(last_observation, action, reward, is_terminal, priority)
 
 
-class ShardedRainbowLearner(RainbowLearner):
+class ShardedRainbowLearner(sharded_learner.ShardedLearner, RainbowLearner):
   """`RainbowLearner` on ONE global prioritized batch sharded over the ranks of
   torch.distributed (SURVEY.md section 8(d), config 5 fed by config 4's sampler).
 
@@ -362,53 +338,17 @@ class ShardedRainbowLearner(RainbowLearner):
   included.  Errors latched on the device (a share beyond `max_rows`, a peer that did not
   answer) are raised by `check()`, which `sync_target()` calls.  Pass `exchange`
   (`PeerExchange.emulated`) to run the phases of several ranks on one device without
-  torch.distributed (tests); `reduce()` then is the caller's.
+  torch.distributed (tests); `reduce()` then is the caller's.  The rank plumbing is
+  `sharded_learner.ShardedLearner`'s.
   """
 
   def __init__(self, num_actions, batch_size=32, max_rows=None, exchange=None,
                group=None, exchange_timeout_s=2.0, ddp=False, **kwargs):
-    torch = _torch()
-    import torch.distributed as dist  # pylint: disable=g-import-not-at-top
-    from dopamine_b200.replay_memory import sharded_replay  # pylint: disable=g-import-not-at-top
-    if ddp:
-      raise ValueError('the sharded learner reduces its gradients itself (ddp=False)')
-    self._dist = dist if exchange is None else None
-    if exchange is None:
-      if not (dist.is_available() and dist.is_initialized()):
-        raise RuntimeError('ShardedRainbowLearner needs torch.distributed initialised')
-      exchange = sharded_replay.PeerExchange(group=group, timeout_s=exchange_timeout_s)
-    self._group = group
+    exchange = self._connect(exchange, group, exchange_timeout_s, ddp)
     RainbowLearner.__init__(self, num_actions, batch_size=batch_size, **kwargs)
-    self.exchange = exchange
-    self.rank, self.world = exchange.rank, exchange.world
-    self.sharded = sharded_replay.ShardedPrioritizedReplay(
-        self.memory, rank=self.rank, world_size=self.world,
-        seed=kwargs.get('seed', 0), exchange=exchange)
-    self.max_rows = (sharded_replay.share_bound(batch_size, self.world)
-                     if max_rows is None else min(int(max_rows), int(batch_size)))
-    params = list(self.online.parameters())
-    if self._dist is not None:
-      with torch.no_grad():
-        for p in params:
-          self._dist.broadcast(p, 0, group=group)
-      RainbowLearner.sync_target(self)
-    # every gradient views one flat buffer; the partial loss rides at its end
-    total = sum(p.numel() for p in params)
-    self._flat = torch.zeros(total + 1, dtype=torch.float32, device='cuda')
-    offset = 0
-    for p in params:
-      p.grad = self._flat[offset:offset + p.numel()].view_as(p)
-      offset += p.numel()
-    self.loss = self._flat[total:]
-    self._sample = None
+    self._shard(exchange, max_rows, kwargs.get('seed', 0))
 
-  # -- phases ------------------------------------------------------------------------
-  def sample(self):
-    """(slots, count, batch tuple, min_probability) of this rank's share."""
-    self._sample = self.sharded.sample_transition_batch_sharded(self.batch_size,
-                                                                self.max_rows)
-    return self._sample
-
+  # -- phases (sample, reduce: ShardedLearner's) ----------------------------------------
   def loss_backward(self):
     """Networks, sharded loss and backward: the flat buffer holds this rank's partial
     gradients and partial mean.  Returns the per-row priorities."""
@@ -428,10 +368,6 @@ class ShardedRainbowLearner(RainbowLearner):
     self.loss.copy_(mean.detach().view(1))
     return priorities
 
-  def reduce(self):
-    """The one all-reduce of the update: gradients and loss summed over the ranks."""
-    self._dist.all_reduce(self._flat, group=self._group)
-
   def apply(self, priorities):
     """Adam on the reduced gradients, then this rank's priority write-back."""
     self.optimizer.step()
@@ -448,16 +384,3 @@ class ShardedRainbowLearner(RainbowLearner):
     if not self._cuda_graph or self._graph is None:
       self.updates += 1
     return self.loss
-
-  def check(self):
-    """Raises what the device latched since the last check (synchronises); also
-    verifies that backward left every gradient in the flat buffer."""
-    lo, hi = self._flat.data_ptr(), self._flat.data_ptr() + 4 * self._flat.numel()
-    for p in self.online.parameters():
-      if p.grad is None or not lo <= p.grad.data_ptr() < hi:
-        raise RuntimeError('a gradient left the all-reduced buffer')
-    self.sharded.check()
-
-  def sync_target(self):
-    self.check()
-    RainbowLearner.sync_target(self)

@@ -18,6 +18,14 @@
 // as the reference's elementwise ops form it (no FMA contraction); the sums over t and
 // t' are accumulated in f64 in a fixed order and rounded once, which is within 1 ulp
 // of any f32 summation order the reference's reductions may use.
+//
+// Sharded mode (b2r_iqn_loss_sharded): the rows are one rank's share of a global batch.
+// Only the first min(*count, batch) CTAs compute a row, and the gradient scale and the
+// mean divide by the global batch instead of `batch`.  Per row that is the arithmetic of
+// the unsharded launch on the whole global batch, so a computed row's loss, next_action
+// and gradient rows are the same bits; CTAs past the count write zero gradient rows and
+// loss 0.  The mean is this rank's part of the global mean.  An unsharded launch is the
+// case count = NULL, global_batch = batch.
 #include "common.cuh"
 
 namespace b2r {
@@ -28,6 +36,8 @@ constexpr int kIqnMaxSamples = 256;  // N, N' <= 256
 
 struct IqnArgs {
   b2r_iqn_args u;
+  const int32_t *count;  // nullable: rows = min(*count, batch), else batch
+  int global_batch;      // divisor of the mean and of its gradient
   unsigned int *ticket;
 };
 
@@ -35,6 +45,34 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
+}
+
+// ---- mean over the batch (:315): the last CTA to finish sums loss[0, rows) in a fixed
+// order and divides by the global batch (every CTA calls; s_red, s_last in shared memory).
+__device__ __forceinline__ void iqn_mean(const IqnArgs &a, int rows, double *s_red,
+                                         bool *s_last) {
+  if (a.u.mean_loss == nullptr) return;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const unsigned int done = atomicAdd(a.ticket, 1u);
+    *s_last = (done == gridDim.x - 1);
+  }
+  __syncthreads();
+  if (!*s_last) return;
+  __threadfence();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  double acc = 0.0;
+  for (int k = threadIdx.x; k < rows; k += blockDim.x) acc += (double)__ldcg(a.u.loss + k);
+  acc = warp_sum_f64(acc);
+  if (lane == 0) s_red[warp] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double total = 0.0;
+    for (int k = 0; k < kIqnWarps; ++k) total += s_red[k];
+    *a.u.mean_loss = (float)(total / (double)a.global_batch);
+    *a.ticket = 0u;  // ready for the next launch
+  }
 }
 
 __global__ void __launch_bounds__(kIqnWarps * 32) iqn_loss_kernel(IqnArgs a) {
@@ -52,6 +90,17 @@ __global__ void __launch_bounds__(kIqnWarps * 32) iqn_loss_kernel(IqnArgs a) {
   pdl_release();
   pdl_acquire();
   const int b = blockIdx.x;
+  const int rows = a.count ? min(*a.count, B) : B;
+  if (b >= rows) {  // a padded row of a shard: zero gradient rows, loss 0, no next_action
+    if (a.u.grad_quantile_values)
+      for (int k = threadIdx.x; k < N * A; k += blockDim.x) {
+        const int t = k / A;
+        a.u.grad_quantile_values[((size_t)t * B + b) * A + (k - t * A)] = 0.f;
+      }
+    if (threadIdx.x == 0) a.u.loss[b] = 0.f;
+    iqn_mean(a, rows, s_red, &s_last);
+    return;
+  }
 
   // ---- greedy next action (:176-188): mean over the K samples, first maximum.
   // Warp w sums the samples k = w (mod 4) of 32 actions at a time; warp 0 adds the four
@@ -135,7 +184,7 @@ __global__ void __launch_bounds__(kIqnWarps * 32) iqn_loss_kernel(IqnArgs a) {
   }
   __syncthreads();
   if (warp == 0) {
-    const double grad_scale = -1.0 / ((double)kappa * (double)NP * (double)B);
+    const double grad_scale = -1.0 / ((double)kappa * (double)NP * (double)a.global_batch);
     double row_sum = 0.0;
     for (int t = lane; t < N; t += 32) {
       double acc = s_acc[0][t], gacc = s_gacc[0][t];
@@ -155,31 +204,38 @@ __global__ void __launch_bounds__(kIqnWarps * 32) iqn_loss_kernel(IqnArgs a) {
     if (lane == 0) a.u.loss[b] = (float)(row_sum / (double)NP);
   }
 
-  // ---- mean over the batch (:315): the last CTA to finish reduces in a fixed order
-  if (a.u.mean_loss == nullptr) return;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int done = atomicAdd(a.ticket, 1u);
-    s_last = (done == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  double acc = 0.0;
-  for (int k = threadIdx.x; k < B; k += blockDim.x) acc += (double)__ldcg(a.u.loss + k);
-  acc = warp_sum_f64(acc);
-  if (lane == 0) s_red[warp] = acc;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double total = 0.0;
-    for (int k = 0; k < kIqnWarps; ++k) total += s_red[k];
-    *a.u.mean_loss = (float)(total / (double)B);
-    *a.ticket = 0u;  // ready for the next launch
-  }
+  iqn_mean(a, rows, s_red, &s_last);
 }
 
 unsigned int *g_iqn_ticket = nullptr;
+
+// The checks and the launch of both entry points; count = NULL: unsharded.
+int iqn_launch(const b2r_iqn_args *args, const int32_t *count, int global_batch,
+               cudaStream_t stream) {
+  if (!args || args->batch <= 0 || args->num_actions <= 0 || args->num_tau_samples <= 0 ||
+      args->num_tau_prime_samples <= 0 || args->num_quantile_samples <= 0)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "bad IQN shape");
+  if (args->num_tau_samples > kIqnMaxSamples || args->num_tau_prime_samples > kIqnMaxSamples)
+    return fail(B2R_ERR_UNSUPPORTED, "more than 256 tau samples are not supported");
+  if (!(args->kappa > 0.f))
+    return fail(B2R_ERR_INVALID_ARGUMENT, "kappa must be positive");
+  if (!args->action_quantile_values || !args->target_quantile_values ||
+      !args->online_quantile_values || !args->quantiles || !args->actions ||
+      !args->rewards || !args->terminals || !args->loss)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "a required IQN pointer is NULL");
+  if (!g_iqn_ticket) {
+    B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&g_iqn_ticket), 4));
+    B2R_CUDA(cudaMemset(g_iqn_ticket, 0, 4));
+  }
+  IqnArgs a;
+  a.u = *args;
+  a.count = count;
+  a.global_batch = global_batch;
+  a.ticket = g_iqn_ticket;
+  B2R_CUDA(launch(iqn_loss_kernel, dim3(args->batch), dim3(kIqnWarps * 32), 0, stream, a));
+  B2R_LAUNCHED();
+  return B2R_OK;
+}
 
 }  // namespace
 }  // namespace b2r
@@ -188,27 +244,13 @@ using b2r::as_stream;
 using b2r::fail;
 
 extern "C" int b2r_iqn_loss(const b2r_iqn_args *args, b2r_stream stream) {
-  if (!args || args->batch <= 0 || args->num_actions <= 0 || args->num_tau_samples <= 0 ||
-      args->num_tau_prime_samples <= 0 || args->num_quantile_samples <= 0)
-    return fail(B2R_ERR_INVALID_ARGUMENT, "bad IQN shape");
-  if (args->num_tau_samples > b2r::kIqnMaxSamples ||
-      args->num_tau_prime_samples > b2r::kIqnMaxSamples)
-    return fail(B2R_ERR_UNSUPPORTED, "more than 256 tau samples are not supported");
-  if (!(args->kappa > 0.f))
-    return fail(B2R_ERR_INVALID_ARGUMENT, "kappa must be positive");
-  if (!args->action_quantile_values || !args->target_quantile_values ||
-      !args->online_quantile_values || !args->quantiles || !args->actions ||
-      !args->rewards || !args->terminals || !args->loss)
-    return fail(B2R_ERR_INVALID_ARGUMENT, "a required IQN pointer is NULL");
-  if (!b2r::g_iqn_ticket) {
-    B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b2r::g_iqn_ticket), 4));
-    B2R_CUDA(cudaMemset(b2r::g_iqn_ticket, 0, 4));
-  }
-  b2r::IqnArgs a;
-  a.u = *args;
-  a.ticket = b2r::g_iqn_ticket;
-  B2R_CUDA(b2r::launch(b2r::iqn_loss_kernel, dim3(args->batch), dim3(b2r::kIqnWarps * 32), 0,
-                       as_stream(stream), a));
-  B2R_LAUNCHED();
-  return B2R_OK;
+  return b2r::iqn_launch(args, nullptr, args ? args->batch : 0, as_stream(stream));
+}
+
+extern "C" int b2r_iqn_loss_sharded(const b2r_iqn_args *args, const int32_t *count,
+                                    int32_t global_batch, b2r_stream stream) {
+  if (!args) return fail(B2R_ERR_INVALID_ARGUMENT, "args is NULL");
+  if (!count) return fail(B2R_ERR_INVALID_ARGUMENT, "a shard's loss needs count");
+  if (global_batch < 1) return fail(B2R_ERR_INVALID_ARGUMENT, "global_batch must be >= 1");
+  return b2r::iqn_launch(args, count, global_batch, as_stream(stream));
 }

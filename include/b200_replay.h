@@ -651,6 +651,21 @@ typedef struct {
 } b2r_iqn_args;
 int b2r_iqn_loss(const b2r_iqn_args *args, b2r_stream stream);
 
+/* The loss of one shard of a global batch of `global_batch` strata, as
+ * b2r_sample_transition_batch_sharded_device samples it (IQN's replay is the prioritized
+ * buffer with unit priorities, implicit_quantile.gin:23-24).  The same arithmetic per
+ * row as b2r_iqn_loss; args->batch is the rank's max_rows (the row stride of every
+ * (samples * batch, A) matrix) and *count (DEVICE, required) its row count.  Rows
+ * b < count get the loss, next_action and gradient rows b2r_iqn_loss gives that
+ * transition on the whole global batch (the gradient scale is
+ * -1 / (kappa * N' * global_batch)); rows b >= count get loss 0 and zero gradient rows,
+ * and their next_action is not written.  mean_loss = (sum over this rank's rows of
+ * loss) / global_batch.  IQN has no importance weights, so nothing is exchanged:
+ * summed over the ranks, the means and the gradients are the global batch's (:315).
+ * DEVICE pointers; asynchronous; can be captured in a CUDA graph. */
+int b2r_iqn_loss_sharded(const b2r_iqn_args *args, const int32_t *count,
+                         int32_t global_batch, b2r_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,10 +1,14 @@
-"""ms per update and transitions/s of ShardedRainbowLearner at 1/2/4/8 GPUs: a global
-batch of 32 rows per GPU, a replay shard of 1M transitions per GPU, eager and
-replayed as a CUDA graph.  Also reports the rows the networks computed (max_rows per
-rank, the padding that keeps the shapes static) next to the useful rows (the global
-batch), and the card's name and power limit read in the same run.
+"""ms per update and transitions/s of ShardedRainbowLearner (`--agent rainbow`) or
+ShardedIQNLearner (`--agent iqn`) at 1/2/4/8 GPUs: a global batch of 32 rows per GPU, a
+replay shard of 1M transitions per GPU, eager and replayed as a CUDA graph.  Also reports
+the rows the networks computed (max_rows per rank, the padding that keeps the shapes
+static) next to the useful rows (the global batch), and the card's name and power limit
+read in the same run.  With `--agent iqn` the shards have unit priorities (IQN's replay),
+the tau counts are IQNLearner's defaults (N = N' = K = 32), and the run also times plain
+IQNLearner.train_step() at batch 32 on one GPU, the N = 1 baseline.
 
-  python profiles/micro/sharded_learner.py [--gpus 1,2,4,8] [--steps 200] [--out F]
+  python profiles/micro/sharded_learner.py [--agent rainbow|iqn] [--gpus 1,2,4,8]
+      [--steps 200] [--out F]
 
 Each configuration runs in fresh processes (one per GPU, NCCL); rank 0 times `--steps`
 updates between CUDA events after `--warmup` updates.  The frames of the shards are
@@ -29,7 +33,7 @@ CAPACITY = 1000000
 ACTIONS = 18
 
 
-def _shard(cap, seed, batch):
+def _shard(cap, seed, batch, unit_priorities=False):
   from dopamine_b200.replay_memory import prioritized_replay_buffer as prb
   rng = np.random.RandomState(seed)
   mem = prb.OutOfGraphPrioritizedReplayBuffer(
@@ -40,15 +44,65 @@ def _shard(cap, seed, batch):
   mem._store['terminal'] = (rng.rand(cap) < 0.01).astype(np.uint8)
   mem.add_count = cap + 1000
   mem.invalid_range = np.array([(1000 - 3 + i) % cap for i in range(7)])
-  mem.set_priority(np.arange(cap, dtype=np.int32),
-                   np.sqrt(np.abs(rng.randn(cap)) + 1e-10).astype(np.float32))
+  priorities = (np.ones(cap, dtype=np.float32) if unit_priorities else
+                np.sqrt(np.abs(rng.randn(cap)) + 1e-10).astype(np.float32))
+  mem.set_priority(np.arange(cap, dtype=np.int32), priorities)
   return mem
 
 
-def _worker(rank, world, port, graph, steps, warmup, out_path):
+def _make_learner(agent_name, global_batch, rank, graph):
+  if agent_name == 'iqn':
+    from dopamine_b200.agents.implicit_quantile import learner
+    return learner.ShardedIQNLearner(
+        ACTIONS, batch_size=global_batch,
+        memory=_shard(CAPACITY, 10 + rank, global_batch, unit_priorities=True),
+        replay_capacity=CAPACITY, seed=1, cuda_graph=graph)
+  from dopamine_b200.agents.rainbow import agent
+  return agent.ShardedRainbowLearner(
+      ACTIONS, batch_size=global_batch, memory=_shard(CAPACITY, 10 + rank, global_batch),
+      replay_capacity=CAPACITY, seed=1, cuda_graph=graph)
+
+
+def _time_updates(torch, learner, steps):
+  start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+  start.record()
+  for _ in range(steps):
+    learner.train_step()
+  end.record()
+  torch.cuda.synchronize()
+  return start.elapsed_time(end) / steps
+
+
+def _iqn_settings(learner):
+  return dict(num_tau_samples=learner.num_tau_samples,
+              num_tau_prime_samples=learner.num_tau_prime_samples,
+              num_quantile_samples=learner.num_quantile_samples)
+
+
+def _baseline_worker(rank, steps, warmup, out_path):
+  """Plain IQNLearner.train_step() at batch 32 on one GPU: the N = 1 baseline."""
+  import torch
+  from dopamine_b200.agents.implicit_quantile import learner as iqn_learner
+  torch.cuda.set_device(rank)
+  learner = iqn_learner.IQNLearner(
+      ACTIONS, batch_size=PER_GPU_BATCH, replay_capacity=CAPACITY, seed=1,
+      memory=_shard(CAPACITY, 10, PER_GPU_BATCH, unit_priorities=True))
+  for _ in range(warmup):
+    learner.train_step()
+  torch.cuda.synchronize()
+  ms = _time_updates(torch, learner, steps)
+  result = dict(agent='iqn', learner='IQNLearner', gpus=1, mode='eager', steps=steps,
+                ms_per_update=round(ms, 4),
+                transitions_per_s=round(PER_GPU_BATCH / ms * 1e3, 1),
+                useful_rows=PER_GPU_BATCH, network_rows=PER_GPU_BATCH,
+                capacity_per_gpu=CAPACITY, **_iqn_settings(learner))
+  with open(out_path, 'w') as f:
+    json.dump(result, f)
+
+
+def _worker(rank, world, port, agent_name, graph, steps, warmup, out_path):
   import torch
   import torch.distributed as dist
-  from dopamine_b200.agents.rainbow import agent
   torch.cuda.set_device(rank)
   os.environ['MASTER_ADDR'] = '127.0.0.1'
   os.environ['MASTER_PORT'] = str(port)
@@ -56,28 +110,23 @@ def _worker(rank, world, port, graph, steps, warmup, out_path):
                           device_id=torch.device('cuda', rank))
   try:
     global_batch = PER_GPU_BATCH * world
-    learner = agent.ShardedRainbowLearner(
-        ACTIONS, batch_size=global_batch, memory=_shard(CAPACITY, 10 + rank, global_batch),
-        replay_capacity=CAPACITY, seed=1, cuda_graph=graph)
+    learner = _make_learner(agent_name, global_batch, rank, graph)
     for _ in range(warmup):
       learner.train_step()
     torch.cuda.synchronize()
     dist.barrier()
-    start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    start.record()
-    for _ in range(steps):
-      learner.train_step()
-    end.record()
-    torch.cuda.synchronize()
+    ms = _time_updates(torch, learner, steps)
     learner.check()
-    ms = start.elapsed_time(end) / steps
     if rank == 0:
-      result = dict(gpus=world, mode='graph' if graph else 'eager', steps=steps,
+      result = dict(agent=agent_name, learner=type(learner).__name__, gpus=world,
+                    mode='graph' if graph else 'eager', steps=steps,
                     ms_per_update=round(ms, 4),
                     transitions_per_s=round(global_batch / ms * 1e3, 1),
                     useful_rows=global_batch, max_rows_per_rank=learner.max_rows,
-                    network_rows=learner.max_rows * world,
+                    network_rows=learner.max_rows * world, capacity_per_gpu=CAPACITY,
                     loss=float(learner.loss.item()))
+      if agent_name == 'iqn':
+        result.update(_iqn_settings(learner))
       with open(out_path, 'w') as f:
         json.dump(result, f)
     dist.barrier()
@@ -95,6 +144,7 @@ def main():
   import torch
   import torch.multiprocessing as mp
   p = argparse.ArgumentParser()
+  p.add_argument('--agent', choices=('rainbow', 'iqn'), default='rainbow')
   p.add_argument('--gpus', default='1,2,4,8')
   p.add_argument('--steps', type=int, default=200)
   p.add_argument('--warmup', type=int, default=20)
@@ -108,35 +158,40 @@ def main():
   lines = [json.dumps(dict(cards=card))]
   print(lines[0], flush=True)
   tmp = os.environ.get('TMPDIR', '/tmp')
+  ctx = mp.get_context('spawn')
+
+  def run(target, world, args, desc):
+    procs = [ctx.Process(target=target, args=(r,) + args) for r in range(world)]
+    for q in procs:
+      q.start()
+    for q in procs:
+      q.join(timeout=1200)
+    for q in procs:
+      if q.is_alive():
+        q.terminate()
+        q.join(timeout=60)
+    codes = [q.exitcode for q in procs]
+    if any(c != 0 for c in codes):
+      lines.append(json.dumps(dict(desc, failed=codes)))
+    else:
+      with open(args[-1]) as f:
+        lines.append(f.read())
+    print(lines[-1], flush=True)
+
+  if a.agent == 'iqn':
+    run(_baseline_worker, 1, (a.steps, a.warmup, os.path.join(tmp, 'iqn_baseline.json')),
+        dict(agent='iqn', learner='IQNLearner', gpus=1, mode='eager'))
   for n in [int(x) for x in a.gpus.split(',')]:
     if n > torch.cuda.device_count():
-      lines.append(json.dumps(dict(gpus=n, skipped='only {} devices'.format(
-          torch.cuda.device_count()))))
+      lines.append(json.dumps(dict(agent=a.agent, gpus=n, skipped='only {} devices'
+                                   .format(torch.cuda.device_count()))))
       print(lines[-1], flush=True)
       continue
     for graph in (False, True):
-      out_path = os.path.join(tmp, 'sharded_learner_{}_{}.json'.format(n, int(graph)))
-      ctx = mp.get_context('spawn')
-      port = _free_port()
-      procs = [ctx.Process(target=_worker,
-                           args=(r, n, port, graph, a.steps, a.warmup, out_path))
-               for r in range(n)]
-      for q in procs:
-        q.start()
-      for q in procs:
-        q.join(timeout=1200)
-      for q in procs:
-        if q.is_alive():
-          q.terminate()
-          q.join(timeout=60)
-      codes = [q.exitcode for q in procs]
-      if any(c != 0 for c in codes):
-        lines.append(json.dumps(dict(gpus=n, mode='graph' if graph else 'eager',
-                                     failed=codes)))
-      else:
-        with open(out_path) as f:
-          lines.append(f.read())
-      print(lines[-1], flush=True)
+      out_path = os.path.join(tmp, 'sharded_learner_{}_{}_{}.json'.format(
+          a.agent, n, int(graph)))
+      run(_worker, n, (n, _free_port(), a.agent, graph, a.steps, a.warmup, out_path),
+          dict(agent=a.agent, gpus=n, mode='graph' if graph else 'eager'))
   if a.out:
     os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
     with open(a.out, 'w') as f:
