@@ -229,6 +229,12 @@ SIGNATURES = {
         c_void_p, c_void_p, c_int32, c_uint64, c_uint64, P(Batch), c_void_p, c_void_p,
         c_int32, c_void_p, c_void_p]),
     'b2r_dqn_loss': (c_int, [P(DqnArgs), c_void_p]),
+    'b2r_dqn_loss_sharded': (c_int, [P(DqnArgs), c_int32, c_void_p]),
+    'b2r_sample_transition_batch_uniform_sharded_device': (c_int, [
+        c_void_p, c_void_p, c_int32, c_uint64, c_uint64, P(Batch), c_void_p, c_void_p,
+        c_int32, c_void_p]),
+    'b2r_exchange_publish_uniform_device': (c_int, [c_void_p, c_void_p, c_int32, c_uint64,
+                                                     c_uint64, c_int32, c_void_p]),
     'b2r_train_step_device': (c_int, [c_void_p, c_int32, c_uint64, c_uint64,
                                       P(Batch), P(C51Args), c_void_p]),
     'b2r_stack_to_planes_device': (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_int32,

@@ -35,7 +35,7 @@ def cumulative_gamma(gamma, update_horizon):
 
 
 def dqn_loss(online_q, target_q, actions, rewards, terminals, cumulative_gamma,  # pylint: disable=redefined-outer-name
-             want_target=False, want_grad=False, want_mean=True, out=None):
+             want_target=False, want_grad=False, want_mean=True, out=None, sharded=None):
   """Bellman target + Huber loss for one batch, on the device.
 
   Args:
@@ -43,6 +43,12 @@ def dqn_loss(online_q, target_q, actions, rewards, terminals, cumulative_gamma, 
     target_q: (B, A) f32 CUDA, target network on `next_state`.
     actions: (B,) int32; rewards: (B,) f32 n-step returns; terminals: (B,) uint8.
     cumulative_gamma: gamma ** update_horizon.
+    sharded: (global_batch, count) — the B rows are one rank's share of a global batch
+      of `global_batch` transitions, as `ShardedUniformReplay.sample_transition_batch_
+      sharded` returns it (b2r_dqn_loss_sharded): the first `count` rows ((1,) int32
+      CUDA tensor) are valid, the mean and its gradient are this rank's part of the
+      global batch's (divisor global_batch), rows past the count get loss 0 and zero
+      gradients.
   Returns:
     dict with 'loss' (B,), optionally 'mean_loss' (scalar), 'target' (B,),
     'grad_q' (B, A) = d mean(loss) / d online_q.
@@ -54,6 +60,13 @@ def dqn_loss(online_q, target_q, actions, rewards, terminals, cumulative_gamma, 
   assert target_q.dtype == torch.float32 and target_q.is_cuda
   assert actions.dtype == torch.int32 and rewards.dtype == torch.float32
   assert terminals.dtype == torch.uint8
+  if sharded is not None:
+    global_batch, count = sharded
+    if (not isinstance(count, torch.Tensor) or count.dtype != torch.int32 or
+        not count.is_cuda or tuple(count.shape) != (1,)):
+      raise ValueError('count must be a (1,) int32 CUDA tensor')
+    if int(global_batch) < 1:
+      raise ValueError('global_batch must be >= 1, got {}'.format(global_batch))
   dev = online_q.device
   if out is None:
     out = {'loss': torch.empty(b, dtype=torch.float32, device=dev)}
@@ -75,8 +88,13 @@ def dqn_loss(online_q, target_q, actions, rewards, terminals, cumulative_gamma, 
   args.target = out['target'].data_ptr() if 'target' in out else None
   args.mean_loss = out['mean_loss'].data_ptr() if 'mean_loss' in out else None
   args.grad_q = out['grad_q'].data_ptr() if 'grad_q' in out else None
-  _native.check(_native.lib().b2r_dqn_loss(ctypes.byref(args),
-                                           _native.current_stream()))
+  if sharded is None:
+    _native.check(_native.lib().b2r_dqn_loss(ctypes.byref(args),
+                                             _native.current_stream()))
+    return out
+  args.batch_count = count.data_ptr()
+  _native.check(_native.lib().b2r_dqn_loss_sharded(ctypes.byref(args), int(global_batch),
+                                                   _native.current_stream()))
   return out
 
 
@@ -86,16 +104,17 @@ class DQNLoss(object):
   _fn = None
 
   @classmethod
-  def apply(cls, online_q, target_q, actions, rewards, terminals, gamma_n):
+  def _function(cls):
     if cls._fn is None:
       torch = _torch()
 
       class _Fn(torch.autograd.Function):
 
         @staticmethod
-        def forward(ctx, online_q, target_q, actions, rewards, terminals, gamma_n):  # pylint: disable=redefined-outer-name
+        def forward(ctx, online_q, target_q, actions, rewards, terminals, gamma_n,  # pylint: disable=redefined-outer-name
+                    sharded):
           out = dqn_loss(online_q.detach(), target_q.detach(), actions, rewards,
-                         terminals, gamma_n, want_grad=True)
+                         terminals, gamma_n, want_grad=True, sharded=sharded)
           ctx.save_for_backward(out['grad_q'])
           ctx.mark_non_differentiable(out['loss'])
           return out['mean_loss'], out['loss']
@@ -103,10 +122,28 @@ class DQNLoss(object):
         @staticmethod
         def backward(ctx, grad_mean, *unused):
           (grad_q,) = ctx.saved_tensors
-          return grad_q * grad_mean, None, None, None, None, None
+          return (grad_q * grad_mean,) + (None,) * 6
 
       cls._fn = _Fn
-    return cls._fn.apply(online_q, target_q, actions, rewards, terminals, gamma_n)
+    return cls._fn
+
+  @classmethod
+  def apply(cls, online_q, target_q, actions, rewards, terminals, gamma_n):
+    return cls._function().apply(online_q, target_q, actions, rewards, terminals, gamma_n,
+                                 None)
+
+
+class ShardedDQNLoss(DQNLoss):
+  """`DQNLoss` over one rank's share of a sharded global batch (b2r_dqn_loss_sharded):
+  `mean, loss = ShardedDQNLoss.apply(..., gamma_n, sharded)` with `sharded` =
+  (global_batch, count) as in `dqn_loss`.  `mean` is this rank's partial mean (its rows'
+  losses over the global batch size) and backward gives its gradient; summed over the
+  ranks both are the global batch's."""
+
+  @classmethod
+  def apply(cls, online_q, target_q, actions, rewards, terminals, gamma_n, sharded):  # pylint: disable=arguments-differ
+    return cls._function().apply(online_q, target_q, actions, rewards, terminals, gamma_n,
+                                 tuple(sharded))
 
 
 # ------------------------------------------------------------- actor side ----

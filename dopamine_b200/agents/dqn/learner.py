@@ -6,12 +6,15 @@ through PyTorch behind the hand-written input kernel), the uniform replay buffer
 Bellman target + Huber loss as ONE kernel (`dqn_loss`, csrc/dqn.cu), TensorFlow's centred
 RMSProp with the reference's numbers, and the target sync.  Same structure as
 `agents/rainbow/agent.RainbowLearner`; the acting side is `dqn_agent.ActingLoop`.
+`ShardedDQNLearner` trains on one global uniform batch drawn over the GPUs' replay shards.
 """
 import math
 
+from dopamine_b200.agents import sharded_learner
 from dopamine_b200.agents.dqn import dqn_agent
 from dopamine_b200.agents.rainbow import agent as conv
 from dopamine_b200.replay_memory import circular_replay_buffer
+from dopamine_b200.replay_memory import sharded_replay
 
 
 def _torch():
@@ -203,3 +206,73 @@ class DQNLearner(object):
       self.sync_target()
     self.training_steps += 1
     return loss
+
+
+class ShardedDQNLearner(sharded_learner.ShardedLearner, DQNLearner):
+  """`DQNLearner` on ONE global batch sharded over the ranks of torch.distributed.
+
+  Every rank owns one uniform replay shard of `replay_capacity` transitions (the
+  reference's `OutOfGraphReplayBuffer`, dqn_agent.py:265-281) and a peer-memory exchange.
+  `batch_size` is the GLOBAL batch: the reference's uniform draws with rejection
+  (circular_replay_buffer.py:436-477) over a virtual buffer whose index range is the
+  concatenation of the shards' ranges (`ShardedUniformReplay`), so the update is the
+  reference's update (dqn_agent.py:283-322) on one batch uniform over the union of the
+  shards' valid transitions.  One update:
+    1. `sample()`: sharded uniform sampler + frame copies into `max_rows` rows (default
+       `share_bound`);
+    2. `loss_backward()`: the target net on `next_state`, the online net on `state`, both
+       on `max_rows` rows, then the sharded Bellman target + Huber loss (mean and
+       gradient over the global batch, zero gradients for padded rows) and backward into
+       one flat buffer;
+    3. `reduce()`: ONE all-reduce (sum) of that buffer — every gradient and, appended,
+       the partial loss, so the reported loss is the global mean;
+    4. `apply()`: TF-form centred RMSProp.  There are no priorities to write back.
+  `cuda_graph=True` captures the whole update, all-reduce included; `step_cadence()` is
+  `DQNLearner`'s.  Errors latched on the device are raised by `check()`, which
+  `sync_target()` calls.  Pass `exchange` (`PeerExchange.emulated`) to run the phases of
+  several ranks on one device without torch.distributed (tests): each rank's sampler then
+  needs the two publish-ahead phases of every rank first (`self.sharded.publish`), and
+  `reduce()` is the caller's.
+  """
+
+  def __init__(self, num_actions, batch_size=32, max_rows=None, exchange=None,
+               group=None, exchange_timeout_s=2.0, ddp=False, cuda_graph=False,
+               **kwargs):
+    exchange = self._connect(exchange, group, exchange_timeout_s, ddp)
+    DQNLearner.__init__(self, num_actions, batch_size=batch_size, **kwargs)
+    self._cuda_graph = bool(cuda_graph)
+    self._graph = None
+    self._static_loss = None
+    self._shard(exchange, max_rows, kwargs.get('seed', 0),
+                sharded_replay.ShardedUniformReplay)
+
+  # -- phases (sample, reduce: ShardedLearner's) ----------------------------------------
+  def loss_backward(self):
+    """Networks, sharded loss and backward: the flat buffer holds this rank's partial
+    gradients and partial mean.  Returns the per-row losses."""
+    torch = _torch()
+    _, count, batch = self._sample
+    state, action, reward, next_state, _, _, terminal = batch[:7]
+    with torch.no_grad():
+      target_q = self.target(next_state)
+    online_q = self.online(state)
+    mean, rows = dqn_agent.ShardedDQNLoss.apply(online_q, target_q, action, reward,
+                                                terminal, self.cumulative_gamma,
+                                                (self.batch_size, count))
+    self._flat.zero_()
+    mean.backward()  # (accumulates into the views of the flat buffer)
+    self.loss.copy_(mean.detach().view(1))
+    return rows
+
+  def apply(self):
+    """RMSProp on the reduced gradients."""
+    self.optimizer.step()
+
+  def _update(self):
+    self.sample()
+    self.loss_backward()
+    self.reduce()
+    self.apply()
+    if not self._cuda_graph or self._graph is None:
+      self.updates += 1
+    return self.loss

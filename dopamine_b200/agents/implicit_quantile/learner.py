@@ -18,6 +18,7 @@ from dopamine_b200.agents.dqn import learner as dqn_learner
 from dopamine_b200.agents.implicit_quantile import implicit_quantile_agent as iqn
 from dopamine_b200.agents.rainbow import agent as conv
 from dopamine_b200.replay_memory import prioritized_replay_buffer
+from dopamine_b200.replay_memory import sharded_replay
 
 
 def _torch():
@@ -198,7 +199,7 @@ class ShardedIQNLearner(sharded_learner.ShardedLearner, IQNLearner):
       self.optimizer = conv.make_tf_adam(self.online.parameters(), lr=adam['lr'],
                                          epsilon=adam['epsilon'], capturable=True)
     seed = kwargs.get('seed', 0)
-    self._shard(exchange, max_rows, seed)
+    self._shard(exchange, max_rows, seed, sharded_replay.ShardedPrioritizedReplay)
     self._generator = torch.Generator(device='cuda')
     self._generator.manual_seed(
         int(np.random.SeedSequence([int(seed), self.rank]).generate_state(1)[0]))

@@ -26,6 +26,7 @@ from dopamine_b200.agents import sharded_learner
 from dopamine_b200.agents.dqn import dqn_agent
 from dopamine_b200.agents.rainbow import rainbow_agent
 from dopamine_b200.replay_memory import prioritized_replay_buffer
+from dopamine_b200.replay_memory import sharded_replay
 
 
 def _torch():
@@ -346,7 +347,8 @@ class ShardedRainbowLearner(sharded_learner.ShardedLearner, RainbowLearner):
                group=None, exchange_timeout_s=2.0, ddp=False, **kwargs):
     exchange = self._connect(exchange, group, exchange_timeout_s, ddp)
     RainbowLearner.__init__(self, num_actions, batch_size=batch_size, **kwargs)
-    self._shard(exchange, max_rows, kwargs.get('seed', 0))
+    self._shard(exchange, max_rows, kwargs.get('seed', 0),
+                sharded_replay.ShardedPrioritizedReplay)
 
   # -- phases (sample, reduce: ShardedLearner's) ----------------------------------------
   def loss_backward(self):

@@ -1,6 +1,7 @@
 """What the learners share beyond their loss: the update replayed as one CUDA graph, and
 the rank plumbing of a data-parallel learner on ONE global batch sharded over the ranks
-(`agent.ShardedRainbowLearner`, `learner.ShardedIQNLearner`)."""
+(`agent.ShardedRainbowLearner`, `learner.ShardedIQNLearner`,
+`learner.ShardedDQNLearner`)."""
 
 
 def _torch():
@@ -22,13 +23,17 @@ class GraphedUpdate(object):
       return self._update()
     if self._graph is None:
       self._capture()
-    self.memory._flush()  # pylint: disable=protected-access
+    self._flush_replay()
     self._graph.replay()
     self.updates += 1
     return self._static_loss
 
   def _graph_generators(self):
     return ()
+
+  def _flush_replay(self):
+    """Applies the replay's staged adds (the graph's sampler reads the ring)."""
+    self.memory._flush()  # pylint: disable=protected-access
 
   def _capture(self):
     torch = _torch()
@@ -39,7 +44,7 @@ class GraphedUpdate(object):
         self._update()
     torch.cuda.current_stream().wait_stream(side)
     torch.cuda.synchronize()
-    self.memory._flush()  # pylint: disable=protected-access
+    self._flush_replay()
     self._graph = torch.cuda.CUDAGraph()
     for generator in self._graph_generators():  # each replay draws fresh numbers
       self._graph.register_generator_state(generator)
@@ -48,9 +53,9 @@ class GraphedUpdate(object):
 
 
 class ShardedLearner(GraphedUpdate):
-  """The rank plumbing of a learner whose `batch_size` is the GLOBAL batch, its strata
-  apportioned over the ranks' replay shards (`ShardedPrioritizedReplay`).  Every rank
-  owns one shard and a peer-memory exchange; parameters start as rank 0's; every
+  """The rank plumbing of a learner whose `batch_size` is the GLOBAL batch, drawn over
+  the ranks' replay shards (`ShardedPrioritizedReplay`, `ShardedUniformReplay`).  Every
+  rank owns one shard and a peer-memory exchange; parameters start as rank 0's; every
   gradient views one flat buffer whose last entry is the partial loss, so `reduce()` is
   ONE all-reduce.  The learner calls `_connect()` before, and `_shard()` after, the
   single-GPU learner's constructor, and provides `loss_backward()`, `apply()` and
@@ -73,15 +78,16 @@ class ShardedLearner(GraphedUpdate):
     self._group = group
     return exchange
 
-  def _shard(self, exchange, max_rows, seed):
-    """The sharded replay over `self.memory`, rank 0's parameters (and target) on every
-    rank, and the flat gradient buffer."""
+  def _shard(self, exchange, max_rows, seed, replay_class):
+    """The sharded replay over `self.memory` (`replay_class`: `ShardedPrioritizedReplay`
+    or `ShardedUniformReplay`), rank 0's parameters (and target) on every rank, and the
+    flat gradient buffer."""
     torch = _torch()
     from dopamine_b200.replay_memory import sharded_replay  # pylint: disable=g-import-not-at-top
     self.exchange = exchange
     self.rank, self.world = exchange.rank, exchange.world
-    self.sharded = sharded_replay.ShardedPrioritizedReplay(
-        self.memory, rank=self.rank, world_size=self.world, seed=seed, exchange=exchange)
+    self.sharded = replay_class(self.memory, rank=self.rank, world_size=self.world,
+                                seed=seed, exchange=exchange)
     self.max_rows = (sharded_replay.share_bound(self.batch_size, self.world)
                      if max_rows is None else min(int(max_rows), int(self.batch_size)))
     params = list(self.online.parameters())
@@ -100,9 +106,13 @@ class ShardedLearner(GraphedUpdate):
     self.loss = self._flat[total:]
     self._sample = None
 
+  def _flush_replay(self):
+    self.sharded.flush()
+
   # -- phases ------------------------------------------------------------------------
   def sample(self):
-    """(slots, count, batch tuple, min_probability) of this rank's share."""
+    """This rank's share: (slots, count, batch tuple) and, from a prioritized shard,
+    min_probability."""
     self._sample = self.sharded.sample_transition_batch_sharded(self.batch_size,
                                                                 self.max_rows)
     return self._sample

@@ -11,7 +11,8 @@
 using b2r::fail;
 
 namespace {
-// totals [2][kMaxShards][2 words], then local minima [2][kMaxShards] (tree.cuh)
+// totals [2][kMaxShards][2 words], then local minima [2][kMaxShards], then the uniform
+// sampler's rejection lists [2][kMaxShards][1 + kRejListWords] (tree.cuh)
 constexpr size_t kMailboxBytes = b2r::kMailboxWords * sizeof(uint64_t);
 }
 
@@ -124,6 +125,15 @@ int b2r_exchange_publish_device(b2r_exchange *x, b2r_buffer *buf, b2r_stream str
   if (!x->connected) return fail(B2R_ERR_INVALID_ARGUMENT, "the exchange is not connected");
   B2R_TRY(b2r::flush_queue(buf, b2r::as_stream(stream)));
   return b2r::launch_exchange_publish(x, buf, b2r::as_stream(stream));
+}
+
+int b2r_exchange_publish_uniform_device(b2r_exchange *x, b2r_buffer *buf,
+                                        int32_t global_batch, uint64_t seed,
+                                        uint64_t offset, int32_t phase, b2r_stream stream) {
+  B2R_TRY(b2r::check_uniform_sharded(buf, x, global_batch));
+  if (phase != 0 && phase != 1) return fail(B2R_ERR_INVALID_ARGUMENT, "phase must be 0 or 1");
+  return b2r::launch_uniform_sharded(buf, x, global_batch, seed, offset, phase, nullptr,
+                                     nullptr, nullptr, 0, b2r::as_stream(stream));
 }
 
 }  // extern "C"

@@ -684,6 +684,11 @@ int b2r_check(b2r_buffer *b, b2r_stream stream) {
       return fail(B2R_ERR_UNSUPPORTED,
                   "a sharded step's share of the global batch (%lld strata) outgrew the "
                   "rows its outputs hold (max_rows)", (long long)st[1]);
+    if (st[0] == B2R_ERR_TOO_FEW_TRANSITIONS)
+      return fail(B2R_ERR_TOO_FEW_TRANSITIONS,
+                  "Cannot sample a batch: no shard holds more than stack size (%d) + "
+                  "update_horizon (%d) transitions.",
+                  b->cfg.stack_size, b->cfg.update_horizon);
     if (st[0] == B2R_ERR_INDEX_RANGE)
       return fail(B2R_ERR_INDEX_RANGE,
                   "row %lld of the batch holds an action outside [0, num_actions)",

@@ -401,6 +401,16 @@ int launch_sample_sharded(b2r_buffer *buf, int32_t global_batch, int32_t num_sha
                           const b2r_batch *scalars = nullptr,
                           float *min_prob_out = nullptr, int32_t max_rows = 0,
                           const PreSync *pre = nullptr, bool publish_min = false);
+// Sharded uniform sampling (sample.cu: uniform_sharded_kernel).  check_uniform_sharded:
+// the host-side refusals shared by the sampling call and the publish-ahead.
+// mode 0 / 1: publish-ahead of the span / the rejection list of the exchange's next step
+// (ranks emulated by sequential launches); 2: the sampler, which closes the step.
+int check_uniform_sharded(const b2r_buffer *buf, const b2r_exchange *x,
+                          int32_t global_batch);
+int launch_uniform_sharded(b2r_buffer *buf, const b2r_exchange *x, int32_t global_batch,
+                           uint64_t seed, uint64_t offset, int mode, int32_t *out_idx,
+                           int32_t *out_slots, int32_t *out_count, int32_t out_cap,
+                           cudaStream_t stream);
 void fill_valid_ctx(const b2r_buffer *buf, ValidCtx *ctx);
 int ensure_ctx(b2r_buffer *buf, cudaStream_t stream);
 // tree.cu: largest batch the one-CTA tree kernel takes, and the fused flush launch

@@ -1624,6 +1624,332 @@ int launch_exchange_publish(const b2r_exchange *x, const b2r_buffer *b,
   return B2R_OK;
 }
 
+// ---- Sharded UNIFORM sampling: one global batch of circular_replay_buffer.py:462-470 over
+// a virtual buffer whose index range is the concatenation of the shards' ranges.
+//
+// Rank g's span is n_g = max(0, max_id_g - min_id_g) (CRB:449-460, from the device
+// validity context, so a replayed graph sees new adds); N = sum of the spans.  Draw j is
+// u_j = philox_uniform53(seed, offset + step, j) with `step` the exchange's step number,
+// o_j = min((int64)(u_j N), N - 1), owned by the rank the scan `o < n_g ? g : o -= n_g`
+// stops at, candidate (min_id_owner + o) mod capacity.  The draws are processed in order
+// while accepted < batch and rejected < max_sample_attempts; the k-th accepted draw is
+// global row k.  Only the owner of a draw knows whether it is valid, so the ranks agree on
+// the accepted draws in two rounds over the mailbox:
+//   1. spans: the totals words (exchange_publish / exchange_collect, f64 payload);
+//   2. rejections: every rank evaluates the draws it owns in [0, batch + max_attempts) —
+//      every draw the loop could process — and publishes the ascending ordinals of its
+//      invalid ones, the first max_attempts of them (kRejWordsOffset region).
+// With rejects_before(j) summed over the G lists (binary searches), an owned valid draw j
+// is kept iff j - rejects_before(j) < batch and rejects_before(j) < max_attempts, as row
+// j - rejects_before(j).  Both quantities only grow with j, so the kept draws are a
+// prefix of the rank's valid draws.  A rank stops evaluating once it has `batch` valid
+// draws (a later draw's row is >= batch) or max_attempts invalid ones (a later draw has
+// rejects_before >= max_attempts): what it leaves out of its list changes no decision.
+namespace {
+
+constexpr int kUniformShardThreads = 1024;
+enum { kUniformPublishSpan = 0, kUniformPublishRejections = 1, kUniformSample = 2 };
+
+struct UniformShardArgs {
+  const ValidCtx *valid_dev;
+  ExchangeArgs xchg;
+  int world, rank;
+  int batch;  // global batch
+  int max_attempts;
+  uint64_t seed, offset;
+  int mode;
+  int out_cap;
+  int32_t *out_idx, *out_slots, *count_out;
+  int32_t *own_j, *own_idx;  // scratch [batch]: this rank's valid draws, ascending
+  int32_t *lists;            // scratch [world * kRejListWords]: the collected lists
+  int64_t *latched;
+};
+
+__device__ __forceinline__ uint64_t rej_word(int32_t value, uint64_t seq) {
+  return ((uint64_t)(uint32_t)value << 32) | (uint32_t)seq;
+}
+
+// Polls one mailbox word until it carries step `seq` (value returned) or the timeout
+// passes (latches B2R_ERR_EXCHANGE for rank g, returns `missing`).
+__device__ __forceinline__ int32_t poll_rej_word(const ExchangeArgs &x, const uint64_t *src,
+                                                 uint64_t seq, int g, int32_t missing,
+                                                 int64_t *latched) {
+  if (x.timeout_ns <= 0) return missing;
+  const bool broken = latched != nullptr && latched[0] == B2R_ERR_EXCHANGE;
+  const uint64_t t0 = global_timer_ns();
+  while (!broken) {
+    const uint64_t w = ld_sys_u64(src);
+    if ((uint32_t)w == (uint32_t)seq) return (int32_t)(w >> 32);
+    if (global_timer_ns() - t0 > (uint64_t)x.timeout_ns) break;
+  }
+  if (latched != nullptr) {
+    latched[0] = B2R_ERR_EXCHANGE;
+    latched[1] = g;
+  }
+  return missing;
+}
+
+__global__ void __launch_bounds__(kUniformShardThreads)
+    uniform_sharded_kernel(const __grid_constant__ UniformShardArgs a) {
+  __shared__ ValidCtx s_valid;
+  __shared__ double s_spans[kMaxShards];
+  __shared__ int64_t s_span[kMaxShards];
+  __shared__ int warp_counts[32];
+  __shared__ int32_t s_rej[kRejListWords];
+  __shared__ int s_start[kMaxShards + 1];
+  __shared__ int s_published, s_stale, s_kept;
+  pdl_release();
+  pdl_acquire();  // (everything below publishes: after griddepcontrol.wait)
+  for (int w = threadIdx.x; w < (int)(sizeof(ValidCtx) / 8); w += blockDim.x)
+    reinterpret_cast<uint64_t *>(&s_valid)[w] =
+        reinterpret_cast<const uint64_t *>(a.valid_dev)[w];
+  const uint64_t xseq = *a.xchg.seq + 1;
+  if (threadIdx.x == 0) {
+    s_published = 0;
+    s_stale = 0;
+    s_kept = 0;
+  }
+  __syncthreads();
+  const ValidCtx &c = s_valid;
+  // uniform_bounds (CRB:449-460) on the device
+  int64_t min_id, max_id;
+  if (c.add_count >= c.capacity) {
+    min_id = c.cursor - c.capacity + c.stack - 1;
+    max_id = c.cursor - c.horizon;
+  } else {
+    min_id = c.stack - 1;
+    max_id = c.cursor - c.horizon;
+  }
+  const int64_t span = max_id > min_id ? max_id - min_id : 0;
+
+  // ---- round 1: spans
+  if (threadIdx.x < 32) {
+    if (a.mode == kUniformPublishSpan)
+      exchange_publish(a.xchg, a.world, a.rank, (double)span, xseq);
+    else
+      exchange_publish_if_needed(a.xchg, a.world, a.rank, (double)span, xseq, a.latched);
+  }
+  if (a.mode == kUniformPublishSpan) return;
+  exchange_collect(a.xchg, a.world, a.rank, (double)span, xseq, s_spans, a.latched);
+  __syncthreads();
+  if (threadIdx.x < a.world) s_span[threadIdx.x] = (int64_t)s_spans[threadIdx.x];
+  __syncthreads();
+  int64_t total = 0;
+  for (int g = 0; g < a.world; ++g) total += s_span[g];
+  if (total == 0) {  // CRB:457-460 on every shard
+    if (threadIdx.x == 0 && a.mode == kUniformSample) {
+      *a.count_out = 0;
+      if (a.latched && a.latched[0] == 0) {
+        a.latched[0] = B2R_ERR_TOO_FEW_TRANSITIONS;
+        a.latched[1] = 0;
+      }
+      *a.xchg.seq = xseq;
+    }
+    return;
+  }
+
+  // ---- this rank's draws of the window: ordinals of the invalid ones, valid ones
+  const uint64_t draw_offset = a.offset + xseq;
+  const int window = a.batch + a.max_attempts;
+  int n_rej = 0, n_ok = 0;  // (block-uniform)
+  for (int base = 0; base < window && n_rej < a.max_attempts && n_ok < a.batch;
+       base += blockDim.x) {
+    const int j = base + threadIdx.x;
+    bool mine = false, ok = false;
+    int64_t idx = 0;
+    if (j < window) {
+      const double u = philox_uniform53(a.seed, draw_offset, (uint64_t)j);
+      int64_t o = (int64_t)(u * (double)total);
+      if (o >= total) o = total - 1;
+      int g = 0;
+      while (g < a.world - 1 && o >= s_span[g]) o -= s_span[g++];
+      if (g == a.rank) {
+        mine = true;
+        idx = wrap_index(min_id + o, c.capacity);  // `% replay_capacity`, CRB:466
+        ok = is_valid_transition(c, idx);
+      }
+    }
+    int tile_rej, tile_ok;
+    const int rej_pos = n_rej + block_scan_flag(mine && !ok, warp_counts, &tile_rej);
+    const int ok_pos = n_ok + block_scan_flag(mine && ok, warp_counts, &tile_ok);
+    if (mine && !ok && rej_pos < a.max_attempts) s_rej[rej_pos] = j;
+    if (mine && ok && ok_pos < a.batch && a.mode == kUniformSample) {
+      a.own_j[ok_pos] = j;
+      a.own_idx[ok_pos] = (int32_t)idx;
+    }
+    n_rej = min(n_rej + tile_rej, a.max_attempts);
+    n_ok = min(n_ok + tile_ok, a.batch);
+  }
+  __syncthreads();
+
+  // ---- round 2: the rejection list, unless a publish-ahead of this step has sent it
+  const size_t parity_base = kRejWordsOffset + (size_t)(xseq & 1) * kMaxShards * kRejSlotWords;
+  const size_t my_slot = parity_base + (size_t)a.rank * kRejSlotWords;
+  if (a.mode == kUniformSample) {
+    if (threadIdx.x == 0) {
+      const uint64_t w = ld_sys_u64(a.xchg.local + my_slot);
+      if ((uint32_t)w == (uint32_t)xseq) {
+        s_published = 1;
+        if ((int32_t)(w >> 32) != n_rej) s_stale = 1;
+      }
+    }
+    __syncthreads();
+    // published ahead: it must be what this launch found (else the buffer changed in
+    // between and the peers decided on another list)
+    if (s_published)
+      for (int k = threadIdx.x; k < n_rej; k += blockDim.x)
+        if (ld_sys_u64(a.xchg.local + my_slot + 1 + k) != rej_word(s_rej[k], xseq)) s_stale = 1;
+  }
+  if (!s_published) {
+    const int words = 1 + n_rej;
+    for (int t = threadIdx.x; t < a.world * words; t += blockDim.x) {
+      const int g = t / words, k = t - g * words;
+      uint64_t *box = g == a.rank ? a.xchg.local : a.xchg.peer[g];
+      st_sys_u64(box + my_slot + k, rej_word(k == 0 ? n_rej : s_rej[k - 1], xseq));
+    }
+  }
+  if (a.mode == kUniformPublishRejections) return;
+  __syncthreads();
+  if (threadIdx.x == 0 && s_stale && a.latched && a.latched[0] == 0) {
+    a.latched[0] = B2R_ERR_STALE_TOTAL;
+    a.latched[1] = a.rank;
+  }
+
+  // ---- the peers' lists: counts, then every ordinal (each word polled for its tag)
+  if (threadIdx.x < a.world) {
+    const int g = threadIdx.x;
+    int cnt = n_rej;
+    if (g != a.rank) {
+      cnt = poll_rej_word(a.xchg, a.xchg.local + parity_base + (size_t)g * kRejSlotWords,
+                          xseq, g, 0, a.latched);
+      cnt = min(max(cnt, 0), a.max_attempts);
+    }
+    s_start[g + 1] = cnt;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    s_start[0] = 0;
+    for (int g = 0; g < a.world; ++g) s_start[g + 1] += s_start[g];
+  }
+  __syncthreads();
+  const int n_lists = s_start[a.world];
+  for (int t = threadIdx.x; t < n_lists; t += blockDim.x) {
+    int g = 0;
+    while (s_start[g + 1] <= t) ++g;
+    const int k = t - s_start[g];
+    a.lists[t] = g == a.rank
+                     ? s_rej[k]
+                     : poll_rej_word(a.xchg,
+                                     a.xchg.local + parity_base + (size_t)g * kRejSlotWords +
+                                         1 + k,
+                                     xseq, g, window, a.latched);
+  }
+  __syncthreads();
+  // invalid draws before draw j, over every rank's list
+  auto rejects_before = [&](int j) {
+    int r = 0;
+    for (int g = 0; g < a.world; ++g) {
+      int lo = s_start[g], hi = s_start[g + 1];
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (a.lists[mid] < j) lo = mid + 1; else hi = mid;
+      }
+      r += lo - s_start[g];
+    }
+    return r;
+  };
+
+  // ---- this rank's rows: the kept prefix of its valid draws
+  int kept = 0;
+  for (int k = threadIdx.x; k < n_ok; k += blockDim.x) {
+    const int j = a.own_j[k];
+    const int rb = rejects_before(j);
+    if (j - rb < a.batch && rb < a.max_attempts) {
+      ++kept;
+      if (k < a.out_cap) {
+        a.out_slots[k] = j - rb;
+        a.out_idx[k] = a.own_idx[k];
+      }
+    }
+  }
+  if (kept) atomicAdd(&s_kept, kept);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    // Did the loop end short (CRB:471-475)?  It stops at the max_attempts-th rejection
+    // j_A - 1 if that comes before the batch is full: j_A - max_attempts accepted.
+    int accepted = a.batch;
+    if (n_lists >= a.max_attempts) {
+      int lo = 0, hi = window;
+      while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (rejects_before(mid) >= a.max_attempts) hi = mid; else lo = mid + 1;
+      }
+      if (rejects_before(lo) >= a.max_attempts) accepted = min(accepted, lo - a.max_attempts);
+    }
+    const int rows = s_kept;
+    *a.count_out = min(rows, a.out_cap);
+    if (a.latched && a.latched[0] == 0) {
+      if (accepted < a.batch) {
+        a.latched[0] = B2R_ERR_SAMPLE_ATTEMPTS;
+        a.latched[1] = accepted;
+      } else if (rows > a.out_cap) {  // a share beyond the caller's outputs
+        a.latched[0] = B2R_ERR_UNSUPPORTED;
+        a.latched[1] = rows;
+      }
+    }
+    *a.xchg.seq = xseq;
+  }
+}
+
+}  // namespace
+
+int check_uniform_sharded(const b2r_buffer *b, const b2r_exchange *x, int32_t global_batch) {
+  if (!b) return fail(B2R_ERR_INVALID_ARGUMENT, "buffer is NULL");
+  if (!x) return fail(B2R_ERR_INVALID_ARGUMENT, "exchange is NULL");
+  if (global_batch < 1 || global_batch > 60000)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "global_batch must be in [1, 60000]");
+  if (x->early_publish)
+    return fail(B2R_ERR_INVALID_ARGUMENT,
+                "the exchange has early publish on: it would send tree totals where the "
+                "uniform sampler exchanges spans");
+  if (!x->connected) return fail(B2R_ERR_INVALID_ARGUMENT, "the exchange is not connected");
+  if (b->cfg.max_sample_attempts > kRejListWords)
+    return fail(B2R_ERR_UNSUPPORTED,
+                "max_sample_attempts %d is above %d, the rejection list a shard can publish",
+                b->cfg.max_sample_attempts, kRejListWords);
+  return B2R_OK;
+}
+
+int launch_uniform_sharded(b2r_buffer *b, const b2r_exchange *x, int32_t global_batch,
+                           uint64_t seed, uint64_t offset, int mode, int32_t *out_idx,
+                           int32_t *out_slots, int32_t *out_count, int32_t out_cap,
+                           cudaStream_t s) {
+  B2R_TRY(flush_queue(b, s));
+  B2R_TRY(ensure_ctx(b, s));
+  B2R_TRY(ensure_inv_slots(b, 2 * (int64_t)global_batch + (int64_t)x->world * kRejListWords));
+  UniformShardArgs a;
+  a.valid_dev = b->ctx_dev;
+  fill_exchange_args(x, &a.xchg);
+  a.world = x->world;
+  a.rank = x->rank;
+  a.batch = global_batch;
+  a.max_attempts = b->cfg.max_sample_attempts > 0 ? b->cfg.max_sample_attempts : 0;
+  a.seed = seed;
+  a.offset = offset;
+  a.mode = mode;
+  a.out_cap = out_cap;
+  a.out_idx = out_idx;
+  a.out_slots = out_slots;
+  a.count_out = out_count;
+  a.own_j = b->inv_slots;
+  a.own_idx = a.own_j + global_batch;
+  a.lists = a.own_idx + global_batch;
+  a.latched = b->status;
+  B2R_CUDA(launch(uniform_sharded_kernel, dim3(1), dim3(kUniformShardThreads), 0, s, a));
+  B2R_LAUNCHED();
+  return B2R_OK;
+}
+
 }  // namespace b2r
 
 using b2r::as_stream;
@@ -1782,6 +2108,26 @@ int b2r_sample_indices_sharded_p2p_device(b2r_buffer *b, b2r_exchange *x,
                                     query01, n_retry, retry_u01, seed, offset,
                                     out_slots, out_indices, out_count,
                                     as_stream(stream));
+}
+
+int b2r_sample_transition_batch_uniform_sharded_device(
+    b2r_buffer *b, b2r_exchange *x, int32_t global_batch, uint64_t seed, uint64_t offset,
+    const b2r_batch *out, int32_t *out_slots, int32_t *out_count, int32_t max_rows,
+    b2r_stream stream) {
+  if (!b) return fail(B2R_ERR_INVALID_ARGUMENT, "buffer is NULL");
+  if (!x) return fail(B2R_ERR_INVALID_ARGUMENT, "exchange is NULL");
+  if (!out || !out->indices)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "out and out->indices are required");
+  if (!out_slots) return fail(B2R_ERR_INVALID_ARGUMENT, "out_slots is NULL");
+  if (!out_count) return fail(B2R_ERR_INVALID_ARGUMENT, "out_count is NULL");
+  if (max_rows < 0) return fail(B2R_ERR_INVALID_ARGUMENT, "max_rows must be >= 0");
+  B2R_TRY(b2r::check_uniform_sharded(b, x, global_batch));
+  const int32_t cap = max_rows > 0 && max_rows < global_batch ? max_rows : global_batch;
+  cudaStream_t s = as_stream(stream);
+  B2R_TRY(b2r::launch_uniform_sharded(b, x, global_batch, seed, offset,
+                                      b2r::kUniformSample, out->indices, out_slots,
+                                      out_count, cap, s));
+  return b2r::launch_gather(b, cap, out->indices, out, s, out_count);
 }
 
 }  // extern "C"

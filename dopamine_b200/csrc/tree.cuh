@@ -327,7 +327,15 @@ __device__ __forceinline__ void exchange_publish(const ExchangeArgs &x, int worl
 // [2 parities][world] words after the totals; a word is the f32 value in the high half
 // and the step number in the low half, written with ONE 8-byte store.
 constexpr int kMinWordsOffset = 2 * kMaxShards * 2;
-constexpr int kMailboxWords = kMinWordsOffset + 2 * kMaxShards;
+// Third region: the rejection lists of the sharded uniform sampler (sample.cu:
+// uniform_sharded_kernel).  Layout [2 parities][kMaxShards][1 count word + kRejListWords
+// ordinal words]; every word is (value:32 | step:32), written with ONE 8-byte store, so a
+// reader polls each word it needs until it carries the step's number.  kRejListWords
+// bounds a buffer's max_sample_attempts (the reference's default is 1000).
+constexpr int kRejWordsOffset = kMinWordsOffset + 2 * kMaxShards;
+constexpr int kRejListWords = 1024;
+constexpr int kRejSlotWords = 1 + kRejListWords;
+constexpr int kMailboxWords = kRejWordsOffset + 2 * kMaxShards * kRejSlotWords;
 
 #ifdef __CUDACC__
 // Called by ONE thread: stores this rank's local minimum of step `seq` into every peer's

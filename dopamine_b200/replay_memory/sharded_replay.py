@@ -1,4 +1,4 @@
-"""Prioritized replay sharded over the GPUs of one box (SURVEY.md section 8e).
+"""Replay sharded over the GPUs of one box (SURVEY.md section 8e).
 
 The reference is single-process; this is the only multi-GPU piece of the path.
 Every rank owns a complete `OutOfGraphPrioritizedReplayBuffer` shard (its own
@@ -16,6 +16,10 @@ batch is drawn as if the G shard trees hung under one more tree level:
 
 The number of strata a shard serves is data dependent and stays on the device
 (`count`); downstream kernels take it from there.
+
+`ShardedUniformReplay` does the same for the uniform `OutOfGraphReplayBuffer`
+(circular_replay_buffer.py:436-477): one global batch of uniform draws over the
+concatenated index ranges of the shards.
 """
 import ctypes
 
@@ -98,6 +102,15 @@ class PeerExchange(object):
     (needed only when the ranks are emulated by sequential launches)."""
     _native.check(self._lib.b2r_exchange_publish_device(
         self._h, memory._h, _native.current_stream()))  # pylint: disable=protected-access
+
+  def publish_uniform(self, memory, global_batch, seed, phase):
+    """Publish-ahead of the uniform sampler's rounds for the next step (ranks emulated by
+    sequential launches): phase 0 sends `memory`'s span; phase 1, once every rank has
+    run phase 0, sends its rejection list (b2r_exchange_publish_uniform_device).
+    `global_batch` and `seed` are those of the coming `ShardedUniformReplay` call."""
+    _native.check(self._lib.b2r_exchange_publish_uniform_device(
+        self._h, memory._h, int(global_batch), int(seed), 0, int(phase),  # pylint: disable=protected-access
+        _native.current_stream()))
 
   def __del__(self):
     if getattr(self, '_h', None):
@@ -203,6 +216,10 @@ class ShardedPrioritizedReplay(object):
         min_probability.data_ptr(), _native.current_stream()))
     return slots, self._count, arrays, min_probability
 
+  def flush(self):
+    """Applies the staged adds (before a CUDA graph replay)."""
+    self.memory._flush()  # pylint: disable=protected-access
+
   def check(self):
     """Raises the error latched by an earlier asynchronous call (a share beyond
     max_rows, a peer that did not answer in time, ...).  Synchronises."""
@@ -213,6 +230,70 @@ class ShardedPrioritizedReplay(object):
     _native.check(self._lib.b2r_set_priority_device_counted(
         self._h, indices.numel(), count.data_ptr(), indices.data_ptr(),
         priorities.data_ptr(), _native.current_stream()))
+
+
+class ShardedUniformReplay(object):
+  """ONE global uniform batch over one `OutOfGraphReplayBuffer` shard per rank.
+
+  The batch is the reference's uniform batch (circular_replay_buffer.py:436-477) of a
+  virtual buffer whose index range is the concatenation of the shards' ranges: every rank
+  draws the same Philox candidates over the summed spans, each candidate belongs to the
+  shard its offset lands in, and the ranks agree on which draws were accepted by
+  exchanging their spans and the ordinals of their rejected draws over the peer mailboxes
+  inside the sampling kernel (b2r_sample_transition_batch_uniform_sharded_device).  The
+  result is uniform over the union of the shards' valid transitions."""
+
+  def __init__(self, memory, rank, world_size, seed, exchange):
+    import torch
+    if exchange is None:
+      raise ValueError('ShardedUniformReplay needs a PeerExchange')
+    self.memory = memory
+    self.exchange = exchange
+    self.rank = int(rank)
+    self.world = int(world_size)
+    self.seed = int(seed)
+    self._lib = _native.lib()
+    self._h = memory._h  # pylint: disable=protected-access
+    self._count = torch.zeros(1, dtype=torch.int32, device='cuda')
+    self._torch = torch
+    self._share_out = None
+
+  def sample_transition_batch_sharded(self, global_batch, max_rows=None):
+    """This rank's share of a global uniform batch in one call: sampler, scalar columns
+    and frame copies.  Returns (slots, count, batch tuple), CUDA tensors sized by
+    `max_rows` rows (default `share_bound`); rows [0, count) are this rank's accepted
+    draws in global row order, slots[r] their global row, the rest are left from earlier
+    calls.  The tensors are reused by every call with the same sizes (static for CUDA
+    graphs)."""
+    torch = self._torch
+    global_batch = int(global_batch)
+    rows = (share_bound(global_batch, self.world) if max_rows is None
+            else min(int(max_rows), global_batch))
+    key = (global_batch, rows)
+    if self._share_out is None or self._share_out[0] != key:
+      _, arrays, batch = self.memory._alloc_outputs(rows, True)  # pylint: disable=protected-access
+      self._share_out = (key, torch.zeros(rows, dtype=torch.int32, device='cuda'),
+                         tuple(arrays), batch)
+    _, slots, arrays, batch = self._share_out
+    _native.check(self._lib.b2r_sample_transition_batch_uniform_sharded_device(
+        self._h, self.exchange._h, global_batch, self.seed, 0,  # pylint: disable=protected-access
+        ctypes.byref(batch), slots.data_ptr(), self._count.data_ptr(), rows,
+        _native.current_stream()))
+    return slots, self._count, arrays
+
+  def publish(self, global_batch, phase):
+    """`PeerExchange.publish_uniform` for this shard (emulated ranks)."""
+    self.exchange.publish_uniform(self.memory, global_batch, self.seed, phase)
+
+  def flush(self):
+    """Applies the staged adds (before a CUDA graph replay)."""
+    _native.check(self._lib.b2r_flush(self._h, _native.current_stream()))
+
+  def check(self):
+    """Raises the error latched by an earlier asynchronous call (a share beyond
+    max_rows, attempts exhausted, too few transitions, a peer that did not answer in
+    time, ...).  Synchronises."""
+    _native.check(self._lib.b2r_check(self._h, _native.current_stream()))
 
 
 def share_bound(global_batch, world, slack=1.5, extra=32):

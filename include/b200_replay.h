@@ -395,6 +395,44 @@ int b2r_sample_transition_batch_sharded_device(b2r_buffer *buf, b2r_exchange *ex
                                                int32_t max_rows, float *min_probability,
                                                b2r_stream stream);
 
+/* Sharded UNIFORM replay: this rank's share of ONE global batch of `global_batch`
+ * transitions drawn as OutOfGraphReplayBuffer draws them (CRB:436-477) from a virtual
+ * buffer whose index range is the concatenation of the shards' ranges.  Rank g's span is
+ * n_g = max(0, max_id_g - min_id_g) (CRB:449-460, read on the device), N = sum of the
+ * spans.  Draw j is u_j = philox_uniform53(seed, offset + step, j), with `step` the
+ * exchange's step number (its step counter + 1; every sampling call over the exchange
+ * closes one step); o_j = min((int64)(u_j * N), N - 1); the owner is the rank the scan
+ * "o < n_g ? g : o -= n_g" in rank order stops at; the candidate is
+ * (min_id_owner + o) mod capacity.  Draws are processed in order while accepted <
+ * global_batch and rejected < max_sample_attempts (CRB:464-470); draw j is accepted iff
+ * it is a valid transition of its owner's shard, and the k-th accepted draw is global
+ * row k.  For one rank this is the mapping of b2r_sample_indices_device.
+ * The ranks agree on the accepted draws in two rounds over the exchange's mailboxes,
+ * inside the sampling kernel: the spans, then each rank's ordinals of rejected draws.
+ * This rank's rows are its accepted draws in row order: out->indices[r] the index,
+ * out_slots[r] the global row, *out_count (DEVICE) their number; the scalar columns and
+ * frames of those rows are gathered into `out` (rows past the count are left alone).
+ * max_rows: rows the outputs hold (0 = global_batch); a larger share serves max_rows rows
+ * and latches B2R_ERR_UNSUPPORTED.  No shard with enough transitions latches
+ * B2R_ERR_TOO_FEW_TRANSITIONS, a loop that ends short B2R_ERR_SAMPLE_ATTEMPTS (on every
+ * rank alike), a peer that does not answer in time B2R_ERR_EXCHANGE (b2r_check).
+ * Refused before any device work: a buffer with max_sample_attempts above 1024, an
+ * exchange with early publish on.  DEVICE pointers; asynchronous; can be captured in a
+ * CUDA graph. */
+int b2r_sample_transition_batch_uniform_sharded_device(
+    b2r_buffer *buf, b2r_exchange *exchange, int32_t global_batch, uint64_t seed,
+    uint64_t offset, const b2r_batch *out, int32_t *out_slots, int32_t *out_count,
+    int32_t max_rows, b2r_stream stream);
+/* Publish-ahead of the uniform sampler's rounds for the exchange's NEXT step, for ranks
+ * emulated by sequential launches on one device: phase 0 publishes this rank's span;
+ * phase 1 (after every rank's phase 0) collects the spans and publishes the rank's
+ * rejection list.  The sampling call then republishes nothing (a list published ahead
+ * that no longer matches the buffer latches B2R_ERR_STALE_TOTAL).  Same arguments as the
+ * sampling call.  Asynchronous. */
+int b2r_exchange_publish_uniform_device(b2r_exchange *exchange, b2r_buffer *buf,
+                                        int32_t global_batch, uint64_t seed,
+                                        uint64_t offset, int32_t phase, b2r_stream stream);
+
 /* Variants whose element count lives on the DEVICE (*count <= max_...): what a
  * shard serves of a global batch is only known there.  Rows past *count are
  * skipped.  Asynchronous. */
@@ -480,6 +518,16 @@ typedef struct {
   const int32_t *batch_count;   /* NULL, or DEVICE count <= batch of rows       */
 } b2r_dqn_args;
 int b2r_dqn_loss(const b2r_dqn_args *args, b2r_stream stream);
+/* The loss of one shard of a global batch of `global_batch` transitions, as
+ * b2r_sample_transition_batch_uniform_sharded_device samples it.  args->batch is the
+ * rank's max_rows and args->batch_count (DEVICE, required) its row count.  Rows b < count
+ * get the loss, target and gradient row b2r_dqn_loss gives that transition on the whole
+ * global batch (gradient clip(e, -1, 1) / global_batch); rows b >= count get loss 0 and
+ * zero gradient rows, their target is not written.  mean_loss = (sum over this rank's
+ * rows of loss, in f64, rounded once) / global_batch: summed over the ranks, the means and
+ * the gradients are the global batch's (DQ:321).  DEVICE pointers; asynchronous. */
+int b2r_dqn_loss_sharded(const b2r_dqn_args *args, int32_t global_batch,
+                         b2r_stream stream);
 
 /* ------------------------------------------------------------------------- */
 /* The whole hot path in one call (SURVEY.md 3.2: what one sess.run(train_op)   */

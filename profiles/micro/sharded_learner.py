@@ -1,13 +1,17 @@
-"""ms per update and transitions/s of ShardedRainbowLearner (`--agent rainbow`) or
-ShardedIQNLearner (`--agent iqn`) at 1/2/4/8 GPUs: a global batch of 32 rows per GPU, a
+"""ms per update and transitions/s of ShardedRainbowLearner (`--agent rainbow`),
+ShardedIQNLearner (`--agent iqn`) or ShardedDQNLearner (`--agent dqn`) at 1/2/4/8 GPUs: a
+global batch of 32 rows per GPU, a
 replay shard of 1M transitions per GPU, eager and replayed as a CUDA graph.  Also reports
 the rows the networks computed (max_rows per rank, the padding that keeps the shapes
 static) next to the useful rows (the global batch), and the card's name and power limit
 read in the same run.  With `--agent iqn` the shards have unit priorities (IQN's replay),
 the tau counts are IQNLearner's defaults (N = N' = K = 32), and the run also times plain
-IQNLearner.train_step() at batch 32 on one GPU, the N = 1 baseline.
+IQNLearner.train_step() at batch 32 on one GPU, the N = 1 baseline.  With `--agent dqn`
+the shards are uniform OutOfGraphReplayBuffers (DQN's replay), the eager runs also time
+`sample()` alone (the sharded uniform sampler and the frame copies), and the baseline is
+plain DQNLearner.train_step() at batch 32.
 
-  python profiles/micro/sharded_learner.py [--agent rainbow|iqn] [--gpus 1,2,4,8]
+  python profiles/micro/sharded_learner.py [--agent rainbow|iqn|dqn] [--gpus 1,2,4,8]
       [--steps 200] [--out F]
 
 Each configuration runs in fresh processes (one per GPU, NCCL); rank 0 times `--steps`
@@ -50,7 +54,27 @@ def _shard(cap, seed, batch, unit_priorities=False):
   return mem
 
 
+def _uniform_shard(cap, seed, batch):
+  from dopamine_b200.replay_memory import circular_replay_buffer as crb
+  rng = np.random.RandomState(seed)
+  mem = crb.OutOfGraphReplayBuffer(
+      (84, 84), 4, cap, batch, update_horizon=3, gamma=0.99, output='torch',
+      rng='device', seed=seed, reuse_outputs=True)
+  mem._store['action'] = rng.randint(0, ACTIONS, size=cap).astype(np.int32)
+  mem._store['reward'] = np.clip(rng.randn(cap), -1, 1).astype(np.float32)
+  mem._store['terminal'] = (rng.rand(cap) < 0.01).astype(np.uint8)
+  mem.add_count = cap + 1000
+  mem.invalid_range = np.array([(1000 - 3 + i) % cap for i in range(7)])
+  return mem
+
+
 def _make_learner(agent_name, global_batch, rank, graph):
+  if agent_name == 'dqn':
+    from dopamine_b200.agents.dqn import learner
+    return learner.ShardedDQNLearner(
+        ACTIONS, batch_size=global_batch,
+        memory=_uniform_shard(CAPACITY, 10 + rank, global_batch),
+        replay_capacity=CAPACITY, update_horizon=3, seed=1, cuda_graph=graph)
   if agent_name == 'iqn':
     from dopamine_b200.agents.implicit_quantile import learner
     return learner.ShardedIQNLearner(
@@ -79,23 +103,32 @@ def _iqn_settings(learner):
               num_quantile_samples=learner.num_quantile_samples)
 
 
-def _baseline_worker(rank, steps, warmup, out_path):
-  """Plain IQNLearner.train_step() at batch 32 on one GPU: the N = 1 baseline."""
+def _baseline_worker(rank, agent_name, steps, warmup, out_path):
+  """Plain IQNLearner / DQNLearner .train_step() at batch 32 on one GPU: the N = 1
+  baseline."""
   import torch
-  from dopamine_b200.agents.implicit_quantile import learner as iqn_learner
   torch.cuda.set_device(rank)
-  learner = iqn_learner.IQNLearner(
-      ACTIONS, batch_size=PER_GPU_BATCH, replay_capacity=CAPACITY, seed=1,
-      memory=_shard(CAPACITY, 10, PER_GPU_BATCH, unit_priorities=True))
+  if agent_name == 'dqn':
+    from dopamine_b200.agents.dqn import learner as dqn_learner
+    learner = dqn_learner.DQNLearner(
+        ACTIONS, batch_size=PER_GPU_BATCH, replay_capacity=CAPACITY, update_horizon=3,
+        seed=1, memory=_uniform_shard(CAPACITY, 10, PER_GPU_BATCH))
+  else:
+    from dopamine_b200.agents.implicit_quantile import learner as iqn_learner
+    learner = iqn_learner.IQNLearner(
+        ACTIONS, batch_size=PER_GPU_BATCH, replay_capacity=CAPACITY, seed=1,
+        memory=_shard(CAPACITY, 10, PER_GPU_BATCH, unit_priorities=True))
   for _ in range(warmup):
     learner.train_step()
   torch.cuda.synchronize()
   ms = _time_updates(torch, learner, steps)
-  result = dict(agent='iqn', learner='IQNLearner', gpus=1, mode='eager', steps=steps,
-                ms_per_update=round(ms, 4),
+  result = dict(agent=agent_name, learner=type(learner).__name__, gpus=1, mode='eager',
+                steps=steps, ms_per_update=round(ms, 4),
                 transitions_per_s=round(PER_GPU_BATCH / ms * 1e3, 1),
                 useful_rows=PER_GPU_BATCH, network_rows=PER_GPU_BATCH,
-                capacity_per_gpu=CAPACITY, **_iqn_settings(learner))
+                capacity_per_gpu=CAPACITY)
+  if agent_name == 'iqn':
+    result.update(_iqn_settings(learner))
   with open(out_path, 'w') as f:
     json.dump(result, f)
 
@@ -116,6 +149,16 @@ def _worker(rank, world, port, agent_name, graph, steps, warmup, out_path):
     torch.cuda.synchronize()
     dist.barrier()
     ms = _time_updates(torch, learner, steps)
+    sample_ms = None
+    if agent_name == 'dqn' and not graph:  # the sampler and the frame copies alone
+      start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+      dist.barrier()
+      start.record()
+      for _ in range(steps):
+        learner.sample()
+      end.record()
+      torch.cuda.synchronize()
+      sample_ms = start.elapsed_time(end) / steps
     learner.check()
     if rank == 0:
       result = dict(agent=agent_name, learner=type(learner).__name__, gpus=world,
@@ -127,6 +170,8 @@ def _worker(rank, world, port, agent_name, graph, steps, warmup, out_path):
                     loss=float(learner.loss.item()))
       if agent_name == 'iqn':
         result.update(_iqn_settings(learner))
+      if sample_ms is not None:
+        result['sample_ms'] = round(sample_ms, 4)
       with open(out_path, 'w') as f:
         json.dump(result, f)
     dist.barrier()
@@ -144,7 +189,7 @@ def main():
   import torch
   import torch.multiprocessing as mp
   p = argparse.ArgumentParser()
-  p.add_argument('--agent', choices=('rainbow', 'iqn'), default='rainbow')
+  p.add_argument('--agent', choices=('rainbow', 'iqn', 'dqn'), default='rainbow')
   p.add_argument('--gpus', default='1,2,4,8')
   p.add_argument('--steps', type=int, default=200)
   p.add_argument('--warmup', type=int, default=20)
@@ -178,9 +223,10 @@ def main():
         lines.append(f.read())
     print(lines[-1], flush=True)
 
-  if a.agent == 'iqn':
-    run(_baseline_worker, 1, (a.steps, a.warmup, os.path.join(tmp, 'iqn_baseline.json')),
-        dict(agent='iqn', learner='IQNLearner', gpus=1, mode='eager'))
+  if a.agent in ('iqn', 'dqn'):
+    run(_baseline_worker, 1,
+        (a.agent, a.steps, a.warmup, os.path.join(tmp, a.agent + '_baseline.json')),
+        dict(agent=a.agent, gpus=1, mode='eager'))
   for n in [int(x) for x in a.gpus.split(',')]:
     if n > torch.cuda.device_count():
       lines.append(json.dumps(dict(agent=a.agent, gpus=n, skipped='only {} devices'
