@@ -130,6 +130,9 @@ struct LossArgs {
   // The write-back behind this kernel is resident already and waits to hear that the
   // sampled indices are final (tree.cuh: TreeGo); go.go == nullptr: nobody does.
   TreeGo go;
+  // c51_post_tree_kernel<true>: where the first half left the log-probabilities, and the
+  // word that says it has (replay.cuh)
+  StageGate stage;
 };
 
 __device__ __forceinline__ uint64_t timer_ns() {
@@ -848,6 +851,8 @@ c51_loss_rows_kernel(LossArgs a) {
 // Scratch per row (kPreRow floats): [0, 64) probabilities of the greedy next action,
 // [64, 128) online softmax statistics, (max, log of the denominator) per action for the
 // first 32 actions (c51_pre_kernel only; stats == 0 in PostArgs: the tail computes them).
+// A staged tail (StageGate) also gets the online log-probabilities of every action, in a
+// buffer of their own (PreArgs::logp).
 constexpr int kPreRow = 2 * kRowAtoms;
 
 struct PreArgs {
@@ -862,6 +867,10 @@ struct PreArgs {
   // page-locked memory (no copy calls on the host); the tail then reads its one row of
   // online logits per transition from this copy instead of crossing PCIe again.
   float *online_copy;
+  // nullable (c51_pre_kernel): [rows][c51_logp_stride] log_softmax of every action's online
+  // logits, and StageGate::done, counted when they are all there
+  float *logp;
+  unsigned int *staged_done;
 };
 
 // CTA per row, warp per action (rows below 128: latency-bound).
@@ -939,6 +948,13 @@ __global__ void __launch_bounds__(1024) c51_pre_kernel(PreArgs a) {
       st.y = logf(osum);
       *reinterpret_cast<float2 *>(a.scratch + (size_t)b * kPreRow + kRowAtoms + 2 * act) = st;
     }
+    if (a.logp != nullptr) {  // (the tail's expression, with the statistics above)
+      const float lse = logf(osum);
+      float *lrow = a.logp + (size_t)b * c51_logp_stride(A, N) + act * N;
+#pragma unroll
+      for (int t = 0; t < PL; ++t)
+        if (lane + 32 * t < N) lrow[lane + 32 * t] = __fsub_rn(__fsub_rn(xo[t], mo), lse);
+    }
     float qpart = 0.f;
 #pragma unroll
     for (int t = 0; t < PL; ++t) {
@@ -983,7 +999,7 @@ __global__ void __launch_bounds__(1024) c51_pre_kernel(PreArgs a) {
       if (lane + 32 * t < N) a.scratch[(size_t)b * kPreRow + lane + 32 * t] = bp[t];
   }
   B2R_MARK_END(8);
-  pre_sync_signal(a.sync);
+  pre_sync_signal(a.sync, a.staged_done);
 }
 
 // Warp per row, G lanes per action (rows from 128 up: bound by instruction issue).
@@ -1081,51 +1097,19 @@ __global__ void __launch_bounds__(kRowWarps * 32) c51_pre_rows_kernel(PreArgs a)
 constexpr int kProjTerms = 5;  // Bellman atoms within dz of an output atom, with slack
                               // (gamma^n >= 2/3: 2 / (gamma^n) + 2 <= 5; wider: the loop)
 
-// One row of the tail by one warp.  bestp_row / sup_row: this warp's shared-memory rows
-// ([kRowAtoms] floats each).  Writes the row's outputs and returns its new priority.
-__device__ __forceinline__ float c51_post_row(const LossArgs &a,
-                                              const float *__restrict__ scratch,
-                                              int have_stats, int b, int rows, int lane,
-                                              float pmin, float *bestp_row, float *sup_row) {
+// The part of a row's tail that follows its scalars and the log-probabilities of its
+// chosen action: Bellman support, projection, cross entropy and the row's outputs.
+// LEAN: neither the projected target nor a gradient row is asked for (compile-time: the
+// staged instance the fused step runs at the agent's batch).
+template <bool LEAN>
+__device__ __forceinline__ float c51_post_finish(const LossArgs &a, int b, int rows, int lane,
+                                                 const float (&zl)[2], float r, float term,
+                                                 float w, const float (&lgp)[2],
+                                                 bool bad_action, int chosen, float eo0,
+                                                 float eo1, float den_o,
+                                                 const float *bestp_row, float *sup_row) {
   const int N = a.u.num_atoms, A = a.u.num_actions;
-  const float *__restrict__ z = a.u.support;
   float prio_out = 0.f;
-  // ---- round trip 1
-  int chosen = a.u.actions[b];
-  const float r = a.u.rewards[b];
-  const float term = (float)a.u.terminals[b];
-  const float my_prob = a.u.sampling_probabilities ? a.u.sampling_probabilities[b] : 1.f;
-  float zl[2], bp[2];
-#pragma unroll
-  for (int t = 0; t < 2; ++t) {
-    const int i = lane + 32 * t;
-    zl[t] = i < N ? z[i] : 0.f;
-    bp[t] = i < N ? scratch[(size_t)b * kPreRow + i] : 0.f;
-  }
-  float2 st = make_float2(0.f, 0.f);  // lane = action: (max, log denominator)
-  if (have_stats && lane < A)
-    st = *reinterpret_cast<const float2 *>(scratch + (size_t)b * kPreRow + kRowAtoms + 2 * lane);
-  // importance weight (RA:279-280): needs the probabilities only — two square roots and
-  // three divisions that are in flight while the second round trip and the projection run
-  float w = 1.f;
-  if (a.u.sampling_probabilities) {
-    const float wmax = __fdiv_rn(1.0f, sqrtf(__fadd_rn(pmin, 1e-10f)));
-    const float raw = __fdiv_rn(1.0f, sqrtf(__fadd_rn(my_prob, 1e-10f)));
-    w = __fdiv_rn(raw, wmax);
-  }
-  B2R_MARK(13);
-  // an action outside [0, A) (tf.gather_nd raises): evaluated for action 0, zero loss,
-  // B2R_ERR_INDEX_RANGE latched
-  const bool bad_action = chosen < 0 || chosen >= A;
-  if (bad_action) chosen = 0;
-  // ---- round trip 2
-  const float *__restrict__ orow = a.u.online_logits + ((size_t)b * A + chosen) * N;
-  float xo[2];
-#pragma unroll
-  for (int t = 0; t < 2; ++t) xo[t] = lane + 32 * t < N ? orow[lane + 32 * t] : kLogitPad;
-#pragma unroll
-  for (int t = 0; t < 2; ++t)
-    if (lane + 32 * t < N) bestp_row[lane + 32 * t] = bp[t];
   // Bellman support (rainbow_agent.py:229-235)
   const float live = __fsub_rn(1.0f, term);
   const float gwt = __fmul_rn(a.u.cumulative_gamma, live);
@@ -1133,26 +1117,6 @@ __device__ __forceinline__ float c51_post_row(const LossArgs &a,
   for (int t = 0; t < 2; ++t)
     if (lane + 32 * t < N) sup_row[lane + 32 * t] = __fadd_rn(r, __fmul_rn(gwt, zl[t]));
   __syncwarp();
-  // log_softmax of the chosen action's online logits (rainbow_agent.py:262-271)
-  float mo, lse, eo0 = 0.f, eo1 = 0.f, den_o = 1.f;
-  if (have_stats && chosen < 32) {
-    mo = __shfl_sync(0xffffffffu, st.x, chosen);
-    lse = __shfl_sync(0xffffffffu, st.y, chosen);
-    if (a.u.grad_logits) {
-      eo0 = expf(__fsub_rn(xo[0], mo));
-      eo1 = expf(__fsub_rn(xo[1], mo));
-      den_o = group_sum<32>(__fadd_rn(eo0, eo1));
-    }
-  } else {
-    mo = group_max<32>(fmaxf(xo[0], xo[1]));
-    eo0 = expf(__fsub_rn(xo[0], mo));
-    eo1 = expf(__fsub_rn(xo[1], mo));
-    den_o = group_sum<32>(__fadd_rn(eo0, eo1));  // pads add exactly 0
-    lse = logf(den_o);
-  }
-  const float lgp[2] = {__fsub_rn(__fsub_rn(xo[0], mo), lse),
-                        __fsub_rn(__fsub_rn(xo[1], mo), lse)};
-  B2R_MARK(14);
 
   // projection (RA:381-494): see c51_loss_rows_kernel for the interval argument
   const float *sup = sup_row, *next_p = bestp_row;
@@ -1243,7 +1207,7 @@ __device__ __forceinline__ float c51_post_row(const LossArgs &a,
   for (int t = 0; t < 2; ++t) {
     const int i = lane + 32 * t;
     if (i < N) {
-      if (a.u.target) a.u.target[(size_t)b * N + i] = tg[t];
+      if (!LEAN && a.u.target) a.u.target[(size_t)b * N + i] = tg[t];
       ce_part = __fadd_rn(ce_part, __fmul_rn(tg[t], lgp[t]));
       tsum_part = __fadd_rn(tsum_part, tg[t]);
     }
@@ -1272,7 +1236,7 @@ __device__ __forceinline__ float c51_post_row(const LossArgs &a,
     if (a.u.weights) a.u.weights[b] = w;
     a.weighted[b] = __fmul_rn(w, ce);
   }
-  if (a.u.grad_logits) {
+  if (!LEAN && a.u.grad_logits) {
     const float scale = __fmul_rn(w, __fdiv_rn(1.0f, (float)rows));
     float *g = a.u.grad_logits + (size_t)b * A * N;
     float v[2] = {0.f, 0.f};
@@ -1293,6 +1257,135 @@ __device__ __forceinline__ float c51_post_row(const LossArgs &a,
     }
   }
   return prio_out;
+}
+
+// One row of the tail by one warp.  bestp_row / sup_row: this warp's shared-memory rows
+// ([kRowAtoms] floats each).  Writes the row's outputs and returns its new priority.
+__device__ __forceinline__ float c51_post_row(const LossArgs &a,
+                                              const float *__restrict__ scratch,
+                                              int have_stats, int b, int rows, int lane,
+                                              float pmin, float *bestp_row, float *sup_row) {
+  const int N = a.u.num_atoms, A = a.u.num_actions;
+  const float *__restrict__ z = a.u.support;
+  // ---- round trip 1
+  int chosen = a.u.actions[b];
+  const float r = a.u.rewards[b];
+  const float term = (float)a.u.terminals[b];
+  const float my_prob = a.u.sampling_probabilities ? a.u.sampling_probabilities[b] : 1.f;
+  float zl[2], bp[2];
+#pragma unroll
+  for (int t = 0; t < 2; ++t) {
+    const int i = lane + 32 * t;
+    zl[t] = i < N ? z[i] : 0.f;
+    bp[t] = i < N ? scratch[(size_t)b * kPreRow + i] : 0.f;
+  }
+  float2 st = make_float2(0.f, 0.f);  // lane = action: (max, log denominator)
+  if (have_stats && lane < A)
+    st = *reinterpret_cast<const float2 *>(scratch + (size_t)b * kPreRow + kRowAtoms + 2 * lane);
+  // importance weight (RA:279-280): needs the probabilities only — two square roots and
+  // three divisions that are in flight while the second round trip and the projection run
+  float w = 1.f;
+  if (a.u.sampling_probabilities) {
+    const float wmax = __fdiv_rn(1.0f, sqrtf(__fadd_rn(pmin, 1e-10f)));
+    const float raw = __fdiv_rn(1.0f, sqrtf(__fadd_rn(my_prob, 1e-10f)));
+    w = __fdiv_rn(raw, wmax);
+  }
+  B2R_MARK(13);
+  // an action outside [0, A) (tf.gather_nd raises): evaluated for action 0, zero loss,
+  // B2R_ERR_INDEX_RANGE latched
+  const bool bad_action = chosen < 0 || chosen >= A;
+  if (bad_action) chosen = 0;
+  // ---- round trip 2
+  const float *__restrict__ orow = a.u.online_logits + ((size_t)b * A + chosen) * N;
+  float xo[2];
+#pragma unroll
+  for (int t = 0; t < 2; ++t) xo[t] = lane + 32 * t < N ? orow[lane + 32 * t] : kLogitPad;
+#pragma unroll
+  for (int t = 0; t < 2; ++t)
+    if (lane + 32 * t < N) bestp_row[lane + 32 * t] = bp[t];
+  // log_softmax of the chosen action's online logits (rainbow_agent.py:262-271)
+  float mo, lse, eo0 = 0.f, eo1 = 0.f, den_o = 1.f;
+  if (have_stats && chosen < 32) {
+    mo = __shfl_sync(0xffffffffu, st.x, chosen);
+    lse = __shfl_sync(0xffffffffu, st.y, chosen);
+    if (a.u.grad_logits) {
+      eo0 = expf(__fsub_rn(xo[0], mo));
+      eo1 = expf(__fsub_rn(xo[1], mo));
+      den_o = group_sum<32>(__fadd_rn(eo0, eo1));
+    }
+  } else {
+    mo = group_max<32>(fmaxf(xo[0], xo[1]));
+    eo0 = expf(__fsub_rn(xo[0], mo));
+    eo1 = expf(__fsub_rn(xo[1], mo));
+    den_o = group_sum<32>(__fadd_rn(eo0, eo1));  // pads add exactly 0
+    lse = logf(den_o);
+  }
+  const float lgp[2] = {__fsub_rn(__fsub_rn(xo[0], mo), lse),
+                        __fsub_rn(__fsub_rn(xo[1], mo), lse)};
+  B2R_MARK(14);
+  return c51_post_finish<false>(a, b, rows, lane, zl, r, term, w, lgp, bad_action, chosen,
+                                eo0, eo1, den_o, bestp_row, sup_row);
+}
+
+// A staged row (c51_post_tree_kernel<true>), ahead of the sampler's end: the greedy
+// action's probabilities into bestp_row, the log-probabilities of all actions into
+// logp_row ([c51_logp_stride / 4] float4s), the support into zl.  L2 loads (__ldcg): the
+// first half's rows arrive through memory, not across a kernel boundary.
+__device__ __forceinline__ void c51_stage_row(const LossArgs &a, const float *scratch, int b,
+                                              int lane, float *bestp_row, float4 *logp_row,
+                                              float (&zl)[2]) {
+  const int N = a.u.num_atoms;
+  const int words = c51_logp_stride(a.u.num_actions, N) / 4;
+  const float4 *src = reinterpret_cast<const float4 *>(a.stage.logp) + (size_t)b * words;
+  constexpr int kBurst = 8;  // float4 loads in flight per lane
+  for (int base = 0; base < words; base += 32 * kBurst) {
+    float4 v[kBurst];
+#pragma unroll
+    for (int u = 0; u < kBurst; ++u) {
+      const int k = base + 32 * u + lane;
+      if (k < words) v[u] = __ldcg(src + k);
+    }
+#pragma unroll
+    for (int u = 0; u < kBurst; ++u) {
+      const int k = base + 32 * u + lane;
+      if (k < words) logp_row[k] = v[u];
+    }
+  }
+#pragma unroll
+  for (int t = 0; t < 2; ++t) {
+    const int i = lane + 32 * t;
+    zl[t] = i < N ? __ldcg(a.u.support + i) : 0.f;
+    if (i < N) bestp_row[i] = __ldcg(scratch + (size_t)b * kPreRow + i);
+  }
+  __syncwarp();  // (the chosen action's row is read across lanes)
+}
+
+// The rest of a staged row, behind the sampler: ONE round trip for the sampled scalars,
+// then the chosen action's log-probabilities from shared memory.
+__device__ __forceinline__ float c51_post_staged_row(const LossArgs &a, int b, int rows,
+                                                     int lane, const float (&zl)[2],
+                                                     const float *bestp_row, float *sup_row,
+                                                     const float *logp_row) {
+  const int N = a.u.num_atoms, A = a.u.num_actions;
+  int chosen = a.u.actions[b];
+  const float r = a.u.rewards[b];
+  const float term = (float)a.u.terminals[b];
+  float w = 1.f;
+  if (a.u.sampling_probabilities) {  // (RA:279-280)
+    const float pmin = *a.u.min_probability;
+    const float my_prob = a.u.sampling_probabilities[b];
+    const float wmax = __fdiv_rn(1.0f, sqrtf(__fadd_rn(pmin, 1e-10f)));
+    const float raw = __fdiv_rn(1.0f, sqrtf(__fadd_rn(my_prob, 1e-10f)));
+    w = __fdiv_rn(raw, wmax);
+  }
+  // (as in c51_post_row: an action outside [0, A) is evaluated for action 0)
+  const bool bad_action = chosen < 0 || chosen >= A;
+  if (bad_action) chosen = 0;
+  B2R_MARK_CTA(13, 1);
+  const float lgp[2] = {lane < N ? logp_row[chosen * N + lane] : 0.f,
+                        lane + 32 < N ? logp_row[chosen * N + lane + 32] : 0.f};
+  return c51_post_finish<true>(a, b, rows, lane, zl, r, term, w, lgp, bad_action, chosen, 0.f,
+                               0.f, 1.f, bestp_row, sup_row);
 }
 
 // The tail: one warp per row, kRowWarps rows per CTA, lanes own atoms lane and lane + 32.
@@ -1379,9 +1472,13 @@ c51_post_kernel(LossArgs a, const float *__restrict__ scratch, int have_stats) {
 // shared memory), one cluster barrier replaces the kernel boundary, and CTA 0 finishes
 // the update (tree_update_tiny_finish).  Measured (profiles/r2/README.md): 15.3 us per
 // step at batch 32 against 16.3 us with the tail and the write-back as two kernels.
+// STAGED (c51_tail_can_stage, no row count on the device): every row CTA stages its rows'
+// inputs from the first half (StageGate) BEFORE its griddepcontrol.wait, while the
+// sampler still runs, and is left with one round trip for the sampled scalars behind it.
 constexpr int kPostClusterCtas = 8;
 constexpr int kPostRowWarps = 5;  // rows per row CTA: 7 row CTAs x 5 >= 32 rows
 
+template <bool STAGED>
 __global__ void __launch_bounds__(1024)
 c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_stats) {
   __shared__ float s_bestp[kPostRowWarps][kRowAtoms];
@@ -1389,13 +1486,31 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
   __shared__ float s_prio[kTinyBatch];      // (CTA 0's copy is the one that is used)
   __shared__ float s_weighted[kTinyBatch];
   __shared__ __align__(8) uint64_t s_arrived;  // mbarrier: the rows' words have landed
+  __shared__ bool s_gate;
+  extern __shared__ float4 s_logp[];  // STAGED: [kPostRowWarps][c51_logp_stride / 4]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const bool tree_cta = blockIdx.x == 0;
   B2R_MARK(10);
   if (tree_cta && threadIdx.x == 0) mbar_init(&s_arrived, 1);
   cluster_arrive_relaxed();  // (nobody sends before the mbarrier exists: waited for below)
+  // STAGED: the row this warp owns (at most 32 rows: one per row warp), staged ahead of the
+  // sampler's end once the first half of this step has ended (StageGate; the ticket is
+  // taken before the dependents may start, and they start once it has ended: the tails of
+  // later steps do not pile up resident behind this one)
+  float zl[2] = {0.f, 0.f};
+  float4 *logp_row = s_logp + (size_t)warp * (c51_logp_stride(a.u.num_actions, a.u.num_atoms) / 4);
+  const int srow = (int)(blockIdx.x - 1) * kPostRowWarps + warp;
+  const bool stages = STAGED && !tree_cta && warp < kPostRowWarps && srow < a.u.batch;
+  if (STAGED) {
+    if (threadIdx.x == 0) s_gate = stage_gate_wait(a.stage);
+    __syncthreads();
+  }
   pdl_release();
+  const bool early = STAGED && s_gate;
+  if (early && stages) c51_stage_row(a, scratch, srow, lane, s_bestp[warp], logp_row, zl);
+  if (STAGED) B2R_MARK_CTA(15, 1);
   pdl_acquire();
+  if (STAGED && !early && stages) c51_stage_row(a, scratch, srow, lane, s_bestp[warp], logp_row, zl);
   B2R_MARK(11);
   // (a shard's step: the row count is on the device, and the write-back rides along only
   // when it turns out to be at most 32 rows — else the tree kernel behind this one does it)
@@ -1415,6 +1530,13 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
       // one word per row (two with the mean loss) will arrive
       if (threadIdx.x == 0) mbar_arrive_expect(&s_arrived, (uint32_t)rows * (want_mean ? 8u : 4u));
       tree_update_tiny_issue(a.tree, warp, lane, &tl);
+    }
+  } else if (STAGED) {
+    if (stages) {
+      prio = c51_post_staged_row(a, srow, rows, lane, zl, s_bestp[warp], s_sup[warp],
+                                 reinterpret_cast<const float *>(logp_row));
+      my_row = srow;
+      if (want_mean) weighted = a.weighted[srow];
     }
   } else if (warp < kPostRowWarps) {
     const float pmin = a.u.sampling_probabilities ? *a.u.min_probability : INFINITY;
@@ -1576,14 +1698,25 @@ bool c51_can_split(const b2r_c51_args *args) {
 
 int c51_scratch_floats_per_row() { return kPreRow; }
 
+// The staged tail (c51_post_tree_kernel<true>) is the lean instance — no target, no
+// gradient — over at most 32 rows, and keeps every action's log-probabilities of its five
+// rows in shared memory (at most 40 KB: 32 actions x 64 atoms).
+bool c51_tail_can_stage(const b2r_c51_args *args) {
+  return args->batch <= kTinyBatch && args->batch_count == nullptr &&
+         args->grad_logits == nullptr && args->target == nullptr &&
+         args->num_actions <= 32 && args->num_atoms <= kRowAtoms;
+}
+
 // First half over `rows` rows of logits; scratch: device [rows][kPreRow] floats.  Sets
 // *have_stats when the launch leaves the online softmax statistics in the scratch.
 int c51_pre_launch(const b2r_c51_args *args, int rows, float *scratch, const PreSync &sync,
                    cudaStream_t s, int *have_stats, const float *online_src,
-                   float *online_copy) {
+                   float *online_copy, const StageGate *stage) {
   if (!args || rows <= 0 || !scratch || !args->target_logits || !args->online_logits ||
       !args->support)
     return fail(B2R_ERR_INVALID_ARGUMENT, "bad C51 arguments");
+  if (stage != nullptr && (rows >= 128 || !stage->done || !stage->logp))
+    return fail(B2R_ERR_INVALID_ARGUMENT, "a staged first half covers fewer than 128 rows");
   PreArgs a;
   a.target_logits = args->target_logits;
   a.online_logits = online_src != nullptr ? online_src : args->online_logits;
@@ -1595,6 +1728,8 @@ int c51_pre_launch(const b2r_c51_args *args, int rows, float *scratch, const Pre
   a.num_atoms = args->num_atoms;
   a.warps = args->num_actions < 32 ? args->num_actions : 32;
   a.sync = sync;
+  a.logp = stage != nullptr ? stage->logp : nullptr;
+  a.staged_done = stage != nullptr ? stage->done : nullptr;
   if (rows >= 128) {
     const dim3 grid((rows + kRowWarps - 1) / kRowWarps), block(kRowWarps * 32);
     if (args->num_atoms == 51)
@@ -1631,7 +1766,8 @@ bool c51_post_takes_tree(const b2r_c51_args *args, const b2r_tree *tree,
 int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_stats,
                     cudaStream_t s, int64_t *err, int32_t *count_copy, b2r_tree *tree,
                     const int32_t *indices, unsigned int *tree_done,
-                    const b2r_exchange *publish, float *loss_host, const TreeGo *go) {
+                    const b2r_exchange *publish, float *loss_host, const TreeGo *go,
+                    const StageGate *stage) {
   if (!args || args->batch <= 0 || !scratch)
     return fail(B2R_ERR_INVALID_ARGUMENT, "bad C51 shape");
   if (args->batch_count && args->mean_weighted_loss)
@@ -1648,6 +1784,12 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
   a.tree_done = nullptr;
   a.loss_host = loss_host;
   if (go != nullptr) a.go = *go;
+  if (stage != nullptr) {
+    if (tree == nullptr || !c51_tail_can_stage(args) || !stage->done || !stage->tickets ||
+        !stage->logp)
+      return fail(B2R_ERR_INVALID_ARGUMENT, "this tail cannot stage its inputs");
+    a.stage = *stage;
+  }
   a.warps = 0;
   B2R_TRY(ensure_loss_scratch(args->batch));
   a.weighted = g_weighted;
@@ -1678,9 +1820,17 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
     }
     int warps = tree->depth + 1;
     if (warps < kPostRowWarps) warps = kPostRowWarps;
-    B2R_CUDA(launch_prio_cluster(c51_post_tree_kernel, dim3(kPostClusterCtas),
-                                 dim3(warps * 32), 0, s, chain_priority(),
-                                 kPostClusterCtas, a, scratch, have_stats));
+    if (stage != nullptr) {
+      const size_t smem = (size_t)kPostRowWarps *
+                          c51_logp_stride(args->num_actions, args->num_atoms) * sizeof(float);
+      B2R_CUDA(launch_prio_cluster(c51_post_tree_kernel<true>, dim3(kPostClusterCtas),
+                                   dim3(warps * 32), smem, s, chain_priority(),
+                                   kPostClusterCtas, a, scratch, have_stats));
+    } else {
+      B2R_CUDA(launch_prio_cluster(c51_post_tree_kernel<false>, dim3(kPostClusterCtas),
+                                   dim3(warps * 32), 0, s, chain_priority(),
+                                   kPostClusterCtas, a, scratch, have_stats));
+    }
     B2R_LAUNCHED();
     return B2R_OK;
   }

@@ -428,8 +428,8 @@ int b2r_create(const b2r_config *cfg, b2r_buffer **out) {
     B2R_CUDA(cudaStreamCreateWithPriority(&b->side2, cudaStreamNonBlocking, greatest));
     B2R_CUDA(cudaStreamCreateWithPriority(&b->side3, cudaStreamNonBlocking, greatest));
   }
-  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->pre_sync), 16));
-  B2R_CUDA(cudaMemset(b->pre_sync, 0, 16));
+  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->pre_sync), 32));
+  B2R_CUDA(cudaMemset(b->pre_sync, 0, 32));
   for (int k = 0; k < 2; ++k)
     B2R_CUDA(cudaEventCreateWithFlags(&b->ev_slot_free[k], cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_c51_fork, cudaEventDisableTiming));
@@ -472,6 +472,7 @@ int b2r_destroy(b2r_buffer *b) {
   if (b->ev_c51_fork) cudaEventDestroy(b->ev_c51_fork);
   if (b->ev_c51_pre) cudaEventDestroy(b->ev_c51_pre);
   if (b->c51_bestp) cudaFree(b->c51_bestp);
+  if (b->c51_logp) cudaFree(b->c51_logp);
   if (b->pre_sync) cudaFree(b->pre_sync);
   if (b->idx_ring) cudaFree(b->idx_ring);
   for (int k = 0; k < 2; ++k)

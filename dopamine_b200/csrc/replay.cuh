@@ -81,6 +81,31 @@ struct PreSync {
   unsigned int *ticket;  // CTAs finished in the running first-half launch
 };
 
+// The agent's batch (at most 32 rows, no gradient): the loss tail stages what the first
+// half left for it — the greedy action's probabilities and the online log-probabilities
+// of EVERY action — while the sampler is still running, so that only the sampled scalars
+// are fetched behind the sampler (c51.cu: c51_post_tree_kernel).  The tail is resident
+// long before the first half of its step has ended and the scratch is rewritten every
+// step, so it waits for a launch NUMBER, as the early write-back does (TreeGo): every
+// staged first half counts itself in `done` when its last CTA leaves; every CTA of a
+// staged tail takes a ticket before it lets its dependents start, so ticket / CTAs is
+// the launch's number k (launches never interleave their tickets), and the CTA stages
+// once done >= k + 1.  (The first halves of consecutive steps run on one stream, so they
+// complete in order; with the trainer's direct I/O the next one may have completed too.)
+// Staged first halves and staged tails are launched in pairs by the same host call.
+// The scratch is two halves by step parity: the first half of step n + 1 writes the other
+// half, and that of step n + 2 is ordered behind the tail of step n (stream order, or
+// DirectIO::first_half_after) — no first half overwrites rows a tail may still read.
+struct StageGate {
+  unsigned int *done = nullptr;           // staged first halves completed (monotone)
+  unsigned long long *tickets = nullptr;  // CTAs of staged tails started (monotone)
+  float *logp = nullptr;  // [rows][c51_logp_stride] log-probabilities, action-major
+};
+// Row stride of StageGate::logp: whole 16-byte words, so a row moves as float4s.
+__host__ __device__ __forceinline__ int c51_logp_stride(int actions, int atoms) {
+  return (actions * atoms + 3) & ~3;
+}
+
 // Row-by-row hand-over from the sampling kernel to the kernels that consume its rows in
 // the same step (the frame copies; see per_sample_warp_kernel and
 // gather_stack4_u8_kernel).  Those kernels are programmatic dependents of the sampler:
@@ -123,15 +148,30 @@ __device__ __forceinline__ uint32_t ld_acquire_u32(const unsigned int *p) {
   asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
 }
-// Last statement of a first-half CTA (every thread calls it).
-__device__ __forceinline__ void pre_sync_signal(const PreSync &p) {
+// Last statement of a first-half CTA (every thread calls it).  staged_done (nullable):
+// StageGate::done of a staged first half.
+__device__ __forceinline__ void pre_sync_signal(const PreSync &p,
+                                                unsigned int *staged_done = nullptr) {
   __threadfence();
   __syncthreads();
   if (threadIdx.x == 0 && atomicAdd(p.ticket, 1u) == gridDim.x - 1) {
     *p.ticket = 0u;  // ready for the next launch
     __threadfence();
+    if (staged_done != nullptr) st_release_u32(staged_done, *staged_done + 1u);
     st_release_u32(p.done, *p.done + 1u);
   }
+}
+// By thread 0 of every CTA of a staged tail, BEFORE the CTA lets its dependents start:
+// takes the ticket and waits for the first half of this launch's step (StageGate).  False
+// after 2 s (a first half that never ran must not hang the GPU): the caller then stages
+// behind its griddepcontrol.wait, when the sampler's own wait for the first half is over.
+__device__ __forceinline__ bool stage_gate_wait(const StageGate &g) {
+  const unsigned long long ticket = atomicAdd(g.tickets, 1ull);
+  const unsigned int launch = (unsigned int)(ticket / gridDim.x) + 1u;
+  const long long t0 = clock64();
+  while ((int)(ld_acquire_u32(g.done) - launch) < 0)
+    if (clock64() - t0 > 4000000000ll) return false;
+  return true;
 }
 // Called by the sampler's closing thread (ONE thread) before the kernel ends.  Gives up
 // after 2 s: a first half that never ran must not hang the GPU (the tail then reads stale
@@ -324,7 +364,10 @@ struct b2r_buffer {
   float *c51_bestp = nullptr;  // device [2 halves][c51_bestp_rows][64 probabilities | 64 stats]
   int64_t c51_bestp_rows = 0;
   int c51_half = 0;            // half the next step's first half writes
-  unsigned int *pre_sync = nullptr;  // device [4]: PreSync done, seen, ticket
+  unsigned int *pre_sync = nullptr;  // device [8]: PreSync done, seen, ticket, tree_done,
+                                     // StageGate done, -, tickets (64 bits)
+  float *c51_logp = nullptr;         // device [2 halves][c51_logp_half]: StageGate::logp
+  int64_t c51_logp_half = 0;
   // Deferred frame copies (b2r_set_deferred_frames): the copies of a fused step are not
   // joined into the caller's stream when the call returns but when b2r_join_frames is
   // called (or staged adds are flushed: they overwrite ring slots the copies may still

@@ -143,6 +143,11 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   PreSync pre_sync = {nullptr, nullptr, nullptr};
   int have_stats = 0;
   float *scratch = nullptr;
+  // The agent's batch: the tail stages the first half's rows ahead of the sampler's end
+  // (StageGate, replay.cuh; the tail and the write-back are then one cluster, below).
+  const bool staged = split_loss && !shard && c51_post_takes_tree(&loss, b->tree) &&
+                      c51_tail_can_stage(&loss);
+  StageGate stage;
   if (split_loss) {
     // (two halves of scratch: with direct I/O the first half of step n + 1 is not
     // ordered behind the tail of step n, which may still be reading its rows)
@@ -162,6 +167,25 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
     }
     scratch = b->c51_bestp + (size_t)(b->c51_half & 1) * (size_t)b->c51_bestp_rows *
                                  c51_scratch_floats_per_row();
+    if (staged) {
+      const int64_t half =
+          (int64_t)rows_cap * c51_logp_stride(loss.num_actions, loss.num_atoms);
+      if (b->c51_logp_half < half) {
+        if (b->c51_logp) {
+          B2R_CUDA(cudaStreamSynchronize(b->side3));
+          B2R_CUDA(cudaStreamSynchronize(s));
+          cudaFree(b->c51_logp);
+        }
+        b->c51_logp = nullptr;
+        b->c51_logp_half = 0;
+        B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->c51_logp),
+                            2 * (size_t)half * sizeof(float)));
+        b->c51_logp_half = half;
+      }
+      stage.done = b->pre_sync + 4;
+      stage.tickets = reinterpret_cast<unsigned long long *>(b->pre_sync + 6);
+      stage.logp = b->c51_logp + (size_t)(b->c51_half & 1) * (size_t)b->c51_logp_half;
+    }
     b->c51_half ^= 1;
     pre_sync.done = b->pre_sync;
     pre_sync.seen = b->pre_sync + 1;
@@ -173,12 +197,14 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
         B2R_CUDA(cudaStreamWaitEvent(b->side3, direct->first_half_after, 0));
       if (wait_before_loss) B2R_CUDA(cudaStreamWaitEvent(b->side3, wait_before_loss, 0));
       B2R_TRY(c51_pre_launch(&loss, rows_cap, scratch, pre_sync, b->side3, &have_stats,
-                             direct->online_src, direct->online_copy));
+                             direct->online_src, direct->online_copy,
+                             staged ? &stage : nullptr));
     } else {
       B2R_CUDA(cudaEventRecord(b->ev_c51_fork, s));
       B2R_CUDA(cudaStreamWaitEvent(b->side3, b->ev_c51_fork, 0));
       if (wait_before_loss) B2R_CUDA(cudaStreamWaitEvent(b->side3, wait_before_loss, 0));
-      B2R_TRY(c51_pre_launch(&loss, rows_cap, scratch, pre_sync, b->side3, &have_stats));
+      B2R_TRY(c51_pre_launch(&loss, rows_cap, scratch, pre_sync, b->side3, &have_stats,
+                             nullptr, nullptr, staged ? &stage : nullptr));
       B2R_CUDA(cudaEventRecord(b->ev_c51_pre, b->side3));
     }
   }
@@ -325,7 +351,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
                             tail_writeback || tail_counted ? b->tree : nullptr,
                             out->indices, tree_done, tail_counted ? early : nullptr,
                             direct ? direct->loss_host : nullptr,
-                            early_tree ? &tree_go : nullptr));
+                            early_tree ? &tree_go : nullptr, staged ? &stage : nullptr));
   else if (tail_writeback)
     B2R_TRY(c51_loss_launch(&loss, s, b->tree, out->indices));
   else if (!(debug_skip() & 1))

@@ -628,13 +628,18 @@ int c51_loss_launch(const b2r_c51_args *args, cudaStream_t stream, b2r_tree *tre
 // alone, over `rows` rows, into scratch ([rows][c51_scratch_floats_per_row()] floats),
 // signalling `sync` when done ...
 struct PreSync;
+struct StageGate;
 bool c51_can_split(const b2r_c51_args *args);
 int c51_scratch_floats_per_row();
+// Can the tail of this batch stage its inputs ahead of the sampler's end (StageGate)?
+// (Also needs the tail and the write-back as one cluster: c51_post_takes_tree.)
+bool c51_tail_can_stage(const b2r_c51_args *args);
 // online_src / online_copy (nullable): read the online logits from there (the caller's
 // page-locked host memory) and leave a device copy for the tail.
+// stage (nullable): also leave every action's log-probabilities for a staged tail.
 int c51_pre_launch(const b2r_c51_args *args, int rows, float *scratch, const PreSync &sync,
                    cudaStream_t stream, int *have_stats, const float *online_src = nullptr,
-                   float *online_copy = nullptr);
+                   float *online_copy = nullptr, const StageGate *stage = nullptr);
 // ... and the tail over the sampled rows.  err (nullable): asynchronous error latch.
 // tree != nullptr (c51_post_takes_tree: batches of at most 32 rows): the tail and
 // set_priority(indices, priorities) as one thread-block cluster.
@@ -648,6 +653,6 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
                     b2r_tree *tree = nullptr, const int32_t *indices = nullptr,
                     unsigned int *tree_done = nullptr,
                     const b2r_exchange *publish = nullptr, float *loss_host = nullptr,
-                    const TreeGo *go = nullptr);
+                    const TreeGo *go = nullptr, const StageGate *stage = nullptr);
 
 }  // namespace b2r

@@ -20,7 +20,8 @@ NAMES = {
     'gather': {0: 'G start (CTA 0)', 1: 'G acquired', 5: 'G CTA 0 stored', 6: 'G END'},
     'c51': {0: 'L-pre start', 1: 'L-pre acquired', 3: 'L softmaxes', 5: 'L projection',
             8: 'L-pre END', 10: 'L-tail start', 11: 'L-tail acquired', 12: 'L-tail loss END',
-            9: 'L-tail tree END', 13: 'L-tail row scalars in', 14: 'L-tail log-softmax done'},
+            9: 'L-tail tree END', 13: 'L-tail row scalars in', 14: 'L-tail log-softmax done',
+            15: 'L-tail staged'},
     'tree': {30: 'T tiny start', 7: 'T tiny / one-CTA END',
              0: 'T one-CTA start', 1: 'T one-CTA acquired', 5: 'T one-CTA leaf level done',
              12: 'P presort start',
