@@ -111,11 +111,8 @@ struct LossArgs {
   float *weighted;        // scratch (B,): w_b * loss_b, reduced by the last CTA
   unsigned int *ticket;   // scratch: CTAs finished (self-resetting)
   int warps;              // warps per CTA = min(num_actions, 32)
-  // Priority write-back at the tail of the loss kernel (batches of at most 32 rows:
-  // the fused step at the agent's batch size).  The last CTA to finish its row runs the
-  // match-based tree update over the priorities the grid has just produced — one kernel
-  // boundary less on a chain of three short kernels.
-  int fuse_tree;
+  // c51_post_tree_kernel: the priority write-back that the cluster applies behind the
+  // tail (batches of at most 32 rows: the fused step at the agent's batch size)
   UpdateArgs<int32_t, float> tree;
   int64_t *err;  // nullable: asynchronous error latch (an action outside [0, A))
   int32_t *count_copy;  // nullable: receives the row count (c51_post_kernel)
@@ -234,12 +231,8 @@ constexpr int kMaxAtomsPerLane = 4;  // num_atoms <= 128
 
 // PL = atoms per lane (2 covers C51's 51 atoms; fewer unrolled copies = less
 // straight-line code to fetch on a cold instruction cache).
-// The large-batch instance runs a third of the warps per row (<= 11 warps) and wants
-// many rows resident per SM: bounds that keep it at 32 registers (10 CTAs of 192
-// threads per SM); the small-batch instance runs one warp per action.
-template <int PL, bool FAST>
-__global__ void __launch_bounds__(FAST ? 384 : 1024, FAST ? 5 : 1)
-c51_loss_kernel(LossArgs a) {
+template <int PL>
+__global__ void __launch_bounds__(1024, 1) c51_loss_kernel(LossArgs a) {
   extern __shared__ float smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x;
@@ -322,12 +315,12 @@ c51_loss_kernel(LossArgs a) {
 #pragma unroll
       for (int t = 0; t < PL; ++t)
         if (lane + 32 * t < N) mo = fmaxf(mo, xo[t]);
-      mo = warp_max<FAST>(mo);
+      mo = warp_max(mo);
       float ps = 0.f;
 #pragma unroll
       for (int t = 0; t < PL; ++t)
         if (lane + 32 * t < N) ps = __fadd_rn(ps, expf(__fsub_rn(xo[t], mo)));
-      const float den_o = warp_sum<FAST>(ps);
+      const float den_o = warp_sum(ps);
       const float lse = logf(den_o);
 #pragma unroll
       for (int t = 0; t < PL; ++t) {
@@ -344,7 +337,7 @@ c51_loss_kernel(LossArgs a) {
     float m = -INFINITY;
 #pragma unroll
     for (int t = 0; t < PL; ++t) m = fmaxf(m, xt[t]);
-    m = warp_max<FAST>(m);
+    m = warp_max(m);
     float e[PL];
     float psum = 0.f;
 #pragma unroll
@@ -353,7 +346,7 @@ c51_loss_kernel(LossArgs a) {
       e[t] = ok ? expf(__fsub_rn(xt[t], m)) : 0.f;
       if (ok) psum = __fadd_rn(psum, e[t]);
     }
-    const float denom = warp_sum<FAST>(psum);
+    const float denom = warp_sum(psum);
     float qpart = 0.f;
 #pragma unroll
     for (int t = 0; t < PL; ++t) {
@@ -362,7 +355,7 @@ c51_loss_kernel(LossArgs a) {
         qpart = __fadd_rn(qpart, __fmul_rn(zl[t], e[t]));
       }
     }
-    const float q = warp_sum<FAST>(qpart);
+    const float q = warp_sum(qpart);
     if (best_a < 0 || q > best_q) {  // strict > keeps the first maximum
       best_q = q;
       best_a = act;
@@ -520,9 +513,8 @@ c51_loss_kernel(LossArgs a) {
 
   B2R_MARK(7);
   B2R_MARK_END(8);
-  // ---- the last CTA to finish: mean weighted loss, reduced in a fixed order, and
-  // (fuse_tree) the priority write-back.
-  if (a.u.mean_weighted_loss == nullptr && !a.fuse_tree) return;
+  // ---- the last CTA to finish: mean weighted loss, reduced in a fixed order
+  if (a.u.mean_weighted_loss == nullptr) return;
   __threadfence();
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -533,11 +525,6 @@ c51_loss_kernel(LossArgs a) {
   __syncthreads();
   if (!s_last) return;
   __threadfence();
-  if (a.fuse_tree) {
-    tree_update_tiny_body<false>(a.tree);
-    B2R_MARK_END(9);
-  }
-  if (a.u.mean_weighted_loss == nullptr) return;
   mean_of_weighted(a.weighted, sharded ? rows : a.u.batch,
                    (float)(sharded ? a.sh.global_batch : a.u.batch), s_red,
                    a.u.mean_weighted_loss);
@@ -1606,32 +1593,13 @@ int b2r_c51_project(int32_t batch, int32_t num_atoms, const float *supports,
 }  // extern "C"
 
 namespace b2r {
-
-// Can the write-back of this batch ride at the tail of its loss kernel?
-bool c51_can_fuse_writeback(const b2r_c51_args *args, const b2r_tree *tree) {
-  // Off unless B2R_FUSE_WRITEBACK=1: measured on one B200 in one process
-  // (profiles/r2/README.md), the fence + ticket by which the last CTA finds out that it
-  // is the last costs what the kernel boundary it replaces costs (17.4 vs 17.2 us per
-  // step at batch 32).
-  static const bool on = [] {
-    const char *e = std::getenv("B2R_FUSE_WRITEBACK");
-    return e != nullptr && std::atoi(e) != 0;
-  }();
-  return on && tree != nullptr && args->batch <= kTinyBatch && args->batch_count == nullptr &&
-         tree_tiny_enabled() && tree->depth + 1 <= 32 && args->num_atoms <= 64;
-}
-
-int c51_loss_launch(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
-                    const int32_t *indices);
-int launch_loss(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
-                const int32_t *indices, const ShardedLoss &sh);
-
+int launch_loss(const b2r_c51_args *args, cudaStream_t s, const ShardedLoss &sh);
 }  // namespace b2r
 
 extern "C" {
 
 int b2r_c51_loss(const b2r_c51_args *args, b2r_stream stream) {
-  return b2r::c51_loss_launch(args, as_stream(stream), nullptr, nullptr);
+  return b2r::launch_loss(args, as_stream(stream), b2r::ShardedLoss());
 }
 
 int b2r_c51_loss_sharded(const b2r_c51_args *args, b2r_exchange *exchange,
@@ -1654,7 +1622,7 @@ int b2r_c51_loss_sharded(const b2r_c51_args *args, b2r_exchange *exchange,
   sh.seq = exchange->seq;
   sh.timeout_ns = exchange->timeout_ns;
   sh.latched = exchange->latched;
-  return b2r::launch_loss(args, as_stream(stream), nullptr, nullptr, sh);
+  return b2r::launch_loss(args, as_stream(stream), sh);
 }
 
 }  // extern "C"
@@ -1678,21 +1646,14 @@ static int ensure_loss_scratch(int batch) {
 }
 
 // ---- the loss in two halves (see c51_pre_kernel) ----
+// Largest batch that splits.  Measured per step, one kernel against two halves
+// (profiles/r2/README.md): 16.8 / 16.0 us at batch 32, 27.9 / 25.7 at 256, 39.5 / 37.1 at
+// 1024 (deferred copies), but 111 / 119 at 4096, where the first half's 1024 CTAs take
+// issue slots from the sampler that everything else waits for.
+constexpr int kC51SplitMax = 2048;
+
 bool c51_can_split(const b2r_c51_args *args) {
-  // B2R_C51_SPLIT=0 keeps the one-kernel loss in the fused step (comparison runs);
-  // B2R_C51_SPLIT_MAX: largest batch that splits.  Measured per step, one kernel against
-  // two halves (profiles/r2/README.md): 16.8 / 16.0 us at batch 32, 27.9 / 25.7 at 256,
-  // 39.5 / 37.1 at 1024 (deferred copies), but 111 / 119 at 4096, where the first half's
-  // 1024 CTAs take issue slots from the sampler that everything else waits for.
-  static const bool on = [] {
-    const char *e = std::getenv("B2R_C51_SPLIT");
-    return e == nullptr || std::atoi(e) != 0;
-  }();
-  static const int split_max = [] {
-    const char *e = std::getenv("B2R_C51_SPLIT_MAX");
-    return e ? std::atoi(e) : 2048;
-  }();
-  return on && args->batch <= split_max && args->num_atoms >= 2 &&
+  return args->batch <= kC51SplitMax && args->num_atoms >= 2 &&
          args->num_atoms <= kRowAtoms && args->num_actions > 0;
 }
 
@@ -1750,16 +1711,11 @@ int c51_pre_launch(const b2r_c51_args *args, int rows, float *scratch, const Pre
 // device-side count is expected to be about that many.
 bool c51_post_takes_tree(const b2r_c51_args *args, const b2r_tree *tree,
                          int64_t expected_rows) {
-  // B2R_POST_TREE=0: tail and write-back as two kernels (comparison runs)
-  static const bool on = [] {
-    const char *e = std::getenv("B2R_POST_TREE");
-    return e == nullptr || std::atoi(e) != 0;
-  }();
   const bool counted = args->batch_count != nullptr;
   const bool small = counted ? (expected_rows >= 0 && expected_rows <= kTinyBatch &&
                                 args->batch <= 256 && args->mean_weighted_loss == nullptr)
                              : args->batch <= kTinyBatch;
-  return on && tree != nullptr && small && tree_tiny_enabled() && tree->depth + 1 <= 32 &&
+  return tree != nullptr && small && tree->depth + 1 <= 32 &&
          (args->sampling_probabilities == nullptr || args->min_probability != nullptr);
 }
 
@@ -1778,7 +1734,6 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
     return fail(B2R_ERR_INVALID_ARGUMENT, "a required C51 pointer is NULL");
   LossArgs a;
   a.u = *args;
-  a.fuse_tree = 0;
   a.err = err;
   a.count_copy = count_copy;
   a.tree_done = nullptr;
@@ -1798,7 +1753,6 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
     if (args->batch_count != nullptr && tree_done == nullptr)
       return fail(B2R_ERR_INVALID_ARGUMENT, "a counted batch needs the tree_done flag");
     set_tree_window(tree->heap, (size_t)tree->leaves * 16);
-    a.fuse_tree = 1;
     a.tree_done = tree_done;
     a.tree.heap = tree->heap;
     a.tree.depth = tree->depth;
@@ -1840,14 +1794,13 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
   return B2R_OK;
 }
 
-// tree != nullptr (c51_can_fuse_writeback): also set_priority(indices, priorities).
-int c51_loss_launch(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
-                    const int32_t *indices) {
-  return launch_loss(args, s, tree, indices, ShardedLoss());
-}
+// From 128 rows up: one warp per row (c51_loss_rows_kernel).  Measured with 10 launches
+// per graph (profiles/r1/README.md): at batch 32 the CTA-per-row kernel and a rows
+// kernel tie (5.95 us), at 256 the rows kernel wins once the logits no longer sit in L2
+// (10.2 -> 7.0 us).
+constexpr int kC51RowsMin = 128;
 
-int launch_loss(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
-                const int32_t *indices, const ShardedLoss &sh) {
+int launch_loss(const b2r_c51_args *args, cudaStream_t s, const ShardedLoss &sh) {
   if (!args || args->batch <= 0 || args->num_atoms < 2 || args->num_actions <= 0)
     return fail(B2R_ERR_INVALID_ARGUMENT, "bad C51 shape");
   if (args->batch_count && args->mean_weighted_loss && sh.global_batch == 0)
@@ -1860,87 +1813,37 @@ int launch_loss(const b2r_c51_args *args, cudaStream_t s, b2r_tree *tree,
   b2r::LossArgs a;
   a.u = *args;
   a.sh = sh;
-  a.fuse_tree = 0;
   a.err = nullptr;
   a.count_copy = nullptr;
   a.tree_done = nullptr;
   a.loss_host = nullptr;
-  if (tree != nullptr) {
-    if (!c51_can_fuse_writeback(args, tree))
-      return fail(B2R_ERR_INVALID_ARGUMENT, "this batch cannot fuse its write-back");
-    set_tree_window(tree->heap, (size_t)tree->leaves * 16);
-    a.fuse_tree = 1;
-    a.tree.heap = tree->heap;
-    a.tree.depth = tree->depth;
-    a.tree.leaves = tree->leaves;
-    a.tree.n = args->batch;
-    a.tree.padded = 32;
-    a.tree.indices = indices;
-    a.tree.values = args->priorities;
-    a.tree.mode = nullptr;
-    a.tree.k_base = 0;
-    a.tree.delta = tree->delta;
-    a.tree.max_rec = tree->max_rec;
-    a.tree.status = tree->status;
-    a.tree.n_dev = nullptr;
-  }
   // Small batches are latency-bound: one warp per action.  Large batches are
   // throughput-bound: a third of that, so more rows are resident per SM.
   a.warps = args->num_actions < 32 ? args->num_actions : 32;
   if (args->batch > 256) a.warps = (a.warps + 2) / 3;
-  int threads = a.warps * 32;
-  if (a.fuse_tree && threads < 32 * (tree->depth + 1)) threads = 32 * (tree->depth + 1);
+  const int threads = a.warps * 32;
   const size_t smem = ((size_t)a.warps + 5) * args->num_atoms * sizeof(float);
   if (smem > 48 * 1024 || args->num_atoms > 32 * b2r::kMaxAtomsPerLane)
     return fail(B2R_ERR_UNSUPPORTED, "num_atoms above 128 is not supported");
   B2R_TRY(ensure_loss_scratch(args->batch));
   a.weighted = b2r::g_weighted;
   a.ticket = b2r::g_ticket;
-  // From 128 rows up: one warp per row (B2R_C51_ROWS_MIN overrides the threshold,
-  // B2R_C51_GROUP = 4 | 16 picks another lanes-per-action instance).  Measured with
-  // 10 launches per graph (profiles/r1/README.md): at batch 32 the CTA-per-row kernel
-  // and the G = 4 instance tie (5.95 us), at 256 the rows kernel wins once the logits
-  // no longer sit in L2 (10.2 -> 7.0 us).
-  static const int rows_min = [] {
-    const char *e = std::getenv("B2R_C51_ROWS_MIN");
-    return e ? std::atoi(e) : 128;
-  }();
-  static const int rows_group = [] {
-    const char *e = std::getenv("B2R_C51_GROUP");
-    return e ? std::atoi(e) : 8;
-  }();
-  if (args->batch >= rows_min && args->num_atoms <= b2r::kRowAtoms) {
+  if (args->batch >= kC51RowsMin && args->num_atoms <= b2r::kRowAtoms) {
     const int blocks = (args->batch + b2r::kRowWarps - 1) / b2r::kRowWarps;
     const dim3 grid(blocks), block(b2r::kRowWarps * 32);
-    if (rows_group == 16)
-      B2R_CUDA(b2r::launch(b2r::c51_loss_rows_kernel<16, 0>, grid, block, 0, s, a));
-    else if (rows_group == 4 && args->num_atoms == 51)
-      B2R_CUDA(b2r::launch(b2r::c51_loss_rows_kernel<4, 51>, grid, block, 0, s, a));
-    else if (args->num_atoms == 51)
+    if (args->num_atoms == 51)
       B2R_CUDA(b2r::launch(b2r::c51_loss_rows_kernel<8, 51>, grid, block, 0, s, a));
     else
       B2R_CUDA(b2r::launch(b2r::c51_loss_rows_kernel<8, 0>, grid, block, 0, s, a));
     B2R_LAUNCHED();
     return B2R_OK;
   }
-  static const int force_fast = [] {
-    const char *e = std::getenv("B2R_C51_FAST");
-    return e ? std::atoi(e) : -1;
-  }();
-  // (the unrolled instance is compiled for at most 384 threads per CTA)
-  const bool fast = (force_fast >= 0 ? force_fast != 0 : args->batch > 256) &&
-                    threads <= 384;
-  if (args->num_atoms <= 64) {
-    if (fast)
-      B2R_CUDA(b2r::launch(b2r::c51_loss_kernel<2, true>, dim3(args->batch),
-                           dim3(threads), smem, s, a));
-    else
-      B2R_CUDA(b2r::launch(b2r::c51_loss_kernel<2, false>, dim3(args->batch),
-                           dim3(threads), smem, s, a));
-  } else {
-    B2R_CUDA(b2r::launch(b2r::c51_loss_kernel<4, false>, dim3(args->batch),
-                         dim3(threads), smem, s, a));
-  }
+  if (args->num_atoms <= 64)
+    B2R_CUDA(b2r::launch(b2r::c51_loss_kernel<2>, dim3(args->batch), dim3(threads), smem,
+                         s, a));
+  else
+    B2R_CUDA(b2r::launch(b2r::c51_loss_kernel<4>, dim3(args->batch), dim3(threads), smem,
+                         s, a));
   B2R_LAUNCHED();
   return B2R_OK;
 }

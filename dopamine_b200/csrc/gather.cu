@@ -39,8 +39,6 @@ struct GatherArgs {
   int32_t scalar_rows;   // grid rows of appended scalar CTAs (0: frames only)
   ScalarArgs sc;
   const int32_t *count;  // nullable: device-side number of rows (<= batch)
-  RowFlags flags;        // desc == nullptr: wait for the preceding kernel as a whole
-  int64_t *latched;      // nullable: asynchronous error latch (hand-over time-out)
 };
 
 // [a0 a1 a2 a3] x4 frames -> 4 words [a_p b_p c_p d_p], p = 0..3.
@@ -84,43 +82,21 @@ template <bool SCALARS>
 __global__ void __launch_bounds__(128, 12) gather_stack4_u8_kernel(const __grid_constant__ GatherArgs a) {
   B2R_MARK(0);
   pdl_release();
-  int64_t i;
-  int length;
   const int b = blockIdx.y;
-  if (!SCALARS && a.flags.desc != nullptr) {
-    // Row hand-over (RowFlags): this grid is a programmatic dependent of the sampler and
-    // was started while the sampler runs; a CTA goes as soon as ITS row's descriptor —
-    // index and trajectory length in one word — is there.
-    __shared__ uint64_t s_desc;
-    if (threadIdx.x == 0) {
-      bool timed_out;
-      s_desc = row_flags_wait(a.flags, b, &timed_out);
-      if (timed_out && a.latched != nullptr && a.latched[0] == 0)
-        a.latched[0] = B2R_ERR_CUDA;
-    }
-    __syncthreads();
-    const uint64_t d = s_desc;
-    if (d == 0ull) return;
-    i = (int64_t)(uint32_t)d;
-    length = (int)((d >> 32) & 0xff);
-    B2R_MARK(1);
-    B2R_MARK(2);
-  } else {
-    pdl_acquire();
-    B2R_MARK(1);
-    const int rows = a.count ? min(*a.count, a.batch) : a.batch;
-    if (SCALARS && blockIdx.y >= a.batch) {  // appended scalar CTAs: one thread per transition
-      const int r = ((blockIdx.y - a.batch) * gridDim.x + blockIdx.x) * blockDim.x +
-                    threadIdx.x;
-      if (r < rows) write_scalars(a.sc, r, a.indices[r]);
-      return;
-    }
-    if (b >= rows) return;
-    i = a.indices[b];
-    bool ends;
-    length = trajectory_length(a.term_flag, i, a.horizon, a.capacity, &ends);
-    B2R_MARK(2);
+  pdl_acquire();
+  B2R_MARK(1);
+  const int rows = a.count ? min(*a.count, a.batch) : a.batch;
+  if (SCALARS && blockIdx.y >= a.batch) {  // appended scalar CTAs: one thread per transition
+    const int r = ((blockIdx.y - a.batch) * gridDim.x + blockIdx.x) * blockDim.x +
+                  threadIdx.x;
+    if (r < rows) write_scalars(a.sc, r, a.indices[r]);
+    return;
   }
+  if (b >= rows) return;
+  const int64_t i = a.indices[b];
+  bool ends;
+  const int length = trajectory_length(a.term_flag, i, a.horizon, a.capacity, &ends);
+  B2R_MARK(2);
 
   const int chunks = (int)(a.obs_bytes >> 4);
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -330,16 +306,6 @@ int gather_variant(int batch) {
   return 1;
 }
 
-// Will launch_gather(frames_only) run the kernel that understands RowFlags?
-bool gather_takes_row_flags(const b2r_buffer *b) {
-  static const bool reg_forced = [] {
-    const char *e = std::getenv("B2R_GATHER");
-    return e != nullptr && std::strcmp(e, "reg") == 0;
-  }();
-  return b->cfg.stack_size == 4 && b->cfg.obs_itemsize == 1 &&
-         (b->cfg.obs_bytes & 15) == 0 && reg_forced;
-}
-
 void fill_scalar_args(const b2r_buffer *b, const b2r_batch *out, ScalarArgs *sc) {
   sc->capacity = b->cfg.capacity;
   sc->horizon = b->cfg.update_horizon;
@@ -382,12 +348,9 @@ void fill_scalar_args(const b2r_buffer *b, const b2r_batch *out, ScalarArgs *sc)
 
 int launch_gather(b2r_buffer *b, int32_t batch, const int32_t *indices_dev,
                   const b2r_batch *out, cudaStream_t stream,
-                  const int32_t *count_dev, bool frames_only, const RowFlags *flags) {
+                  const int32_t *count_dev, bool frames_only) {
   GatherArgs a;
   a.count = count_dev;
-  a.flags.desc = nullptr;
-  a.flags.tag_word = a.flags.final_word = nullptr;
-  a.latched = b->status;
   a.capacity = b->cfg.capacity;
   a.stack = b->cfg.stack_size;
   a.horizon = b->cfg.update_horizon;
@@ -428,21 +391,15 @@ int launch_gather(b2r_buffer *b, int32_t batch, const int32_t *indices_dev,
     // + rows of scalar CTAs (one thread per transition)
     a.scalar_rows = frames_only ? 0 : (batch + nx * 128 - 1) / (nx * 128);
     dim3 grid(nx, batch + a.scalar_rows);
-    if (frames_only && flags != nullptr && count_dev == nullptr) a.flags = *flags;
     if (frames_only) {  // beside the chain: lowest priority
       // While the copies are short next to the chain (up to ~1.5k rows) each copy CTA
       // claims 56 KB of shared memory it does not use: at most 4 of them then share an
       // SM, which leaves the chain's CTAs their occupancy (65 -> 58 us per step at
       // batch 1024).  Beyond that the copies themselves bound the step and run
-      // unrestricted (capping costs 146 -> 162 us at 4096).  B2R_GATHER_PAD_KB
-      // overrides.
-      static const int pad_env = [] {
-        const char *e = std::getenv("B2R_GATHER_PAD_KB");
-        return e ? std::atoi(e) : -1;
-      }();
-      const int pad_kb = pad_env >= 0 ? pad_env : (batch > 64 && batch <= 1536 ? 56 : 0);
+      // unrestricted (capping costs 146 -> 162 us at 4096).
+      const int pad_kb = batch > 64 && batch <= 1536 ? 56 : 0;
       static bool pad_ready = false;
-      if (pad_kb > 48 && !pad_ready) {
+      if (pad_kb > 0 && !pad_ready) {
         B2R_CUDA(cudaFuncSetAttribute(gather_stack4_u8_kernel<false>,
                                       cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       pad_kb * 1024));

@@ -149,7 +149,7 @@ int flush_queue(b2r_buffer *b, cudaStream_t stream, bool split,
   // per update): ONE launch that reads the staging buffer straight from pinned host
   // memory — tree update in CTA 0, row writes in the others (tree.cu).
   if (b->tree != nullptr && !split && s->host_dev != nullptr &&
-      b->q_entries <= kFusedFlushMax && std::getenv("B2R_NO_FUSED_FLUSH") == nullptr) {
+      b->q_entries <= kFusedFlushMax) {
     Header hh = header_of(s->host_dev, b->queue_cap);
     AddParams p;
     p.n_entries = b->q_entries;
@@ -265,33 +265,6 @@ int ensure_inv_slots(b2r_buffer *b, int64_t n) {
   b->inv_slots = nullptr;
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->inv_slots), (size_t)n * 4));
   b->inv_slots_cap = n;
-  return B2R_OK;
-}
-
-int row_flags_for(b2r_buffer *b, int64_t rows, RowFlags *out) {
-  // Off unless B2R_ROW_FLAGS=1: measured (profiles/r2/README.md), starting the copies
-  // row by row gains 0.4-1 us of a 33 us sampler + copies pair at batch 1024 and costs
-  // 2 us at batch 32, where the sampler's first CTA has to hold back its dependents.
-  static const bool on = [] {
-    const char *e = std::getenv("B2R_ROW_FLAGS");
-    return e != nullptr && std::atoi(e) != 0;
-  }();
-  out->desc = nullptr;
-  out->tag_word = out->final_word = nullptr;
-  if (!on) return B2R_OK;
-  if (rows > b->row_flags_cap) {
-    if (b->row_flags) cudaFree(b->row_flags);
-    b->row_flags = nullptr;
-    b->row_flags_cap = 0;
-    int64_t cap = 4096;
-    while (cap < rows) cap *= 2;
-    B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->row_flags), (size_t)(cap + 4) * 8));
-    B2R_CUDA(cudaMemset(b->row_flags, 0, (size_t)(cap + 4) * 8));
-    b->row_flags_cap = cap;
-  }
-  out->tag_word = b->row_flags;
-  out->final_word = b->row_flags + 1;
-  out->desc = reinterpret_cast<uint64_t *>(b->row_flags + 8);
   return B2R_OK;
 }
 
@@ -425,7 +398,6 @@ int b2r_create(const b2r_config *cfg, b2r_buffer **out) {
   {
     int least = 0, greatest = 0;
     cudaDeviceGetStreamPriorityRange(&least, &greatest);
-    B2R_CUDA(cudaStreamCreateWithPriority(&b->side2, cudaStreamNonBlocking, greatest));
     B2R_CUDA(cudaStreamCreateWithPriority(&b->side3, cudaStreamNonBlocking, greatest));
   }
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->pre_sync), 32));
@@ -434,7 +406,6 @@ int b2r_create(const b2r_config *cfg, b2r_buffer **out) {
     B2R_CUDA(cudaEventCreateWithFlags(&b->ev_slot_free[k], cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_c51_fork, cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_c51_pre, cudaEventDisableTiming));
-  B2R_CUDA(cudaEventCreateWithFlags(&b->ev_join2, cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_pre, cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_h2d, cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_rows, cudaEventDisableTiming));
@@ -454,7 +425,6 @@ int b2r_destroy(b2r_buffer *b) {
     if (b->staging[k].dev) cudaFree(b->staging[k].dev);
     if (b->staging[k].done) cudaEventDestroy(b->staging[k].done);
   }
-  if (b->row_flags) cudaFree(b->row_flags);
   if (b->inv_slots) cudaFree(b->inv_slots);
   cudaFree(b->info);
   cudaFree(b->status);
@@ -466,8 +436,6 @@ int b2r_destroy(b2r_buffer *b) {
   if (b->side) cudaStreamDestroy(b->side);
   if (b->ev_fork) cudaEventDestroy(b->ev_fork);
   if (b->ev_join) cudaEventDestroy(b->ev_join);
-  if (b->side2) cudaStreamDestroy(b->side2);
-  if (b->ev_join2) cudaEventDestroy(b->ev_join2);
   if (b->side3) cudaStreamDestroy(b->side3);
   if (b->ev_c51_fork) cudaEventDestroy(b->ev_c51_fork);
   if (b->ev_c51_pre) cudaEventDestroy(b->ev_c51_pre);

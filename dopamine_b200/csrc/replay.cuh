@@ -106,42 +106,9 @@ __host__ __device__ __forceinline__ int c51_logp_stride(int actions, int atoms) 
   return (actions * atoms + 3) & ~3;
 }
 
-// Row-by-row hand-over from the sampling kernel to the kernels that consume its rows in
-// the same step (the frame copies; see per_sample_warp_kernel and
-// gather_stack4_u8_kernel).  Those kernels are programmatic dependents of the sampler:
-// the hardware starts their CTAs once every sampler CTA is running, and instead of
-// waiting for the sampler to END they wait for the row they need.  The sampler leaves
-// one 8-byte descriptor per row, written with a single store:
-//   [63:40] the step's tag (device draw counter + 1, folded to 24 bits, never 0)
-//   [39:32] trajectory length L (circular_replay_buffer.py:517-527)
-//   [31:0]  the sampled index
-// so a consumer that sees the tag has everything it needs to address the frames: no
-// acquire, no second load of the index, no terminal look-up.  The sampler's first CTA
-// publishes the tag in tag_word before it lets the dependents start; final_word == tag
-// says that the sampler is finished (rows that never got a descriptor — a latched
-// failure — are then skipped).
-struct RowFlags {
-  uint64_t *desc;        // [rows]; nullptr: no hand-over (wait for the whole kernel)
-  uint32_t *tag_word;
-  uint32_t *final_word;
-};
-
 #ifdef __CUDACC__
 __device__ __forceinline__ void st_release_u32(uint32_t *p, uint32_t v) {
   asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ void st_release_u64(uint64_t *p, uint64_t v) {
-  asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ uint32_t ld_volatile_u32(const uint32_t *p) {
-  uint32_t v;
-  asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint64_t ld_volatile_u64(const uint64_t *p) {
-  uint64_t v;
-  asm volatile("ld.volatile.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
 }
 __device__ __forceinline__ uint32_t ld_acquire_u32(const unsigned int *p) {
   uint32_t v;
@@ -205,34 +172,6 @@ __device__ __forceinline__ void pre_sync_consume(const PreSync &p, const PreSync
       if (clock64() - t0 > 4000000000ll) break;
   }
   *p.seen = k.seen + 1u;
-}
-// 24-bit form of the step tag, never 0 (a descriptor that was never written is 0)
-__device__ __forceinline__ uint32_t row_tag24(uint32_t tag) { return tag % 0xffffffu + 1u; }
-__device__ __forceinline__ uint64_t row_descriptor(uint32_t tag, int length, int64_t idx) {
-  return ((uint64_t)row_tag24(tag) << 40) | ((uint64_t)(length & 0xff) << 32) |
-         (uint64_t)(uint32_t)idx;
-}
-// Called by ONE thread: the descriptor of row `row` of this step once it is there, 0 if
-// the sampler finished without it (or after 2 s: a hung producer must not hang the GPU;
-// *timed_out says which).
-__device__ __forceinline__ uint64_t row_flags_wait(const RowFlags &f, int row,
-                                                   bool *timed_out) {
-  *timed_out = false;
-  uint64_t d = ld_volatile_u64(f.desc + row);   // (both loads in flight together)
-  const uint32_t tag = ld_volatile_u32(f.tag_word);
-  const long long t0 = clock64();
-  while (true) {
-    if ((uint32_t)(d >> 40) == row_tag24(tag)) return d;
-    if (ld_volatile_u32(f.final_word) == tag) {
-      d = ld_volatile_u64(f.desc + row);
-      return (uint32_t)(d >> 40) == row_tag24(tag) ? d : 0ull;
-    }
-    if (clock64() - t0 > 4000000000ll) {
-      *timed_out = true;
-      return 0ull;
-    }
-    d = ld_volatile_u64(f.desc + row);
-  }
 }
 #endif
 
@@ -352,10 +291,6 @@ struct b2r_buffer {
   // fused step: the frame copies run on `side`, forked/joined with these events
   cudaStream_t side = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  // ... and the write-back's grouping pass (needs the indices only) on `side2`, beside
-  // the loss kernel
-  cudaStream_t side2 = nullptr;
-  cudaEvent_t ev_join2 = nullptr;
   cudaEvent_t ev_pre = nullptr, ev_h2d = nullptr, ev_rows = nullptr;  // split flush
   // ... and the half of the C51 loss that needs the network outputs only on `side3`,
   // beside the sampler (c51.cu: c51_pre_kernel)
@@ -384,8 +319,6 @@ struct b2r_buffer {
   cudaEvent_t ev_slot_free[2] = {nullptr, nullptr};
   bool slot_busy[2] = {false, false};
   float *min_prob = nullptr;    // device: min sampling probability of the last batch
-  uint32_t *row_flags = nullptr;  // device: tag word, final word, desc[row] (RowFlags)
-  int64_t row_flags_cap = 0;
   // Device copy of the validity context (add_count, cursor, invalid_range): the
   // prioritized sampler reads it from here, so a captured CUDA graph stays valid
   // while adds move the cursor.  Refreshed by every flush (the image rides in the
@@ -456,26 +389,19 @@ int launch_uniform_sharded(b2r_buffer *buf, const b2r_exchange *x, int32_t globa
                            cudaStream_t stream);
 void fill_valid_ctx(const b2r_buffer *buf, ValidCtx *ctx);
 int ensure_ctx(b2r_buffer *buf, cudaStream_t stream);
-// tree.cu: largest batch the one-CTA tree kernel takes, and the fused flush launch
-// (priorities of n new rows + their row writes, staging read zero-copy).
-int tree_small_max();
+// tree.cu: the fused flush launch (priorities of n new rows + their row writes, staging
+// read zero-copy).
 int flush_fused(b2r_tree *tree, int n, const int64_t *slots, const double *prio,
                 const uint8_t *mode, const AddParams &rows, int row_blocks_per_entry,
                 cudaStream_t stream, const b2r_exchange *publish = nullptr);
 int ensure_inv_slots(b2r_buffer *buf, int64_t n);
-// Row flags for `rows` rows (RowFlags; all fields nullptr when the hand-over is off:
-// B2R_ROW_FLAGS=0, the thread sampler).
-int row_flags_for(b2r_buffer *buf, int64_t rows, RowFlags *out);
-bool sampler_hands_over_rows(int strata);  // sample.cu: that sampler publishes RowFlags
-bool gather_takes_row_flags(const b2r_buffer *buf);  // gather.cu
 int launch_gather(b2r_buffer *buf, int32_t batch, const int32_t *indices_dev,
                   const b2r_batch *out, cudaStream_t stream,
-                  const int32_t *count_dev = nullptr, bool frames_only = false,
-                  const RowFlags *flags = nullptr);
+                  const int32_t *count_dev = nullptr, bool frames_only = false);
 int launch_sample(b2r_buffer *buf, int32_t batch, bool philox, uint64_t seed,
                   uint64_t offset, const double *strat_dev,
                   const double *retry_dev, int32_t n_retry, int32_t *out_idx_dev,
                   int32_t *info_dev, cudaStream_t stream,
                   const b2r_batch *scalars = nullptr, float *min_prob_out = nullptr,
-                  const RowFlags *flags = nullptr, const PreSync *pre = nullptr);
+                  const PreSync *pre = nullptr);
 }  // namespace b2r

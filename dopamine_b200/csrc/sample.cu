@@ -70,8 +70,6 @@ struct PerSampleArgs {
   // 1.0 / batch as IEEE double division gives it (np.linspace's step), computed on the
   // host: an fp64 division is a ~500-cycle subroutine on the device.
   double step;
-  // Row-by-row hand-over to the step's consumers (warp sampler, Philox draws only).
-  RowFlags flags;
   // Fused step: the first half of the C51 loss runs beside this kernel; the closing
   // thread waits for it before the kernel ends (PreSync; done == nullptr: nothing to wait
   // for).
@@ -678,28 +676,14 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int warps = blockDim.x >> 5;
   B2R_MARK(10);
-  const bool hand_over = a.flags.desc != nullptr && a.counter != nullptr && a.with_scalars &&
-                         a.sc.fast;
-  if (hand_over && blockIdx.x == 0) {
-    // CTA 0 names the step before it lets the dependents start (RowFlags)
-    pdl_acquire();
-    if (threadIdx.x == 0) {
-      st_release_u32(a.flags.tag_word, (uint32_t)(*a.counter + 1));
-      __threadfence();
-    }
-    __syncthreads();
-    pdl_release();
-  } else {
-    pdl_release();
-    pdl_acquire();
-  }
+  pdl_release();
+  pdl_acquire();
   B2R_MARK(11);
   // every load of the prologue is issued before the first one is used; the nodes of
   // the first descent round (levels 1..5 under the root) ride along
   WarpCtx ctx;
   warp_ctx_issue(a.valid_dev, lane, &ctx);
   const uint64_t draws_before = a.counter ? *a.counter : 0ull;
-  const uint32_t row_tag = (uint32_t)(draws_before + 1);
   const bool exchange = a.xchg.local != nullptr && a.num_shards > 1;
   uint64_t xseq = 0;
   if (exchange) xseq = *a.xchg.seq + 1;
@@ -737,7 +721,6 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       if (a.counter) *a.counter = draws_before + 1;
       if (exchange) *a.xchg.seq = xseq;
       if (a.latched && a.latched[0] == 0) a.latched[0] = B2R_ERR_EMPTY_TREE;
-      if (hand_over) st_release_u32(a.flags.final_word, row_tag);
       pre_sync_consume(a.pre);
     }
     if (CLUSTER) cluster_wait();
@@ -903,12 +886,9 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
         else ws.inv_flag[pos] = valid ? 0 : 1;
         if (valid) {
           float p = INFINITY;
-          int length = 0;
-          if (fast_scalars) p = finish_scalars(a.sc, pos, idx, row, &length);
+          if (fast_scalars) p = finish_scalars(a.sc, pos, idx, row);
           else if (a.with_scalars) p = write_scalars(a.sc, pos, idx);
           my_min = fminf(my_min, p);
-          if (hand_over)
-            st_release_u64(a.flags.desc + pos, row_descriptor(row_tag, length, idx));
         }
       } else if (CLUSTER) {
         st_async_u32(&s_cl_spec_idx[pos - n_mine], (uint32_t)(int32_t)idx, &s_arrived, 0);
@@ -971,7 +951,6 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
         if (a.count_out) *a.count_out = n_mine;
         if (want_min) *a.min_prob_out = m;
         if (want_min) publish_local_min(a, exchange, m, xseq);
-        if (hand_over) st_release_u32(a.flags.final_word, row_tag);
         pre_sync_consume(a.pre, peek);
       }
       B2R_MARK_ANY(20);
@@ -1085,16 +1064,13 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       const int idx = n_spec > 0 ? s_spec_idx[r] : ld_scratch<CLUSTER>(ws.spec_idx + r);
       const int slot = ws.inv_list[j];
       a.out_idx[slot] = idx;
-      int length = 0;
       if (fast_scalars) {  // one round trip for every input of the row
         ScalarLoads row;
         load_scalars(a.sc, idx, &row);
-        fix_min = fminf(fix_min, finish_scalars(a.sc, slot, idx, row, &length));
+        fix_min = fminf(fix_min, finish_scalars(a.sc, slot, idx, row));
       } else if (a.with_scalars) {
         fix_min = fminf(fix_min, write_scalars(a.sc, slot, idx));
       }
-      if (hand_over)
-        st_release_u64(a.flags.desc + slot, row_descriptor(row_tag, length, idx));
       if (j == num_invalid - 1) s_draws_used = r + 1;
     }
     if (threadIdx.x == 0 && spec_done == budget) {
@@ -1126,16 +1102,13 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       if (active && valid && ord < num_invalid) {
         const int slot = ws.inv_list[ord];
         a.out_idx[slot] = (int32_t)idx;
-        int length = 0;
         if (fast_scalars) {
           ScalarLoads row;
           load_scalars(a.sc, idx, &row);
-          fix_min = fminf(fix_min, finish_scalars(a.sc, slot, idx, row, &length));
+          fix_min = fminf(fix_min, finish_scalars(a.sc, slot, idx, row));
         } else if (a.with_scalars) {
           fix_min = fminf(fix_min, write_scalars(a.sc, slot, idx));
         }
-        if (hand_over)
-          st_release_u64(a.flags.desc + slot, row_descriptor(row_tag, length, idx));
         if (ord == num_invalid - 1) s_draws_used = r + 1;
       }
       if (active && r == budget - 1) {
@@ -1168,18 +1141,13 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
           a.out_idx[next_slot] = s_last_idx;
           if (a.with_scalars && s_last_idx >= 0 && s_last_idx < ctx.capacity) {
             // (the reference hands this invalid index on: so do the consumers' rows)
-            int length = 0;
             if (fast_scalars) {
               ScalarLoads row;
               load_scalars(a.sc, s_last_idx, &row);
-              fix_min = fminf(fix_min,
-                              finish_scalars(a.sc, next_slot, s_last_idx, row, &length));
+              fix_min = fminf(fix_min, finish_scalars(a.sc, next_slot, s_last_idx, row));
             } else {
               fix_min = fminf(fix_min, write_scalars(a.sc, next_slot, s_last_idx));
             }
-            if (hand_over)
-              st_release_u64(a.flags.desc + next_slot,
-                             row_descriptor(row_tag, length, s_last_idx));
           }
           if (num_invalid > found + 1) {
             status = B2R_ERR_SAMPLE_ATTEMPTS;
@@ -1212,7 +1180,6 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       publish_local_min(a, exchange, m, xseq);
     }
   }
-  if (hand_over && threadIdx.x == 0) st_release_u32(a.flags.final_word, row_tag);
   if (threadIdx.x == 0) pre_sync_consume(a.pre);
   B2R_MARK_ANY(20);
 }
@@ -1330,45 +1297,21 @@ static void sample_shape(int batch, int *threads, int *tiles) {
   }
 }
 
-// 1 (default): a warp per stratum (per_sample_warp_kernel); 0: a thread per stratum
-// over shared-memory-staged top levels (per_sample_kernel; B2R_SAMPLER=thread).
-// Caller-supplied queries of a SHARDED batch always take the thread kernel: their
-// owners need not be monotone in the stratum index, so the rank's rows are compacted
-// by one CTA.
-static int sampler_variant() {
-  static const int v = [] {
-    const char *e = std::getenv("B2R_SAMPLER");
-    return e != nullptr && std::strcmp(e, "thread") == 0 ? 0 : 1;
-  }();
-  return v;
-}
-
-// Largest number of strata the warp sampler takes.  Every instruction of it serves ONE
-// stratum, so from a few thousand strata on it is bound by instruction issue (4096
-// warps x ~2 k instructions = 14 k cycles on 592 schedulers) and the thread-per-stratum
-// kernel, 32 strata per instruction, is the faster one again: measured in the fused
-// step at 4096, 116 us against 109 us (profiles/r2/README.md).  B2R_SAMPLER_WARP_MAX
-// overrides.
-static int sampler_warp_max() {
-  static const int v = [] {
-    const char *e = std::getenv("B2R_SAMPLER_WARP_MAX");
-    return e ? std::atoi(e) : 2048;
-  }();
-  return v;
-}
-
-bool sampler_hands_over_rows(int strata) {
-  return sampler_variant() == 1 && strata <= sampler_warp_max();
-}
+// Largest number of strata the warp sampler (per_sample_warp_kernel) takes; above, a
+// thread per stratum over shared-memory-staged top levels (per_sample_kernel).  Every
+// instruction of the warp sampler serves ONE stratum, so from a few thousand strata on it
+// is bound by instruction issue (4096 warps x ~2 k instructions = 14 k cycles on 592
+// schedulers) and the thread-per-stratum kernel, 32 strata per instruction, is the faster
+// one again: measured in the fused step at 4096, 116 us against 109 us
+// (profiles/r2/README.md).  Caller-supplied queries of a SHARDED batch always take the
+// thread kernel: their owners need not be monotone in the stratum index, so the rank's
+// rows are compacted by one CTA.
+constexpr int kSamplerWarpMax = 2048;
 
 // Grid and scratch of the warp sampler for `strata` expected strata and outputs of
 // `cap` rows.
 static int warp_sampler_setup(b2r_buffer *b, int strata, int cap, WarpScratch *ws,
                               int *threads, int *ctas) {
-  static const bool use_cluster = [] {
-    const char *e = std::getenv("B2R_SAMPLER_CLUSTER");
-    return e == nullptr || std::atoi(e) != 0;
-  }();
   int warps = strata <= 64 ? 4 : 8;
   // replacement draws evaluated up front: a pick is invalid with probability ~0.3 % in
   // an Atari-like memory (a terminal among the three frames before it)
@@ -1376,7 +1319,7 @@ static int warp_sampler_setup(b2r_buffer *b, int strata, int cap, WarpScratch *w
   if (spec < 4) spec = 4;
   if (spec > kSpecMax) spec = kSpecMax;
   ws->cluster = 0;
-  if (use_cluster && strata + 4 <= 64 && cap <= kClusterCap) {
+  if (strata + 4 <= 64 && cap <= kClusterCap) {
     // one cluster of 8 CTAs; the warps left over after the strata draw replacements
     ws->cluster = 1;
     *ctas = 8;
@@ -1401,18 +1344,15 @@ static int warp_sampler_setup(b2r_buffer *b, int strata, int cap, WarpScratch *w
 
 // Two register budgets: 126 registers (no spills, 16 warps per SM) while every warp of
 // the launch is resident anyway; 64 registers (a few spills outside the descent, 32 warps
-// per SM) for the batches that would otherwise need a second wave.
-// B2R_SAMPLER_WAVE_CTAS overrides the switch point.
+// per SM) for the batches that would otherwise need a second wave: 296 CTAs, two per SM.
+constexpr int kSamplerWaveCtas = 296;
+
 static cudaError_t launch_warp_sampler(int ctas, int threads, cudaStream_t stream,
                                        const PerSampleArgs &a, const WarpScratch &ws) {
-  static const int wave_ctas = [] {
-    const char *e = std::getenv("B2R_SAMPLER_WAVE_CTAS");
-    return e ? std::atoi(e) : 296;
-  }();
   if (ws.cluster)
     return launch_prio_cluster(per_sample_warp_kernel<2, true>, dim3(ctas), dim3(threads),
                                0, stream, chain_priority(), ctas, a, ws);
-  if (ctas > wave_ctas)
+  if (ctas > kSamplerWaveCtas)
     return launch(per_sample_warp_kernel<4, false>, dim3(ctas), dim3(threads), 0, stream,
                   a, ws);
   return launch(per_sample_warp_kernel<2, false>, dim3(ctas), dim3(threads), 0, stream, a,
@@ -1423,13 +1363,12 @@ int launch_sample(b2r_buffer *b, int32_t batch, bool philox, uint64_t seed,
                   uint64_t offset, const double *strat_dev,
                   const double *retry_dev, int32_t n_retry, int32_t *out_idx_dev,
                   int32_t *info_dev, cudaStream_t stream,
-                  const b2r_batch *scalars, float *min_prob_out, const RowFlags *flags,
-                  const PreSync *pre) {
+                  const b2r_batch *scalars, float *min_prob_out, const PreSync *pre) {
   int threads, tiles;
   sample_shape(batch, &threads, &tiles);
   if (tiles > kMaxTiles)
     return fail(B2R_ERR_UNSUPPORTED, "batch above %d is not supported", kMaxTiles * 128);
-  const bool by_warp = sampler_variant() == 1 && batch <= sampler_warp_max();
+  const bool by_warp = batch <= kSamplerWarpMax;
   PerSampleArgs a;
   WarpScratch ws;
   if (by_warp)
@@ -1472,9 +1411,6 @@ int launch_sample(b2r_buffer *b, int32_t batch, bool philox, uint64_t seed,
   a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
   if (pre != nullptr) a.pre = *pre;
   a.xchg.local = nullptr;
-  a.flags.desc = nullptr;
-  a.flags.tag_word = a.flags.final_word = nullptr;
-  if (flags != nullptr && by_warp && philox) a.flags = *flags;
   if (scalars) {
     fill_scalar_args(b, scalars, &a.sc);
     if (a.sc.indices_out == out_idx_dev) a.sc.indices_out = nullptr;
@@ -1526,10 +1462,9 @@ int launch_sample_sharded(b2r_buffer *b, int32_t global_batch, int32_t num_shard
   // Philox strata: the warp sampler over this rank's stratum range (see shard_ranges).
   // Caller-supplied queries (any order): one CTA of the thread kernel walks every tile
   // and compacts this rank's strata with block scans (tiles of 128 over many CTAs with
-  // the range search for Philox strata when B2R_SAMPLER=thread).
+  // the range search for Philox strata above kSamplerWarpMax).
   // (a rank's expected share decides, not the global batch)
-  const bool by_warp = sampler_variant() == 1 && query01 == nullptr &&
-                       global_batch / num_shards <= sampler_warp_max();
+  const bool by_warp = query01 == nullptr && global_batch / num_shards <= kSamplerWarpMax;
   const bool ranges = query01 == nullptr && num_shards > 1 &&
                       (by_warp || global_batch > 256);
   const int cap = max_rows > 0 && max_rows < global_batch ? max_rows : global_batch;
@@ -1589,8 +1524,6 @@ int launch_sample_sharded(b2r_buffer *b, int32_t global_batch, int32_t num_shard
   a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
   if (pre != nullptr) a.pre = *pre;
   a.xchg.local = nullptr;
-  a.flags.desc = nullptr;
-  a.flags.tag_word = a.flags.final_word = nullptr;
   if (x && x->world > 1) fill_exchange_args(x, &a.xchg);
   if (scalars) {
     fill_scalar_args(b, scalars, &a.sc);

@@ -42,25 +42,7 @@ static HostTrace g_host_trace;
 // stream beside the tree update).  Measured at batch 32 (e2e_breakdown.py): 49.7 us
 // per update unsplit, 54.7 us split — the side stream also carries the forked frame
 // copies, and the extra event hops cost more than the 3 us row kernel they hide.
-// B2R_SPLIT_MIN overrides.
-static int split_min() {
-  static const int v = [] {
-    const char *e = std::getenv("B2R_SPLIT_MIN");
-    return e ? std::atoi(e) : 64;
-  }();
-  return v;
-}
-
-// Profiling switch (never set in production): B2R_DEBUG_SKIP is a bit mask of step
-// kernels to leave out — 1 loss, 2 write-back, 4 its grouping pass, 8 frame copies — to
-// see what each costs the others when they share the GPU.
-static int debug_skip() {
-  static const int v = [] {
-    const char *e = std::getenv("B2R_DEBUG_SKIP");
-    return e ? std::atoi(e) : 0;
-  }();
-  return v;
-}
+constexpr int kSplitMin = 64;
 
 // One shard of a sharded replay: `batch` is then the GLOBAL batch, this rank's rows
 // are compacted at the front of `out` and counted on the device.
@@ -136,7 +118,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   // sampler; the tail that needs the sampled rows follows the sampler (c51.cu).
   // (A shard does not know its row count before it has sampled: the first half covers
   // every row its logits hold.)
-  const bool split_loss = !sample_only && !debug_skip() && c51_can_split(&loss);
+  const bool split_loss = !sample_only && c51_can_split(&loss);
   if (direct != nullptr && direct->online_src != nullptr && !split_loss)
     return fail(B2R_ERR_INVALID_ARGUMENT, "direct logits need the loss in two halves");
   const bool unjoined = direct != nullptr && split_loss;  // (see DirectIO)
@@ -218,7 +200,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
                                       shard->exchange->world > 1
                                   ? shard->exchange
                                   : nullptr;
-  if (!early) B2R_TRY(flush_queue(b, s, batch > split_min()));
+  if (!early) B2R_TRY(flush_queue(b, s, batch > kSplitMin));
   const bool flush_behind = early != nullptr && b->q_entries > 0;
   g_host_trace.lap(2);
   // Deferred frame copies: the copies read their indices from a private ring slot (the
@@ -253,14 +235,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
     if (b->slot_busy[ring_slot])
       B2R_CUDA(cudaStreamWaitEvent(s, b->ev_slot_free[ring_slot], 0));
   }
-  // Frame copies start row by row as the sampler finalises rows (RowFlags) when the
-  // fast gather path will run: stack 4, 1-byte pixels, 16-byte frames, register variant.
-  RowFlags flags = {nullptr, nullptr, nullptr};
-  const bool frames_wanted =
-      (out->state != nullptr || out->next_state != nullptr) && !(debug_skip() & 8);
-  if (!shard && !deferred && frames_wanted && sampler_hands_over_rows(batch) &&
-      gather_takes_row_flags(b))
-    B2R_TRY(row_flags_for(b, batch, &flags));
+  const bool frames = out->state != nullptr || out->next_state != nullptr;
   if (shard)
     B2R_TRY(launch_sample_sharded(
         b, batch, shard->exchange->world, shard->exchange->rank, nullptr,
@@ -270,51 +245,31 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   else
     B2R_TRY(launch_sample(b, batch, true, seed, offset, nullptr, nullptr, 0,
                           sample_idx, b->info, s, out, b->min_prob,
-                          flags.desc ? &flags : nullptr, split_loss ? &pre_sync : nullptr));
+                          split_loss ? &pre_sync : nullptr));
   g_host_trace.lap(3);
-  const bool frames = frames_wanted;
-  // The write-back groups the batch by tree node on every level — which needs the
-  // sampled indices, not the new priorities: that half runs on a second forked stream
-  // while the loss kernel works, and the write-back proper only applies the values.
   int64_t expected_rows =
       shard ? (batch + shard->exchange->world - 1) / shard->exchange->world : -1;
   if (expected_rows > rows_cap) expected_rows = rows_cap;
-  // Up to B2R_TREE_EARLY_MAX rows (default 1024, the kernel's largest batch; 0: never):
-  // ONE write-back kernel behind the loss tail that is resident early and groups the batch
-  // ahead of its values (tree.cu, kEarly; the loss tail tells it when the indices are
-  // final — TreeGo).  Above (and with B2R_TREE_EARLY=0) the grouping runs as a small kernel
-  // of its own on a forked stream and is joined in front of the write-back proper.
+  // Behind a split loss, up to 1024 rows (tree_early_takes): ONE write-back kernel behind
+  // the loss tail that is resident early and groups the batch ahead of its values
+  // (tree.cu, kEarly; the loss tail tells it when the indices are final — TreeGo).
   // (At 1024 rows, where the frame copies bound the step: 33.2 us with the TMA copies,
-  // 36.8 us with the side-stream grouping and the register copies under their occupancy
-  // cap, 40.1 us with this kernel beside the capped register copies —
-  // profiles/r2/out/run63.txt, run71.txt, run72.txt.)
-  static const int tree_early_max = [] {
-    const char *e = std::getenv("B2R_TREE_EARLY_MAX");
-    const char *off = std::getenv("B2R_TREE_EARLY");
-    if (off != nullptr && std::atoi(off) == 0) return 0;
-    return e != nullptr ? std::atoi(e) : 1024;
-  }();
-  const bool groupable =
-      !sample_only && tree_can_presort(rows_cap, expected_rows) && !(debug_skip() & 6);
-  const int64_t likely_rows = expected_rows >= 0 ? expected_rows : rows_cap;
-  const bool early_tree = groupable && split_loss && likely_rows <= tree_early_max;
-  const bool presort = groupable && !early_tree;
+  // 36.8 us with a separate grouping kernel on a forked stream and the register copies
+  // under their occupancy cap, 40.1 us with this kernel beside the capped register
+  // copies — profiles/r2/out/run63.txt, run71.txt, run72.txt.)
+  // Behind the one-kernel loss the write-back is the plain kFull launch: that kernel lets
+  // its dependents start at its first instruction, while the sampler may still be writing
+  // the indices.
+  const bool early_tree = split_loss && tree_early_takes(rows_cap, expected_rows);
   const TreeGo tree_go = early_tree ? tree_go_of(b->tree) : TreeGo();
-  if (frames || presort) B2R_CUDA(cudaEventRecord(b->ev_fork, s));
-  if (presort) {
-    B2R_CUDA(cudaStreamWaitEvent(b->side2, b->ev_fork, 0));
-    B2R_TRY((tree_apply<int32_t, float>(b->tree, rows_cap, out->indices, nullptr, nullptr,
-                                        b->side2, count, expected_rows, 1)));
-    B2R_CUDA(cudaEventRecord(b->ev_join2, b->side2));
-  }
   if (frames) {
+    B2R_CUDA(cudaEventRecord(b->ev_fork, s));
     B2R_CUDA(cudaStreamWaitEvent(b->side, b->ev_fork, 0));
     // (deferred: the first half of the loss rejoins through the copies' stream, so that
     // the next sampler's only parent in a captured graph is this step's write-back)
     if (deferred && split_loss && !unjoined)
       B2R_CUDA(cudaStreamWaitEvent(b->side, b->ev_c51_pre, 0));
-    B2R_TRY(launch_gather(b, rows_cap, sample_idx, out, b->side, count, true,
-                          flags.desc ? &flags : nullptr));
+    B2R_TRY(launch_gather(b, rows_cap, sample_idx, out, b->side, count, true));
     B2R_CUDA(cudaEventRecord(b->ev_join, b->side));
     if (deferred) {
       b->frames_pending = true;
@@ -334,16 +289,13 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   // tail's only parent in a captured graph is the sampler: it keeps its programmatic
   // early launch.  Its stream rejoins below, with the frame copies.)
   if (!split_loss && wait_before_loss) B2R_CUDA(cudaStreamWaitEvent(s, wait_before_loss, 0));
-  // (B2R_FUSE_WRITEBACK=1, unsplit loss only: write-back at the tail of the loss kernel)
   // (split loss, at most 32 rows: tail and write-back as one thread-block cluster)
   // A shard's step (row count on the device): the cluster applies the write-back when
   // the count turns out to be at most 32 and the one-CTA tree kernel launched behind it
   // then returns at once (`tree_done`).
   const bool tail_counted = split_loss && shard != nullptr && !flush_behind &&
                             c51_post_takes_tree(&loss, b->tree, expected_rows);
-  const bool tail_writeback =
-      split_loss ? (!shard && c51_post_takes_tree(&loss, b->tree))
-                 : (!shard && !debug_skip() && c51_can_fuse_writeback(&loss, b->tree));
+  const bool tail_writeback = split_loss && !shard && c51_post_takes_tree(&loss, b->tree);
   unsigned int *tree_done = tail_counted ? b->pre_sync + 3 : nullptr;
   if (split_loss)
     B2R_TRY(c51_post_launch(&loss, scratch, have_stats, s, b->status,
@@ -352,17 +304,14 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
                             out->indices, tree_done, tail_counted ? early : nullptr,
                             direct ? direct->loss_host : nullptr,
                             early_tree ? &tree_go : nullptr, staged ? &stage : nullptr));
-  else if (tail_writeback)
-    B2R_TRY(c51_loss_launch(&loss, s, b->tree, out->indices));
-  else if (!(debug_skip() & 1))
+  else
     B2R_TRY(b2r_c51_loss(&loss, s));
   if (loss_done) B2R_CUDA(cudaEventRecord(loss_done, s));
   g_host_trace.lap(5);
-  if (presort) B2R_CUDA(cudaStreamWaitEvent(s, b->ev_join2, 0));
-  if (!(debug_skip() & 2) && !tail_writeback)
+  if (!tail_writeback)
     B2R_TRY((tree_apply<int32_t, float>(b->tree, rows_cap, out->indices, loss.priorities,
                                         nullptr, s, count, expected_rows,
-                                        presort ? 2 : (early_tree ? 3 : 0),
+                                        early_tree ? kEarly : kFull,
                                         flush_behind ? nullptr : early, tree_done,
                                         early_tree)));
   if (flush_behind) B2R_TRY(flush_queue(b, s, false, early));
@@ -726,8 +675,7 @@ int b2r_trainer_step_host(b2r_trainer *t, const float *online_logits,
   // two records covers both)
   b2r_c51_args probe = t->c51;  // (c51.batch is the rows behind the sampler)
   const bool through_first_half = !t->cfg.use_graph && b2r::c51_can_split(&probe);
-  static const bool loss_copy = std::getenv("B2R_TRAINER_LOSS_COPY") != nullptr;
-  const bool kernel_writes_losses = through_first_half && t->ring_dev != nullptr && !loss_copy;
+  const bool kernel_writes_losses = through_first_half && t->ring_dev != nullptr;
   if (n >= 2)
     B2R_CUDA(cudaStreamWaitEvent(
         t->copy, kernel_writes_losses ? t->ev_done[(size_t)((n - 2) % t->ring)]
@@ -747,7 +695,7 @@ int b2r_trainer_step_host(b2r_trainer *t, const float *online_logits,
                          n >= 2 ? t->ev_done[(size_t)((n - 2) % t->ring)] : nullptr};
   // ... and then the tail writes the per-row losses into this step's page-locked result
   // slot itself (33 words over PCIe): no result copy, no result-copy stream; the event
-  // the host collects on is recorded behind the tail.  B2R_TRAINER_LOSS_COPY=1: the copy.
+  // the host collects on is recorded behind the tail.
   const int slot = (int)(n % t->ring);
   if (kernel_writes_losses)
     hints.loss_host = t->ring_dev + (size_t)slot * (t->cfg.logit_rows + 1);
@@ -766,7 +714,7 @@ int b2r_trainer_step_host(b2r_trainer *t, const float *online_logits,
   } else if (t->cfg.use_graph && n >= 2) {
     // Everything host-dependent (staged adds, validity context) goes first, eagerly;
     // the replayed graph reads it from HBM.
-    B2R_TRY(b2r::flush_queue(t->buf, s, t->cfg.batch > b2r::split_min()));
+    B2R_TRY(b2r::flush_queue(t->buf, s, t->cfg.batch > b2r::kSplitMin));
     B2R_TRY(b2r::ensure_ctx(t->buf, s));
     if (!t->exec[set]) B2R_TRY(capture_step(t, set));
     B2R_CUDA(cudaStreamWaitEvent(s, t->ev_in[set], 0));

@@ -170,7 +170,7 @@ using BigCfg1024 = BigCfg<256, 4>;
 // kEarly, up to 1024 entries: one entry per thread.  These kernels are chains of dependent
 // instructions (ncu: 13 cycles per instruction and warp, 2 warps per scheduler with
 // 256 x 4); a thread with one entry runs a quarter of them and the schedulers have eight
-// warps to pick from (B2R_TREE_WIDE=0: 256 x 4).
+// warps to pick from.
 using BigCfgWide = BigCfg<1024, 1>;
 static_assert(BigCfg4096::kChunk == kTreeChunk, "chunk size");
 
@@ -564,7 +564,7 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_kernel(UpdateArgs<I, 
   // sharing the GPU with the frame copies of the same step (a cooperative grid starts
   // only once every CTA of it can be resident).
   __shared__ int s_role;
-  B2R_MARK(a.phase == kPresort ? 12 : 13);
+  B2R_MARK(13);
   pdl_release();
   pdl_acquire();
   if (threadIdx.x == 0) s_role = (int)atomicInc(a.sync_words, (unsigned)a.depth);
@@ -585,26 +585,6 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_kernel(UpdateArgs<I, 
   // A chunk beyond the device-side count (sharded replay: the host launches for the
   // largest possible count) has nothing to do; every CTA sees the same n.
   if (n <= 0) return;
-  if (a.phase == kPresort) {
-    // group the n entries by their node on this level and leave the lists in HBM
-    uint32_t key[kBigItems], val[kBigItems];
-    const int shift0 = a.depth - level;
-#pragma unroll
-    for (int j = 0; j < kBigItems; ++j) {
-      const int k = threadIdx.x * kBigItems + j;
-      key[j] = k < n ? (uint32_t)((int64_t)a.indices[k] >> shift0) : 0xffffffffu;
-      val[j] = (uint32_t)k;
-    }
-    if (level != 0) BigSort(sm.g.sort).Sort(key, val, 0, level);
-    uint32_t *dst = a.sorted + (size_t)level * 2 * C::kChunk;
-#pragma unroll
-    for (int j = 0; j < kBigItems; ++j) {  // thread-contiguous: 16-byte stores
-      dst[threadIdx.x * kBigItems + j] = key[j];
-      dst[C::kChunk + threadIdx.x * kBigItems + j] = val[j];
-    }
-    B2R_MARK_END(14);
-    return;
-  }
   if (threadIdx.x == 0) {
     s_stop = n;
     s_stop_code = 0;
@@ -647,8 +627,6 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_kernel(UpdateArgs<I, 
   B2R_MARK_LVL(23, a.depth - 1);
   B2R_MARK_LVL(29, 0);
   bool leaf_done = false;
-  // kApply: the presorted lists hold all n entries; they serve iff all n are applied
-  const bool presorted = a.phase == kApply && n_eff == n;
   if (is_leaf) {
     // max_recorded_priority = max(value, current) over the applied prefix
     // (before vals[] turns into deltas).
@@ -658,22 +636,14 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_kernel(UpdateArgs<I, 
     for (int off = 16; off > 0; off >>= 1)
       local_max = fmax(local_max, __shfl_xor_sync(0xffffffffu, local_max, off));
     if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = local_max;
-    if (!presorted) leaf_done = leaf_deltas_hashed<C>(a, n_eff, sm.h, vals);
+    leaf_done = leaf_deltas_hashed<C>(a, n_eff, sm.h, vals);
     __syncthreads();
   }
 
   // 3. group by node: thread t holds entries 4t .. 4t+3 (batch order); pads carry
   //    all-ones keys and sit behind every real entry, so they stay last.
   const int shift = a.depth - level;
-  if (presorted) {
-    const uint32_t *src = a.sorted + (size_t)level * 2 * C::kChunk;
-#pragma unroll
-    for (int j = 0; j < kBigItems; ++j) {
-      sm.g.node[threadIdx.x * kBigItems + j] = __ldcg(src + threadIdx.x * kBigItems + j);
-      sm.g.elem[threadIdx.x * kBigItems + j] =
-          __ldcg(src + C::kChunk + threadIdx.x * kBigItems + j);
-    }
-  } else if (!leaf_done) {
+  if (!leaf_done) {
     uint32_t key[kBigItems], val[kBigItems];
 #pragma unroll
     for (int j = 0; j < kBigItems; ++j) {
@@ -1345,7 +1315,7 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_early_kernel(UpdateAr
   constexpr uint32_t kEmpty = 0xffffffffu;
   using Sort = typename C::Sort;
   using Info = DupInfo<C>;
-  static_assert(Info::kWords <= DupInfo<BigCfg4096>::kWords, "scratch (ensure_sorted)");
+  static_assert(Info::kWords <= DupInfo<BigCfgWide>::kWords, "scratch (ensure_sorted)");
   extern __shared__ __align__(16) uint8_t smem_raw[];
   typename C::EarlySmem &sm = *reinterpret_cast<typename C::EarlySmem *>(smem_raw);
   double *vals = sm.vals;
@@ -1463,9 +1433,8 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_early_kernel(UpdateAr
   }
   if (first_bad < n) atomicMin(&s_stop, first_bad);
   int own_pos[kItems];
-  const bool own_list =
-      a.own_lists != 0 && leaf_list_from_sorted<C>(a, n, sm, s_dup, lidx, &ns, scratch, s_scan,
-                                                   a.depth - level, own_pos, who) == 1;
+  const bool own_list = leaf_list_from_sorted<C>(a, n, sm, s_dup, lidx, &ns, scratch, s_scan,
+                                                 a.depth - level, own_pos, who) == 1;
   B2R_PHASE(who, 5);
   B2R_TRACE_COUNT(0, is_leaf);
   B2R_TRACE_COUNT(1, is_leaf && own_list);
@@ -2030,23 +1999,27 @@ int allow_big_smem(K kernel) {
   return B2R_OK;
 }
 
-// One chunk of the cooperative kernel with geometry C.
-template <typename C, typename I, typename V>
+// One chunk of the cooperative kernel with geometry C: tree_update_kernel, or (EARLY,
+// kEarly) tree_update_early_kernel.
+template <typename C, bool EARLY, typename I, typename V>
 int launch_big_chunk(const UpdateArgs<I, V> &a, int depth, cudaStream_t stream) {
-  B2R_TRY((allow_big_smem<C, 0>(tree_update_kernel<I, V, C>)));
-  B2R_TRY((allow_big_smem<C, 1>(tree_update_early_kernel<I, V, C>)));
+  void (*kernel)(UpdateArgs<I, V>);
+  if constexpr (EARLY)
+    kernel = tree_update_early_kernel<I, V, C>;
+  else
+    kernel = tree_update_kernel<I, V, C>;
+  B2R_TRY((allow_big_smem<C, EARLY ? 1 : 0>(kernel)));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(depth + 1);
   cfg.blockDim = dim3(C::kThreads);
-  cfg.dynamicSmemBytes =
-      a.phase == kEarly ? sizeof(typename C::EarlySmem) : sizeof(typename C::Smem);
+  cfg.dynamicSmemBytes = EARLY ? sizeof(typename C::EarlySmem) : sizeof(typename C::Smem);
   cfg.stream = stream;
   cudaLaunchAttribute attr[3];
   int n_attr = 0;
   // Launched early (programmatic dependent launch) only in the 256 x 4 geometry: 21
   // early CTAs of 1024 threads would sit on 21 SMs for the whole loss kernel.
   // (kEarly: starting early is the point — its CTAs are sorting meanwhile.)
-  if (pdl_enabled() && (C::kThreads <= 256 || a.phase == kEarly)) {
+  if (pdl_enabled() && (C::kThreads <= 256 || EARLY)) {
     attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[n_attr++].val.programmaticStreamSerializationAllowed = 1;
   }
@@ -2064,10 +2037,7 @@ int launch_big_chunk(const UpdateArgs<I, V> &a, int depth, cudaStream_t stream) 
   }
   cfg.attrs = attr;
   cfg.numAttrs = n_attr;
-  if (a.phase == kEarly)
-    B2R_CUDA(cudaLaunchKernelEx(&cfg, tree_update_early_kernel<I, V, C>, a));
-  else
-    B2R_CUDA(cudaLaunchKernelEx(&cfg, tree_update_kernel<I, V, C>, a));
+  B2R_CUDA(cudaLaunchKernelEx(&cfg, kernel, a));
   B2R_LAUNCHED();
   return B2R_OK;
 }
@@ -2077,37 +2047,12 @@ int launch_big_chunk(const UpdateArgs<I, V> &a, int depth, cudaStream_t stream) 
 // The one-CTA kernel sorts per warp (cost ~ n log^2 n): it wins for the agent's batch
 // of 32 (4.9 us) and already loses to the 256 x 4 cooperative kernel at 64 entries
 // (10.5 vs 9.2 us; at 256: 43 vs 9.8 us — measured with 10 launches per graph,
-// profiles/r1/README.md).  B2R_TREE_SMALL_MAX overrides the threshold.
-int tree_small_max() {
-  static const int small_max = [] {
-    const char *e = std::getenv("B2R_TREE_SMALL_MAX");
-    int v = e ? std::atoi(e) : 32;
-    return v < 0 ? 0 : (v > kSmallBatch ? kSmallBatch : v);
-  }();
-  return small_max;
-}
-
-// B2R_TREE_TINY=0 sends batches of up to 32 sets through the sorting one-CTA kernel
-// instead of the match-based one (comparison runs).
-bool tree_tiny_enabled() {
-  static const bool on = [] {
-    const char *e = std::getenv("B2R_TREE_TINY");
-    return e == nullptr || std::atoi(e) != 0;
-  }();
-  return on;
-}
+// profiles/r1/README.md).  Largest batch it takes.
+constexpr int kTreeSmallMax = 32;
 
 // Shortest average chain (entries per touched node of a level) that is worth the
 // verified scan: a round costs about as much as 60-80 dependent DADDs.
-// B2R_TREE_SCAN_MIN overrides it (0 = serial chains everywhere).
-int tree_scan_min_chain() {
-  static const int v = [] {
-    const char *e = std::getenv("B2R_TREE_SCAN_MIN");
-    const int x = e ? std::atoi(e) : 32;
-    return x < 0 ? 0 : x;
-  }();
-  return v;
-}
+constexpr int kTreeScanMinChain = 32;
 
 static int allow_small_smem() {
   static bool ready = false;
@@ -2154,38 +2099,29 @@ int flush_fused(b2r_tree *t, int n, const int64_t *slots, const double *prio,
   }
   B2R_CUDA(launch(flush_fused_kernel, dim3(1 + n * row_blocks_per_entry),
                   dim3(32 * (t->depth + 1)), smem, stream, a, rows,
-                  row_blocks_per_entry, (int)(n <= kTinyBatch && tree_tiny_enabled())));
+                  row_blocks_per_entry, (int)(n <= kTinyBatch)));
   B2R_LAUNCHED();
   return B2R_OK;
 }
 
-// Does a batch of n sets (expected_n as in tree_apply) go through the cooperative
-// kernel in ONE chunk, i.e. can its grouping be done ahead of the values?
-bool tree_can_presort(int64_t n, int64_t expected_n) {
-  static const bool on = [] {
-    const char *e = std::getenv("B2R_TREE_PRESORT");
-    return e == nullptr || std::atoi(e) != 0;
-  }();
+// Can the early write-back (kEarly) take a batch of n sets (expected_n as in
+// tree_apply)?  It is the cooperative kernel in ONE chunk of its geometry: batches above
+// the one-CTA kernel's and up to 1024 sets.  Beyond that the frame copies bound the step
+// and the write-back hides behind them anyway.
+// (A launch sized for more entries than are expected — a sharded step's bound on its
+// share — groups its first chunk early, where the expected entries are; chunks behind
+// it, normally empty, run as kFull.)
+bool tree_early_takes(int64_t n, int64_t expected_n) {
   const int64_t likely = expected_n >= 0 ? expected_n : n;
-  if (n <= kSmallBatch && likely <= tree_small_max()) return false;
-  // Beyond the 256 x 4 geometry the frame copies bound the step and the write-back
-  // hides behind them anyway: a second pass would only take SM slots from the copies.
-  static const int64_t presort_max = [] {
-    const char *e = std::getenv("B2R_TREE_PRESORT_MAX");
-    return e ? (int64_t)std::atoi(e) : (int64_t)BigCfg1024::kChunk;
-  }();
-  // (A launch sized for more entries than are expected — a sharded step's bound on its
-  // share — presorts its first chunk, where the expected entries are; chunks behind it,
-  // normally empty, run unsplit.)
-  return on && likely <= BigCfg4096::kChunk && likely <= presort_max;
+  if (n <= kSmallBatch && likely <= kTreeSmallMax) return false;
+  return likely <= BigCfgWide::kChunk;
 }
 
 static int ensure_sorted(b2r_tree *t) {
   if (t->sorted) return B2R_OK;
-  // (the presorted lists of every level; kEarly: the leaf CTA's list of duplicate leaves)
-  size_t words = (size_t)(t->depth + 1) * 2 * BigCfg4096::kChunk;
-  if (words < (size_t)DupInfo<BigCfg4096>::kWords) words = DupInfo<BigCfg4096>::kWords;
-  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&t->sorted), words * sizeof(uint32_t)));
+  // (kEarly: the leaf CTA's list of duplicate leaves)
+  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&t->sorted),
+                      (size_t)DupInfo<BigCfgWide>::kWords * sizeof(uint32_t)));
   return B2R_OK;
 }
 
@@ -2195,16 +2131,15 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
                int64_t expected_n, int phase, const b2r_exchange *publish,
                unsigned int *skip_flag, bool go_by_flag) {
   set_tree_window(t->heap, (size_t)t->leaves * 16);
-  if (phase != kFull) {
-    if (!tree_can_presort(n, expected_n) || mode != nullptr)
-      return fail(B2R_ERR_INVALID_ARGUMENT, "this batch cannot be presorted");
+  if (phase == kEarly) {
+    if (!tree_early_takes(n, expected_n) || mode != nullptr)
+      return fail(B2R_ERR_INVALID_ARGUMENT, "this batch cannot take the early write-back");
     B2R_TRY(ensure_sorted(t));
   }
-  const int small_max = tree_small_max();
   // A device-side count (sharded replay) is only bounded by n on the host: the
   // caller's expectation decides, the one-CTA kernel copes with up to kSmallBatch.
   const int64_t likely = expected_n >= 0 ? expected_n : n;
-  if (n <= kSmallBatch && likely <= small_max) {
+  if (n <= kSmallBatch && likely <= kTreeSmallMax) {
     // latency path: one CTA, one warp per level
     const int padded = padded_size((int)n);
     const size_t smem = (size_t)padded * 8 * (1 + 2 * (size_t)(t->depth + 1));
@@ -2229,13 +2164,13 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
       a.publish_rank = publish->rank;
     }
     a.skip_flag = skip_flag;
-    if (n <= kTinyBatch && tree_tiny_enabled() && skip_flag == nullptr)
+    if (n <= kTinyBatch && skip_flag == nullptr)
       B2R_CUDA(launch(tree_update_tiny_kernel<I, V>, dim3(1), dim3(32 * (t->depth + 1)),
                       0, stream, a));
     else
       B2R_CUDA(launch(tree_update_small_kernel<I, V>, dim3(1),
                       dim3(32 * (t->depth + 1)), smem, stream, a,
-                      (int)(n_dev != nullptr && tree_tiny_enabled() && t->depth + 1 <= 32)));
+                      (int)(n_dev != nullptr && t->depth + 1 <= 32)));
     B2R_LAUNCHED();
     return B2R_OK;
   }
@@ -2244,7 +2179,6 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
   const bool compact = likely <= BigCfg1024::kChunk;
   const int64_t chunk = compact ? BigCfg1024::kChunk : BigCfg4096::kChunk;
   for (int64_t base = 0; base < n; base += chunk) {
-    if (phase == kPresort && base > 0) break;  // (only the first chunk is grouped ahead)
     const int len = (int)((n - base) < chunk ? (n - base) : chunk);
     UpdateArgs<I, V> a;
     a.heap = t->heap;
@@ -2260,27 +2194,18 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
     a.max_rec = t->max_rec;
     a.status = t->status;
     a.n_dev = n_dev;
-    a.scan_min_chain = tree_scan_min_chain();
+    a.scan_min_chain = kTreeScanMinChain;
     a.phase = base == 0 ? phase : kFull;
-    static const int own_lists = [] {
-      const char *e = std::getenv("B2R_TREE_OWN_LISTS");
-      return e == nullptr || std::atoi(e) != 0 ? 1 : 0;
-    }();
-    a.own_lists = own_lists;
     a.tickets = reinterpret_cast<unsigned long long *>(t->sync_words + 12);
     a.go = go_by_flag && a.phase == kEarly ? t->sync_words + 14 : nullptr;
     a.sorted = t->sorted;
     a.sync_words = t->sync_words;
-    static const bool wide = [] {
-      const char *e = std::getenv("B2R_TREE_WIDE");
-      return e == nullptr || std::atoi(e) != 0;
-    }();
-    if (compact && a.phase == kEarly && wide)
-      B2R_TRY((launch_big_chunk<BigCfgWide>(a, t->depth, stream)));
+    if (a.phase == kEarly)  // (tree_early_takes: compact)
+      B2R_TRY((launch_big_chunk<BigCfgWide, true>(a, t->depth, stream)));
     else if (compact)
-      B2R_TRY((launch_big_chunk<BigCfg1024>(a, t->depth, stream)));
+      B2R_TRY((launch_big_chunk<BigCfg1024, false>(a, t->depth, stream)));
     else
-      B2R_TRY((launch_big_chunk<BigCfg4096>(a, t->depth, stream)));
+      B2R_TRY((launch_big_chunk<BigCfg4096, false>(a, t->depth, stream)));
   }
   return B2R_OK;
 }
@@ -2392,7 +2317,7 @@ int b2r_tree_set(b2r_tree *t, int64_t n, const int64_t *indices,
   // promise holds trivially)
   const char *phase_env = std::getenv("B2R_TREE_SET_PHASE");
   const int phase = phase_env != nullptr && std::atoi(phase_env) == b2r::kEarly &&
-                            b2r::tree_can_presort(n, -1)
+                            b2r::tree_early_takes(n, -1)
                         ? b2r::kEarly
                         : b2r::kFull;
   B2R_TRY((b2r::tree_apply<int64_t, double>(

@@ -17,8 +17,8 @@ struct b2r_tree {
   double *max_rec = nullptr;   // device scalar: max_recorded_priority
   int64_t *status = nullptr;   // device [2]: latched error code, offending position
   double *delta = nullptr;     // device scratch: per-element leaf deltas of a chunk
-  uint32_t *sorted = nullptr;  // device scratch: per-level (node, entry) lists of a
-                               // presorted chunk (tree.cu: kPresort / kApply)
+  uint32_t *sorted = nullptr;  // device scratch: the early write-back's list of
+                               // duplicate leaves (tree.cu: kEarly, DupInfo)
   unsigned int *sync_words = nullptr;  // device: level ticket, barrier flag, arrivals,
                                        // pending failure (tree_update_kernel)
   b2r::Bounce bounce;
@@ -372,8 +372,8 @@ __device__ __forceinline__ void tree_go_signal(const TreeGo &g) {
 #endif
 
 #ifdef __CUDACC__
-// Arguments of the batched-set kernels (tree.cu; the tiny body below also runs at the
-// tail of the C51 loss kernel, c51.cu).
+// Arguments of the batched-set kernels (tree.cu; the tiny body below also runs in the
+// C51 loss tail's cluster, c51.cu).
 template <typename I, typename V>
 struct UpdateArgs {
   double *heap;
@@ -391,26 +391,17 @@ struct UpdateArgs {
   // internal levels whose average chain (n >> level) is at least this long run their
   // ordered add-chains as a verified scan (chains_by_verified_scan); 0 = never
   int scan_min_chain = 0;
-  // Two-launch form of the cooperative kernel (the fused step): grouping the entries by
-  // node needs the INDICES only, so it can run while the loss kernel is still producing
-  // the values.  kPresort: every level CTA sorts and leaves (node, entry) in `sorted`
-  // ([level][node | entry][chunk] words), nothing else.  kApply: the level CTAs read
-  // those lists instead of sorting — unless an entry must not be applied (negative value,
-  // index out of range), in which case the lists are ignored and the kernel sorts the
-  // applied prefix itself, as kFull always does.
-  // kEarly (tree_update_early_kernel): ONE launch that does the index-only work ahead of
-  // its griddepcontrol.wait, beside the kernel that produces the values.  The caller
-  // promises that the indices (and n_dev) were final before that kernel let its
+  // kFull: the whole update in tree_update_kernel.  kEarly (tree_update_early_kernel): ONE
+  // launch that does the work that needs the INDICES only (grouping the entries by node)
+  // ahead of its griddepcontrol.wait, beside the kernel that produces the values.  The
+  // caller promises that the indices (and n_dev) were final before that kernel let its
   // dependents start.
   int phase = 0;
-  // kEarly: 0 = never take the path for batches that are grouped by leaf already
-  // (B2R_TREE_OWN_LISTS=0, comparison runs)
-  int own_lists = 1;
   // kEarly: the launch's tickets (always) and, when the kernel in front signals "indices
   // final" through memory instead of through its end, the word to wait on (TreeGo)
   unsigned long long *tickets = nullptr;
   unsigned int *go = nullptr;
-  uint32_t *sorted = nullptr;
+  uint32_t *sorted = nullptr;  // kEarly: b2r_tree::sorted
   // role ticket, barrier flag, barrier arrivals (see tree_update_kernel)
   unsigned int *sync_words = nullptr;
   // Sharded replay: this launch leaves the tree final for the next sharded step, so the
@@ -431,7 +422,7 @@ __device__ __forceinline__ void publish_root(const UpdateArgs<I, V> &a) {
   const double root = *reinterpret_cast<volatile double *>(a.heap + 1);
   exchange_publish(*a.publish, a.publish_world, a.publish_rank, root, *a.publish->seq + 1);
 }
-constexpr int kFull = 0, kPresort = 1, kApply = 2, kEarly = 3;
+constexpr int kFull = 0, kEarly = 3;
 
 // At most 32 sets (the agent's batch, an add flush): entry k lives in lane k of every
 // warp, warp l owns tree level l, and nothing is sorted.  __match_any_sync groups the
@@ -605,9 +596,8 @@ __device__ __forceinline__ void tree_update_tiny_body(const UpdateArgs<I, V> &a)
 // n_dev (nullable): device count, the effective n is min(n, *n_dev).
 // expected_n (>= 0): how many entries the caller expects when only the device knows
 // (n_dev); picks between the one-CTA and the cooperative kernel.
-// phase: 0 = the whole update; 1 = only group the entries by node (needs the indices,
-// not the values: tree_can_presort says whether this batch can); 2 = apply the values
-// over the lists of a phase-1 launch with the same n / indices / n_dev / expected_n.
+// phase: kFull = the whole update; kEarly = the early write-back, resident ahead of the
+// values (tree_early_takes says whether this batch can; see UpdateArgs::phase).
 // publish (nullable, one-CTA kernels only): the launch leaves the tree final for the next
 // sharded step and publishes the new root to the exchange's peers.
 template <typename I, typename V>
@@ -618,12 +608,7 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
                bool go_by_flag = false);
 // What the kernel in front of an early write-back of `t` signals (go_by_flag).
 TreeGo tree_go_of(b2r_tree *t);
-bool tree_can_presort(int64_t n, int64_t expected_n);
-bool tree_tiny_enabled();
-// c51.cu: the C51 loss with the write-back of its priorities at the kernel's tail.
-bool c51_can_fuse_writeback(const b2r_c51_args *args, const b2r_tree *tree);
-int c51_loss_launch(const b2r_c51_args *args, cudaStream_t stream, b2r_tree *tree,
-                    const int32_t *indices);
+bool tree_early_takes(int64_t n, int64_t expected_n);
 // c51.cu: the loss in two halves (the fused step): what depends on the network outputs
 // alone, over `rows` rows, into scratch ([rows][c51_scratch_floats_per_row()] floats),
 // signalling `sync` when done ...
