@@ -5,10 +5,13 @@ defaults of :79-108 and dqn.gin): the Nature DQN network (atari_lib.py:85-105, c
 through PyTorch behind the hand-written input kernel), the uniform replay buffer, the
 Bellman target + Huber loss as ONE kernel (`dqn_loss`, csrc/dqn.cu), TensorFlow's centred
 RMSProp with the reference's numbers, and the target sync.  Same structure as
-`agents/rainbow/agent.RainbowLearner`; the acting side is `dqn_agent.ActingLoop`.
+`agents/rainbow/agent.RainbowLearner`; the acting side is `dqn_agent.ActingLoop`, and
+`DQNAgent` joins the two as the reference's runner creates it for dqn.gin.
 `ShardedDQNLearner` trains on one global uniform batch drawn over the GPUs' replay shards.
 """
 import math
+
+import numpy as np
 
 from dopamine_b200.agents import sharded_learner
 from dopamine_b200.agents.dqn import dqn_agent
@@ -141,12 +144,15 @@ def make_tf_rmsprop(params, lr=0.00025, decay=0.95, momentum=0.0, epsilon=0.0000
   return TFRMSProp()
 
 
-class DQNLearner(object):
-  """Replay + train op of DQNAgent (dqn_agent.py:237-322)."""
+class DQNLearner(sharded_learner.GraphedUpdate):
+  """Replay + train op of DQNAgent (dqn_agent.py:237-322).  With `cuda_graph=True` the
+  whole update (uniform sampler, frame copies, both networks, loss, backward, RMSProp)
+  is captured once and replayed as one CUDA graph (`GraphedUpdate`)."""
 
   def __init__(self, num_actions, observation_shape=(84, 84), stack_size=4, gamma=0.99,
                update_horizon=1, replay_capacity=1000000, batch_size=32,
-               target_update_period=8000, update_period=4, seed=0, memory=None):
+               target_update_period=8000, update_period=4, seed=0, memory=None,
+               cuda_graph=False):
     torch = _torch()
     self.num_actions = num_actions
     self.batch_size = batch_size
@@ -165,6 +171,9 @@ class DQNLearner(object):
     for p in self.target.parameters():
       p.requires_grad_(False)
     self.optimizer = make_tf_rmsprop(self.online.parameters())
+    self._cuda_graph = bool(cuda_graph)
+    self._graph = None
+    self._static_loss = None
     self.training_steps = 0
     self.updates = 0
 
@@ -176,7 +185,8 @@ class DQNLearner(object):
     with _torch().no_grad():
       return self.online(state)
 
-  def train_step(self):
+  # train_step() is GraphedUpdate's
+  def _update(self):
     """dqn_agent.py:283-322: sample -> target net on next_state, online net on state ->
     Bellman target + Huber loss (one kernel) -> backward -> RMSProp.  Returns the mean
     loss (a CUDA tensor, no sync)."""
@@ -191,7 +201,8 @@ class DQNLearner(object):
     self.optimizer.zero_grad(set_to_none=True)
     loss.backward()
     self.optimizer.step()
-    self.updates += 1
+    if not self._cuda_graph or self._graph is None:
+      self.updates += 1
     return loss
 
   def sync_target(self):
@@ -206,6 +217,53 @@ class DQNLearner(object):
       self.sync_target()
     self.training_steps += 1
     return loss
+
+
+class DQNAgent(DQNLearner, dqn_agent.ActingLoop):
+  """`DQNAgent` (dqn_agent.py:76-560) as the reference's runner sees it:
+  `begin_episode(observation)`, `step(reward, observation)`, `end_episode(reward)`,
+  `eval_mode`, `bundle_and_checkpoint`, `unbundle`.  Constructor arguments keep the
+  reference's names and defaults (dqn_agent.py:76-108); `sess`, `tf_device`,
+  `use_staging`, `max_tf_checkpoints_to_keep`, `optimizer` (always TensorFlow's centred
+  RMSProp with dqn.gin's numbers, `make_tf_rmsprop`) and the summary arguments have no
+  meaning here.  `replay_capacity` and `batch_size` are the replay buffer's
+  (`_build_replay_buffer`, dqn_agent.py:265-281, binds them through gin); `seed`,
+  `memory` and `cuda_graph` are `DQNLearner`'s.  Lives here rather than in
+  `dqn_agent.py` because this module imports that one."""
+
+  def __init__(self, sess=None, num_actions=None, observation_shape=(84, 84),
+               observation_dtype=np.uint8, stack_size=4, gamma=0.99, update_horizon=1,
+               min_replay_history=20000, update_period=4, target_update_period=8000,
+               epsilon_fn=dqn_agent.linearly_decaying_epsilon, epsilon_train=0.01,
+               epsilon_eval=0.001, epsilon_decay_period=250000, tf_device='/cpu:*',
+               use_staging=True, max_tf_checkpoints_to_keep=4, optimizer=None,
+               summary_writer=None, summary_writing_frequency=500,
+               replay_capacity=1000000, batch_size=32, seed=0,
+               allow_partial_reload=False, memory=None, cuda_graph=False):
+    del sess, tf_device, use_staging, max_tf_checkpoints_to_keep, optimizer
+    del summary_writer, summary_writing_frequency
+    if num_actions is None:
+      raise ValueError('num_actions is required')
+    if np.dtype(observation_dtype) != np.uint8:
+      raise NotImplementedError('the convolutional network takes uint8 frames')
+    DQNLearner.__init__(
+        self, num_actions, observation_shape=observation_shape, stack_size=stack_size,
+        gamma=gamma, update_horizon=update_horizon, replay_capacity=replay_capacity,
+        batch_size=batch_size, target_update_period=target_update_period,
+        update_period=update_period, seed=seed, memory=memory, cuda_graph=cuda_graph)
+    self._init_acting(observation_shape, stack_size, observation_dtype,
+                      min_replay_history=min_replay_history,
+                      update_period=update_period,
+                      target_update_period=target_update_period,
+                      epsilon_fn=epsilon_fn, epsilon_train=epsilon_train,
+                      epsilon_eval=epsilon_eval,
+                      epsilon_decay_period=epsilon_decay_period,
+                      allow_partial_reload=allow_partial_reload)
+
+  def _store_transition(self, last_observation, action, reward, is_terminal):
+    """dqn_agent.py:460-472: the uniform buffer takes no priority."""
+    if not self.eval_mode:
+      self.store_transition(last_observation, action, reward, is_terminal)
 
 
 class ShardedDQNLearner(sharded_learner.ShardedLearner, DQNLearner):
@@ -239,10 +297,8 @@ class ShardedDQNLearner(sharded_learner.ShardedLearner, DQNLearner):
                group=None, exchange_timeout_s=2.0, ddp=False, cuda_graph=False,
                **kwargs):
     exchange = self._connect(exchange, group, exchange_timeout_s, ddp)
-    DQNLearner.__init__(self, num_actions, batch_size=batch_size, **kwargs)
-    self._cuda_graph = bool(cuda_graph)
-    self._graph = None
-    self._static_loss = None
+    DQNLearner.__init__(self, num_actions, batch_size=batch_size, cuda_graph=cuda_graph,
+                        **kwargs)
     self._shard(exchange, max_rows, kwargs.get('seed', 0),
                 sharded_replay.ShardedUniformReplay)
 

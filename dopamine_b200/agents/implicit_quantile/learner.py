@@ -8,12 +8,15 @@ the target quantile values and the quantile-Huber loss as ONE kernel
 (`quantile_huber_loss`, csrc/iqn.cu), TensorFlow's Adam with the reference's numbers, the
 target sync.  Uniform replay through the prioritized buffer class, as the reference does
 ("IQN currently does not support prioritized replay", implicit_quantile.gin:23-24).
+`ImplicitQuantileAgent` joins `IQNLearner` to the episode interface
+(`dqn_agent.ActingLoop`) as the reference's runner creates it for implicit_quantile.gin.
 """
 import math
 
 import numpy as np
 
 from dopamine_b200.agents import sharded_learner
+from dopamine_b200.agents.dqn import dqn_agent
 from dopamine_b200.agents.dqn import learner as dqn_learner
 from dopamine_b200.agents.implicit_quantile import implicit_quantile_agent as iqn
 from dopamine_b200.agents.rainbow import agent as conv
@@ -72,15 +75,23 @@ def make_implicit_quantile_network(num_actions, quantile_embedding_dim=64,
   return ImplicitQuantileNetwork()
 
 
-class IQNLearner(object):
-  """Replay + train op of ImplicitQuantileAgent (implicit_quantile_agent.py:120-321)."""
+class IQNLearner(sharded_learner.GraphedUpdate):
+  """Replay + train op of ImplicitQuantileAgent (implicit_quantile_agent.py:120-321).
+
+  Eagerly the networks draw their taus with `torch.rand` (atari_lib.py:180-181).  With
+  `cuda_graph=True` the whole update is captured once and replayed as one CUDA graph
+  (`GraphedUpdate`); its taus are then drawn into three static buffers, `online_taus`
+  (N * B, 1), `target_taus` (N' * B, 1) and `action_taus` (K * B, 1), refilled in place
+  at every update from a CUDA generator of the learner seeded from `seed`, so that every
+  replay draws fresh ones.  `q_values` (acting) keeps drawing its own taus and does not
+  move that generator."""
 
   def __init__(self, num_actions, observation_shape=(84, 84), stack_size=4, kappa=1.0,
                num_tau_samples=32, num_tau_prime_samples=32, num_quantile_samples=32,
                quantile_embedding_dim=64, double_dqn=False, gamma=0.99, update_horizon=3,
                replay_capacity=1000000, batch_size=32, target_update_period=8000,
                update_period=4, learning_rate=0.00005, adam_epsilon=0.0003125, seed=0,
-               memory=None):
+               memory=None, cuda_graph=False):
     torch = _torch()
     self.num_actions = num_actions
     self.kappa = kappa
@@ -103,10 +114,38 @@ class IQNLearner(object):
     self.target.load_state_dict(self.online.state_dict())
     for p in self.target.parameters():
       p.requires_grad_(False)
+    self._cuda_graph = bool(cuda_graph)
+    self._graph = None
+    self._static_loss = None
+    # with cuda_graph, Adam's step count lives on the device so that it can be captured
     self.optimizer = conv.make_tf_adam(self.online.parameters(), lr=learning_rate,
-                                       epsilon=adam_epsilon)  # implicit_quantile.gin:26-29
+                                       epsilon=adam_epsilon,  # implicit_quantile.gin:26-29
+                                       capturable=self._cuda_graph)
+    self._generator = None
+    if self._cuda_graph:
+      self._init_taus(batch_size, [seed])
     self.training_steps = 0
     self.updates = 0
+
+  def _init_taus(self, rows, entropy):
+    """The three static tau buffers for `rows` batch rows and the CUDA generator that
+    refills them, seeded from `entropy` (a list of ints)."""
+    torch = _torch()
+    self._generator = torch.Generator(device='cuda')
+    self._generator.manual_seed(
+        int(np.random.SeedSequence([int(e) for e in entropy]).generate_state(1)[0]))
+    taus = lambda samples: torch.zeros(samples * rows, 1, device='cuda')
+    self.online_taus = taus(self.num_tau_samples)
+    self.target_taus = taus(self.num_tau_prime_samples)
+    self.action_taus = taus(self.num_quantile_samples)
+
+  def _draw_taus(self):
+    """Fresh taus in the static buffers (atari_lib.py:180-181)."""
+    for t in (self.online_taus, self.target_taus, self.action_taus):
+      t.uniform_(0., 1., generator=self._generator)
+
+  def _graph_generators(self):
+    return (self._generator,)
 
   def store_transition(self, last_observation, action, reward, is_terminal):
     """rainbow_agent.py:307-337 with the uniform scheme: priority 1."""
@@ -119,7 +158,8 @@ class IQNLearner(object):
       values, _ = self.online(state, self.num_quantile_samples)
       return values.view(self.num_quantile_samples, -1, self.num_actions).mean(0)
 
-  def train_step(self):
+  # train_step() is GraphedUpdate's
+  def _update(self):
     """implicit_quantile_agent.py:166-321: online net on `state` with N taus, target net
     on `next_state` with N' taus, the action-picking net with K taus (target net; online
     with double_dqn) -> greedy next action, target quantile values and quantile-Huber
@@ -127,18 +167,24 @@ class IQNLearner(object):
     torch = _torch()
     batch = self.memory.sample_transition_batch(self.batch_size)
     state, action, reward, next_state, _, _, terminal = batch[:7]
+    online_taus = target_taus = action_taus = None  # eager: drawn inside the networks
+    if self._generator is not None:
+      self._draw_taus()
+      online_taus, target_taus = self.online_taus, self.target_taus
+      action_taus = self.action_taus
     with torch.no_grad():
-      target_values, _ = self.target(next_state, self.num_tau_prime_samples)
+      target_values, _ = self.target(next_state, self.num_tau_prime_samples, target_taus)
       picker = self.online if self.double_dqn else self.target
-      action_values, _ = picker(next_state, self.num_quantile_samples)
-    online_values, quantiles = self.online(state, self.num_tau_samples)
+      action_values, _ = picker(next_state, self.num_quantile_samples, action_taus)
+    online_values, quantiles = self.online(state, self.num_tau_samples, online_taus)
     loss, _ = iqn.QuantileHuberLoss.apply(
         online_values, quantiles, target_values, action_values, action, reward, terminal,
         self.cumulative_gamma, self.kappa)
     self.optimizer.zero_grad(set_to_none=True)
     loss.backward()
     self.optimizer.step()
-    self.updates += 1
+    if not self._cuda_graph or self._graph is None:
+      self.updates += 1
     return loss
 
   def sync_target(self):
@@ -153,6 +199,61 @@ class IQNLearner(object):
       self.sync_target()
     self.training_steps += 1
     return loss
+
+
+class ImplicitQuantileAgent(IQNLearner, dqn_agent.ActingLoop):
+  """`ImplicitQuantileAgent` (implicit_quantile_agent.py, on the acting loop of
+  dqn_agent.py:341-560) as the reference's runner sees it: `begin_episode(observation)`,
+  `step(reward, observation)`, `end_episode(reward)`, `eval_mode`,
+  `bundle_and_checkpoint`, `unbundle`.  IQN's own arguments keep the reference's names
+  and defaults; the `RainbowAgent` arguments the reference forwards through `**kwargs`
+  are explicit here, with implicit_quantile.gin's numbers as `IQNLearner` has them.
+  `sess`, `tf_device`, `use_staging`, `optimizer` (always TensorFlow's Adam,
+  `learning_rate` / `adam_epsilon`) and the summary arguments have no meaning here.
+  Replay is uniform (implicit_quantile.gin:23-24): transitions are stored with priority
+  1.  The greedy action is the first argmax of the mean over `num_quantile_samples`
+  quantile values (`IQNLearner.q_values`, implicit_quantile_agent.py:148-164)."""
+
+  def __init__(self, sess=None, num_actions=None, kappa=1.0, num_tau_samples=32,
+               num_tau_prime_samples=32, num_quantile_samples=32,
+               quantile_embedding_dim=64, double_dqn=False, summary_writer=None,
+               summary_writing_frequency=500, observation_shape=(84, 84),
+               observation_dtype=np.uint8, stack_size=4, gamma=0.99, update_horizon=3,
+               min_replay_history=20000, update_period=4, target_update_period=8000,
+               epsilon_fn=dqn_agent.linearly_decaying_epsilon, epsilon_train=0.01,
+               epsilon_eval=0.001, epsilon_decay_period=250000, tf_device='/cpu:*',
+               use_staging=True, optimizer=None, replay_capacity=1000000, batch_size=32,
+               learning_rate=0.00005, adam_epsilon=0.0003125, seed=0,
+               allow_partial_reload=False, memory=None, cuda_graph=False):
+    del sess, summary_writer, summary_writing_frequency, tf_device, use_staging
+    del optimizer
+    if num_actions is None:
+      raise ValueError('num_actions is required')
+    if np.dtype(observation_dtype) != np.uint8:
+      raise NotImplementedError('the convolutional network takes uint8 frames')
+    IQNLearner.__init__(
+        self, num_actions, observation_shape=observation_shape, stack_size=stack_size,
+        kappa=kappa, num_tau_samples=num_tau_samples,
+        num_tau_prime_samples=num_tau_prime_samples,
+        num_quantile_samples=num_quantile_samples,
+        quantile_embedding_dim=quantile_embedding_dim, double_dqn=double_dqn,
+        gamma=gamma, update_horizon=update_horizon, replay_capacity=replay_capacity,
+        batch_size=batch_size, target_update_period=target_update_period,
+        update_period=update_period, learning_rate=learning_rate,
+        adam_epsilon=adam_epsilon, seed=seed, memory=memory, cuda_graph=cuda_graph)
+    self._init_acting(observation_shape, stack_size, observation_dtype,
+                      min_replay_history=min_replay_history,
+                      update_period=update_period,
+                      target_update_period=target_update_period,
+                      epsilon_fn=epsilon_fn, epsilon_train=epsilon_train,
+                      epsilon_eval=epsilon_eval,
+                      epsilon_decay_period=epsilon_decay_period,
+                      allow_partial_reload=allow_partial_reload)
+
+  def _store_transition(self, last_observation, action, reward, is_terminal):
+    """rainbow_agent.py:307-337 with the uniform scheme: priority 1."""
+    if not self.eval_mode:
+      self.store_transition(last_observation, action, reward, is_terminal)
 
 
 class ShardedIQNLearner(sharded_learner.ShardedLearner, IQNLearner):
@@ -188,7 +289,6 @@ class ShardedIQNLearner(sharded_learner.ShardedLearner, IQNLearner):
   def __init__(self, num_actions, batch_size=32, max_rows=None, exchange=None,
                group=None, exchange_timeout_s=2.0, ddp=False, cuda_graph=False,
                **kwargs):
-    torch = _torch()
     exchange = self._connect(exchange, group, exchange_timeout_s, ddp)
     IQNLearner.__init__(self, num_actions, batch_size=batch_size, **kwargs)
     self._cuda_graph = bool(cuda_graph)
@@ -200,23 +300,13 @@ class ShardedIQNLearner(sharded_learner.ShardedLearner, IQNLearner):
                                          epsilon=adam['epsilon'], capturable=True)
     seed = kwargs.get('seed', 0)
     self._shard(exchange, max_rows, seed, sharded_replay.ShardedPrioritizedReplay)
-    self._generator = torch.Generator(device='cuda')
-    self._generator.manual_seed(
-        int(np.random.SeedSequence([int(seed), self.rank]).generate_state(1)[0]))
-    taus = lambda samples: torch.zeros(samples * self.max_rows, 1, device='cuda')
-    self.online_taus = taus(self.num_tau_samples)
-    self.target_taus = taus(self.num_tau_prime_samples)
-    self.action_taus = taus(self.num_quantile_samples)
-
-  def _graph_generators(self):
-    return (self._generator,)
+    self._init_taus(self.max_rows, [seed, self.rank])
 
   # -- phases (reduce: ShardedLearner's) ----------------------------------------------
   def sample(self):
     """This rank's share of the global batch, then fresh taus (:180-181)."""
     sample = super(ShardedIQNLearner, self).sample()
-    for t in (self.online_taus, self.target_taus, self.action_taus):
-      t.uniform_(0., 1., generator=self._generator)
+    self._draw_taus()
     return sample
 
   def loss_backward(self):

@@ -1185,13 +1185,14 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
 }
 
 struct UniformSampleArgs {
-  ValidCtx valid;
+  // read from HBM (refreshed by every flush), not passed by value: a captured CUDA graph
+  // samples over the transitions added since the capture
+  const ValidCtx *valid_dev;
   int batch;
   int max_attempts;
   int use_philox;
   uint64_t seed, offset;
   uint64_t *counter;
-  int64_t min_id, max_id;      // Philox mode: candidates in [min_id, max_id)
   int n_cand;                  // host mode: number of supplied candidates
   const int64_t *candidates;   // np.random.randint(min_id, max_id) draws
   int32_t *out_idx;
@@ -1202,13 +1203,22 @@ struct UniformSampleArgs {
 // circular_replay_buffer.py:462-470 over a window of candidate draws.
 __global__ void __launch_bounds__(1024) uniform_sample_kernel(UniformSampleArgs a) {
   __shared__ int warp_counts[32];
+  __shared__ ValidCtx s_valid;
   pdl_release();
   pdl_acquire();
+  for (int w = threadIdx.x; w < (int)(sizeof(ValidCtx) / 8); w += blockDim.x)
+    reinterpret_cast<uint64_t *>(&s_valid)[w] =
+        reinterpret_cast<const uint64_t *>(a.valid_dev)[w];
   int accepted = a.counters[0], rejected = a.counters[1], used = 0;
   const uint64_t draws_before = a.counter ? *a.counter : 0ull;
   const uint64_t draw_offset = a.offset + draws_before;
   __syncthreads();
-  const int64_t span = a.max_id - a.min_id;
+  const ValidCtx &c = s_valid;
+  // Philox mode: uniform_bounds (CRB:449-460) on the device; the host has checked that
+  // the span is not empty
+  const int64_t min_id = c.add_count >= c.capacity ? c.cursor - c.capacity + c.stack - 1
+                                                   : c.stack - 1;
+  const int64_t span = c.cursor - c.horizon - min_id;
   int base = 0;
   while (accepted < a.batch && rejected < a.max_attempts &&
          (a.use_philox || base < a.n_cand)) {
@@ -1222,12 +1232,12 @@ __global__ void __launch_bounds__(1024) uniform_sample_kernel(UniformSampleArgs 
         const double u = philox_uniform53(a.seed, draw_offset, (uint64_t)p);
         int64_t off = (int64_t)(u * (double)span);
         if (off >= span) off = span - 1;
-        cand = a.min_id + off;
+        cand = min_id + off;
       } else {
         cand = a.candidates[p];
       }
-      idx = wrap_index(cand, a.valid.capacity);  // `% replay_capacity`, CRB:466
-      valid = is_valid_transition(a.valid, idx);
+      idx = wrap_index(cand, c.capacity);  // `% replay_capacity`, CRB:466
+      valid = is_valid_transition(c, idx);
     }
     int tile_acc, tile_rej, tile_done;
     const int acc_before = accepted + block_scan_flag(active && valid, warp_counts, &tile_acc);
@@ -1913,14 +1923,14 @@ int b2r_sample_indices_uniform(b2r_buffer *b, int32_t batch, int32_t n_cand,
   memcpy(b->bounce.host + off_cnt, cnt, 16);
   B2R_CUDA(cudaMemcpyAsync(b->bounce.dev, b->bounce.host, off_cnt + 16,
                            cudaMemcpyHostToDevice, s));
+  B2R_TRY(b2r::ensure_ctx(b, s));
   b2r::UniformSampleArgs a;
-  b2r::fill_valid_ctx(b, &a.valid);
+  a.valid_dev = b->ctx_dev;
   a.batch = batch;
   a.max_attempts = b->cfg.max_sample_attempts;
   a.use_philox = 0;
   a.seed = a.offset = 0;
   a.counter = nullptr;
-  a.min_id = a.max_id = 0;
   a.n_cand = n_cand;
   a.candidates = reinterpret_cast<const int64_t *>(b->bounce.dev);
   a.out_idx = reinterpret_cast<int32_t *>(b->bounce.dev + off_out);
@@ -1991,9 +2001,11 @@ int b2r_sample_indices_device(b2r_buffer *b, int32_t batch, uint64_t seed,
   if (b->tree)
     return b2r::launch_sample(b, batch, true, seed, offset, nullptr, nullptr, 0,
                               out_indices, b->info, s);
+  int64_t min_id, max_id;  // (the kernel recomputes them from the device context)
+  B2R_TRY(b2r::uniform_bounds(b, &min_id, &max_id));
+  B2R_TRY(b2r::ensure_ctx(b, s));
   b2r::UniformSampleArgs a;
-  b2r::fill_valid_ctx(b, &a.valid);
-  B2R_TRY(b2r::uniform_bounds(b, &a.min_id, &a.max_id));
+  a.valid_dev = b->ctx_dev;
   a.batch = batch;
   a.max_attempts = b->cfg.max_sample_attempts;
   a.use_philox = 1;

@@ -314,9 +314,13 @@ class OutOfGraphReplayBuffer(object):
   def invalid_range(self, value):
     self._set_state(int(self.add_count), value)
 
+  def _flush(self):
+    """Applies the staged adds (and with them the validity context in HBM)."""
+    _native.check(self._lib.b2r_flush(self._h, self._stream()))
+
   def _set_state(self, add_count, invalid):
     invalid = np.ascontiguousarray(np.asarray(invalid).astype(np.int64))
-    _native.check(self._lib.b2r_flush(self._h, self._stream()))
+    self._flush()
     _native.check(self._lib.b2r_set_state(self._h, add_count,
                                           _native.ptr(invalid), len(invalid)))
 

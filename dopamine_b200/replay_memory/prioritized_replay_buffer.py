@@ -130,9 +130,6 @@ class OutOfGraphPrioritizedReplayBuffer(
     self.sum_tree = sum_tree.SumTree(
         replay_capacity, _handle=tree_handle, _before_read=self._flush)
 
-  def _flush(self):
-    _native.check(self._lib.b2r_flush(self._h, self._stream()))
-
   def get_add_args_signature(self):
     parent_add_signature = super(OutOfGraphPrioritizedReplayBuffer,
                                  self).get_add_args_signature()
