@@ -53,6 +53,16 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// The first output atom whose projection interval is open above.  Bellman atoms at or
+// above zlast clip to it, and reach atom i wherever zlast - z_i < dz: the last atom, and
+// also atom N - 2 on the f32 supports whose last spacing rounds below dz = z[1] - z[0]
+// (vmax 10 at 64 or 101 atoms, not at 51).  Their hat there is a few millionths, but
+// the dense form adds it.
+__device__ __forceinline__ int clipped_reach_below_last(float zprev, float zlast, float dz,
+                                                        int n) {
+  return __fsub_rn(zlast, zprev) < dz ? n - 2 : n - 1;
+}
+
 // out[i] = sum_j clip(1 - |clip(s_j, z0, zlast) - z_i| / dz, 0, 1) * w_j
 // (rainbow_agent.py:424-492); s, w in shared memory, i strided over lanes.
 __device__ __forceinline__ float project_atom(const float *s, const float *w,
@@ -408,15 +418,16 @@ __global__ void __launch_bounds__(1024, 1) c51_loss_kernel(LossArgs a) {
   const float *next_p = smem + (size_t)win * N;
   const float z0 = zs[0], zlast = zs[N - 1];
   const float dz = __fsub_rn(zs[1], zs[0]);
+  const int open_above = clipped_reach_below_last(zs[N - 2], zlast, dz, N);
   // The dense form sums hat(i, j) * p_j over all j, but hat is exactly 0 unless
   // |clip(s_j) - z_i| < dz.  The Bellman atoms s_j = r + g * z_j are non-decreasing
   // in j (g = gamma^n (1 - terminal) >= 0), so the j that can reach atom i form one
   // interval: those with s_j inside (z_i - dz, z_i + dz), open-ended below for the
-  // first atom and above for the last one (clipping).  Each thread evaluates the
-  // reference's expression over a conservative superset of its interval (two extra
-  // positions either side cover any rounding of the bounds; terminal rows, where all
-  // s_j coincide, take the whole range) in ascending j.  Skipped terms are exact
-  // zeros, so the sum is the dense form's.
+  // first atom and above for the atoms from open_above up (clipping).  Each thread
+  // evaluates the reference's expression over a conservative superset of its interval
+  // (two extra positions either side cover any rounding of the bounds; terminal rows,
+  // where all s_j coincide, take the whole range) in ascending j.  Skipped terms are
+  // zeros of the dense form, so the sum is its sum in the same order.
 #pragma unroll 1
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     const float zi = zs[i];
@@ -427,7 +438,8 @@ __global__ void __launch_bounds__(1024, 1) c51_loss_kernel(LossArgs a) {
       const float lo = (zi - dz - r - gwt * z0) * inv;
       const float hi = (zi + dz - r - gwt * z0) * inv;
       if (i > 0 && lo > 2.f) jl = min(N - 1, (int)fminf(lo, 1e6f) - 2);
-      if (i < N - 1 && hi < (float)(N - 3)) jh = max(0, (int)fmaxf(hi, -1e6f) + 3);
+      if (i < open_above && hi < (float)(N - 3))
+        jh = min(N - 1, max(0, (int)fmaxf(hi, -1e6f) + 3));  // (N <= 3: hi may be < 0)
     }
     float acc = 0.f;
 #pragma unroll 1
@@ -713,13 +725,14 @@ c51_loss_rows_kernel(LossArgs a) {
     // |clip(s_j) - z_i| < dz, and the Bellman atoms s_j = r + g z_j are non-decreasing
     // in j (g >= 0), so the j that reach atom i form one interval: s_j inside
     // (z_i - dz, z_i + dz), i.e. lo < j < hi in units of atoms, open-ended below for
-    // the first atom and above for the last (clipping).  Each lane sums the
-    // reference's expression in ascending j over [floor(lo), floor(hi) + 1]: one
-    // spare position either side, against a rounding error of lo / hi below 1e-4.
-    // Skipped terms are exact zeros, so the sum is the dense form's.
+    // the first atom and above for the atoms from open_above up (clipping).  Each lane
+    // sums the reference's expression in ascending j over [floor(lo), floor(hi) + 1]:
+    // one spare position either side, against a rounding error of lo / hi below 1e-4.
+    // Skipped terms are zeros of the dense form, so the sum is its sum in the same order.
     const float *sup = s_sup[warp], *next_p = s_bestp[warp];
     const float z0 = z[0], zlast = z[N - 1];
     const float dz = __fsub_rn(z[1], z0);
+    const int open_above = clipped_reach_below_last(z[N - 2], zlast, dz, N);
     float tg[2] = {0.f, 0.f};
     float ce_part = 0.f, tsum_part = 0.f;
 #pragma unroll
@@ -746,7 +759,7 @@ c51_loss_rows_kernel(LossArgs a) {
             const float lo = (zi - dz - r - gwt * z0) * inv;
             const float hi = (zi + dz - r - gwt * z0) * inv;
             if (i > 0 && lo > 0.f) jl = min(N - 1, (int)fminf(lo, 1e6f));
-            if (i < N - 1 && hi < (float)(N - 2)) jh = max(0, (int)fmaxf(hi, -1e6f) + 1);
+            if (i < open_above && hi < (float)(N - 2)) jh = max(0, (int)fmaxf(hi, -1e6f) + 1);
           }
 #pragma unroll 1
           for (int j = jl; j <= jh; ++j) {
@@ -1082,7 +1095,8 @@ __global__ void __launch_bounds__(kRowWarps * 32) c51_pre_rows_kernel(PreArgs a)
 }
 
 constexpr int kProjTerms = 5;  // Bellman atoms within dz of an output atom, with slack
-                              // (gamma^n >= 2/3: 2 / (gamma^n) + 2 <= 5; wider: the loop)
+                              // (gamma^n >= 2/3: 2 / (gamma^n) + 2 <= 5; wider, or atom
+                              // N - 2 open above with clipped mass beyond: the loop)
 
 // The part of a row's tail that follows its scalars and the log-probabilities of its
 // chosen action: Bellman support, projection, cross entropy and the row's outputs.
@@ -1110,7 +1124,9 @@ __device__ __forceinline__ float c51_post_finish(const LossArgs &a, int b, int r
   const float z0 = __shfl_sync(0xffffffffu, zl[0], 0);
   const float z1 = __shfl_sync(0xffffffffu, zl[0], 1);
   const float zlast = __shfl_sync(0xffffffffu, N > 32 ? zl[1] : zl[0], (N - 1) & 31);
+  const float zprev = __shfl_sync(0xffffffffu, N > 33 ? zl[1] : zl[0], (N - 2) & 31);
   const float dz = __fsub_rn(z1, z0);
+  const int open_above = clipped_reach_below_last(zprev, zlast, dz, N);
   float tg[2] = {0.f, 0.f};
   if (gwt == 0.f) {
     // terminal row: every s_j is r, so hat(i, .) is one number, and it is 0 for all but
@@ -1141,7 +1157,7 @@ __device__ __forceinline__ float c51_post_finish(const LossArgs &a, int b, int r
         const float lo = (zl[t] - dz - r - gwt * z0) * inv;
         const float hi = (zl[t] + dz - r - gwt * z0) * inv;
         if (i > 0 && lo > 0.f) jl[t] = min(N - 1, (int)fminf(lo, 1e6f));
-        if (i < N - 1 && hi < (float)(N - 2)) jh[t] = max(0, (int)fmaxf(hi, -1e6f) + 1);
+        if (i < open_above && hi < (float)(N - 2)) jh[t] = max(0, (int)fmaxf(hi, -1e6f) + 1);
       }
     }
     const bool narrow = jh[0] - jl[0] < kProjTerms && jh[1] - jl[1] < kProjTerms;
