@@ -871,6 +871,9 @@ struct PreArgs {
   // logits, and StageGate::done, counted when they are all there
   float *logp;
   unsigned int *staged_done;
+  // The one-stream step (RowsGate): launched behind the sampler, which waits for this
+  // launch's signal before it ends, so the griddepcontrol.wait comes after the signal.
+  int wait_late;
 };
 
 // CTA per row, warp per action (rows below 128: latency-bound).
@@ -883,7 +886,7 @@ __global__ void __launch_bounds__(1024) c51_pre_kernel(PreArgs a) {
   const int N = a.num_atoms, A = a.num_actions, W = a.warps;
   B2R_MARK(0);
   pdl_release();
-  pdl_acquire();
+  if (!a.wait_late) pdl_acquire();
   B2R_MARK(1);
   const float *__restrict__ trow = a.target_logits + (size_t)b * A * N;
   const float *__restrict__ orow = a.online_logits + (size_t)b * A * N;
@@ -1000,6 +1003,7 @@ __global__ void __launch_bounds__(1024) c51_pre_kernel(PreArgs a) {
   }
   B2R_MARK_END(8);
   pre_sync_signal(a.sync, a.staged_done);
+  if (a.wait_late) pdl_acquire();
 }
 
 // Warp per row, G lanes per action (rows from 128 up: bound by instruction issue).
@@ -1489,7 +1493,7 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
   __shared__ float s_prio[kTinyBatch];      // (CTA 0's copy is the one that is used)
   __shared__ float s_weighted[kTinyBatch];
   __shared__ __align__(8) uint64_t s_arrived;  // mbarrier: the rows' words have landed
-  __shared__ bool s_gate;
+  __shared__ bool s_gate, s_rows;
   extern __shared__ float4 s_logp[];  // STAGED: [kPostRowWarps][c51_logp_stride / 4]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const bool tree_cta = blockIdx.x == 0;
@@ -1512,7 +1516,15 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
   const bool early = STAGED && s_gate;
   if (early && stages) c51_stage_row(a, scratch, srow, lane, s_bestp[warp], logp_row, zl);
   if (STAGED) B2R_MARK_CTA(15, 1);
-  pdl_acquire();
+  // The one-stream step: the predecessor is the frame copies, not the sampler — the rows
+  // are there once the sampler has counted its launch (RowsGate); the griddepcontrol.wait
+  // moves to the exits.  (Either gate timed out: behind the wait, the safe order.)
+  const bool gated = STAGED && a.stage.rows.done != nullptr;
+  if (gated) {
+    if (threadIdx.x == 0) s_rows = rows_gate_wait(a.stage.rows);
+    __syncthreads();
+  }
+  if (!gated || !(s_rows && early)) pdl_acquire();
   if (STAGED && !early && stages) c51_stage_row(a, scratch, srow, lane, s_bestp[warp], logp_row, zl);
   B2R_MARK(11);
   // (a shard's step: the row count is on the device, and the write-back rides along only
@@ -1554,7 +1566,10 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
   }
   B2R_MARK_END(12);
   cluster_wait();
-  if (!with_tree) return;
+  if (!with_tree) {
+    if (gated) pdl_acquire();
+    return;
+  }
   if (!tree_cta) {
     // the row's priority (and weighted loss) into CTA 0's shared memory, counted on its
     // mbarrier: no fence, no second barrier
@@ -1562,6 +1577,7 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
       st_async_u32(&s_prio[my_row], __float_as_uint(prio), &s_arrived, 0);
       if (want_mean) st_async_u32(&s_weighted[my_row], __float_as_uint(weighted), &s_arrived, 0);
     }
+    if (gated) pdl_acquire();
     return;
   }
   mbar_wait(&s_arrived, 0);
@@ -1575,6 +1591,7 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
     acc = group_sum<32>(acc);
     if (lane == 0) *a.u.mean_weighted_loss = __fdiv_rn(acc, (float)rows);
   }
+  if (gated) pdl_acquire();
 }
 
 float *g_weighted = nullptr;
@@ -1707,6 +1724,7 @@ int c51_pre_launch(const b2r_c51_args *args, int rows, float *scratch, const Pre
   a.sync = sync;
   a.logp = stage != nullptr ? stage->logp : nullptr;
   a.staged_done = stage != nullptr ? stage->done : nullptr;
+  a.wait_late = stage != nullptr && stage->rows.done != nullptr ? 1 : 0;
   if (rows >= 128) {
     const dim3 grid((rows + kRowWarps - 1) / kRowWarps), block(kRowWarps * 32);
     if (args->num_atoms == 51)

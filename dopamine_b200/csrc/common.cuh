@@ -186,6 +186,21 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
       "r"(parity)
       : "memory");
 }
+// The same with acquire at cluster scope: what the senders wrote before their st.async (whose
+// complete-tx releases at cluster scope), global memory included, happens before what follows.
+__device__ __forceinline__ void mbar_wait_cluster(uint64_t *bar, uint32_t parity) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "WAIT_%=:\n"
+      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n"
+      "@p bra DONE_%=;\n"
+      "bra WAIT_%=;\n"
+      "DONE_%=:\n"
+      "}\n" ::"r"(smem_u32(bar)),
+      "r"(parity)
+      : "memory");
+}
 // word -> the same shared-memory location in CTA `rank` of the cluster, counted on that
 // CTA's mbarrier (both given as THIS CTA's addresses of the corresponding variables)
 __device__ __forceinline__ void st_async_u32(void *local_dst, uint32_t value, uint64_t *local_bar,

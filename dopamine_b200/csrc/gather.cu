@@ -39,6 +39,7 @@ struct GatherArgs {
   int32_t scalar_rows;   // grid rows of appended scalar CTAs (0: frames only)
   ScalarArgs sc;
   const int32_t *count;  // nullable: device-side number of rows (<= batch)
+  RowsGate gate;         // the one-stream step (TMA copies only; done == nullptr: none)
 };
 
 // [a0 a1 a2 a3] x4 frames -> 4 words [a_p b_p c_p d_p], p = 0..3.
@@ -187,8 +188,19 @@ gather_stack4_u8_tma_kernel(const __grid_constant__ GatherArgs a) {
   extern __shared__ __align__(128) uint8_t tma_smem[];
   __shared__ __align__(8) uint64_t bar;
   __shared__ int s_length;
+  __shared__ bool s_rows;
+  B2R_MARK(0);
   pdl_release();
-  pdl_acquire();
+  // The one-stream step: the predecessor is the first half of the loss; the indices are
+  // final once the sampler has counted its launch (RowsGate), and the griddepcontrol.wait
+  // moves to the end (the copies have landed when the step's last kernel completes).
+  const bool gated = a.gate.done != nullptr;
+  if (gated) {
+    if (threadIdx.x == 0) s_rows = rows_gate_wait(a.gate);
+    __syncthreads();
+  }
+  if (!gated || !s_rows) pdl_acquire();
+  B2R_MARK(1);
   const int rows = a.count ? min(*a.count, a.batch) : a.batch;
   if (SCALARS && (int)blockIdx.x >= a.batch) {  // appended scalar CTAs
     const int b = ((int)blockIdx.x - a.batch) * blockDim.x + threadIdx.x;
@@ -236,6 +248,8 @@ gather_stack4_u8_tma_kernel(const __grid_constant__ GatherArgs a) {
       reinterpret_cast<uint4 *>(out_next)[o] = v;
     }
   }
+  B2R_MARK_END(6);
+  if (gated) pdl_acquire();
 }
 
 // General path: any stack size / element size. thread = one observation element.
@@ -346,10 +360,23 @@ void fill_scalar_args(const b2r_buffer *b, const b2r_batch *out, ScalarArgs *sc)
   sc->next_reward_out = static_cast<float *>(out->next_reward);
 }
 
+// Gated copies always launch this many CTAs (those beyond the batch only take their ticket):
+// a launch's number is ticket / CTAs only while every launch has the same grid.
+constexpr int kGatedCopyCtas = kTinyBatch;
+
+bool gather_can_gate(const b2r_buffer *b, int32_t batch) {
+  return batch <= kGatedCopyCtas && b->cfg.stack_size == 4 && b->cfg.obs_itemsize == 1 && (b->cfg.obs_bytes & 15) == 0 &&
+         gather_variant(batch) == 1 &&
+         (size_t)kTmaMaxFrames * (size_t)b->cfg.obs_bytes <= 200 * 1024;
+}
+
 int launch_gather(b2r_buffer *b, int32_t batch, const int32_t *indices_dev,
                   const b2r_batch *out, cudaStream_t stream,
-                  const int32_t *count_dev, bool frames_only) {
+                  const int32_t *count_dev, bool frames_only, const RowsGate *gate) {
+  if (gate != nullptr && (count_dev != nullptr || !frames_only || !gather_can_gate(b, batch)))
+    return fail(B2R_ERR_INVALID_ARGUMENT, "only the TMA frame copies of a counted batch gate");
   GatherArgs a;
+  if (gate != nullptr) a.gate = *gate;
   a.count = count_dev;
   a.capacity = b->cfg.capacity;
   a.stack = b->cfg.stack_size;
@@ -378,7 +405,7 @@ int launch_gather(b2r_buffer *b, int32_t batch, const int32_t *indices_dev,
       ready = true;
     }
     a.scalar_rows = frames_only ? 0 : (batch + kTmaThreads - 1) / kTmaThreads;
-    dim3 grid(batch + a.scalar_rows);
+    dim3 grid(gate != nullptr ? kGatedCopyCtas : batch + a.scalar_rows);
     if (frames_only)
       B2R_CUDA(launch_prio(gather_stack4_u8_tma_kernel<false>, grid, dim3(kTmaThreads),
                            tma_bytes, stream, 0, a));

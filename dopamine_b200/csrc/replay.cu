@@ -400,8 +400,8 @@ int b2r_create(const b2r_config *cfg, b2r_buffer **out) {
     cudaDeviceGetStreamPriorityRange(&least, &greatest);
     B2R_CUDA(cudaStreamCreateWithPriority(&b->side3, cudaStreamNonBlocking, greatest));
   }
-  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->pre_sync), 32));
-  B2R_CUDA(cudaMemset(b->pre_sync, 0, 32));
+  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->pre_sync), 64));
+  B2R_CUDA(cudaMemset(b->pre_sync, 0, 64));
   for (int k = 0; k < 2; ++k)
     B2R_CUDA(cudaEventCreateWithFlags(&b->ev_slot_free[k], cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_c51_fork, cudaEventDisableTiming));

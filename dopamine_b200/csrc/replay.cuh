@@ -75,6 +75,10 @@ __device__ __forceinline__ int block_scan_flag(bool flag, int *warp_counts,
 // (acquire) before the kernel ends, and the tail has the sampler as its only parent.
 // The first half is a few microseconds of work that starts together with the sampler,
 // so the wait normally finds the bump already there.
+// Only the fork/join step needs this hand-shake for its ordering; the one-stream step
+// (step.cu: train_step, RowsGate) orders the first half behind the sampler on the stream
+// and keeps the sampler's wait only so that `done` and `seen` advance the same way on both
+// paths, which may alternate on one buffer.
 struct PreSync {
   unsigned int *done;    // first-half launches completed (monotone); nullptr: no hand-shake
   unsigned int *seen;    // ... consumed by a sampler (touched by its closing thread only)
@@ -96,10 +100,30 @@ struct PreSync {
 // The scratch is two halves by step parity: the first half of step n + 1 writes the other
 // half, and that of step n + 2 is ordered behind the tail of step n (stream order, or
 // DirectIO::first_half_after) — no first half overwrites rows a tail may still read.
+// The one-stream step (step.cu: train_step at the agent's batch with its frame copies joined
+// and nothing else to wait for): sampler, first half, frame copies and tail run in this order
+// on the caller's stream, each launched programmatically behind the one before, so that every
+// kernel node of a captured step has ONE parent and keeps its early launch — the next step's
+// sampler included.  The copies and the tail no longer learn from their predecessor's
+// completion that the sampled rows are there: the sampler's closing thread counts its launch
+// in `done` (release) once every row, the minimum and the counters are final, and every CTA
+// of a gated copy or tail launch takes a ticket (ticket / CTAs = its launch number k, as in
+// StageGate) and reads the rows once done >= k + 1.  Samplers, copies and tails of this kind
+// are launched together by one host call, and only by it: the counts stay paired.
+// Completion stays transitive: the first half, the copies and the tail each pass their
+// griddepcontrol.wait before they exit (the first half after it has signalled the sampler),
+// so "tail n complete" means all of step n is complete, the copies included.  The sampler lets
+// its dependents launch only after its own griddepcontrol.wait: the first half of step n + 1
+// then starts after the tail of step n has ended, never while it reads the scratch half.
+struct RowsGate {
+  unsigned int *done = nullptr;           // sampler launches with final rows (monotone)
+  unsigned long long *tickets = nullptr;  // CTAs of this consumer's gated launches (monotone)
+};
 struct StageGate {
   unsigned int *done = nullptr;           // staged first halves completed (monotone)
   unsigned long long *tickets = nullptr;  // CTAs of staged tails started (monotone)
   float *logp = nullptr;  // [rows][c51_logp_stride] log-probabilities, action-major
+  RowsGate rows;  // the one-stream step (done == nullptr: the fork/join step)
 };
 // Row stride of StageGate::logp: whole 16-byte words, so a row moves as float4s.
 __host__ __device__ __forceinline__ int c51_logp_stride(int actions, int atoms) {
@@ -139,6 +163,23 @@ __device__ __forceinline__ bool stage_gate_wait(const StageGate &g) {
   while ((int)(ld_acquire_u32(g.done) - launch) < 0)
     if (clock64() - t0 > 4000000000ll) return false;
   return true;
+}
+// By thread 0 of every CTA of a gated copy or tail launch (RowsGate), before it reads a row.
+// False after 2 s: the caller then falls back to its griddepcontrol.wait, which in the
+// one-stream order is behind the sampler's completion (correct, only late).
+__device__ __forceinline__ bool rows_gate_wait(const RowsGate &g) {
+  const unsigned long long ticket = atomicAdd(g.tickets, 1ull);
+  const unsigned int launch = (unsigned int)(ticket / gridDim.x) + 1u;
+  const long long t0 = clock64();
+  while ((int)(ld_acquire_u32(g.done) - launch) < 0) {
+    if (clock64() - t0 > 4000000000ll) return false;
+    __nanosleep(32);
+  }
+  return true;
+}
+// The sampler's last word (RowsGate::done): release, no round trip.
+__device__ __forceinline__ void rows_gate_publish(unsigned int *done) {
+  asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(done) : "memory");
 }
 // Called by the sampler's closing thread (ONE thread) before the kernel ends.  Gives up
 // after 2 s: a first half that never ran must not hang the GPU (the tail then reads stale
@@ -299,8 +340,9 @@ struct b2r_buffer {
   float *c51_bestp = nullptr;  // device [2 halves][c51_bestp_rows][64 probabilities | 64 stats]
   int64_t c51_bestp_rows = 0;
   int c51_half = 0;            // half the next step's first half writes
-  unsigned int *pre_sync = nullptr;  // device [8]: PreSync done, seen, ticket, tree_done,
-                                     // StageGate done, -, tickets (64 bits)
+  unsigned int *pre_sync = nullptr;  // device [16]: PreSync done, seen, ticket, tree_done,
+                                     // StageGate done, -, tickets (64 bits), RowsGate done,
+                                     // -, copy tickets (64 bits), tail tickets (64 bits), -, -
   float *c51_logp = nullptr;         // device [2 halves][c51_logp_half]: StageGate::logp
   int64_t c51_logp_half = 0;
   // Deferred frame copies (b2r_set_deferred_frames): the copies of a fused step are not
@@ -395,13 +437,19 @@ int flush_fused(b2r_tree *tree, int n, const int64_t *slots, const double *prio,
                 const uint8_t *mode, const AddParams &rows, int row_blocks_per_entry,
                 cudaStream_t stream, const b2r_exchange *publish = nullptr);
 int ensure_inv_slots(b2r_buffer *buf, int64_t n);
+// gate (nullable): frame copies of the one-stream step (RowsGate); only the TMA copies
+// (gather_can_gate) take one.
 int launch_gather(b2r_buffer *buf, int32_t batch, const int32_t *indices_dev,
                   const b2r_batch *out, cudaStream_t stream,
-                  const int32_t *count_dev = nullptr, bool frames_only = false);
+                  const int32_t *count_dev = nullptr, bool frames_only = false,
+                  const RowsGate *gate = nullptr);
+bool gather_can_gate(const b2r_buffer *buf, int32_t batch);
+// rows_done (nullable): RowsGate::done of the one-stream step (batches of the warp sampler,
+// with scalars and the minimum).
 int launch_sample(b2r_buffer *buf, int32_t batch, bool philox, uint64_t seed,
                   uint64_t offset, const double *strat_dev,
                   const double *retry_dev, int32_t n_retry, int32_t *out_idx_dev,
                   int32_t *info_dev, cudaStream_t stream,
                   const b2r_batch *scalars = nullptr, float *min_prob_out = nullptr,
-                  const PreSync *pre = nullptr);
+                  const PreSync *pre = nullptr, unsigned int *rows_done = nullptr);
 }  // namespace b2r

@@ -80,6 +80,10 @@ struct PerSampleArgs {
   // Exchange mode: the closing thread also stores min_prob_out's value into every peer's
   // mailbox for this step (b2r_sample_transition_batch_sharded_device).
   int publish_min;
+  // nullable: RowsGate::done of the one-stream step (replay.cuh), counted by the closing
+  // thread when rows, minimum and counters are final.  The kernel then lets its dependents
+  // launch only after its own griddepcontrol.wait.
+  unsigned int *rows_done;
 };
 
 // The local minimum of step `seq`, for the peers' sharded loss (b2r_c51_loss_sharded).
@@ -676,8 +680,9 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int warps = blockDim.x >> 5;
   B2R_MARK(10);
-  pdl_release();
+  if (a.rows_done == nullptr) pdl_release();
   pdl_acquire();
+  if (a.rows_done != nullptr) pdl_release();
   B2R_MARK(11);
   // every load of the prologue is issued before the first one is used; the nodes of
   // the first descent round (levels 1..5 under the root) ride along
@@ -722,6 +727,7 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       if (exchange) *a.xchg.seq = xseq;
       if (a.latched && a.latched[0] == 0) a.latched[0] = B2R_ERR_EMPTY_TREE;
       pre_sync_consume(a.pre);
+      if (a.rows_done != nullptr) rows_gate_publish(a.rows_done);
     }
     if (CLUSTER) cluster_wait();
     return;
@@ -899,6 +905,14 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       }
     }
   }
+  // The one-stream step: the copies and the tail read these rows once the closing thread has
+  // counted the launch (RowsGate), not behind the kernel's completion.  The order comes
+  // without a fence per row: every CTA sends its minimum word behind the barrier below,
+  // after all of its rows; the complete-tx of an st.async releases at cluster scope; CTA 0
+  // waits for every word with acquire at cluster scope (mbar_wait_cluster); and the closing
+  // thread counts the launch with a release at GPU scope, which passes on what it has
+  // acquired.  (Plain grids: the fence + ticket election below orders the rows before the
+  // last CTA.)
   B2R_MARK(16);
   if (want_min) {
     if (lane == 0) s_wmin[warp] = my_min;
@@ -917,7 +931,10 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
     // (the closing thread's look at the first half of the loss travels with the wait)
     PreSyncPeek peek = {0u, 1u};
     if (threadIdx.x == 0) peek = pre_sync_peek(a.pre);
-    mbar_wait(&s_arrived, 0);
+    if (a.rows_done != nullptr)
+      mbar_wait_cluster(&s_arrived, 0);
+    else
+      mbar_wait(&s_arrived, 0);
     ws.inv_flag = s_flag;
     ws.spec_idx = s_cl_spec_idx;
     ws.spec_valid = s_cl_spec_valid;
@@ -942,6 +959,9 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
         for (int o = 16; o > 0; o >>= 1) m = fminf(m, __shfl_xor_sync(full, m, o));
       }
       if (lane == 0) {
+        if (want_min) *a.min_prob_out = m;
+        // (rows and minimum are final: the count goes first, its release waits for them only)
+        if (a.rows_done != nullptr) rows_gate_publish(a.rows_done);
         if (a.counter) *a.counter = draws_before + 1;
         if (exchange) *a.xchg.seq = xseq;
         a.info[0] = B2R_OK;
@@ -949,7 +969,6 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
         a.info[2] = 0;
         a.info[3] = n_mine;
         if (a.count_out) *a.count_out = n_mine;
-        if (want_min) *a.min_prob_out = m;
         if (want_min) publish_local_min(a, exchange, m, xseq);
         pre_sync_consume(a.pre, peek);
       }
@@ -1120,6 +1139,7 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       __syncthreads();
     }
   }
+  if (a.rows_done != nullptr) __threadfence();  // (the fix-ups, before the count)
   __syncthreads();
   B2R_MARK_ANY(19);
   if (threadIdx.x == 0) {
@@ -1180,7 +1200,10 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
       publish_local_min(a, exchange, m, xseq);
     }
   }
-  if (threadIdx.x == 0) pre_sync_consume(a.pre);
+  if (threadIdx.x == 0) {
+    pre_sync_consume(a.pre);
+    if (a.rows_done != nullptr) rows_gate_publish(a.rows_done);
+  }
   B2R_MARK_ANY(20);
 }
 
@@ -1373,12 +1396,16 @@ int launch_sample(b2r_buffer *b, int32_t batch, bool philox, uint64_t seed,
                   uint64_t offset, const double *strat_dev,
                   const double *retry_dev, int32_t n_retry, int32_t *out_idx_dev,
                   int32_t *info_dev, cudaStream_t stream,
-                  const b2r_batch *scalars, float *min_prob_out, const PreSync *pre) {
+                  const b2r_batch *scalars, float *min_prob_out, const PreSync *pre,
+                  unsigned int *rows_done) {
   int threads, tiles;
   sample_shape(batch, &threads, &tiles);
   if (tiles > kMaxTiles)
     return fail(B2R_ERR_UNSUPPORTED, "batch above %d is not supported", kMaxTiles * 128);
   const bool by_warp = batch <= kSamplerWarpMax;
+  if (rows_done != nullptr && (!by_warp || !scalars || !min_prob_out))
+    return fail(B2R_ERR_INVALID_ARGUMENT,
+                "only the warp sampler with scalars and the minimum counts its rows");
   PerSampleArgs a;
   WarpScratch ws;
   if (by_warp)
@@ -1418,6 +1445,7 @@ int launch_sample(b2r_buffer *b, int32_t batch, bool philox, uint64_t seed,
   a.shard_ranges = 0;
   a.out_cap = batch;
   a.publish_min = 0;
+  a.rows_done = rows_done;
   a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
   if (pre != nullptr) a.pre = *pre;
   a.xchg.local = nullptr;
@@ -1531,6 +1559,7 @@ int launch_sample_sharded(b2r_buffer *b, int32_t global_batch, int32_t num_shard
   a.shard_ranges = ranges ? 1 : 0;
   a.out_cap = cap;
   a.publish_min = publish_min ? 1 : 0;
+  a.rows_done = nullptr;
   a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
   if (pre != nullptr) a.pre = *pre;
   a.xchg.local = nullptr;

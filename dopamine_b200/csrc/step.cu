@@ -9,7 +9,9 @@
 // the next step's sampler needs this step's write-back.  The frame stacks feed the
 // network, not this chain.  So the sampler emits the scalar columns itself, the
 // chain sample -> loss -> write-back runs on the caller's stream, and the HBM-bound
-// frame copies run beside it on a forked stream, joined before the call returns.
+// frame copies run beside it on a forked stream, joined before the call returns —
+// except at the agent's batch, where every kernel goes on the caller's stream (RowsGate,
+// replay.cuh: a joined fork would give the next step's sampler three parents).
 #include "gather.cuh"
 
 #include <cmath>
@@ -129,6 +131,17 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   // (StageGate, replay.cuh; the tail and the write-back are then one cluster, below).
   const bool staged = split_loss && !shard && c51_post_takes_tree(&loss, b->tree) &&
                       c51_tail_can_stage(&loss);
+  // The one-stream step (RowsGate, replay.cuh): sampler -> first half -> frame copies ->
+  // tail + write-back, all on `s`, every kernel launched programmatically behind the one
+  // before — in a captured graph every node then has ONE parent, and the next step's
+  // sampler keeps its early launch.  Only where nothing else joins the step: copies joined
+  // before the call returns, no direct I/O, no event to wait for.  (Programmatic launch is
+  // required: the sampler's closing thread waits for the first half, launched behind it.)
+  const bool frames = out->state != nullptr || out->next_state != nullptr;
+  const bool one_stream = staged && frames && !b->deferred_frames && direct == nullptr &&
+                          wait_before_loss == nullptr && pdl_enabled() &&
+                          gather_can_gate(b, rows_cap);
+  RowsGate copy_gate;
   StageGate stage;
   if (split_loss) {
     // (two halves of scratch: with direct I/O the first half of step n + 1 is not
@@ -167,12 +180,20 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
       stage.done = b->pre_sync + 4;
       stage.tickets = reinterpret_cast<unsigned long long *>(b->pre_sync + 6);
       stage.logp = b->c51_logp + (size_t)(b->c51_half & 1) * (size_t)b->c51_logp_half;
+      if (one_stream) {
+        stage.rows.done = b->pre_sync + 8;
+        stage.rows.tickets = reinterpret_cast<unsigned long long *>(b->pre_sync + 12);
+        copy_gate.done = b->pre_sync + 8;
+        copy_gate.tickets = reinterpret_cast<unsigned long long *>(b->pre_sync + 10);
+      }
     }
     b->c51_half ^= 1;
     pre_sync.done = b->pre_sync;
     pre_sync.seen = b->pre_sync + 1;
     pre_sync.ticket = b->pre_sync + 2;
-    if (unjoined) {
+    if (one_stream) {
+      // (launched behind the sampler, below)
+    } else if (unjoined) {
       // nothing on `s` feeds the first half: it waits only for whoever last read the
       // buffers it writes (the tail two steps back) and for the logits
       if (direct->first_half_after)
@@ -235,7 +256,6 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
     if (b->slot_busy[ring_slot])
       B2R_CUDA(cudaStreamWaitEvent(s, b->ev_slot_free[ring_slot], 0));
   }
-  const bool frames = out->state != nullptr || out->next_state != nullptr;
   if (shard)
     B2R_TRY(launch_sample_sharded(
         b, batch, shard->exchange->world, shard->exchange->rank, nullptr,
@@ -245,7 +265,11 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   else
     B2R_TRY(launch_sample(b, batch, true, seed, offset, nullptr, nullptr, 0,
                           sample_idx, b->info, s, out, b->min_prob,
-                          split_loss ? &pre_sync : nullptr));
+                          split_loss ? &pre_sync : nullptr,
+                          one_stream ? copy_gate.done : nullptr));
+  if (one_stream)
+    B2R_TRY(c51_pre_launch(&loss, rows_cap, scratch, pre_sync, s, &have_stats, nullptr,
+                           nullptr, &stage));
   g_host_trace.lap(3);
   int64_t expected_rows =
       shard ? (batch + shard->exchange->world - 1) / shard->exchange->world : -1;
@@ -262,7 +286,9 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   // the indices.
   const bool early_tree = split_loss && tree_early_takes(rows_cap, expected_rows);
   const TreeGo tree_go = early_tree ? tree_go_of(b->tree) : TreeGo();
-  if (frames) {
+  if (one_stream) {
+    B2R_TRY(launch_gather(b, rows_cap, sample_idx, out, s, nullptr, true, &copy_gate));
+  } else if (frames) {
     B2R_CUDA(cudaEventRecord(b->ev_fork, s));
     B2R_CUDA(cudaStreamWaitEvent(b->side, b->ev_fork, 0));
     // (deferred: the first half of the loss rejoins through the copies' stream, so that
@@ -315,8 +341,8 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
                                         flush_behind ? nullptr : early, tree_done,
                                         early_tree)));
   if (flush_behind) B2R_TRY(flush_queue(b, s, false, early));
-  if (frames && !deferred) B2R_CUDA(cudaStreamWaitEvent(s, b->ev_join, 0));
-  if (split_loss && !unjoined && !(deferred && frames))
+  if (frames && !deferred && !one_stream) B2R_CUDA(cudaStreamWaitEvent(s, b->ev_join, 0));
+  if (split_loss && !unjoined && !(deferred && frames) && !one_stream)
     B2R_CUDA(cudaStreamWaitEvent(s, b->ev_c51_pre, 0));
   g_host_trace.lap(6);
   return B2R_OK;
