@@ -142,55 +142,27 @@ struct LossArgs {
   StageGate stage;
 };
 
-__device__ __forceinline__ uint64_t timer_ns() {
-  uint64_t t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
-}
-
 // Minimum of `own` and the peers' local minima of the current step (see ShardedLoss).  A
 // peer's word carries the step number in-band: a stale or early word is waited on, never
 // read as a value.  A peer that does not publish within the timeout latches
 // B2R_ERR_EXCHANGE (later launches then skip the wait) and is left out.
 __device__ __noinline__ float sharded_min_probability(const ShardedLoss &x, float own) {
   const uint64_t seq = *x.seq;
-  const uint32_t tag = (uint32_t)seq;
   const uint64_t *box = x.mins + (size_t)(seq & 1) * x.world;
   float m = own;
   for (int g = 0; g < x.world; ++g) {
-    if (g == x.rank) continue;
-    bool broken = x.timeout_ns <= 0 || (x.latched != nullptr && x.latched[0] == B2R_ERR_EXCHANGE);
-    const uint64_t t0 = timer_ns();
-    while (!broken) {
-      const uint64_t w = ld_sys_u64(box + g);
-      if ((uint32_t)w == tag) {
-        m = fminf(m, __uint_as_float((uint32_t)(w >> 32)));
-        break;
-      }
-      if (timer_ns() - t0 > (uint64_t)x.timeout_ns) {
-        if (x.latched != nullptr) {
-          x.latched[0] = B2R_ERR_EXCHANGE;
-          x.latched[1] = g;
-        }
-        broken = true;
-      }
+    if (g == x.rank || x.timeout_ns <= 0 ||
+        (x.latched != nullptr && x.latched[0] == B2R_ERR_EXCHANGE))
+      continue;
+    uint64_t w;
+    if (poll_tagged_word(box + g, seq, x.timeout_ns, &w)) {
+      m = fminf(m, __uint_as_float((uint32_t)(w >> 32)));
+    } else if (x.latched != nullptr) {
+      x.latched[0] = B2R_ERR_EXCHANGE;
+      x.latched[1] = g;
     }
   }
   return m;
-}
-
-// Last CTA of a launch to get here (every thread calls; s_last in shared memory).
-__device__ __forceinline__ bool last_cta(unsigned int *ticket, bool *s_last) {
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int done = atomicAdd(ticket, 1u);
-    *s_last = (done == gridDim.x - 1);
-    if (*s_last) *ticket = 0u;  // ready for the next launch
-  }
-  __syncthreads();
-  if (*s_last) __threadfence();
-  return *s_last;
 }
 
 // By the last CTA: sum of weighted[0, n) in a fixed order (thread t takes k = t mod
@@ -526,17 +498,7 @@ __global__ void __launch_bounds__(1024, 1) c51_loss_kernel(LossArgs a) {
   B2R_MARK(7);
   B2R_MARK_END(8);
   // ---- the last CTA to finish: mean weighted loss, reduced in a fixed order
-  if (a.u.mean_weighted_loss == nullptr) return;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int done = atomicAdd(a.ticket, 1u);
-    s_last = (done == gridDim.x - 1);
-    if (s_last) *a.ticket = 0u;  // ready for the next launch
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
+  if (a.u.mean_weighted_loss == nullptr || !last_cta(a.ticket, &s_last)) return;
   mean_of_weighted(a.weighted, sharded ? rows : a.u.batch,
                    (float)(sharded ? a.sh.global_batch : a.u.batch), s_red,
                    a.u.mean_weighted_loss);
@@ -868,10 +830,10 @@ struct PreArgs {
   // online logits per transition from this copy instead of crossing PCIe again.
   float *online_copy;
   // nullable (c51_pre_kernel): [rows][c51_logp_stride] log_softmax of every action's online
-  // logits, and StageGate::done, counted when they are all there
+  // logits, and StageGate::first_half.done, counted when they are all there
   float *logp;
   unsigned int *staged_done;
-  // The one-stream step (RowsGate): launched behind the sampler, which waits for this
+  // The one-stream step (StageGate::rows): launched behind the sampler, which waits for this
   // launch's signal before it ends, so the griddepcontrol.wait comes after the signal.
   int wait_late;
 };
@@ -1446,16 +1408,7 @@ c51_post_kernel(LossArgs a, const float *__restrict__ scratch, int have_stats) {
   B2R_MARK_END(12);
 
   // ---- mean weighted loss: the last CTA to finish reduces in a fixed order.
-  if (a.u.mean_weighted_loss == nullptr) return;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int done = atomicAdd(a.ticket, 1u);
-    s_last = (done == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
+  if (a.u.mean_weighted_loss == nullptr || !last_cta(a.ticket, &s_last, false)) return;
   float acc = 0.f;
   for (int k = threadIdx.x; k < a.u.batch; k += blockDim.x)
     acc = __fadd_rn(acc, __ldcg(a.weighted + k));
@@ -1508,23 +1461,15 @@ c51_post_tree_kernel(LossArgs a, const float *__restrict__ scratch, int have_sta
   float4 *logp_row = s_logp + (size_t)warp * (c51_logp_stride(a.u.num_actions, a.u.num_atoms) / 4);
   const int srow = (int)(blockIdx.x - 1) * kPostRowWarps + warp;
   const bool stages = STAGED && !tree_cta && warp < kPostRowWarps && srow < a.u.batch;
-  if (STAGED) {
-    if (threadIdx.x == 0) s_gate = stage_gate_wait(a.stage);
-    __syncthreads();
-  }
+  const bool early = STAGED && cta_gate_wait<0>(a.stage.first_half, &s_gate);
   pdl_release();
-  const bool early = STAGED && s_gate;
   if (early && stages) c51_stage_row(a, scratch, srow, lane, s_bestp[warp], logp_row, zl);
   if (STAGED) B2R_MARK_CTA(15, 1);
   // The one-stream step: the predecessor is the frame copies, not the sampler — the rows
-  // are there once the sampler has counted its launch (RowsGate); the griddepcontrol.wait
+  // are there once the sampler has counted its launch (StageGate::rows); the griddepcontrol.wait
   // moves to the exits.  (Either gate timed out: behind the wait, the safe order.)
   const bool gated = STAGED && a.stage.rows.done != nullptr;
-  if (gated) {
-    if (threadIdx.x == 0) s_rows = rows_gate_wait(a.stage.rows);
-    __syncthreads();
-  }
-  if (!gated || !(s_rows && early)) pdl_acquire();
+  if (!(gated && cta_gate_wait<32>(a.stage.rows, &s_rows) && early)) pdl_acquire();
   if (STAGED && !early && stages) c51_stage_row(a, scratch, srow, lane, s_bestp[warp], logp_row, zl);
   B2R_MARK(11);
   // (a shard's step: the row count is on the device, and the write-back rides along only
@@ -1709,7 +1654,7 @@ int c51_pre_launch(const b2r_c51_args *args, int rows, float *scratch, const Pre
   if (!args || rows <= 0 || !scratch || !args->target_logits || !args->online_logits ||
       !args->support)
     return fail(B2R_ERR_INVALID_ARGUMENT, "bad C51 arguments");
-  if (stage != nullptr && (rows >= 128 || !stage->done || !stage->logp))
+  if (stage != nullptr && (rows >= 128 || !stage->first_half.done || !stage->logp))
     return fail(B2R_ERR_INVALID_ARGUMENT, "a staged first half covers fewer than 128 rows");
   PreArgs a;
   a.target_logits = args->target_logits;
@@ -1723,7 +1668,7 @@ int c51_pre_launch(const b2r_c51_args *args, int rows, float *scratch, const Pre
   a.warps = args->num_actions < 32 ? args->num_actions : 32;
   a.sync = sync;
   a.logp = stage != nullptr ? stage->logp : nullptr;
-  a.staged_done = stage != nullptr ? stage->done : nullptr;
+  a.staged_done = stage != nullptr ? stage->first_half.done : nullptr;
   a.wait_late = stage != nullptr && stage->rows.done != nullptr ? 1 : 0;
   if (rows >= 128) {
     const dim3 grid((rows + kRowWarps - 1) / kRowWarps), block(kRowWarps * 32);
@@ -1774,8 +1719,8 @@ int c51_post_launch(const b2r_c51_args *args, const float *scratch, int have_sta
   a.loss_host = loss_host;
   if (go != nullptr) a.go = *go;
   if (stage != nullptr) {
-    if (tree == nullptr || !c51_tail_can_stage(args) || !stage->done || !stage->tickets ||
-        !stage->logp)
+    if (tree == nullptr || !c51_tail_can_stage(args) || !stage->first_half.done ||
+        !stage->first_half.tickets || !stage->logp)
       return fail(B2R_ERR_INVALID_ARGUMENT, "this tail cannot stage its inputs");
     a.stage = *stage;
   }

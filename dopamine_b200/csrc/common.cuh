@@ -6,6 +6,7 @@
 
 #include <atomic>
 #include <cstdarg>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -226,16 +227,102 @@ __device__ __forceinline__ void pdl_acquire() {
   asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
+// ---- hand-over of a few words between kernels through global memory ---------------------
+// A signaller publishes a word with release; its consumers poll it with acquire, and what
+// the signaller wrote before the release is visible to them once they have seen the word.
+__device__ __forceinline__ void st_release_u32(unsigned int *p, unsigned int v) {
+  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int *p) {
+  unsigned int v;
+  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+// Peer memory (NVLink / NVSwitch): relaxed at system scope.
+__device__ __forceinline__ void st_sys_u64(uint64_t *p, uint64_t v) {
+  asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ uint64_t ld_sys_u64(const uint64_t *p) {
+  uint64_t v;
+  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+
+__device__ __forceinline__ uint64_t global_timer_ns() {
+  uint64_t t;
+  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
+  return t;
+}
+
+// How long a consumer polls a hand-over word before it gives up: 4e9 clock64 cycles, about
+// 2 s at the B200's clocks.  A signaller that never ran (its launch failed, and the caller has
+// been told) must not hang the GPU; every consumer has a safe fallback, normally its
+// griddepcontrol.wait.
+constexpr long long kSpinLimit = 4000000000ll;
+
+// Polls *word with acquire until ready(value) holds: false once kSpinLimit has passed.
+// kBackoffNs > 0: a __nanosleep between polls.
+template <int kBackoffNs = 0, typename Ready>
+__device__ __forceinline__ bool poll_acquire(const unsigned int *word, Ready ready) {
+  const long long t0 = clock64();
+  while (!ready(ld_acquire_u32(word))) {
+    if (clock64() - t0 > kSpinLimit) return false;
+    if (kBackoffNs > 0) __nanosleep(kBackoffNs);
+  }
+  return true;
+}
+
+// Polls a peer-memory mailbox word until its low 32 bits carry step `seq`: true with the word
+// in *w, false once timeout_ns of %globaltimer have passed.
+__device__ __forceinline__ bool poll_tagged_word(const uint64_t *src, uint64_t seq,
+                                                 int64_t timeout_ns, uint64_t *w) {
+  const uint64_t t0 = global_timer_ns();
+  for (;;) {
+    *w = ld_sys_u64(src);
+    if ((uint32_t)*w == (uint32_t)seq) return true;
+    if (global_timer_ns() - t0 > (uint64_t)timeout_ns) return false;
+  }
+}
+
+// Launch numbers from tickets: every CTA of a launch takes one ticket before it lets its
+// dependents start, so the tickets of consecutive launches never interleave.  `launch` is the
+// launch's number counted from 1, `arrival` the CTA's place within its launch.
+struct LaunchTicket {
+  unsigned int launch, arrival;
+};
+__device__ __forceinline__ LaunchTicket launch_ticket(unsigned long long *tickets,
+                                                      unsigned int ctas) {
+  const unsigned long long t = atomicAdd(tickets, 1ull);
+  return {(unsigned int)(t / ctas) + 1u, (unsigned int)(t % ctas)};
+}
+
+// Last-CTA election, by thread 0 of every CTA of the launch: true in the CTA that arrives
+// last.  rearm: that CTA resets the ticket for the next launch at once; a caller that passes
+// false resets it itself, later (the next launch takes its tickets behind its own
+// griddepcontrol.wait, so any point before this launch ends will do).
+__device__ __forceinline__ bool arrive_last(unsigned int *ticket, bool rearm = true) {
+  const bool last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+  if (rearm && last) *ticket = 0u;
+  return last;
+}
+// The same for the whole CTA (every thread calls it; s_last in shared memory): the CTA that
+// arrives last sees everything the others wrote before they arrived.
+__device__ __forceinline__ bool last_cta(unsigned int *ticket, bool *s_last, bool rearm = true) {
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) *s_last = arrive_last(ticket, rearm);
+  __syncthreads();
+  const bool last = *s_last;
+  if (last) __threadfence();
+  return last;
+}
+
 // ---- optional phase tracing (build with -DB2R_TRACE; never in the shipped .so) ---
 #ifdef B2R_TRACE
 // -DB2R_TRACE_GT: marks are %globaltimer nanoseconds (one clock for all kernels and
 // SMs: a timeline of the whole step); otherwise clock64 cycles of the marking SM.
 #ifdef B2R_TRACE_GT
-__device__ __forceinline__ long long b2r_now() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return (long long)t;
-}
+__device__ __forceinline__ long long b2r_now() { return (long long)global_timer_ns(); }
 #else
 __device__ __forceinline__ long long b2r_now() { return clock64(); }
 #endif

@@ -39,7 +39,7 @@ struct GatherArgs {
   int32_t scalar_rows;   // grid rows of appended scalar CTAs (0: frames only)
   ScalarArgs sc;
   const int32_t *count;  // nullable: device-side number of rows (<= batch)
-  RowsGate gate;         // the one-stream step (TMA copies only; done == nullptr: none)
+  LaunchGate gate;         // the one-stream step (TMA copies only; done == nullptr: none)
 };
 
 // [a0 a1 a2 a3] x4 frames -> 4 words [a_p b_p c_p d_p], p = 0..3.
@@ -192,14 +192,11 @@ gather_stack4_u8_tma_kernel(const __grid_constant__ GatherArgs a) {
   B2R_MARK(0);
   pdl_release();
   // The one-stream step: the predecessor is the first half of the loss; the indices are
-  // final once the sampler has counted its launch (RowsGate), and the griddepcontrol.wait
-  // moves to the end (the copies have landed when the step's last kernel completes).
+  // final once the sampler has counted its launch (StageGate::rows), and the
+  // griddepcontrol.wait moves to the end (the copies have landed when the step's last
+  // kernel completes).
   const bool gated = a.gate.done != nullptr;
-  if (gated) {
-    if (threadIdx.x == 0) s_rows = rows_gate_wait(a.gate);
-    __syncthreads();
-  }
-  if (!gated || !s_rows) pdl_acquire();
+  if (!(gated && cta_gate_wait<32>(a.gate, &s_rows))) pdl_acquire();
   B2R_MARK(1);
   const int rows = a.count ? min(*a.count, a.batch) : a.batch;
   if (SCALARS && (int)blockIdx.x >= a.batch) {  // appended scalar CTAs
@@ -372,7 +369,7 @@ bool gather_can_gate(const b2r_buffer *b, int32_t batch) {
 
 int launch_gather(b2r_buffer *b, int32_t batch, const int32_t *indices_dev,
                   const b2r_batch *out, cudaStream_t stream,
-                  const int32_t *count_dev, bool frames_only, const RowsGate *gate) {
+                  const int32_t *count_dev, bool frames_only, const LaunchGate *gate) {
   if (gate != nullptr && (count_dev != nullptr || !frames_only || !gather_can_gate(b, batch)))
     return fail(B2R_ERR_INVALID_ARGUMENT, "only the TMA frame copies of a counted batch gate");
   GatherArgs a;

@@ -51,16 +51,7 @@ __device__ __forceinline__ double warp_sum_f64(double v) {
 // order and divides by the global batch (every CTA calls; s_red, s_last in shared memory).
 __device__ __forceinline__ void iqn_mean(const IqnArgs &a, int rows, double *s_red,
                                          bool *s_last) {
-  if (a.u.mean_loss == nullptr) return;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned int done = atomicAdd(a.ticket, 1u);
-    *s_last = (done == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (!*s_last) return;
-  __threadfence();
+  if (a.u.mean_loss == nullptr || !last_cta(a.ticket, s_last, false)) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   double acc = 0.0;
   for (int k = threadIdx.x; k < rows; k += blockDim.x) acc += (double)__ldcg(a.u.loss + k);

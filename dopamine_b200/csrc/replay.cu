@@ -382,8 +382,6 @@ int b2r_create(const b2r_config *cfg, b2r_buffer **out) {
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->info), 64));
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->status), 16));
   B2R_CUDA(cudaMemset(b->status, 0, 16));
-  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->ticket), 4));
-  B2R_CUDA(cudaMemset(b->ticket, 0, 4));
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->shard_counter), 8));
   B2R_CUDA(cudaMemset(b->shard_counter, 0, 8));
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->draw_counter), 8));
@@ -400,8 +398,8 @@ int b2r_create(const b2r_config *cfg, b2r_buffer **out) {
     cudaDeviceGetStreamPriorityRange(&least, &greatest);
     B2R_CUDA(cudaStreamCreateWithPriority(&b->side3, cudaStreamNonBlocking, greatest));
   }
-  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->pre_sync), 64));
-  B2R_CUDA(cudaMemset(b->pre_sync, 0, 64));
+  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&b->sync), sizeof(b2r::StepSync)));
+  B2R_CUDA(cudaMemset(b->sync, 0, sizeof(b2r::StepSync)));
   for (int k = 0; k < 2; ++k)
     B2R_CUDA(cudaEventCreateWithFlags(&b->ev_slot_free[k], cudaEventDisableTiming));
   B2R_CUDA(cudaEventCreateWithFlags(&b->ev_c51_fork, cudaEventDisableTiming));
@@ -430,7 +428,6 @@ int b2r_destroy(b2r_buffer *b) {
   cudaFree(b->status);
   cudaFree(b->draw_counter);
   cudaFree(b->shard_counter);
-  cudaFree(b->ticket);
   cudaFree(b->min_prob);
   cudaFree(b->ctx_dev);
   if (b->side) cudaStreamDestroy(b->side);
@@ -441,7 +438,7 @@ int b2r_destroy(b2r_buffer *b) {
   if (b->ev_c51_pre) cudaEventDestroy(b->ev_c51_pre);
   if (b->c51_bestp) cudaFree(b->c51_bestp);
   if (b->c51_logp) cudaFree(b->c51_logp);
-  if (b->pre_sync) cudaFree(b->pre_sync);
+  if (b->sync) cudaFree(b->sync);
   if (b->idx_ring) cudaFree(b->idx_ring);
   for (int k = 0; k < 2; ++k)
     if (b->ev_slot_free[k]) cudaEventDestroy(b->ev_slot_free[k]);

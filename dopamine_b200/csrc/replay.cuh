@@ -76,7 +76,7 @@ __device__ __forceinline__ int block_scan_flag(bool flag, int *warp_counts,
 // The first half is a few microseconds of work that starts together with the sampler,
 // so the wait normally finds the bump already there.
 // Only the fork/join step needs this hand-shake for its ordering; the one-stream step
-// (step.cu: train_step, RowsGate) orders the first half behind the sampler on the stream
+// (step.cu: train_step, StageGate::rows) orders the first half behind the sampler on the stream
 // and keeps the sampler's wait only so that `done` and `seen` advance the same way on both
 // paths, which may alternate on one buffer.
 struct PreSync {
@@ -115,81 +115,81 @@ struct PreSync {
 // so "tail n complete" means all of step n is complete, the copies included.  The sampler lets
 // its dependents launch only after its own griddepcontrol.wait: the first half of step n + 1
 // then starts after the tail of step n has ended, never while it reads the scratch half.
-struct RowsGate {
-  unsigned int *done = nullptr;           // sampler launches with final rows (monotone)
-  unsigned long long *tickets = nullptr;  // CTAs of this consumer's gated launches (monotone)
+// Both gates are LaunchGates: one opens for the launch numbered k (launch_ticket, counted
+// from 1) once `done` >= k.
+struct LaunchGate {
+  unsigned int *done = nullptr;           // signaller launches completed (monotone)
+  unsigned long long *tickets = nullptr;  // CTAs of the gated launches started (monotone)
 };
 struct StageGate {
-  unsigned int *done = nullptr;           // staged first halves completed (monotone)
-  unsigned long long *tickets = nullptr;  // CTAs of staged tails started (monotone)
+  LaunchGate first_half;  // staged first halves completed / CTAs of staged tails started
   float *logp = nullptr;  // [rows][c51_logp_stride] log-probabilities, action-major
-  RowsGate rows;  // the one-stream step (done == nullptr: the fork/join step)
+  // the one-stream step: sampler launches with final rows / CTAs of gated tails
+  // (rows.done == nullptr: the fork/join step)
+  LaunchGate rows;
 };
 // Row stride of StageGate::logp: whole 16-byte words, so a row moves as float4s.
 __host__ __device__ __forceinline__ int c51_logp_stride(int actions, int atoms) {
   return (actions * atoms + 3) & ~3;
 }
 
+// The hand-over words of the fused step (step.cu), one set per buffer, zeroed at creation.
+struct StepSync {
+  unsigned int pre_done, pre_seen, pre_ticket;  // PreSync
+  unsigned int tree_done;  // UpdateArgs::skip_flag of a shard's one-CTA write-back
+  unsigned int stage_done, unused0;
+  unsigned long long stage_tickets;  // StageGate::first_half
+  unsigned int rows_done, unused1;   // StageGate::rows and the gated copies
+  unsigned long long copy_tickets, tail_tickets;
+  unsigned int sample_ticket;  // last-CTA election of the sample kernels
+};
+static_assert(offsetof(StepSync, stage_tickets) % 8 == 0 &&
+                  offsetof(StepSync, copy_tickets) % 8 == 0 &&
+                  offsetof(StepSync, tail_tickets) == 48 && sizeof(StepSync) == 64,
+              "StepSync keeps its word order");
+
 #ifdef __CUDACC__
-__device__ __forceinline__ void st_release_u32(uint32_t *p, uint32_t v) {
-  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ uint32_t ld_acquire_u32(const unsigned int *p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
 // Last statement of a first-half CTA (every thread calls it).  staged_done (nullable):
-// StageGate::done of a staged first half.
+// StageGate::first_half.done of a staged first half.
 __device__ __forceinline__ void pre_sync_signal(const PreSync &p,
                                                 unsigned int *staged_done = nullptr) {
   __threadfence();
   __syncthreads();
-  if (threadIdx.x == 0 && atomicAdd(p.ticket, 1u) == gridDim.x - 1) {
-    *p.ticket = 0u;  // ready for the next launch
+  if (threadIdx.x == 0 && arrive_last(p.ticket)) {
     __threadfence();
     if (staged_done != nullptr) st_release_u32(staged_done, *staged_done + 1u);
     st_release_u32(p.done, *p.done + 1u);
   }
 }
-// By thread 0 of every CTA of a staged tail, BEFORE the CTA lets its dependents start:
-// takes the ticket and waits for the first half of this launch's step (StageGate).  False
-// after 2 s (a first half that never ran must not hang the GPU): the caller then stages
-// behind its griddepcontrol.wait, when the sampler's own wait for the first half is over.
-__device__ __forceinline__ bool stage_gate_wait(const StageGate &g) {
-  const unsigned long long ticket = atomicAdd(g.tickets, 1ull);
-  const unsigned int launch = (unsigned int)(ticket / gridDim.x) + 1u;
-  const long long t0 = clock64();
-  while ((int)(ld_acquire_u32(g.done) - launch) < 0)
-    if (clock64() - t0 > 4000000000ll) return false;
-  return true;
+// By thread 0 of every CTA of a gated launch, BEFORE the CTA lets its dependents start: takes
+// the ticket and waits for the signaller of this launch's step.  False after kSpinLimit: the
+// caller then falls back to its griddepcontrol.wait, which is behind the signaller's own
+// completion or wait (correct, only late).  kBackoffNs: poll_acquire.
+template <int kBackoffNs>
+__device__ __forceinline__ bool gate_wait(const LaunchGate &g) {
+  const unsigned int launch = launch_ticket(g.tickets, gridDim.x).launch;
+  return poll_acquire<kBackoffNs>(g.done, [=](unsigned v) { return (int)(v - launch) >= 0; });
 }
-// By thread 0 of every CTA of a gated copy or tail launch (RowsGate), before it reads a row.
-// False after 2 s: the caller then falls back to its griddepcontrol.wait, which in the
-// one-stream order is behind the sampler's completion (correct, only late).
-__device__ __forceinline__ bool rows_gate_wait(const RowsGate &g) {
-  const unsigned long long ticket = atomicAdd(g.tickets, 1ull);
-  const unsigned int launch = (unsigned int)(ticket / gridDim.x) + 1u;
-  const long long t0 = clock64();
-  while ((int)(ld_acquire_u32(g.done) - launch) < 0) {
-    if (clock64() - t0 > 4000000000ll) return false;
-    __nanosleep(32);
-  }
-  return true;
+// The same for the whole CTA (every thread calls it; s_ok in shared memory).  The staged
+// tail spins; the one-stream step's copies and tail back off 32 ns between polls (measured
+// that way).
+template <int kBackoffNs>
+__device__ __forceinline__ bool cta_gate_wait(const LaunchGate &g, bool *s_ok) {
+  if (threadIdx.x == 0) *s_ok = gate_wait<kBackoffNs>(g);
+  __syncthreads();
+  return *s_ok;
 }
-// The sampler's last word (RowsGate::done): release, no round trip.
+// The sampler's last word (StageGate::rows.done): release, no round trip.
 __device__ __forceinline__ void rows_gate_publish(unsigned int *done) {
   asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(done) : "memory");
 }
 // Called by the sampler's closing thread (ONE thread) before the kernel ends.  Gives up
-// after 2 s: a first half that never ran must not hang the GPU (the tail then reads stale
-// rows; the launch error that caused it has been reported to the caller).
+// after kSpinLimit: a first half that never ran must not hang the GPU (the tail then reads
+// stale rows; the launch error that caused it has been reported to the caller).
 __device__ __forceinline__ void pre_sync_consume(const PreSync &p) {
   if (p.done == nullptr) return;
   const unsigned int seen = *p.seen;
-  const long long t0 = clock64();
-  while (ld_acquire_u32(p.done) == seen)
-    if (clock64() - t0 > 4000000000ll) break;
+  poll_acquire(p.done, [=](unsigned v) { return v != seen; });
   *p.seen = seen + 1u;
 }
 // The same in two steps, so that the two loads are in flight long before the closing
@@ -207,11 +207,8 @@ __device__ __forceinline__ PreSyncPeek pre_sync_peek(const PreSync &p) {
 }
 __device__ __forceinline__ void pre_sync_consume(const PreSync &p, const PreSyncPeek &k) {
   if (p.done == nullptr) return;
-  if (k.done == k.seen) {  // not yet when we looked: wait now
-    const long long t0 = clock64();
-    while (ld_acquire_u32(p.done) == k.seen)
-      if (clock64() - t0 > 4000000000ll) break;
-  }
+  if (k.done == k.seen)  // not yet when we looked: wait now
+    poll_acquire(p.done, [=](unsigned v) { return v != k.seen; });
   *p.seen = k.seen + 1u;
 }
 #endif
@@ -324,7 +321,6 @@ struct b2r_buffer {
   int64_t inv_slots_cap = 0;
   int32_t *info = nullptr;      // device [4]: status, fail slot, draws used, count
   int64_t *status = nullptr;    // device [2]: latched asynchronous error
-  unsigned int *ticket = nullptr;   // device: last-CTA election of the sample kernel
   uint64_t *shard_counter = nullptr;  // device: like draw_counter, for sharded draws
                                       // (advances in lockstep on every rank)
   uint64_t *draw_counter = nullptr;  // device: bumps per Philox sample launch, so a
@@ -340,9 +336,7 @@ struct b2r_buffer {
   float *c51_bestp = nullptr;  // device [2 halves][c51_bestp_rows][64 probabilities | 64 stats]
   int64_t c51_bestp_rows = 0;
   int c51_half = 0;            // half the next step's first half writes
-  unsigned int *pre_sync = nullptr;  // device [16]: PreSync done, seen, ticket, tree_done,
-                                     // StageGate done, -, tickets (64 bits), RowsGate done,
-                                     // -, copy tickets (64 bits), tail tickets (64 bits), -, -
+  b2r::StepSync *sync = nullptr;     // device
   float *c51_logp = nullptr;         // device [2 halves][c51_logp_half]: StageGate::logp
   int64_t c51_logp_half = 0;
   // Deferred frame copies (b2r_set_deferred_frames): the copies of a fused step are not
@@ -437,14 +431,14 @@ int flush_fused(b2r_tree *tree, int n, const int64_t *slots, const double *prio,
                 const uint8_t *mode, const AddParams &rows, int row_blocks_per_entry,
                 cudaStream_t stream, const b2r_exchange *publish = nullptr);
 int ensure_inv_slots(b2r_buffer *buf, int64_t n);
-// gate (nullable): frame copies of the one-stream step (RowsGate); only the TMA copies
+// gate (nullable): frame copies of the one-stream step (StageGate::rows); only the TMA copies
 // (gather_can_gate) take one.
 int launch_gather(b2r_buffer *buf, int32_t batch, const int32_t *indices_dev,
                   const b2r_batch *out, cudaStream_t stream,
                   const int32_t *count_dev = nullptr, bool frames_only = false,
-                  const RowsGate *gate = nullptr);
+                  const LaunchGate *gate = nullptr);
 bool gather_can_gate(const b2r_buffer *buf, int32_t batch);
-// rows_done (nullable): RowsGate::done of the one-stream step (batches of the warp sampler,
+// rows_done (nullable): StageGate::rows.done of the one-stream step (batches of the warp sampler,
 // with scalars and the minimum).
 int launch_sample(b2r_buffer *buf, int32_t batch, bool philox, uint64_t seed,
                   uint64_t offset, const double *strat_dev,

@@ -80,7 +80,7 @@ struct PerSampleArgs {
   // Exchange mode: the closing thread also stores min_prob_out's value into every peer's
   // mailbox for this step (b2r_sample_transition_batch_sharded_device).
   int publish_min;
-  // nullable: RowsGate::done of the one-stream step (replay.cuh), counted by the closing
+  // nullable: StageGate::rows.done of the one-stream step (replay.cuh), counted by the closing
   // thread when rows, minimum and counters are final.  The kernel then lets its dependents
   // launch only after its own griddepcontrol.wait.
   unsigned int *rows_done;
@@ -90,12 +90,6 @@ struct PerSampleArgs {
 __device__ __forceinline__ void publish_local_min(const PerSampleArgs &a, bool exchange,
                                                   float m, uint64_t seq) {
   if (a.publish_min && exchange) exchange_publish_min(a.xchg, a.num_shards, a.rank, m, seq);
-}
-
-__device__ __forceinline__ uint64_t global_timer_ns() {
-  uint64_t t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
 }
 
 // Receiving half of the all-gather of shard totals (tree.cuh: exchange_publish): thread g
@@ -188,7 +182,8 @@ __global__ void __launch_bounds__(MAX_THREADS) per_sample_kernel(const __grid_co
   __shared__ float warp_mins[32];
   __shared__ double s_totals[kMaxShards];
   __shared__ int s_first[2];
-  __shared__ int s_draws_used, s_last_idx, s_last_valid, s_is_last;
+  __shared__ int s_draws_used, s_last_idx, s_last_valid;
+  __shared__ bool s_is_last;
   __shared__ int tile_start[kMaxTiles + 1];
 
   __shared__ ValidCtx s_valid;
@@ -240,9 +235,7 @@ __global__ void __launch_bounds__(MAX_THREADS) per_sample_kernel(const __grid_co
   if (grand_total == 0.0 || (a.num_shards == 1 && local_total == 0.0)) {
     // sum_tree.py:159-160 (every CTA takes this branch together; the last one to
     // arrive advances the step counters, which every CTA read on entry)
-    if (threadIdx.x == 0 &&
-        (gridDim.x == 1 || atomicAdd(a.ticket, 1u) == gridDim.x - 1)) {
-      if (gridDim.x > 1) *a.ticket = 0u;
+    if (threadIdx.x == 0 && (gridDim.x == 1 || arrive_last(a.ticket))) {
       a.info[0] = B2R_ERR_EMPTY_TREE;
       a.info[1] = 0; a.info[2] = 0; a.info[3] = 0;
       if (a.count_out) *a.count_out = 0;
@@ -419,13 +412,7 @@ __global__ void __launch_bounds__(MAX_THREADS) per_sample_kernel(const __grid_co
 
   // ---- only the last CTA to finish goes on
   if (gridDim.x > 1) {
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0)
-      s_is_last = atomicAdd(a.ticket, 1u) == gridDim.x - 1;
-    __syncthreads();
-    if (!s_is_last) return;
-    __threadfence();
+    if (!last_cta(a.ticket, &s_is_last, false)) return;
   } else {
     __syncthreads();
   }
@@ -673,7 +660,8 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
   __shared__ int warp_counts[32];
   __shared__ float warp_mins[32];
   __shared__ int s_draw_of[kSpecMax], s_spec_idx[kSpecMax];
-  __shared__ int s_draws_used, s_last_idx, s_last_valid, s_is_last;
+  __shared__ int s_draws_used, s_last_idx, s_last_valid;
+  __shared__ bool s_is_last;
   __shared__ ValidCtx s_valid;  // thread-per-draw retry rounds only
 
   const unsigned full = 0xffffffffu;
@@ -715,9 +703,7 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
   if (grand_total == 0.0 || (a.num_shards == 1 && local_total == 0.0)) {
     // sum_tree.py:159-160; every CTA takes this branch, the last to arrive closes
     if (threadIdx.x == 0 &&
-        (CLUSTER ? blockIdx.x == 0
-                 : (gridDim.x == 1 || atomicAdd(a.ticket, 1u) == gridDim.x - 1))) {
-      if (!CLUSTER && gridDim.x > 1) *a.ticket = 0u;
+        (CLUSTER ? blockIdx.x == 0 : (gridDim.x == 1 || arrive_last(a.ticket)))) {
       a.info[0] = B2R_ERR_EMPTY_TREE;
       a.info[1] = 0; a.info[2] = 0; a.info[3] = 0;
       if (a.count_out) *a.count_out = 0;
@@ -906,7 +892,7 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
     }
   }
   // The one-stream step: the copies and the tail read these rows once the closing thread has
-  // counted the launch (RowsGate), not behind the kernel's completion.  The order comes
+  // counted the launch (StageGate::rows), not behind the kernel's completion.  The order comes
   // without a fence per row: every CTA sends its minimum word behind the barrier below,
   // after all of its rows; the complete-tx of an st.async releases at cluster scope; CTA 0
   // waits for every word with acquire at cluster scope (mbar_wait_cluster); and the closing
@@ -979,12 +965,7 @@ per_sample_warp_kernel(const __grid_constant__ PerSampleArgs a,
     for (int p = threadIdx.x; p < n_mine; p += blockDim.x) s_flag[p] = (uint8_t)s_flag32[p];
     __syncthreads();
   } else if (gridDim.x > 1) {
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) s_is_last = atomicAdd(a.ticket, 1u) == gridDim.x - 1;
-    __syncthreads();
-    if (!s_is_last) return;
-    __threadfence();
+    if (!last_cta(a.ticket, &s_is_last, false)) return;
   } else {
     __syncthreads();
   }
@@ -1432,7 +1413,7 @@ int launch_sample(b2r_buffer *b, int32_t batch, bool philox, uint64_t seed,
     a.tile_counts = b->inv_slots + (int64_t)tiles * threads;
     a.tile_min = reinterpret_cast<float *>(a.tile_counts + kMaxTiles);
   }
-  a.ticket = b->ticket;
+  a.ticket = &b->sync->sample_ticket;
   a.info = info_dev;
   a.latched = philox ? b->status : nullptr;
   a.num_shards = 1;
@@ -1546,7 +1527,7 @@ int launch_sample_sharded(b2r_buffer *b, int32_t global_batch, int32_t num_shard
   a.strat_query01 = query01;
   a.retry_u01 = retry_u01;
   a.out_idx = out_indices;
-  a.ticket = b->ticket;
+  a.ticket = &b->sync->sample_ticket;
   a.info = b->info;
   a.latched = b->status;
   a.num_shards = num_shards;
@@ -1648,12 +1629,8 @@ __device__ __forceinline__ int32_t poll_rej_word(const ExchangeArgs &x, const ui
                                                  int64_t *latched) {
   if (x.timeout_ns <= 0) return missing;
   const bool broken = latched != nullptr && latched[0] == B2R_ERR_EXCHANGE;
-  const uint64_t t0 = global_timer_ns();
-  while (!broken) {
-    const uint64_t w = ld_sys_u64(src);
-    if ((uint32_t)w == (uint32_t)seq) return (int32_t)(w >> 32);
-    if (global_timer_ns() - t0 > (uint64_t)x.timeout_ns) break;
-  }
+  uint64_t w;
+  if (!broken && poll_tagged_word(src, seq, x.timeout_ns, &w)) return (int32_t)(w >> 32);
   if (latched != nullptr) {
     latched[0] = B2R_ERR_EXCHANGE;
     latched[1] = g;

@@ -10,8 +10,8 @@
 // network, not this chain.  So the sampler emits the scalar columns itself, the
 // chain sample -> loss -> write-back runs on the caller's stream, and the HBM-bound
 // frame copies run beside it on a forked stream, joined before the call returns —
-// except at the agent's batch, where every kernel goes on the caller's stream (RowsGate,
-// replay.cuh: a joined fork would give the next step's sampler three parents).
+// except at the agent's batch, where every kernel goes on the caller's stream
+// (StageGate::rows, replay.cuh: a joined fork would give the next step's sampler three parents).
 #include "gather.cuh"
 
 #include <cmath>
@@ -131,7 +131,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   // (StageGate, replay.cuh; the tail and the write-back are then one cluster, below).
   const bool staged = split_loss && !shard && c51_post_takes_tree(&loss, b->tree) &&
                       c51_tail_can_stage(&loss);
-  // The one-stream step (RowsGate, replay.cuh): sampler -> first half -> frame copies ->
+  // The one-stream step (StageGate::rows, replay.cuh): sampler -> first half -> frame copies ->
   // tail + write-back, all on `s`, every kernel launched programmatically behind the one
   // before — in a captured graph every node then has ONE parent, and the next step's
   // sampler keeps its early launch.  Only where nothing else joins the step: copies joined
@@ -141,7 +141,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   const bool one_stream = staged && frames && !b->deferred_frames && direct == nullptr &&
                           wait_before_loss == nullptr && pdl_enabled() &&
                           gather_can_gate(b, rows_cap);
-  RowsGate copy_gate;
+  LaunchGate copy_gate;
   StageGate stage;
   if (split_loss) {
     // (two halves of scratch: with direct I/O the first half of step n + 1 is not
@@ -177,20 +177,15 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
                             2 * (size_t)half * sizeof(float)));
         b->c51_logp_half = half;
       }
-      stage.done = b->pre_sync + 4;
-      stage.tickets = reinterpret_cast<unsigned long long *>(b->pre_sync + 6);
+      stage.first_half = {&b->sync->stage_done, &b->sync->stage_tickets};
       stage.logp = b->c51_logp + (size_t)(b->c51_half & 1) * (size_t)b->c51_logp_half;
       if (one_stream) {
-        stage.rows.done = b->pre_sync + 8;
-        stage.rows.tickets = reinterpret_cast<unsigned long long *>(b->pre_sync + 12);
-        copy_gate.done = b->pre_sync + 8;
-        copy_gate.tickets = reinterpret_cast<unsigned long long *>(b->pre_sync + 10);
+        stage.rows = {&b->sync->rows_done, &b->sync->tail_tickets};
+        copy_gate = {&b->sync->rows_done, &b->sync->copy_tickets};
       }
     }
     b->c51_half ^= 1;
-    pre_sync.done = b->pre_sync;
-    pre_sync.seen = b->pre_sync + 1;
-    pre_sync.ticket = b->pre_sync + 2;
+    pre_sync = {&b->sync->pre_done, &b->sync->pre_seen, &b->sync->pre_ticket};
     if (one_stream) {
       // (launched behind the sampler, below)
     } else if (unjoined) {
@@ -322,7 +317,7 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
   const bool tail_counted = split_loss && shard != nullptr && !flush_behind &&
                             c51_post_takes_tree(&loss, b->tree, expected_rows);
   const bool tail_writeback = split_loss && !shard && c51_post_takes_tree(&loss, b->tree);
-  unsigned int *tree_done = tail_counted ? b->pre_sync + 3 : nullptr;
+  unsigned int *tree_done = tail_counted ? &b->sync->tree_done : nullptr;
   if (split_loss)
     B2R_TRY(c51_post_launch(&loss, scratch, have_stats, s, b->status,
                             shard && count != shard->out_count ? shard->out_count : nullptr,

@@ -429,39 +429,29 @@ __device__ __forceinline__ bool chains_by_verified_scan(double *__restrict__ lev
 template <typename I, typename V>
 __device__ __forceinline__ void leaf_publishes(const UpdateArgs<I, V> &a, int n, int n_eff,
                                                int stop_code) {
-  long long *pending = reinterpret_cast<long long *>(a.sync_words + 4);
+  long long *pending = a.sync->pending;
   if (threadIdx.x == 0) {
     pending[0] = n_eff < n ? stop_code : 0;
     pending[1] = a.k_base + n_eff;
   }
   __threadfence();
   __syncthreads();
-  if (threadIdx.x == 0) {
-    asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(a.sync_words + 1), "r"(1u)
-                 : "memory");
-  }
+  if (threadIdx.x == 0) st_release_u32(&a.sync->leaf_flag, 1u);
   B2R_MARK_ANY(10);
 }
 
 // Returns (to every thread) the number of entries the leaf CTA applied.
 template <typename I, typename V>
 __device__ __forceinline__ int levels_wait_for_leaf(const UpdateArgs<I, V> &a) {
-  long long *pending = reinterpret_cast<long long *>(a.sync_words + 4);
+  const long long *pending = a.sync->pending;
   __shared__ int s_applied;
   if (threadIdx.x == 0) {
-    unsigned seen = 0;
-    const long long t0 = clock64();
-    do {
-      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];"
-                   : "=r"(seen)
-                   : "l"(a.sync_words + 1)
-                   : "memory");
-    } while (seen == 0 && clock64() - t0 < 4000000000ll);  // (2 s: never hang the GPU)
-    if (seen == 0 && a.status[0] == 0) a.status[0] = B2R_ERR_CUDA;
+    const bool seen = poll_acquire(&a.sync->leaf_flag, [](unsigned v) { return v != 0u; });
+    if (!seen && a.status[0] == 0) a.status[0] = B2R_ERR_CUDA;
     s_applied = seen ? (int)(pending[1] - a.k_base) : 0;
     // the last level to leave re-arms the flag for the next launch
-    if (atomicInc(a.sync_words + 2, (unsigned)a.depth - 1) == (unsigned)a.depth - 1) {
-      a.sync_words[1] = 0u;
+    if (atomicInc(&a.sync->level_arrivals, (unsigned)a.depth - 1) == (unsigned)a.depth - 1) {
+      a.sync->leaf_flag = 0u;
       if (pending[0] != 0 && a.status[0] == 0) {
         a.status[0] = pending[0];
         a.status[1] = pending[1];
@@ -567,7 +557,7 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_kernel(UpdateArgs<I, 
   B2R_MARK(13);
   pdl_release();
   pdl_acquire();
-  if (threadIdx.x == 0) s_role = (int)atomicInc(a.sync_words, (unsigned)a.depth);
+  if (threadIdx.x == 0) s_role = (int)atomicInc(&a.sync->role_ticket, (unsigned)a.depth);
   __syncthreads();
   const int level = s_role == 0 ? a.depth : s_role - 1;
   const bool is_leaf = level == a.depth;
@@ -1328,16 +1318,15 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_early_kernel(UpdateAr
   __shared__ uint32_t s_listed;
   __shared__ ScanSmem s_scan;
   uint32_t *info = a.sorted;
-  unsigned int *list_flag = a.sync_words + 8, *ended = a.sync_words + 9;
-  unsigned int *fetched = a.sync_words + 10;  // level CTAs that have their leaves
+  TreeSync &sync = *a.sync;
   B2R_MARK(13);
   // The last CTA to leave re-arms the list's flag and the count of level CTAs that have
   // their leaves (everybody is past both then), and counts the launch (TreeGo).
   auto leave = [&]() {
-    if (threadIdx.x == 0 && atomicInc(ended, (unsigned)a.depth) == (unsigned)a.depth) {
-      *list_flag = 0u;
-      *fetched = 0u;
-      atomicAdd(a.sync_words + 15, 1u);
+    if (threadIdx.x == 0 && atomicInc(&sync.ended, (unsigned)a.depth) == (unsigned)a.depth) {
+      sync.list_flag = 0u;
+      sync.fetched = 0u;
+      atomicAdd(&sync.completed, 1u);
     }
   };
   // A ticket first, dependents second: the next early write-back can only start once
@@ -1347,20 +1336,12 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_early_kernel(UpdateAr
   // behind each other (each lets the next start from its first instruction) and sit on
   // the SMs waiting — bounded to one step ahead this way.
   if (threadIdx.x == 0) {
-    const unsigned long long ticket = atomicAdd(a.tickets, 1ull);
-    const unsigned int ctas = (unsigned)a.depth + 1u;
-    s_role = (int)(ticket % ctas);
+    const LaunchTicket t = launch_ticket(a.tickets, (unsigned)a.depth + 1u);
+    s_role = (int)t.arrival;
     s_listed = 1u;
-    if (a.go != nullptr) {
-      // resident ahead of the indices: wait to hear that they are final (TreeGo)
-      const unsigned int launch = (unsigned int)(ticket / ctas) + 1u;
-      unsigned int seen = 0;
-      const long long t0 = clock64();
-      do {
-        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(a.go) : "memory");
-      } while (seen != launch && clock64() - t0 < 4000000000ll);  // (2 s: never hang)
-      s_listed = seen == launch ? 1u : 0u;
-    }
+    // resident ahead of the indices: wait to hear that they are final (TreeGo)
+    if (a.go != nullptr)
+      s_listed = poll_acquire(a.go, [&](unsigned v) { return v == t.launch; }) ? 1u : 0u;
   }
   __syncthreads();
   pdl_release();
@@ -1460,7 +1441,7 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_early_kernel(UpdateAr
     }
     B2R_PHASE(who, 8);
     __syncthreads();
-    if (!is_leaf && threadIdx.x == 0) atomicAdd(fetched, 1u);
+    if (!is_leaf && threadIdx.x == 0) atomicAdd(&sync.fetched, 1u);
     B2R_PHASE(who, 9);
     const bool head = (int)threadIdx.x < ndup &&
                       (threadIdx.x == 0 ||
@@ -1486,19 +1467,13 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_early_kernel(UpdateAr
     listed = leaf_hashed_prepare<C>(a, n, sm.h, s_dup, &leaf_prep, &s_stop, info);
     __threadfence();
     __syncthreads();
-    if (threadIdx.x == 0)
-      asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(list_flag), "r"(1u) : "memory");
+    if (threadIdx.x == 0) st_release_u32(&sync.list_flag, 1u);
     ndup = listed ? s_dup.ndup : 0;
   } else {
     group_level<C>(a, level, n, sm, &prep, &s_stop, s_scan);
     B2R_LEVEL_TIME(0, level);
     if (threadIdx.x == 0) {
-      unsigned seen = 0;
-      const long long t0 = clock64();
-      do {
-        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(seen) : "l"(list_flag)
-                     : "memory");
-      } while (seen == 0 && clock64() - t0 < 4000000000ll);  // (2 s: never hang the GPU)
+      const bool seen = poll_acquire(&sync.list_flag, [](unsigned v) { return v != 0u; });
       s_listed = seen ? __ldcg(info + Info::kCount) : Info::kOverflow;
     }
     __syncthreads();
@@ -1568,15 +1543,10 @@ __global__ void __launch_bounds__(C::kThreads) tree_update_early_kernel(UpdateAr
   // (own lists: the level CTAs take the old leaves from the tree, so the new ones wait
   // until all of them have theirs — which they have had since before the values came)
   if (own_list && is_leaf) {
-    if (threadIdx.x == 0) {
-      unsigned have = 0;
-      const long long t0 = clock64();
-      do {
-        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(have) : "l"(fetched)
-                     : "memory");
-      } while (have < (unsigned)a.depth && clock64() - t0 < 4000000000ll);
-      if (have < (unsigned)a.depth && a.status[0] == 0) a.status[0] = B2R_ERR_CUDA;
-    }
+    if (threadIdx.x == 0 &&
+        !poll_acquire(&sync.fetched, [&](unsigned v) { return v >= (unsigned)a.depth; }) &&
+        a.status[0] == 0)
+      a.status[0] = B2R_ERR_CUDA;
     __syncthreads();
   }
   B2R_TRACE_COUNT(2, is_leaf && listed && n_eff == n);
@@ -2196,10 +2166,10 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
     a.n_dev = n_dev;
     a.scan_min_chain = kTreeScanMinChain;
     a.phase = base == 0 ? phase : kFull;
-    a.tickets = reinterpret_cast<unsigned long long *>(t->sync_words + 12);
-    a.go = go_by_flag && a.phase == kEarly ? t->sync_words + 14 : nullptr;
+    a.tickets = &t->sync->early_tickets;
+    a.go = go_by_flag && a.phase == kEarly ? &t->sync->go : nullptr;
     a.sorted = t->sorted;
-    a.sync_words = t->sync_words;
+    a.sync = t->sync;
     if (a.phase == kEarly)  // (tree_early_takes: compact)
       B2R_TRY((launch_big_chunk<BigCfgWide, true>(a, t->depth, stream)));
     else if (compact)
@@ -2225,8 +2195,8 @@ template int tree_apply<int32_t, double>(b2r_tree *, int64_t, const int32_t *,
 
 TreeGo tree_go_of(b2r_tree *t) {
   TreeGo g;
-  g.completed = t->sync_words + 15;
-  g.go = t->sync_words + 14;
+  g.completed = &t->sync->completed;
+  g.go = &t->sync->go;
   return g;
 }
 
@@ -2264,8 +2234,8 @@ int b2r_tree_create(int64_t capacity, b2r_tree **out) {
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&t->status), 16));
   B2R_CUDA(cudaMemset(t->status, 0, 16));
   B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&t->delta), b2r::kTreeChunk * 8));
-  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&t->sync_words), 64));
-  B2R_CUDA(cudaMemset(t->sync_words, 0, 64));
+  B2R_CUDA(cudaMalloc(reinterpret_cast<void **>(&t->sync), sizeof(b2r::TreeSync)));
+  B2R_CUDA(cudaMemset(t->sync, 0, sizeof(b2r::TreeSync)));
   const double one = 1.0;  // ST:89
   B2R_CUDA(cudaMemcpy(t->max_rec, &one, 8, cudaMemcpyHostToDevice));
   *out = t;
@@ -2279,7 +2249,7 @@ int b2r_tree_destroy(b2r_tree *t) {
   cudaFree(t->status);
   cudaFree(t->delta);
   if (t->sorted) cudaFree(t->sorted);
-  cudaFree(t->sync_words);
+  cudaFree(t->sync);
   t->bounce.release();
   delete t;
   return B2R_OK;

@@ -9,6 +9,26 @@
 // the children of h are 2h and 2h+1, and the 4 grandchildren / 8
 // great-grandchildren of a node start on 32 B / 64 B boundaries, which the
 // speculative descent below relies on.  16 MB for capacity 1M: L2-resident.
+namespace b2r {
+// The tree kernels' hand-over words (tree.cu), zeroed at creation; each protocol re-arms
+// its words for the next launch.
+struct TreeSync {
+  // tree_update_kernel: levels handed out in order of arrival, the leaf CTA's one-way
+  // barrier flag and the count of levels past it
+  unsigned int role_ticket, leaf_flag, level_arrivals, unused0;
+  long long pending[2];  // failure of the leaf CTA: stop code, first entry not applied
+  // tree_update_early_kernel: the leaf CTA's list of duplicates is out, CTAs that have
+  // left, level CTAs that have their leaves; the launches' tickets (launch_ticket)
+  unsigned int list_flag, ended, fetched, unused1;
+  unsigned long long early_tickets;
+  unsigned int go, completed;  // TreeGo
+};
+static_assert(offsetof(TreeSync, pending) % 8 == 0 &&
+                  offsetof(TreeSync, early_tickets) % 8 == 0 &&
+                  offsetof(TreeSync, go) == 56 && sizeof(TreeSync) == 64,
+              "TreeSync keeps its word order");
+}  // namespace b2r
+
 struct b2r_tree {
   int64_t capacity = 0;
   int depth = 0;          // levels = depth + 1
@@ -19,8 +39,7 @@ struct b2r_tree {
   double *delta = nullptr;     // device scratch: per-element leaf deltas of a chunk
   uint32_t *sorted = nullptr;  // device scratch: the early write-back's list of
                                // duplicate leaves (tree.cu: kEarly, DupInfo)
-  unsigned int *sync_words = nullptr;  // device: level ticket, barrier flag, arrivals,
-                                       // pending failure (tree_update_kernel)
+  b2r::TreeSync *sync = nullptr;  // device
   b2r::Bounce bounce;
 };
 
@@ -286,14 +305,6 @@ struct ExchangeArgs {
 };
 
 #ifdef __CUDACC__
-__device__ __forceinline__ void st_sys_u64(uint64_t *p, uint64_t v) {
-  asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ uint64_t ld_sys_u64(const uint64_t *p) {
-  uint64_t v;
-  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
 // All-gather of one fp64 per rank through peer memory (NVLink / NVSwitch), sending half:
 // thread g (= threadIdx.x & 31 < world) stores this rank's root total straight into rank
 // g's mailbox.  Each total travels as two 8-byte words that carry half of the payload and
@@ -367,7 +378,7 @@ struct TreeGo {
 __device__ __forceinline__ void tree_go_signal(const TreeGo &g) {
   if (g.go == nullptr) return;
   const unsigned int launch = *reinterpret_cast<const volatile unsigned int *>(g.completed) + 1u;
-  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(g.go), "r"(launch) : "memory");
+  st_release_u32(g.go, launch);
 }
 #endif
 
@@ -402,8 +413,7 @@ struct UpdateArgs {
   unsigned long long *tickets = nullptr;
   unsigned int *go = nullptr;
   uint32_t *sorted = nullptr;  // kEarly: b2r_tree::sorted
-  // role ticket, barrier flag, barrier arrivals (see tree_update_kernel)
-  unsigned int *sync_words = nullptr;
+  TreeSync *sync = nullptr;
   // Sharded replay: this launch leaves the tree final for the next sharded step, so the
   // warp that writes the root publishes it to the peers (ExchangeArgs::pub; one-CTA
   // kernels only).  nullptr: nothing to publish.

@@ -1,7 +1,7 @@
-"""The fused step at the agent's batch on ONE stream (csrc/replay.cuh: RowsGate; csrc/step.cu:
-train_step): sampler -> first half of the loss -> frame copies -> tail + write-back, each
-launched programmatically behind the one before, so that every kernel of a captured step
-has one parent and the next step's sampler keeps its early launch.
+"""The fused step at the agent's batch on ONE stream (csrc/replay.cuh: StageGate::rows;
+csrc/step.cu: train_step): sampler -> first half of the loss -> frame copies -> tail +
+write-back, each launched programmatically behind the one before, so that every kernel of
+a captured step has one parent and the next step's sampler keeps its early launch.
 
 The CPU part models the hand-overs under the edges the hardware gives: a kernel launches
 once its predecessor has let its dependents start, and passes its griddepcontrol.wait

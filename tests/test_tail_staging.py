@@ -1,5 +1,5 @@
 """The loss tail of the fused step at the agent's batch stages its inputs from the first
-half of the loss while the sampler is still running (csrc/replay.cuh: StageGate;
+half of the loss while the sampler is still running (csrc/replay.cuh: StageGate::first_half;
 csrc/c51.cu: c51_post_tree_kernel<true>).
 
 The CPU part models the hand-shake.  The first half of step k runs on a side stream and

@@ -1,5 +1,6 @@
 """CPU model of the "indices are final" hand-shake between the loss tail and the early tree
-write-back (csrc/tree.cuh: TreeGo, tree_go_signal; csrc/tree.cu: tree_update_early_kernel).
+write-back (csrc/tree.cuh: TreeGo, tree_go_signal, the words TreeSync::go and ::completed;
+csrc/tree.cu: tree_update_early_kernel, whose tickets come from launch_ticket).
 
 The write-back of step k is RESIDENT while the sampler and the loss tail of step k still
 run — and, one programmatic launch further, so may be the write-back of step k + 1 while
