@@ -76,14 +76,18 @@ def dqn_loss(online_q, target_q, actions, rewards, terminals, cumulative_gamma, 
       out['target'] = torch.empty(b, dtype=torch.float32, device=dev)
     if want_grad:
       out['grad_q'] = torch.empty(b, a, dtype=torch.float32, device=dev)
+  # the contiguous copies of strided inputs live until the launch: a copy freed at once
+  # goes back to torch's allocator, which hands its memory to the next input's copy
+  keep = [target_q.contiguous(), online_q.contiguous(), actions.contiguous(),
+          rewards.contiguous(), terminals.contiguous()]
   args = _native.DqnArgs()
   args.batch, args.num_actions = b, a
   args.cumulative_gamma = float(np.float32(cumulative_gamma))
-  args.target_q = target_q.contiguous().data_ptr()
-  args.online_q = online_q.contiguous().data_ptr()
-  args.actions = actions.contiguous().data_ptr()
-  args.rewards = rewards.contiguous().data_ptr()
-  args.terminals = terminals.contiguous().data_ptr()
+  args.target_q = keep[0].data_ptr()
+  args.online_q = keep[1].data_ptr()
+  args.actions = keep[2].data_ptr()
+  args.rewards = keep[3].data_ptr()
+  args.terminals = keep[4].data_ptr()
   args.loss = out['loss'].data_ptr()
   args.target = out['target'].data_ptr() if 'target' in out else None
   args.mean_loss = out['mean_loss'].data_ptr() if 'mean_loss' in out else None

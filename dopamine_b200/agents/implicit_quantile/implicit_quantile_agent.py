@@ -55,6 +55,8 @@ def quantile_huber_loss(online_quantile_values, quantiles, target_quantile_value
   if not kappa > 0:
     raise ValueError('kappa must be positive, got {}'.format(kappa))
   batch = actions.shape[0]
+  if batch < 1:
+    raise ValueError('batch must be >= 1, got {}'.format(batch))
   num_actions = online_quantile_values.shape[1]
   for name, x in (('online_quantile_values', online_quantile_values),
                   ('target_quantile_values', target_quantile_values),

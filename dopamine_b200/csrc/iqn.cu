@@ -95,9 +95,13 @@ __global__ void __launch_bounds__(kIqnWarps * 32) iqn_loss_kernel(IqnArgs a) {
 
   // ---- greedy next action (:176-188): mean over the K samples, first maximum.
   // Warp w sums the samples k = w (mod 4) of 32 actions at a time; warp 0 adds the four
-  // partial sums in warp order, divides and keeps the running first maximum.
+  // partial sums in warp order, divides and keeps the running first maximum.  A lane
+  // takes its first action whatever its q, so a row whose means are all -inf or NaN
+  // still yields an action in [0, A) (all -inf: action 0, as argmax gives) and never
+  // gathers the target at the sentinel's column.
+  constexpr int kNoAction = 0x7fffffff;
   float best_q = -INFINITY;
-  int best_a = 0x7fffffff;
+  int best_a = kNoAction;
   for (int base = 0; base < A; base += 32) {
     const int act = base + lane;
     double sum = 0.0;
@@ -111,7 +115,8 @@ __global__ void __launch_bounds__(kIqnWarps * 32) iqn_loss_kernel(IqnArgs a) {
 #pragma unroll
       for (int w = 1; w < kIqnWarps; ++w) total += s_q[w][lane];
       const float q = __fdiv_rn((float)total, (float)K);
-      if (q > best_q) {  // ascending act: strict > keeps the first maximum
+      // ascending act: strict > keeps the first maximum
+      if (best_a == kNoAction || q > best_q) {
         best_q = q;
         best_a = act;
       }
@@ -123,7 +128,9 @@ __global__ void __launch_bounds__(kIqnWarps * 32) iqn_loss_kernel(IqnArgs a) {
     for (int o = 16; o > 0; o >>= 1) {
       const float q2 = __shfl_xor_sync(0xffffffffu, best_q, o);
       const int a2 = __shfl_xor_sync(0xffffffffu, best_a, o);
-      if (q2 > best_q || (q2 == best_q && a2 < best_a)) {
+      // & and | rather than && and ||: one predicate, no branch in each step
+      if ((a2 != kNoAction) &
+          ((best_a == kNoAction) | (q2 > best_q) | ((q2 == best_q) & (a2 < best_a)))) {
         best_q = q2;
         best_a = a2;
       }
