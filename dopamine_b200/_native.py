@@ -212,6 +212,10 @@ SIGNATURES = {
     'b2r_store_write': (c_int, [c_void_p, c_int32, c_int64, c_int64, c_void_p,
                                 c_void_p]),
     'b2r_store_device_ptr': (c_void_p, [c_void_p, c_int32]),
+    'b2r_ckpt_save_column': (c_int, [c_void_p, c_int32, c_int32, c_int32, P(c_int64),
+                                     c_void_p]),
+    'b2r_ckpt_load_column': (c_int, [c_void_p, c_int32, c_int32, c_int64, c_int32,
+                                     c_void_p]),
     'b2r_sample_indices_sharded_device': (c_int, [
         c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_int32,
         c_void_p, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p]),

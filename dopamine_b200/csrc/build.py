@@ -8,7 +8,7 @@ PKG = os.path.dirname(HERE)
 ROOT = os.path.dirname(PKG)
 LIB = os.path.join(PKG, 'libb200replay.so')
 SOURCES = ['common.cu', 'tree.cu', 'replay.cu', 'sample.cu', 'gather.cu',
-           'c51.cu', 'dqn.cu', 'step.cu', 'exchange.cu', 'actor.cu', 'iqn.cu']
+           'c51.cu', 'dqn.cu', 'step.cu', 'exchange.cu', 'actor.cu', 'iqn.cu', 'ckpt.cu']
 HEADERS = ['common.cuh', 'tree.cuh', 'replay.cuh', 'gather.cuh',
            os.path.join(ROOT, 'include', 'b200_replay.h')]
 

@@ -273,6 +273,27 @@ int ensure_inv_slots(b2r_buffer *b, int64_t n) {
 using b2r::as_stream;
 using b2r::fail;
 
+namespace b2r {
+int refresh_terminal_mirror(b2r_buffer *b, int64_t row0, int64_t nrows, cudaStream_t s) {
+  // `in` of a store write may be a device pointer, and a checkpoint load writes the
+  // column from a kernel, so the rows are read back from the store itself.
+  const int64_t rb = b->col[B2R_COL_TERMINAL].row_bytes;
+  std::vector<uint8_t> rows((size_t)(nrows * rb));
+  B2R_CUDA(cudaMemcpyAsync(rows.data(), b->col[B2R_COL_TERMINAL].dev + row0 * rb,
+                           rows.size(), cudaMemcpyDeviceToHost, s));
+  B2R_CUDA(cudaStreamSynchronize(s));
+  for (int64_t k = 0; k < nrows; ++k)
+    b->term_is_one[row0 + k] = terminal_equals_one(rows.data() + k * rb,
+                                                   b->cfg.terminal_itemsize);
+  if (b->term_flag_owned && nrows > 0) {
+    term_flag_rebuild_kernel<<<(unsigned)((nrows + 255) / 256), 256, 0, s>>>(
+        b->col[B2R_COL_TERMINAL].dev, b->cfg.terminal_itemsize, row0, nrows, b->term_flag);
+    B2R_LAUNCHED();
+  }
+  return B2R_OK;
+}
+}  // namespace b2r
+
 extern "C" {
 
 int b2r_create(const b2r_config *cfg, b2r_buffer **out) {
@@ -598,27 +619,11 @@ int b2r_store_write(b2r_buffer *b, int32_t column, int64_t row0, int64_t nrows,
   const int64_t rb = b->col[column].row_bytes;
   B2R_CUDA(cudaMemcpyAsync(b->col[column].dev + row0 * rb, in,
                            (size_t)(nrows * rb), cudaMemcpyDefault, s));
-  if (column == B2R_COL_TERMINAL) {
-    // keep the host mirror of `terminal == 1` (CRB:255) in step; `in` may be a
-    // device pointer, so read the rows back from the store itself.
-    std::vector<uint8_t> rows((size_t)(nrows * rb));
-    B2R_CUDA(cudaMemcpyAsync(rows.data(), b->col[column].dev + row0 * rb,
-                             rows.size(), cudaMemcpyDeviceToHost, s));
-    B2R_CUDA(cudaStreamSynchronize(s));
-    for (int64_t k = 0; k < nrows; ++k)
-      b->term_is_one[row0 + k] = b2r::terminal_equals_one(
-          rows.data() + k * rb, b->cfg.terminal_itemsize);
-    if (b->term_flag_owned && nrows > 0) {
-      b2r::term_flag_rebuild_kernel<<<(unsigned)((nrows + 255) / 256), 256, 0,
-                                      s>>>(b->col[3].dev,
-                                           b->cfg.terminal_itemsize, row0, nrows,
-                                           b->term_flag);
-      B2R_LAUNCHED();
-    }
-  }
+  if (column == B2R_COL_TERMINAL) B2R_TRY(b2r::refresh_terminal_mirror(b, row0, nrows, s));
   B2R_CUDA(cudaStreamSynchronize(s));
   return B2R_OK;
 }
+
 
 const void *b2r_store_device_ptr(b2r_buffer *b, int32_t column) {
   if (column < 0 || column >= b->num_columns) return nullptr;

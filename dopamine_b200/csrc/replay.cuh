@@ -394,6 +394,10 @@ namespace b2r {
 // tree_apply).
 int flush_queue(b2r_buffer *buf, cudaStream_t stream, bool split = false,
                 const b2r_exchange *publish = nullptr);
+// Keeps the host mirror of `terminal == 1` (CRB:255) and the 1-byte terminal flags in step
+// with terminal rows [row0, row0 + nrows) of the store after they were overwritten.
+int refresh_terminal_mirror(b2r_buffer *buf, int64_t row0, int64_t nrows,
+                            cudaStream_t stream);
 // Makes `stream` wait for every deferred frame copy queued so far (no-op otherwise).
 int join_frames(b2r_buffer *buf, cudaStream_t stream);
 void fill_exchange_args(const b2r_exchange *x, ExchangeArgs *out);

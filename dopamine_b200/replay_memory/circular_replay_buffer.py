@@ -21,10 +21,13 @@ What is different on purpose:
 import collections
 import ctypes
 import gzip
+import io
 import math
 import os
 import pickle
+import struct
 import sys
+import zlib
 
 import numpy as np
 
@@ -43,6 +46,43 @@ def invalid_range(cursor, replay_capacity, stack_size, update_horizon):
   return np.array(
       [(cursor - update_horizon + i) % replay_capacity
        for i in range(stack_size + update_horizon)])
+
+
+# Blocked gzip store files: every member starts with this header (FLG = FEXTRA, MTIME 0,
+# XFL 0, OS 255, one 'BC' subfield of 2 bytes) followed by BSIZE = member size - 1.
+_BGZF_PREFIX = b'\x1f\x8b\x08\x04\x00\x00\x00\x00\x00\xff\x06\x00BC\x02\x00'
+BGZF_HEADER_BYTES = len(_BGZF_PREFIX) + 2
+
+
+def npy_header(shape, dtype):
+  """The bytes `np.save(f, a, allow_pickle=False)` writes before the data of a
+  C-contiguous array `a` of this shape and dtype (format 1.0, or 2.0 when the header
+  does not fit 1.0, as np.save chooses)."""
+  fmt = np.lib.format
+  d = {'descr': fmt.dtype_to_descr(np.dtype(dtype)), 'fortran_order': False,
+       'shape': tuple(int(s) for s in shape)}
+  buf = io.BytesIO()
+  try:
+    fmt.write_array_header_1_0(buf, d)
+  except ValueError:
+    buf = io.BytesIO()
+    fmt.write_array_header_2_0(buf, d)
+  return buf.getvalue()
+
+
+def bgzf_member(payload):
+  """`payload` as one blocked-gzip member with a single stored block."""
+  body = (b'\x01' + struct.pack('<HH', len(payload), len(payload) ^ 0xFFFF) +
+          bytes(payload))
+  size = BGZF_HEADER_BYTES + len(body) + 8
+  return (_BGZF_PREFIX + struct.pack('<H', size - 1) + body +
+          struct.pack('<II', zlib.crc32(payload), len(payload)))
+
+
+def _write_all(fd, data):
+  view = memoryview(data)
+  while view:
+    view = view[os.write(fd, view):]
 
 
 def _torch():
@@ -736,24 +776,26 @@ class OutOfGraphReplayBuffer(object):
         checkpointable_elements[member_name] = None
     return checkpointable_elements
 
-  def _checkpoint_value(self, attr):
-    if attr.startswith(STORE_FILENAME_PREFIX):
-      return self._store[attr[len(STORE_FILENAME_PREFIX):]]
-    return getattr(self, attr)
-
   def save(self, checkpoint_dir, iteration_number):
-    """Writes one gzip file per attribute / store array, reference layout."""
+    """Writes one gzip file per attribute / store array, reference layout.
+
+    Store arrays are compressed on the device into blocked gzip (see
+    `_save_store_column`); any gzip reader, the reference's `load` included, reads them
+    as the `np.save` stream of the array."""
     if not os.path.exists(checkpoint_dir):
       return
     for attr in self._return_checkpointable_elements():
       filename = self._generate_filename(checkpoint_dir, attr, iteration_number)
-      value = self._checkpoint_value(attr)
-      with open(filename, 'wb') as f:
-        with gzip.GzipFile(fileobj=f) as outfile:
-          if isinstance(value, np.ndarray):
-            np.save(outfile, value, allow_pickle=False)
-          else:
-            self._pickle_attribute(attr, value, outfile)
+      if attr.startswith(STORE_FILENAME_PREFIX):
+        self._save_store_column(attr[len(STORE_FILENAME_PREFIX):], filename)
+      else:
+        value = getattr(self, attr)
+        with open(filename, 'wb') as f:
+          with gzip.GzipFile(fileobj=f) as outfile:
+            if isinstance(value, np.ndarray):
+              np.save(outfile, value, allow_pickle=False)
+            else:
+              self._pickle_attribute(attr, value, outfile)
       stale_iteration_number = iteration_number - CHECKPOINT_DURATION
       if stale_iteration_number >= 0:
         stale_filename = self._generate_filename(checkpoint_dir, attr,
@@ -764,18 +806,32 @@ class OutOfGraphReplayBuffer(object):
           pass
 
   def load(self, checkpoint_dir, suffix):
-    """Restores from files written by `save` (or by the reference's save)."""
+    """Restores from files written by `save` (or by the reference's save).
+
+    A store file in the blocked layout `save` writes, whose .npy header matches the
+    buffer's storage shape and dtype, is inflated on the device; any other gzip file
+    takes the host path.  Every file is read (blocked ones: inflated and checked on the
+    device without writing) before any state changes, so a load that raises leaves
+    the buffer as it was."""
     save_elements = self._return_checkpointable_elements()
     for attr in save_elements:
       filename = self._generate_filename(checkpoint_dir, attr, suffix)
       if not os.path.exists(filename):
         raise FileNotFoundError('Missing file: {}'.format(filename))
     loaded = {}
+    blocked = {}
     for attr in save_elements:
       filename = self._generate_filename(checkpoint_dir, attr, suffix)
+      if attr.startswith(STORE_FILENAME_PREFIX):
+        name = attr[len(STORE_FILENAME_PREFIX):]
+        offset = self._blocked_data_offset(name, filename)
+        if offset is not None:
+          self._load_store_column(name, filename, offset, verify_only=True)
+          blocked[name] = (filename, offset)
+          continue
       with open(filename, 'rb') as f:
         with gzip.GzipFile(fileobj=f) as infile:
-          current = self._checkpoint_value(attr) if not attr.startswith(
+          current = getattr(self, attr) if not attr.startswith(
               STORE_FILENAME_PREFIX) else None
           if attr.startswith(STORE_FILENAME_PREFIX) or isinstance(
               current, np.ndarray):
@@ -785,12 +841,65 @@ class OutOfGraphReplayBuffer(object):
     for attr, value in loaded.items():
       if attr.startswith(STORE_FILENAME_PREFIX):
         self._store[attr[len(STORE_FILENAME_PREFIX):]] = value
+    for name, (filename, offset) in blocked.items():
+      self._load_store_column(name, filename, offset, verify_only=False)
     self._set_state(int(loaded['add_count']), loaded['invalid_range'])
     for attr, value in loaded.items():
       if attr.startswith(STORE_FILENAME_PREFIX) or attr in ('add_count',
                                                             'invalid_range'):
         continue
       self._restore_attribute(attr, value)
+
+  # -- blocked gzip store files (csrc/ckpt.cu) ----------------------------------------------
+  def _npy_header(self, name):
+    """The bytes `np.save(f, _store[name], allow_pickle=False)` writes before the data."""
+    element = self.get_storage_signature()[self._columns[name]]
+    return npy_header((self._replay_capacity,) + tuple(element.shape), element.type)
+
+  def _save_store_column(self, name, filename):
+    """Member 0 (the .npy header) from the host, members 1.. from the device."""
+    fd = os.open(filename, os.O_WRONLY | os.O_CREAT | os.O_TRUNC, 0o666)
+    try:
+      _write_all(fd, bgzf_member(self._npy_header(name)))
+      written = ctypes.c_int64(0)
+      _native.check(self._lib.b2r_ckpt_save_column(
+          self._h, self._columns[name], fd, 0, ctypes.byref(written), self._stream()))
+    finally:
+      os.close(fd)
+
+  def _blocked_data_offset(self, name, filename):
+    """Where member 1 starts when `filename` is a blocked file of store `name` (member 0
+    a BGZF member holding exactly this buffer's .npy header for it), else None."""
+    with open(filename, 'rb') as f:
+      head = f.read(BGZF_HEADER_BYTES)
+      if (len(head) < BGZF_HEADER_BYTES or
+          head[:BGZF_HEADER_BYTES - 2] != _BGZF_PREFIX[:BGZF_HEADER_BYTES - 2]):
+        return None
+      size = struct.unpack('<H', head[-2:])[0] + 1
+      rest = f.read(size - BGZF_HEADER_BYTES)
+    if size < BGZF_HEADER_BYTES + 8 or len(rest) != size - BGZF_HEADER_BYTES:
+      return None
+    inflater = zlib.decompressobj(-15)
+    try:
+      payload = inflater.decompress(rest[:-8])
+    except zlib.error:
+      return None
+    crc, isize = struct.unpack('<II', rest[-8:])
+    if (not inflater.eof or inflater.unused_data or crc != zlib.crc32(payload) or
+        isize != len(payload) or payload != self._npy_header(name)):
+      return None
+    return size
+
+  def _load_store_column(self, name, filename, offset, verify_only):
+    fd = os.open(filename, os.O_RDONLY)
+    try:
+      status = self._lib.b2r_ckpt_load_column(self._h, self._columns[name], fd, offset,
+                                              1 if verify_only else 0, self._stream())
+    finally:
+      os.close(fd)
+    if status == _native.ERR_INVALID_ARGUMENT:
+      raise gzip.BadGzipFile('{}: {}'.format(filename, _native.last_error()))
+    _native.check(status)
 
   def _restore_attribute(self, attr, value):
     setattr(self, attr, value)

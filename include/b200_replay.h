@@ -302,6 +302,33 @@ int b2r_store_write(b2r_buffer *buf, int32_t column, int64_t row0,
 /* Device address of a column (read-only use by callers that stay on the GPU). */
 const void *b2r_store_device_ptr(b2r_buffer *buf, int32_t column);
 
+/* Checkpoint files of a store column as blocked gzip (save() / load(), CRB:593-687).
+ * The column's bytes (capacity x row bytes) are cut into 65280-byte slices; slice k-1 is
+ * gzip member k, compressed on the device by one CTA: header 1f 8b 08, FLG FEXTRA, MTIME
+ * 0, XFL 0, OS 255, one BGZF extra subfield 'B' 'C' with BSIZE = member size - 1; a raw
+ * deflate body of one fixed-Huffman block, or one stored block where that is smaller
+ * (matches stay inside the member, distances <= 32768); CRC-32 and ISIZE.  Member 0, the
+ * .npy header, is the caller's.  Any gzip reader inflates the whole file as one stream.
+ * Work goes through fixed windows of 1024 members, double-buffered, so device and pinned
+ * scratch do not grow with the capacity and the file I/O overlaps the kernels.
+ *
+ * b2r_ckpt_save_column appends members 1..M to `fd` at its current position and sets
+ * *bytes_out to the bytes appended.  verify_only != 0: writes nothing; every member is
+ * compressed, inflated again on the device and compared with the column (any difference
+ * -> B2R_ERR_INVALID_ARGUMENT), *bytes_out the size the members would take.
+ * b2r_ckpt_load_column reads members 1..M from `fd` at byte `offset` (pread: the file
+ * position does not move) and inflates them straight into the column.  Only members in
+ * the format above are accepted; anything else — a bad header or BSIZE, another block type,
+ * a bad code or distance, a CRC-32 or ISIZE that does not match, a missing member, bytes
+ * after the last one — returns B2R_ERR_INVALID_ARGUMENT naming the member, never a device
+ * fault.  A member is written only after its own checks pass; verify_only != 0 runs every
+ * check and writes nothing, so a caller that verifies first never leaves a column half
+ * loaded.  Both synchronise. */
+int b2r_ckpt_save_column(b2r_buffer *buf, int32_t column, int32_t fd, int32_t verify_only,
+                         int64_t *bytes_out, b2r_stream stream);
+int b2r_ckpt_load_column(b2r_buffer *buf, int32_t column, int32_t fd, int64_t offset,
+                         int32_t verify_only, b2r_stream stream);
+
 /* Sharded replay (SURVEY.md section 8e): one buffer per GPU; shard_totals[g] is
  * rank g's root priority (device array, e.g. straight out of an NCCL all-gather).
  * For each of the global_batch strata i (query01[i] in [0,1], DEVICE), mass =
