@@ -575,13 +575,8 @@ ckpt_inflate_kernel(const uint8_t *__restrict__ in, int64_t in_bytes,
 // ---- host side ---------------------------------------------------------------------------
 // (per call: the attribute belongs to the current device)
 int set_smem_limits() {
-  B2R_CUDA(cudaFuncSetAttribute(ckpt_deflate_kernel,
-                                cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)kDeflateSmem));
-  B2R_CUDA(cudaFuncSetAttribute(ckpt_inflate_kernel,
-                                cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)kInflateSmem));
-  return B2R_OK;
+  B2R_TRY(allow_dynamic_smem(ckpt_deflate_kernel, (int)kDeflateSmem));
+  return allow_dynamic_smem(ckpt_inflate_kernel, (int)kInflateSmem);
 }
 
 // Device and pinned allocations of one call, released on every return path.

@@ -87,7 +87,12 @@ struct TreeWindow {
 TreeWindow &tree_window();
 void set_tree_window(void *base, size_t bytes);  // also reserves the L2 set-aside once
 
-template <typename... Params, typename... Args>
+// launch_prio_cluster options: launch without programmatic stream serialization even where
+// pdl_enabled(); take the tree's L2 window at priority 0 too (the frame copies launch at
+// priority 0 precisely so that they stay out of it).
+constexpr unsigned kLaunchNoPdl = 1u, kLaunchTreeWindow = 2u;
+
+template <unsigned kFlags = 0u, typename... Params, typename... Args>
 cudaError_t launch_prio_cluster(void (*kernel)(Params...), dim3 grid, dim3 block,
                                 size_t smem, cudaStream_t stream, int priority,
                                 int cluster_x, Args &&...args) {
@@ -99,7 +104,7 @@ cudaError_t launch_prio_cluster(void (*kernel)(Params...), dim3 grid, dim3 block
   cudaLaunchAttribute attr[4];
   int n = 0;
   const TreeWindow &w = tree_window();
-  if (w.base != nullptr && priority != 0) {
+  if (w.base != nullptr && (priority != 0 || (kFlags & kLaunchTreeWindow))) {
     attr[n].id = cudaLaunchAttributeAccessPolicyWindow;
     attr[n].val.accessPolicyWindow.base_ptr = w.base;
     attr[n].val.accessPolicyWindow.num_bytes = w.bytes;
@@ -108,7 +113,7 @@ cudaError_t launch_prio_cluster(void (*kernel)(Params...), dim3 grid, dim3 block
     attr[n].val.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
     ++n;
   }
-  if (pdl_enabled()) {
+  if (pdl_enabled() && !(kFlags & kLaunchNoPdl)) {
     attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[n].val.programmaticStreamSerializationAllowed = 1;
     ++n;
@@ -143,6 +148,24 @@ cudaError_t launch(void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem
                    cudaStream_t stream, Args &&...args) {
   return launch_prio(kernel, grid, block, smem, stream, chain_priority(),
                      static_cast<Args &&>(args)...);
+}
+
+// Lets `kernel` launch with up to `bytes` of dynamic shared memory per CTA (above the
+// default 48 KB), on the current device.
+template <typename K>
+int allow_dynamic_smem(K kernel, int bytes) {
+  B2R_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  return B2R_OK;
+}
+// The same once per kernel and process.
+template <auto kKernel>
+int allow_dynamic_smem_once(int bytes) {
+  static bool done = false;
+  if (!done) {
+    B2R_TRY(allow_dynamic_smem(kKernel, bytes));
+    done = true;
+  }
+  return B2R_OK;
 }
 
 // Barrier over the CTAs of a thread-block cluster with release / acquire semantics at

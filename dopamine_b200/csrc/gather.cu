@@ -391,16 +391,8 @@ int launch_gather(b2r_buffer *b, int32_t batch, const int32_t *indices_dev,
   const bool fast = a.stack == 4 && a.obs_itemsize == 1 && (a.obs_bytes & 15) == 0;
   const size_t tma_bytes = (size_t)kTmaMaxFrames * (size_t)a.obs_bytes;
   if (fast && gather_variant(batch) == 1 && tma_bytes <= 200 * 1024) {
-    static bool ready = false;
-    if (!ready) {
-      B2R_CUDA(cudaFuncSetAttribute(gather_stack4_u8_tma_kernel<true>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    200 * 1024));
-      B2R_CUDA(cudaFuncSetAttribute(gather_stack4_u8_tma_kernel<false>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    200 * 1024));
-      ready = true;
-    }
+    B2R_TRY(allow_dynamic_smem_once<gather_stack4_u8_tma_kernel<true>>(200 * 1024));
+    B2R_TRY(allow_dynamic_smem_once<gather_stack4_u8_tma_kernel<false>>(200 * 1024));
     a.scalar_rows = frames_only ? 0 : (batch + kTmaThreads - 1) / kTmaThreads;
     dim3 grid(gate != nullptr ? kGatedCopyCtas : batch + a.scalar_rows);
     if (frames_only)
@@ -422,13 +414,8 @@ int launch_gather(b2r_buffer *b, int32_t batch, const int32_t *indices_dev,
       // batch 1024).  Beyond that the copies themselves bound the step and run
       // unrestricted (capping costs 146 -> 162 us at 4096).
       const int pad_kb = batch > 64 && batch <= 1536 ? 56 : 0;
-      static bool pad_ready = false;
-      if (pad_kb > 0 && !pad_ready) {
-        B2R_CUDA(cudaFuncSetAttribute(gather_stack4_u8_kernel<false>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      pad_kb * 1024));
-        pad_ready = true;
-      }
+      if (pad_kb > 0)
+        B2R_TRY(allow_dynamic_smem_once<gather_stack4_u8_kernel<false>>(pad_kb * 1024));
       B2R_CUDA(launch_prio(gather_stack4_u8_kernel<false>, grid, dim3(128),
                            (size_t)pad_kb * 1024, stream, 0, a));
     }

@@ -403,20 +403,47 @@ int join_frames(b2r_buffer *buf, cudaStream_t stream);
 void fill_exchange_args(const b2r_exchange *x, ExchangeArgs *out);
 int launch_exchange_publish(const b2r_exchange *x, const b2r_buffer *buf,
                             cudaStream_t stream);
-// Sharded sampling.  Totals come from `shard_totals` (device array) or, when `x` is
-// set, from the peer-memory exchange.  `scalars` / `min_prob_out` as in launch_sample;
-// out_count (nullable, device) receives this rank's row count.  max_rows (> 0): rows
-// the caller's outputs hold — a rank whose share of a Philox batch is larger serves the
-// first max_rows and latches B2R_ERR_UNSUPPORTED (0: global_batch rows).
-int launch_sample_sharded(b2r_buffer *buf, int32_t global_batch, int32_t num_shards,
-                          int32_t rank, const double *shard_totals,
-                          const b2r_exchange *x, const double *query01,
-                          int32_t n_retry, const double *retry_u01, uint64_t seed,
-                          uint64_t offset, int32_t *out_slots, int32_t *out_indices,
-                          int32_t *out_count, cudaStream_t stream,
-                          const b2r_batch *scalars = nullptr,
-                          float *min_prob_out = nullptr, int32_t max_rows = 0,
-                          const PreSync *pre = nullptr, bool publish_min = false);
+// One launch of the prioritized sampler (sample.cu), unsharded or one rank of a sharded
+// global batch.  Every pointer is a device pointer.
+struct SampleRequest {
+  int32_t batch = 0;  // strata (the global batch when sharded)
+  // A sharded call (also with one shard): this rank's rows go to out_slots / count_out, and
+  // rows the range search cannot find (caller queries, one shard) are compacted by one CTA.
+  bool sharded = false;
+  int32_t num_shards = 1, rank = 0;
+  // Shard totals from `shard_totals`, or, when `x` is set, from the peer-memory exchange.
+  const double *shard_totals = nullptr;
+  const b2r_exchange *x = nullptr;
+  // Stratified queries in [0, 1] and retry uniforms (the reference's RNG stream);
+  // query01 == nullptr: Philox draws (seed, offset + *counter).
+  const double *query01 = nullptr;
+  const double *retry_u01 = nullptr;
+  int32_t max_attempts = 0;
+  uint64_t seed = 0, offset = 0;
+  // Philox: the device draw counter added to offset and advanced by the launch, so that a
+  // captured CUDA graph draws fresh strata at every replay (b2r_buffer::draw_counter;
+  // sharded calls: shard_counter, which advances in lockstep on all ranks as each makes the
+  // same sequence of sharded calls).
+  uint64_t *counter = nullptr;
+  bool latch = true;       // report asynchronous errors in b2r_buffer::status
+  int32_t *info = nullptr;  // [4]: status, fail slot, retry draws used, count
+  int32_t *out_idx = nullptr;
+  int32_t *out_slots = nullptr;  // nullable: each row's place in the global batch
+  int32_t *count_out = nullptr;  // nullable: this rank's row count
+  // > 0: rows the outputs hold — a rank whose share of a Philox batch is larger serves the
+  // first out_cap and latches B2R_ERR_UNSUPPORTED (0: batch rows).
+  int32_t out_cap = 0;
+  // Scalar columns written as the rows become final, and the batch's smallest sampling
+  // probability (both nullable).
+  const b2r_batch *scalars = nullptr;
+  float *min_prob_out = nullptr;
+  const PreSync *pre = nullptr;  // nullable: the first half of the loss running beside
+  bool publish_min = false;      // store the minimum into every peer's mailbox
+  // nullable: StageGate::rows.done of the one-stream step (batches of the warp sampler,
+  // with scalars and the minimum).
+  unsigned int *rows_done = nullptr;
+};
+int launch_sample(b2r_buffer *buf, const SampleRequest &r, cudaStream_t stream);
 // Sharded uniform sampling (sample.cu: uniform_sharded_kernel).  check_uniform_sharded:
 // the host-side refusals shared by the sampling call and the publish-ahead.
 // mode 0 / 1: publish-ahead of the span / the rejection list of the exchange's next step
@@ -442,12 +469,4 @@ int launch_gather(b2r_buffer *buf, int32_t batch, const int32_t *indices_dev,
                   const int32_t *count_dev = nullptr, bool frames_only = false,
                   const LaunchGate *gate = nullptr);
 bool gather_can_gate(const b2r_buffer *buf, int32_t batch);
-// rows_done (nullable): StageGate::rows.done of the one-stream step (batches of the warp sampler,
-// with scalars and the minimum).
-int launch_sample(b2r_buffer *buf, int32_t batch, bool philox, uint64_t seed,
-                  uint64_t offset, const double *strat_dev,
-                  const double *retry_dev, int32_t n_retry, int32_t *out_idx_dev,
-                  int32_t *info_dev, cudaStream_t stream,
-                  const b2r_batch *scalars = nullptr, float *min_prob_out = nullptr,
-                  const PreSync *pre = nullptr, unsigned int *rows_done = nullptr);
 }  // namespace b2r

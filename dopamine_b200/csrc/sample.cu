@@ -1296,20 +1296,55 @@ int sample_threads(int n) {
   return t;
 }
 
-}  // namespace
-
-// Threads per CTA (= strata per tile).  Small batches: one CTA (at least 256
-// threads, so that staging the top levels is two rounds of loads).  Large batches:
-// tiles of 128 strata, so that the descents spread over many SMs.
-static void sample_shape(int batch, int *threads, int *tiles) {
-  if (batch <= 256) {
-    *threads = 256;
-    *tiles = 1;
-  } else {
-    *threads = 128;
-    *tiles = (batch + 127) / 128;
-  }
+// The request of the b2r_sample_indices_sharded_* entry points, but for the totals.
+SampleRequest sharded_indices_request(b2r_buffer *b, int32_t global_batch,
+                                      const double *query01, int32_t n_retry,
+                                      const double *retry_u01, uint64_t seed,
+                                      uint64_t offset, int32_t *out_slots,
+                                      int32_t *out_indices, int32_t *out_count) {
+  SampleRequest r;
+  r.batch = global_batch;
+  r.sharded = true;
+  r.query01 = query01;
+  r.retry_u01 = retry_u01;
+  r.max_attempts = n_retry;
+  r.seed = seed;
+  r.offset = offset;
+  r.counter = b->shard_counter;
+  r.info = b->info;
+  r.out_idx = out_indices;
+  r.out_slots = out_slots;
+  r.count_out = out_count;
+  return r;
 }
+
+// uniform_sample_kernel over the caller's `candidates` (n_cand of them; no latch, counters
+// in/out) or, candidates == nullptr, over Philox draws of (seed, offset + the buffer's draw
+// counter).
+int launch_uniform_sample(b2r_buffer *b, int batch, uint64_t seed, uint64_t offset,
+                          int n_cand, const int64_t *candidates, int32_t *out_idx,
+                          int32_t *counters, cudaStream_t stream) {
+  const bool philox = candidates == nullptr;
+  UniformSampleArgs a;
+  a.valid_dev = b->ctx_dev;
+  a.batch = batch;
+  a.max_attempts = b->cfg.max_sample_attempts;
+  a.use_philox = philox ? 1 : 0;
+  a.seed = seed;
+  a.offset = offset;
+  a.counter = philox ? b->draw_counter : nullptr;
+  a.n_cand = n_cand;
+  a.candidates = candidates;
+  a.out_idx = out_idx;
+  a.counters = counters;
+  a.latched = philox ? b->status : nullptr;
+  B2R_CUDA(launch(uniform_sample_kernel, dim3(1), dim3(sample_threads(philox ? batch : n_cand)),
+                  0, stream, a));
+  B2R_LAUNCHED();
+  return B2R_OK;
+}
+
+}  // namespace
 
 // Largest number of strata the warp sampler (per_sample_warp_kernel) takes; above, a
 // thread per stratum over shared-memory-staged top levels (per_sample_kernel).  Every
@@ -1361,91 +1396,103 @@ static int warp_sampler_setup(b2r_buffer *b, int strata, int cap, WarpScratch *w
 // per SM) for the batches that would otherwise need a second wave: 296 CTAs, two per SM.
 constexpr int kSamplerWaveCtas = 296;
 
-static cudaError_t launch_warp_sampler(int ctas, int threads, cudaStream_t stream,
-                                       const PerSampleArgs &a, const WarpScratch &ws) {
-  if (ws.cluster)
-    return launch_prio_cluster(per_sample_warp_kernel<2, true>, dim3(ctas), dim3(threads),
-                               0, stream, chain_priority(), ctas, a, ws);
-  if (ctas > kSamplerWaveCtas)
-    return launch(per_sample_warp_kernel<4, false>, dim3(ctas), dim3(threads), 0, stream,
-                  a, ws);
-  return launch(per_sample_warp_kernel<2, false>, dim3(ctas), dim3(threads), 0, stream, a,
-                ws);
-}
-
-int launch_sample(b2r_buffer *b, int32_t batch, bool philox, uint64_t seed,
-                  uint64_t offset, const double *strat_dev,
-                  const double *retry_dev, int32_t n_retry, int32_t *out_idx_dev,
-                  int32_t *info_dev, cudaStream_t stream,
-                  const b2r_batch *scalars, float *min_prob_out, const PreSync *pre,
-                  unsigned int *rows_done) {
-  int threads, tiles;
-  sample_shape(batch, &threads, &tiles);
-  if (tiles > kMaxTiles)
-    return fail(B2R_ERR_UNSUPPORTED, "batch above %d is not supported", kMaxTiles * 128);
-  const bool by_warp = batch <= kSamplerWarpMax;
-  if (rows_done != nullptr && (!by_warp || !scalars || !min_prob_out))
+int launch_sample(b2r_buffer *b, const SampleRequest &r, cudaStream_t stream) {
+  if (!b->tree) return fail(B2R_ERR_UNSUPPORTED, "not a prioritized buffer");
+  if (r.batch <= 0 || r.num_shards <= 0 || r.num_shards > kMaxShards || r.rank < 0 ||
+      r.rank >= r.num_shards)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "bad sharding arguments");
+  if (r.x && !r.x->connected && r.x->world > 1)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "the exchange is not connected");
+  const bool philox = r.query01 == nullptr;
+  const int cap = r.out_cap > 0 && r.out_cap < r.batch ? r.out_cap : r.batch;
+  // The warp sampler up to kSamplerWarpMax strata (sharded: of a rank's expected share,
+  // not of the global batch), over this rank's stratum range for Philox strata (see
+  // shard_ranges).  Sharded caller queries (any order): one CTA of the thread kernel walks
+  // every tile and compacts this rank's strata with block scans; Philox strata above
+  // kSamplerWarpMax: tiles of 128 over many CTAs with the range search.
+  const bool by_warp = (philox || !r.sharded) && r.batch / r.num_shards <= kSamplerWarpMax;
+  const bool ranges = philox && r.num_shards > 1 && (by_warp || r.batch > 256);
+  if (r.rows_done != nullptr && (!by_warp || !r.scalars || !r.min_prob_out))
     return fail(B2R_ERR_INVALID_ARGUMENT,
                 "only the warp sampler with scalars and the minimum counts its rows");
-  PerSampleArgs a;
+  PerSampleArgs a = {};
   WarpScratch ws;
-  if (by_warp)
-    B2R_TRY(warp_sampler_setup(b, batch, batch, &ws, &threads, &tiles));
-  else
-    B2R_TRY(ensure_inv_slots(b, (int64_t)tiles * threads + 2 * kMaxTiles + 8));
+  int threads, ctas;
+  if (by_warp) {
+    // grid for the expected share plus a margin; the warps stride over the rest
+    int expect = r.num_shards > 1
+                     ? r.batch / r.num_shards + r.batch / (4 * r.num_shards) + 8
+                     : r.batch;
+    if (expect > cap) expect = cap;
+    B2R_TRY(warp_sampler_setup(b, expect, cap, &ws, &threads, &ctas));
+  } else {
+    // Threads per CTA (= strata per tile).  Small batches: one CTA (at least 256 threads,
+    // so that staging the top levels is two rounds of loads).  Large batches: tiles of 128
+    // strata, so that the descents spread over many SMs (with ranges, tiles of this rank's
+    // range: the grid follows the capacity of the outputs, not the global batch), or the
+    // one CTA of 1024 threads that compacts a rank's rows.
+    const bool one_cta = r.sharded && !ranges;
+    threads = r.batch <= 256 ? 256 : (one_cta ? 1024 : 128);
+    ctas = ((one_cta ? r.batch : cap) + threads - 1) / threads;
+    if (ctas > kMaxTiles)
+      return r.sharded ? fail(B2R_ERR_UNSUPPORTED, "global batch too large")
+                       : fail(B2R_ERR_UNSUPPORTED, "batch above %d is not supported",
+                              kMaxTiles * 128);
+    B2R_TRY(ensure_inv_slots(b, (int64_t)ctas * threads + 2 * kMaxTiles + 8));
+    a.inv_slots = b->inv_slots;
+    a.tile_counts = b->inv_slots + (int64_t)ctas * threads;
+    a.tile_min = reinterpret_cast<float *>(a.tile_counts + kMaxTiles);
+  }
   a.heap = b->tree->heap;
   a.depth = b->tree->depth;
   B2R_TRY(ensure_ctx(b, stream));
   a.valid_dev = b->ctx_dev;
-  a.batch = batch;
-  a.step = 1.0 / (double)batch;
-  a.max_attempts = philox ? b->cfg.max_sample_attempts : n_retry;
+  a.batch = r.batch;
+  a.step = 1.0 / (double)r.batch;
+  a.max_attempts = r.max_attempts;
   a.use_philox = philox ? 1 : 0;
-  a.seed = seed;
-  a.offset = offset;
-  a.counter = philox ? b->draw_counter : nullptr;
-  a.zero = 0;
-  a.strat_query01 = strat_dev;
-  a.retry_u01 = retry_dev;
-  a.out_idx = out_idx_dev;
-  if (!by_warp) {
-    a.inv_slots = b->inv_slots;
-    a.tile_counts = b->inv_slots + (int64_t)tiles * threads;
-    a.tile_min = reinterpret_cast<float *>(a.tile_counts + kMaxTiles);
-  }
+  a.seed = r.seed;
+  a.offset = r.offset;
+  a.counter = philox ? r.counter : nullptr;
+  a.strat_query01 = r.query01;
+  a.retry_u01 = r.retry_u01;
+  a.out_idx = r.out_idx;
   a.ticket = &b->sync->sample_ticket;
-  a.info = info_dev;
-  a.latched = philox ? b->status : nullptr;
-  a.num_shards = 1;
-  a.rank = 0;
-  a.shard_totals = nullptr;
-  a.out_slots = nullptr;
-  a.with_scalars = scalars != nullptr;
-  a.min_prob_out = min_prob_out;
-  a.count_out = nullptr;
-  a.shard_ranges = 0;
-  a.out_cap = batch;
-  a.publish_min = 0;
-  a.rows_done = rows_done;
-  a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
-  if (pre != nullptr) a.pre = *pre;
-  a.xchg.local = nullptr;
-  if (scalars) {
-    fill_scalar_args(b, scalars, &a.sc);
-    if (a.sc.indices_out == out_idx_dev) a.sc.indices_out = nullptr;
+  a.info = r.info;
+  a.latched = r.latch ? b->status : nullptr;
+  a.num_shards = r.num_shards;
+  a.rank = r.rank;
+  a.shard_totals = r.shard_totals;
+  a.out_slots = r.out_slots;
+  a.with_scalars = r.scalars != nullptr;
+  a.min_prob_out = r.min_prob_out;
+  a.count_out = r.count_out;
+  a.shard_ranges = ranges ? 1 : 0;
+  a.out_cap = cap;
+  a.publish_min = r.publish_min ? 1 : 0;
+  a.rows_done = r.rows_done;
+  if (r.pre != nullptr) a.pre = *r.pre;
+  if (r.x && r.x->world > 1) fill_exchange_args(r.x, &a.xchg);
+  if (r.scalars) {
+    fill_scalar_args(b, r.scalars, &a.sc);
+    if (a.sc.indices_out == r.out_idx) a.sc.indices_out = nullptr;
   }
   set_tree_window(b->tree->heap, (size_t)b->tree->leaves * 16);
-  if (by_warp) {
-    a.inv_slots = nullptr;
-    a.tile_counts = nullptr;
-    a.tile_min = nullptr;
-    B2R_CUDA(launch_warp_sampler(tiles, threads, stream, a, ws));
-    B2R_LAUNCHED();
-    return B2R_OK;
-  }
-  // 3 tree levels per memory round trip (more would bloat the straight-line code,
-  // and a cold instruction cache costs more than the saved round trips).
-  B2R_CUDA(launch(per_sample_kernel<3, 256>, dim3(tiles), dim3(threads), 0, stream, a));
+  if (by_warp && ws.cluster)
+    B2R_CUDA(launch_prio_cluster(per_sample_warp_kernel<2, true>, dim3(ctas), dim3(threads),
+                                 0, stream, chain_priority(), ctas, a, ws));
+  else if (by_warp && ctas > kSamplerWaveCtas)
+    B2R_CUDA(launch(per_sample_warp_kernel<4, false>, dim3(ctas), dim3(threads), 0, stream,
+                    a, ws));
+  else if (by_warp)
+    B2R_CUDA(launch(per_sample_warp_kernel<2, false>, dim3(ctas), dim3(threads), 0, stream,
+                    a, ws));
+  else if (threads != 1024)  // 3 tree levels per memory round trip (more would bloat the
+                             // straight-line code, and a cold instruction cache costs more
+                             // than the saved round trips)
+    B2R_CUDA(launch(per_sample_kernel<3, 256>, dim3(ctas), dim3(threads), 0, stream, a));
+  else
+    B2R_CUDA(launch(per_sample_kernel<3, 1024>, dim3(1), dim3(threads), 0, stream, a));
   B2R_LAUNCHED();
   return B2R_OK;
 }
@@ -1462,104 +1509,6 @@ void fill_exchange_args(const b2r_exchange *x, ExchangeArgs *out) {
   // ranks' strata then no longer partition the batch.
   static const bool nowait = std::getenv("B2R_DEBUG_XCHG_NOWAIT") != nullptr;
   if (nowait) out->timeout_ns = 0;
-}
-
-int launch_sample_sharded(b2r_buffer *b, int32_t global_batch, int32_t num_shards,
-                          int32_t rank, const double *shard_totals,
-                          const b2r_exchange *x, const double *query01,
-                          int32_t n_retry, const double *retry_u01, uint64_t seed,
-                          uint64_t offset, int32_t *out_slots, int32_t *out_indices,
-                          int32_t *out_count, cudaStream_t s,
-                          const b2r_batch *scalars, float *min_prob_out,
-                          int32_t max_rows, const PreSync *pre, bool publish_min) {
-  if (!b->tree) return fail(B2R_ERR_UNSUPPORTED, "not a prioritized buffer");
-  if (global_batch <= 0 || num_shards <= 0 || num_shards > kMaxShards || rank < 0 ||
-      rank >= num_shards)
-    return fail(B2R_ERR_INVALID_ARGUMENT, "bad sharding arguments");
-  if (x && !x->connected && x->world > 1)
-    return fail(B2R_ERR_INVALID_ARGUMENT, "the exchange is not connected");
-  // Philox strata: the warp sampler over this rank's stratum range (see shard_ranges).
-  // Caller-supplied queries (any order): one CTA of the thread kernel walks every tile
-  // and compacts this rank's strata with block scans (tiles of 128 over many CTAs with
-  // the range search for Philox strata above kSamplerWarpMax).
-  // (a rank's expected share decides, not the global batch)
-  const bool by_warp = query01 == nullptr && global_batch / num_shards <= kSamplerWarpMax;
-  const bool ranges = query01 == nullptr && num_shards > 1 &&
-                      (by_warp || global_batch > 256);
-  const int cap = max_rows > 0 && max_rows < global_batch ? max_rows : global_batch;
-  int threads = global_batch <= 256 ? 256 : (ranges ? 128 : 1024);
-  // (with ranges a CTA works on tiles of this rank's range: the grid follows the
-  // capacity of the outputs, not the global batch)
-  int tiles = ((ranges ? cap : global_batch) + threads - 1) / threads;
-  if (tiles > kMaxTiles) return fail(B2R_ERR_UNSUPPORTED, "global batch too large");
-  PerSampleArgs a;
-  WarpScratch ws;
-  if (by_warp) {
-    // grid for the expected share plus a margin; the warps stride over the rest
-    int expect = num_shards > 1 ? global_batch / num_shards + global_batch / (4 * num_shards) + 8
-                                : global_batch;
-    if (expect > cap) expect = cap;
-    B2R_TRY(warp_sampler_setup(b, expect, cap, &ws, &threads, &tiles));
-    a.inv_slots = nullptr;
-    a.tile_counts = nullptr;
-    a.tile_min = nullptr;
-  } else {
-    B2R_TRY(ensure_inv_slots(b, (int64_t)tiles * threads + 2 * kMaxTiles + 8));
-    a.inv_slots = b->inv_slots;
-    a.tile_counts = b->inv_slots + (int64_t)tiles * threads;
-    a.tile_min = reinterpret_cast<float *>(a.tile_counts + kMaxTiles);
-  }
-  a.heap = b->tree->heap;
-  a.depth = b->tree->depth;
-  B2R_TRY(ensure_ctx(b, s));
-  a.valid_dev = b->ctx_dev;
-  a.batch = global_batch;
-  a.step = 1.0 / (double)global_batch;
-  a.max_attempts = n_retry;
-  a.use_philox = (query01 == nullptr) ? 1 : 0;
-  a.seed = seed;
-  a.offset = offset;
-  // Philox mode: the draw number also advances on the device, in lockstep on all
-  // ranks (each makes the same sequence of sharded calls), so a captured CUDA
-  // graph draws fresh, rank-consistent strata at every replay.
-  a.counter = a.use_philox ? b->shard_counter : nullptr;
-  a.zero = 0;
-  a.strat_query01 = query01;
-  a.retry_u01 = retry_u01;
-  a.out_idx = out_indices;
-  a.ticket = &b->sync->sample_ticket;
-  a.info = b->info;
-  a.latched = b->status;
-  a.num_shards = num_shards;
-  a.rank = rank;
-  a.shard_totals = shard_totals;
-  a.out_slots = out_slots;
-  a.with_scalars = scalars != nullptr;
-  a.min_prob_out = min_prob_out;
-  a.count_out = out_count;
-  a.shard_ranges = ranges ? 1 : 0;
-  a.out_cap = cap;
-  a.publish_min = publish_min ? 1 : 0;
-  a.rows_done = nullptr;
-  a.pre.done = a.pre.seen = a.pre.ticket = nullptr;
-  if (pre != nullptr) a.pre = *pre;
-  a.xchg.local = nullptr;
-  if (x && x->world > 1) fill_exchange_args(x, &a.xchg);
-  if (scalars) {
-    fill_scalar_args(b, scalars, &a.sc);
-    if (a.sc.indices_out == out_indices) a.sc.indices_out = nullptr;
-  }
-  set_tree_window(b->tree->heap, (size_t)b->tree->leaves * 16);
-  if (by_warp)
-    B2R_CUDA(launch_warp_sampler(tiles, threads, s, a, ws));
-  else if (global_batch <= 256)
-    B2R_CUDA(launch(per_sample_kernel<3, 256>, dim3(1), dim3(threads), 0, s, a));
-  else if (ranges)
-    B2R_CUDA(launch(per_sample_kernel<3, 256>, dim3(tiles), dim3(threads), 0, s, a));
-  else
-    B2R_CUDA(launch(per_sample_kernel<3, 1024>, dim3(1), dim3(threads), 0, s, a));
-  B2R_LAUNCHED();
-  return B2R_OK;
 }
 
 // Publishes a rank's total for the next exchange step without consuming it.
@@ -1930,21 +1879,10 @@ int b2r_sample_indices_uniform(b2r_buffer *b, int32_t batch, int32_t n_cand,
   B2R_CUDA(cudaMemcpyAsync(b->bounce.dev, b->bounce.host, off_cnt + 16,
                            cudaMemcpyHostToDevice, s));
   B2R_TRY(b2r::ensure_ctx(b, s));
-  b2r::UniformSampleArgs a;
-  a.valid_dev = b->ctx_dev;
-  a.batch = batch;
-  a.max_attempts = b->cfg.max_sample_attempts;
-  a.use_philox = 0;
-  a.seed = a.offset = 0;
-  a.counter = nullptr;
-  a.n_cand = n_cand;
-  a.candidates = reinterpret_cast<const int64_t *>(b->bounce.dev);
-  a.out_idx = reinterpret_cast<int32_t *>(b->bounce.dev + off_out);
-  a.counters = reinterpret_cast<int32_t *>(b->bounce.dev + off_cnt);
-  a.latched = nullptr;
-  B2R_CUDA(b2r::launch(b2r::uniform_sample_kernel, dim3(1),
-                       dim3(b2r::sample_threads(n_cand)), 0, s, a));
-  B2R_LAUNCHED();
+  B2R_TRY(b2r::launch_uniform_sample(
+      b, batch, 0, 0, n_cand, reinterpret_cast<const int64_t *>(b->bounce.dev),
+      reinterpret_cast<int32_t *>(b->bounce.dev + off_out),
+      reinterpret_cast<int32_t *>(b->bounce.dev + off_cnt), s));
   B2R_CUDA(cudaMemcpyAsync(b->bounce.host + off_out, b->bounce.dev + off_out,
                            off_cnt + 16 - off_out, cudaMemcpyDeviceToHost, s));
   B2R_CUDA(cudaStreamSynchronize(s));
@@ -1975,11 +1913,15 @@ int b2r_sample_indices_prioritized(b2r_buffer *b, int32_t batch,
   if (n_retry) memcpy(b->bounce.host + off_retry, retry_u01, (size_t)n_retry * 8);
   B2R_CUDA(cudaMemcpyAsync(b->bounce.dev, b->bounce.host, off_out,
                            cudaMemcpyHostToDevice, s));
-  int32_t *dinfo = reinterpret_cast<int32_t *>(b->bounce.dev + off_info);
-  B2R_TRY(b2r::launch_sample(
-      b, batch, false, 0, 0, reinterpret_cast<const double *>(b->bounce.dev),
-      reinterpret_cast<const double *>(b->bounce.dev + off_retry), n_retry,
-      reinterpret_cast<int32_t *>(b->bounce.dev + off_out), dinfo, s));
+  b2r::SampleRequest r;
+  r.batch = batch;
+  r.query01 = reinterpret_cast<const double *>(b->bounce.dev);
+  r.retry_u01 = reinterpret_cast<const double *>(b->bounce.dev + off_retry);
+  r.max_attempts = n_retry;
+  r.latch = false;
+  r.info = reinterpret_cast<int32_t *>(b->bounce.dev + off_info);
+  r.out_idx = reinterpret_cast<int32_t *>(b->bounce.dev + off_out);
+  B2R_TRY(b2r::launch_sample(b, r, s));
   B2R_CUDA(cudaMemcpyAsync(b->bounce.host + off_out, b->bounce.dev + off_out,
                            off_info + 16 - off_out, cudaMemcpyDeviceToHost, s));
   B2R_CUDA(cudaStreamSynchronize(s));
@@ -2004,30 +1946,23 @@ int b2r_sample_indices_device(b2r_buffer *b, int32_t batch, uint64_t seed,
   if (batch <= 0) return fail(B2R_ERR_INVALID_ARGUMENT, "bad batch");
   cudaStream_t s = as_stream(stream);
   B2R_TRY(b2r::flush_queue(b, s));
-  if (b->tree)
-    return b2r::launch_sample(b, batch, true, seed, offset, nullptr, nullptr, 0,
-                              out_indices, b->info, s);
+  if (b->tree) {
+    b2r::SampleRequest r;
+    r.batch = batch;
+    r.max_attempts = b->cfg.max_sample_attempts;
+    r.seed = seed;
+    r.offset = offset;
+    r.counter = b->draw_counter;
+    r.info = b->info;
+    r.out_idx = out_indices;
+    return b2r::launch_sample(b, r, s);
+  }
   int64_t min_id, max_id;  // (the kernel recomputes them from the device context)
   B2R_TRY(b2r::uniform_bounds(b, &min_id, &max_id));
   B2R_TRY(b2r::ensure_ctx(b, s));
-  b2r::UniformSampleArgs a;
-  a.valid_dev = b->ctx_dev;
-  a.batch = batch;
-  a.max_attempts = b->cfg.max_sample_attempts;
-  a.use_philox = 1;
-  a.seed = seed;
-  a.offset = offset;
-  a.counter = b->draw_counter;
-  a.n_cand = 0;
-  a.candidates = nullptr;
-  a.out_idx = out_indices;
-  a.counters = b->info;
-  a.latched = b->status;
   B2R_CUDA(cudaMemsetAsync(b->info, 0, 16, s));
-  B2R_CUDA(b2r::launch(b2r::uniform_sample_kernel, dim3(1),
-                       dim3(b2r::sample_threads(batch)), 0, s, a));
-  B2R_LAUNCHED();
-  return B2R_OK;
+  return b2r::launch_uniform_sample(b, batch, seed, offset, 0, nullptr, out_indices, b->info,
+                                    s);
 }
 
 int b2r_sample_indices_sharded_device(b2r_buffer *b, int32_t global_batch,
@@ -2040,10 +1975,13 @@ int b2r_sample_indices_sharded_device(b2r_buffer *b, int32_t global_batch,
                                       b2r_stream stream) {
   if (!shard_totals) return fail(B2R_ERR_INVALID_ARGUMENT, "shard_totals is NULL");
   B2R_TRY(b2r::flush_queue(b, as_stream(stream)));
-  return b2r::launch_sample_sharded(b, global_batch, num_shards, rank, shard_totals,
-                                    nullptr, query01, n_retry, retry_u01, seed,
-                                    offset, out_slots, out_indices, out_count,
-                                    as_stream(stream));
+  b2r::SampleRequest r = b2r::sharded_indices_request(
+      b, global_batch, query01, n_retry, retry_u01, seed, offset, out_slots, out_indices,
+      out_count);
+  r.num_shards = num_shards;
+  r.rank = rank;
+  r.shard_totals = shard_totals;
+  return b2r::launch_sample(b, r, as_stream(stream));
 }
 
 int b2r_sample_indices_sharded_p2p_device(b2r_buffer *b, b2r_exchange *x,
@@ -2055,10 +1993,13 @@ int b2r_sample_indices_sharded_p2p_device(b2r_buffer *b, b2r_exchange *x,
                                           b2r_stream stream) {
   if (!x) return fail(B2R_ERR_INVALID_ARGUMENT, "exchange is NULL");
   B2R_TRY(b2r::flush_queue(b, as_stream(stream)));
-  return b2r::launch_sample_sharded(b, global_batch, x->world, x->rank, nullptr, x,
-                                    query01, n_retry, retry_u01, seed, offset,
-                                    out_slots, out_indices, out_count,
-                                    as_stream(stream));
+  b2r::SampleRequest r = b2r::sharded_indices_request(
+      b, global_batch, query01, n_retry, retry_u01, seed, offset, out_slots, out_indices,
+      out_count);
+  r.num_shards = x->world;
+  r.rank = x->rank;
+  r.x = x;
+  return b2r::launch_sample(b, r, as_stream(stream));
 }
 
 int b2r_sample_transition_batch_uniform_sharded_device(

@@ -251,17 +251,31 @@ static int train_step(b2r_buffer *b, int32_t batch, uint64_t seed, uint64_t offs
     if (b->slot_busy[ring_slot])
       B2R_CUDA(cudaStreamWaitEvent(s, b->ev_slot_free[ring_slot], 0));
   }
-  if (shard)
-    B2R_TRY(launch_sample_sharded(
-        b, batch, shard->exchange->world, shard->exchange->rank, nullptr,
-        shard->exchange, nullptr, b->cfg.max_sample_attempts, nullptr, seed, offset,
-        shard->out_slots, sample_idx, const_cast<int32_t *>(count), s, out, min_out,
-        rows_cap, split_loss ? &pre_sync : nullptr, sample_only));
-  else
-    B2R_TRY(launch_sample(b, batch, true, seed, offset, nullptr, nullptr, 0,
-                          sample_idx, b->info, s, out, b->min_prob,
-                          split_loss ? &pre_sync : nullptr,
-                          one_stream ? copy_gate.done : nullptr));
+  SampleRequest req;
+  req.batch = batch;
+  req.max_attempts = b->cfg.max_sample_attempts;
+  req.seed = seed;
+  req.offset = offset;
+  req.counter = shard ? b->shard_counter : b->draw_counter;
+  req.info = b->info;
+  req.out_idx = sample_idx;
+  req.scalars = out;
+  req.pre = split_loss ? &pre_sync : nullptr;
+  if (shard) {
+    req.sharded = true;
+    req.num_shards = shard->exchange->world;
+    req.rank = shard->exchange->rank;
+    req.x = shard->exchange;
+    req.out_slots = shard->out_slots;
+    req.count_out = const_cast<int32_t *>(count);
+    req.out_cap = rows_cap;
+    req.min_prob_out = min_out;
+    req.publish_min = sample_only;
+  } else {
+    req.min_prob_out = b->min_prob;
+    req.rows_done = one_stream ? copy_gate.done : nullptr;
+  }
+  B2R_TRY(launch_sample(b, req, s));
   if (one_stream)
     B2R_TRY(c51_pre_launch(&loss, rows_cap, scratch, pre_sync, s, &have_stats, nullptr,
                            nullptr, &stage));

@@ -1957,59 +1957,47 @@ int padded_size(int n) {
   return p;
 }
 
-template <typename C, int WHICH, typename K>
-int allow_big_smem(K kernel) {
-  static bool done = false;  // per instantiation (WHICH tells kernels of one type apart)
-  if (!done) {
-    B2R_CUDA(cudaFuncSetAttribute(
-        kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-        (int)(WHICH == 1 ? sizeof(typename C::EarlySmem) : sizeof(typename C::Smem))));
-    done = true;
-  }
-  return B2R_OK;
-}
-
 // One chunk of the cooperative kernel with geometry C: tree_update_kernel, or (EARLY,
 // kEarly) tree_update_early_kernel.
 template <typename C, bool EARLY, typename I, typename V>
 int launch_big_chunk(const UpdateArgs<I, V> &a, int depth, cudaStream_t stream) {
-  void (*kernel)(UpdateArgs<I, V>);
-  if constexpr (EARLY)
-    kernel = tree_update_early_kernel<I, V, C>;
-  else
-    kernel = tree_update_kernel<I, V, C>;
-  B2R_TRY((allow_big_smem<C, EARLY ? 1 : 0>(kernel)));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(depth + 1);
-  cfg.blockDim = dim3(C::kThreads);
-  cfg.dynamicSmemBytes = EARLY ? sizeof(typename C::EarlySmem) : sizeof(typename C::Smem);
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[3];
-  int n_attr = 0;
+  constexpr auto kernel = [] {  // (only the kernel used is instantiated)
+    if constexpr (EARLY)
+      return tree_update_early_kernel<I, V, C>;
+    else
+      return tree_update_kernel<I, V, C>;
+  }();
+  constexpr int smem = EARLY ? sizeof(typename C::EarlySmem) : sizeof(typename C::Smem);
+  B2R_TRY(allow_dynamic_smem_once<kernel>(smem));
   // Launched early (programmatic dependent launch) only in the 256 x 4 geometry: 21
   // early CTAs of 1024 threads would sit on 21 SMs for the whole loss kernel.
   // (kEarly: starting early is the point — its CTAs are sorting meanwhile.)
-  if (pdl_enabled() && (C::kThreads <= 256 || EARLY)) {
-    attr[n_attr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n_attr++].val.programmaticStreamSerializationAllowed = 1;
-  }
-  if (chain_priority() != 0) {
-    attr[n_attr].id = cudaLaunchAttributePriority;
-    attr[n_attr++].val.priority = chain_priority();
-  }
-  if (tree_window().base != nullptr) {
-    attr[n_attr].id = cudaLaunchAttributeAccessPolicyWindow;
-    attr[n_attr].val.accessPolicyWindow.base_ptr = tree_window().base;
-    attr[n_attr].val.accessPolicyWindow.num_bytes = tree_window().bytes;
-    attr[n_attr].val.accessPolicyWindow.hitRatio = 1.0f;
-    attr[n_attr].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-    attr[n_attr++].val.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
-  }
-  cfg.attrs = attr;
-  cfg.numAttrs = n_attr;
-  B2R_CUDA(cudaLaunchKernelEx(&cfg, kernel, a));
+  constexpr unsigned flags =
+      kLaunchTreeWindow | (C::kThreads <= 256 || EARLY ? 0u : kLaunchNoPdl);
+  B2R_CUDA(launch_prio_cluster<flags>(kernel, dim3(depth + 1), dim3(C::kThreads), smem,
+                                      stream, chain_priority(), 1, a));
   B2R_LAUNCHED();
   return B2R_OK;
+}
+
+// What every write-back of `t` takes; the launch adds its chunk of the batch and its own
+// fields.  publish: see tree_apply.
+template <typename I, typename V>
+UpdateArgs<I, V> update_args(const b2r_tree *t, const b2r_exchange *publish) {
+  UpdateArgs<I, V> a;
+  a.heap = t->heap;
+  a.depth = t->depth;
+  a.leaves = t->leaves;
+  a.delta = t->delta;
+  a.max_rec = t->max_rec;
+  a.status = t->status;
+  a.sync = t->sync;
+  if (publish != nullptr && publish->world > 1 && publish->connected) {
+    a.publish = publish->args_dev;
+    a.publish_world = publish->world;
+    a.publish_rank = publish->rank;
+  }
+  return a;
 }
 
 }  // namespace
@@ -2024,21 +2012,14 @@ constexpr int kTreeSmallMax = 32;
 // verified scan: a round costs about as much as 60-80 dependent DADDs.
 constexpr int kTreeScanMinChain = 32;
 
+// The one-CTA kernels' dynamic shared memory for kSmallBatch entries at the deepest tree
+// (32 levels).
 static int allow_small_smem() {
-  static bool ready = false;
-  if (!ready) {
-    const int bytes = kSmallBatch * 8 * (1 + 2 * 32);
-    B2R_CUDA(cudaFuncSetAttribute(tree_update_small_kernel<int64_t, double>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-    B2R_CUDA(cudaFuncSetAttribute(tree_update_small_kernel<int32_t, float>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-    B2R_CUDA(cudaFuncSetAttribute(tree_update_small_kernel<int32_t, double>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-    B2R_CUDA(cudaFuncSetAttribute(flush_fused_kernel,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-    ready = true;
-  }
-  return B2R_OK;
+  constexpr int bytes = kSmallBatch * 8 * (1 + 2 * 32);
+  B2R_TRY((allow_dynamic_smem_once<tree_update_small_kernel<int64_t, double>>(bytes)));
+  B2R_TRY((allow_dynamic_smem_once<tree_update_small_kernel<int32_t, float>>(bytes)));
+  B2R_TRY((allow_dynamic_smem_once<tree_update_small_kernel<int32_t, double>>(bytes)));
+  return allow_dynamic_smem_once<flush_fused_kernel>(bytes);
 }
 
 int flush_fused(b2r_tree *t, int n, const int64_t *slots, const double *prio,
@@ -2048,25 +2029,14 @@ int flush_fused(b2r_tree *t, int n, const int64_t *slots, const double *prio,
   B2R_TRY(allow_small_smem());
   const int padded = padded_size(n);
   const size_t smem = (size_t)padded * 8 * (1 + 2 * (size_t)(t->depth + 1));
-  UpdateArgs<int64_t, double> a;
-  a.heap = t->heap;
-  a.depth = t->depth;
-  a.leaves = t->leaves;
+  UpdateArgs<int64_t, double> a = update_args<int64_t, double>(t, publish);
   a.n = n;
   a.padded = padded;
   a.indices = slots;
   a.values = prio;
   a.mode = mode;
   a.k_base = 0;
-  a.delta = t->delta;
-  a.max_rec = t->max_rec;
-  a.status = t->status;
   a.n_dev = nullptr;
-  if (publish != nullptr && publish->world > 1 && publish->connected) {
-    a.publish = publish->args_dev;
-    a.publish_world = publish->world;
-    a.publish_rank = publish->rank;
-  }
   B2R_CUDA(launch(flush_fused_kernel, dim3(1 + n * row_blocks_per_entry),
                   dim3(32 * (t->depth + 1)), smem, stream, a, rows,
                   row_blocks_per_entry, (int)(n <= kTinyBatch)));
@@ -2114,25 +2084,14 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
     const int padded = padded_size((int)n);
     const size_t smem = (size_t)padded * 8 * (1 + 2 * (size_t)(t->depth + 1));
     B2R_TRY(allow_small_smem());
-    UpdateArgs<I, V> a;
-    a.heap = t->heap;
-    a.depth = t->depth;
-    a.leaves = t->leaves;
+    UpdateArgs<I, V> a = update_args<I, V>(t, publish);
     a.n = (int)n;
     a.padded = padded;
     a.indices = indices;
     a.values = values;
     a.mode = mode;
     a.k_base = 0;
-    a.delta = t->delta;
-    a.max_rec = t->max_rec;
-    a.status = t->status;
     a.n_dev = n_dev;
-    if (publish != nullptr && publish->world > 1 && publish->connected) {
-      a.publish = publish->args_dev;
-      a.publish_world = publish->world;
-      a.publish_rank = publish->rank;
-    }
     a.skip_flag = skip_flag;
     if (n <= kTinyBatch && skip_flag == nullptr)
       B2R_CUDA(launch(tree_update_tiny_kernel<I, V>, dim3(1), dim3(32 * (t->depth + 1)),
@@ -2150,26 +2109,19 @@ int tree_apply(b2r_tree *t, int64_t n, const I *indices, const V *values,
   const int64_t chunk = compact ? BigCfg1024::kChunk : BigCfg4096::kChunk;
   for (int64_t base = 0; base < n; base += chunk) {
     const int len = (int)((n - base) < chunk ? (n - base) : chunk);
-    UpdateArgs<I, V> a;
-    a.heap = t->heap;
-    a.depth = t->depth;
-    a.leaves = t->leaves;
+    UpdateArgs<I, V> a = update_args<I, V>(t, publish);
     a.n = len;
     a.padded = (int)chunk;
     a.indices = indices + base;
     a.values = values + base;
     a.mode = mode ? mode + base : nullptr;
     a.k_base = base;
-    a.delta = t->delta;
-    a.max_rec = t->max_rec;
-    a.status = t->status;
     a.n_dev = n_dev;
     a.scan_min_chain = kTreeScanMinChain;
     a.phase = base == 0 ? phase : kFull;
     a.tickets = &t->sync->early_tickets;
     a.go = go_by_flag && a.phase == kEarly ? &t->sync->go : nullptr;
     a.sorted = t->sorted;
-    a.sync = t->sync;
     if (a.phase == kEarly)  // (tree_early_takes: compact)
       B2R_TRY((launch_big_chunk<BigCfgWide, true>(a, t->depth, stream)));
     else if (compact)
