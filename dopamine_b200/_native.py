@@ -27,6 +27,8 @@ ERR_STALE_TOTAL = 11
 QUEUE_FULL = 10
 STREAM_NONE = ctypes.c_void_p(-1)
 IPC_HANDLE_BYTES = 64
+SAMPLER_STATE_VERSION, SAMPLER_STATE_WORDS = 1, 2
+EXCHANGE_STATE_VERSION, EXCHANGE_STATE_WORDS = 1, 1
 
 PRIORITY_EXPLICIT = 0
 PRIORITY_MAX_RECORDED = 1
@@ -216,6 +218,10 @@ SIGNATURES = {
                                      c_void_p]),
     'b2r_ckpt_load_column': (c_int, [c_void_p, c_int32, c_int32, c_int64, c_int32,
                                      c_void_p]),
+    'b2r_sampler_state_get': (c_int, [c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
+    'b2r_sampler_state_set': (c_int, [c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
+    'b2r_exchange_state_get': (c_int, [c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
+    'b2r_exchange_state_set': (c_int, [c_void_p, c_int32, c_void_p, c_int32, c_void_p]),
     'b2r_sample_indices_sharded_device': (c_int, [
         c_void_p, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_int32,
         c_void_p, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p]),

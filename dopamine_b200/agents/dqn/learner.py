@@ -141,6 +141,10 @@ def make_tf_rmsprop(params, lr=0.00025, decay=0.95, momentum=0.0, epsilon=0.0000
         torch._foreach_sub_(ps, update)
       return None
 
+    def load_state_dict(self, state_dict):
+      """In place: a captured update keeps reading the same accumulators."""
+      sharded_learner.load_optimizer_state(self, state_dict)
+
   return TFRMSProp()
 
 

@@ -333,6 +333,18 @@ class ShardedIQNLearner(sharded_learner.ShardedLearner, IQNLearner):
     """Adam on the reduced gradients."""
     self.optimizer.step()
 
+  # -- checkpoints (ShardedLearner's, with this rank's tau generator) ------------------
+  def _rank_state(self):
+    state = super(ShardedIQNLearner, self)._rank_state()
+    state['tau_generator'] = bytes(self._generator.get_state().numpy()).hex()
+    return state
+
+  def _load_rank_state(self, state):
+    torch = _torch()
+    super(ShardedIQNLearner, self)._load_rank_state(state)
+    words = bytearray.fromhex(state['tau_generator'])
+    self._generator.set_state(torch.frombuffer(words, dtype=torch.uint8))  # (in place)
+
   def _update(self):
     self.sample()
     self.loss_backward()

@@ -164,6 +164,28 @@ def make_tf_adam(params, lr, beta1=0.9, beta2=0.999, epsilon=1e-8, capturable=Fa
         torch._foreach_sub_(ps, update)
       return None
 
+    def state_dict(self):
+      """Also holds the step count t, as TensorFlow saves beta1_power / beta2_power."""
+      out = super().state_dict()
+      out['step'] = int(self._t.item()) if capturable and self._t is not None else (
+          self._host_t)
+      return out
+
+    def load_state_dict(self, state_dict):
+      """In place (sharded_learner.load_optimizer_state), the step count included: a
+      captured update keeps reading the same moments and device step count."""
+      state_dict = dict(state_dict)
+      step = state_dict.pop('step', None)
+      sharded_learner.load_optimizer_state(self, state_dict)
+      if step is None:  # a bundle written before the step count was saved
+        return
+      self._host_t = int(step)
+      if capturable:
+        if self._t is None:
+          self._t = torch.zeros((), dtype=torch.float64,
+                                device=self.param_groups[0]['params'][0].device)
+        self._t.fill_(float(step))
+
   return TFAdam()
 
 

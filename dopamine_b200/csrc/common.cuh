@@ -45,6 +45,21 @@ static inline cudaStream_t as_stream(b2r_stream s) {
   return reinterpret_cast<cudaStream_t>(s);
 }
 
+// The refusals of the versioned state get / set pairs (b2r_sampler_state_*,
+// b2r_exchange_state_*), checked before the handle or the device is touched.
+static inline int check_state_words(int32_t version, int32_t known_version, int32_t n_words,
+                                    int32_t known_words, const void *handle,
+                                    const void *words) {
+  if (version != known_version)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "state version %d is not %d", version,
+                known_version);
+  if (n_words != known_words)
+    return fail(B2R_ERR_INVALID_ARGUMENT, "state of %d words, expected %d", n_words,
+                known_words);
+  if (!handle || !words) return fail(B2R_ERR_INVALID_ARGUMENT, "NULL argument");
+  return B2R_OK;
+}
+
 // Pinned host <-> device bounce buffer that grows on demand.
 struct Bounce {
   uint8_t *host = nullptr;

@@ -120,6 +120,27 @@ int b2r_exchange_set_early_publish(b2r_exchange *x, int32_t on) {
   return B2R_OK;
 }
 
+int b2r_exchange_state_get(b2r_exchange *x, int32_t version, uint64_t *words,
+                           int32_t n_words, b2r_stream stream) {
+  B2R_TRY(b2r::check_state_words(version, B2R_EXCHANGE_STATE_VERSION, n_words,
+                                 B2R_EXCHANGE_STATE_WORDS, x, words));
+  B2R_CUDA(cudaMemcpyAsync(words, x->seq, 8, cudaMemcpyDefault, b2r::as_stream(stream)));
+  return B2R_OK;
+}
+
+int b2r_exchange_state_set(b2r_exchange *x, int32_t version, const uint64_t *words,
+                           int32_t n_words, b2r_stream stream) {
+  B2R_TRY(b2r::check_state_words(version, B2R_EXCHANGE_STATE_VERSION, n_words,
+                                 B2R_EXCHANGE_STATE_WORDS, x, words));
+  cudaStream_t s = b2r::as_stream(stream);
+  B2R_CUDA(cudaMemcpyAsync(x->seq, words, 8, cudaMemcpyDefault, s));
+  // every tag in the mailbox becomes 0, and pub[0] = 0 "nothing published": the steps
+  // after any restored step number are >= 1
+  B2R_CUDA(cudaMemsetAsync(x->mailbox, 0, kMailboxBytes, s));
+  B2R_CUDA(cudaMemsetAsync(x->pub, 0, 16, s));
+  return B2R_OK;
+}
+
 int b2r_exchange_publish_device(b2r_exchange *x, b2r_buffer *buf, b2r_stream stream) {
   if (!x || !buf || !buf->tree) return fail(B2R_ERR_INVALID_ARGUMENT, "bad argument");
   if (!x->connected) return fail(B2R_ERR_INVALID_ARGUMENT, "the exchange is not connected");

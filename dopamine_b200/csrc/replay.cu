@@ -739,4 +739,24 @@ int b2r_copy_total_device(b2r_buffer *b, double *dst, b2r_stream stream) {
   return B2R_OK;
 }
 
+int b2r_sampler_state_get(b2r_buffer *b, int32_t version, uint64_t *words, int32_t n_words,
+                          b2r_stream stream) {
+  B2R_TRY(b2r::check_state_words(version, B2R_SAMPLER_STATE_VERSION, n_words,
+                                 B2R_SAMPLER_STATE_WORDS, b, words));
+  cudaStream_t s = as_stream(stream);
+  B2R_CUDA(cudaMemcpyAsync(words, b->draw_counter, 8, cudaMemcpyDefault, s));
+  B2R_CUDA(cudaMemcpyAsync(words + 1, b->shard_counter, 8, cudaMemcpyDefault, s));
+  return B2R_OK;
+}
+
+int b2r_sampler_state_set(b2r_buffer *b, int32_t version, const uint64_t *words,
+                          int32_t n_words, b2r_stream stream) {
+  B2R_TRY(b2r::check_state_words(version, B2R_SAMPLER_STATE_VERSION, n_words,
+                                 B2R_SAMPLER_STATE_WORDS, b, words));
+  cudaStream_t s = as_stream(stream);
+  B2R_CUDA(cudaMemcpyAsync(b->draw_counter, words, 8, cudaMemcpyDefault, s));
+  B2R_CUDA(cudaMemcpyAsync(b->shard_counter, words + 1, 8, cudaMemcpyDefault, s));
+  return B2R_OK;
+}
+
 }  // extern "C"

@@ -813,6 +813,12 @@ class OutOfGraphReplayBuffer(object):
     takes the host path.  Every file is read (blocked ones: inflated and checked on the
     device without writing) before any state changes, so a load that raises leaves
     the buffer as it was."""
+    self._load_apply(self._load_prepare(checkpoint_dir, suffix))
+
+  def _load_prepare(self, checkpoint_dir, suffix):
+    """The reading half of `load`: every file read, blocked store files verified on the
+    device, nothing changed.  Returns what `_load_apply` writes.  A caller restoring
+    several buffers as one checkpoint prepares all of them before applying any."""
     save_elements = self._return_checkpointable_elements()
     for attr in save_elements:
       filename = self._generate_filename(checkpoint_dir, attr, suffix)
@@ -838,6 +844,11 @@ class OutOfGraphReplayBuffer(object):
             loaded[attr] = np.load(infile, allow_pickle=False)
           else:
             loaded[attr] = self._unpickle_attribute(attr, infile)
+    return loaded, blocked
+
+  def _load_apply(self, prepared):
+    """The writing half of `load`, on what `_load_prepare` returned."""
+    loaded, blocked = prepared
     for attr, value in loaded.items():
       if attr.startswith(STORE_FILENAME_PREFIX):
         self._store[attr[len(STORE_FILENAME_PREFIX):]] = value
@@ -849,6 +860,26 @@ class OutOfGraphReplayBuffer(object):
                                                             'invalid_range'):
         continue
       self._restore_attribute(attr, value)
+
+  # -- sampler state (b2r_sampler_state_get / _set) ------------------------------------------
+  def sampler_state(self):
+    """What decides the next draws besides the stored transitions: the device's draw
+    counters (Philox samplers, sharded prioritized sampler) and the host's draw counter
+    of rng='device' sampling.  A dict of plain ints; `set_sampler_state` takes it back."""
+    words = np.zeros(_native.SAMPLER_STATE_WORDS, dtype=np.uint64)
+    _native.check(self._lib.b2r_sampler_state_get(
+        self._h, _native.SAMPLER_STATE_VERSION, _native.ptr(words), len(words),
+        self._stream()))
+    _torch().cuda.current_stream().synchronize()
+    return {'version': _native.SAMPLER_STATE_VERSION,
+            'words': [int(w) for w in words], 'draw_counter': int(self._draw_counter)}
+
+  def set_sampler_state(self, state):
+    """Restores what `sampler_state` returned (stream-ordered on the device)."""
+    words = np.ascontiguousarray(state['words'], dtype=np.uint64)
+    _native.check(self._lib.b2r_sampler_state_set(
+        self._h, int(state['version']), _native.ptr(words), len(words), self._stream()))
+    self._draw_counter = int(state['draw_counter'])
 
   # -- blocked gzip store files (csrc/ckpt.cu) ----------------------------------------------
   def _npy_header(self, name):

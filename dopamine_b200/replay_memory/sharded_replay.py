@@ -112,6 +112,25 @@ class PeerExchange(object):
         self._h, memory._h, int(global_batch), int(seed), 0, int(phase),  # pylint: disable=protected-access
         _native.current_stream()))
 
+  def state(self):
+    """The exchange's step number (b2r_exchange_state_get) as a dict of plain ints."""
+    import torch
+    words = np.zeros(_native.EXCHANGE_STATE_WORDS, dtype=np.uint64)
+    _native.check(self._lib.b2r_exchange_state_get(
+        self._h, _native.EXCHANGE_STATE_VERSION, _native.ptr(words), len(words),
+        _native.current_stream()))
+    torch.cuda.current_stream().synchronize()
+    return {'version': _native.EXCHANGE_STATE_VERSION, 'words': [int(w) for w in words]}
+
+  def set_state(self, state):
+    """Restores what `state` returned and clears this rank's mailbox
+    (b2r_exchange_state_set).  Every rank must restore the same step number, and none
+    may start a step before every rank has restored."""
+    words = np.ascontiguousarray(state['words'], dtype=np.uint64)
+    _native.check(self._lib.b2r_exchange_state_set(
+        self._h, int(state['version']), _native.ptr(words), len(words),
+        _native.current_stream()))
+
   def __del__(self):
     if getattr(self, '_h', None):
       self._lib.b2r_exchange_destroy(self._h)

@@ -329,6 +329,20 @@ int b2r_ckpt_save_column(b2r_buffer *buf, int32_t column, int32_t fd, int32_t ve
 int b2r_ckpt_load_column(b2r_buffer *buf, int32_t column, int32_t fd, int64_t offset,
                          int32_t verify_only, b2r_stream stream);
 
+/* The sampler state of a buffer that only the device holds, for a checkpoint that resumes
+ * the same draws: word 0 the draw counter of the Philox samplers, word 1 the counter of
+ * the sharded prioritized sampler (it advances in lockstep on every rank).  `words` is
+ * B2R_SAMPLER_STATE_WORDS uint64 in host or device memory.  _get copies the counters
+ * into `words` and _set copies `words` into them, both with cudaMemcpyAsync on `stream`
+ * (host memory: synchronise `stream` before reading what _get wrote).  _set refuses a
+ * version or word count other than these before it touches the buffer or the device. */
+#define B2R_SAMPLER_STATE_VERSION 1
+#define B2R_SAMPLER_STATE_WORDS 2
+int b2r_sampler_state_get(b2r_buffer *buf, int32_t version, uint64_t *words,
+                          int32_t n_words, b2r_stream stream);
+int b2r_sampler_state_set(b2r_buffer *buf, int32_t version, const uint64_t *words,
+                          int32_t n_words, b2r_stream stream);
+
 /* Sharded replay (SURVEY.md section 8e): one buffer per GPU; shard_totals[g] is
  * rank g's root priority (device array, e.g. straight out of an NCCL all-gather).
  * For each of the global_batch strata i (query01[i] in [0,1], DEVICE), mass =
@@ -389,6 +403,21 @@ int b2r_exchange_set_timeout(b2r_exchange *exchange, double seconds);
  * published and latches B2R_ERR_STALE_TOTAL instead of letting the ranks apportion
  * the batch from different totals.  Every rank of an exchange must use the same setting. */
 int b2r_exchange_set_early_publish(b2r_exchange *exchange, int32_t on);
+/* The step number of an exchange, for a checkpoint: word 0 is the step counter (its
+ * parity picks the mailbox slot of the next step, its low 32 bits + 1 the tag a peer
+ * polls for).  `words` is B2R_EXCHANGE_STATE_WORDS uint64 in host or device memory,
+ * copied with cudaMemcpyAsync on `stream` as in b2r_sampler_state_get / _set, which also
+ * refuse what these refuse.  _set also clears this rank's mailbox and its record of what
+ * it has published, so that no word written before the restore can carry the tag of a
+ * step after it.  That is safe because every rank restores the same step number: no peer
+ * has published for a step beyond it, and none may do so before every rank's _set has
+ * run (the caller holds the ranks at a barrier in between). */
+#define B2R_EXCHANGE_STATE_VERSION 1
+#define B2R_EXCHANGE_STATE_WORDS 1
+int b2r_exchange_state_get(b2r_exchange *exchange, int32_t version, uint64_t *words,
+                           int32_t n_words, b2r_stream stream);
+int b2r_exchange_state_set(b2r_exchange *exchange, int32_t version, const uint64_t *words,
+                           int32_t n_words, b2r_stream stream);
 /* Publishes this rank's total for the NEXT step without consuming the step (the
  * sampling call publishes again, identically).  Only needed when ranks are
  * emulated by sequential launches on one device, where a launch cannot wait for a
